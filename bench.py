@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark: env steps/sec of fused random playouts,
 twixt(board_size=24), 1 Mi envs per GPU (BASELINE.json configs[3]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch: every env of the rank's
@@ -48,6 +48,7 @@ SEED = 0x7477697854  # "twixT"
 METRIC = "env_steps_per_sec_random_playouts_board24"
 UNIT = "steps/s"
 ALGO_BYTES_PER_STEP = 1328  # 2 * S(24), SURVEY.md section 8(d)
+DUMP_BYTES_MAX = 64 * 10**6 - 4096  # --dump-outputs in all, less room for the .npy headers
 
 
 def _peaks():
@@ -458,6 +459,25 @@ def adapter_latency(TwixTBatch, n, device, args):
     return res
 
 
+def dump_outputs(out_dir, outputs, suffix=""):
+    """Writes what the timed playout handed back in its last step as float32 `<name><suffix>.npy`: `returns`
+    [E, 2] and `lengths` [E] (plies per game, exact in float32).  Seeds and stream ids depend only on the
+    arguments, so two builds run with the same arguments can be compared array for array.  Above
+    DUMP_BYTES_MAX the same seeded sample of envs is taken from every array and its indices go to `env_index`."""
+    import numpy as np
+    arrays = {name: t.cpu().numpy().astype(np.float32) for name, t in outputs.items()}
+    envs = len(next(iter(arrays.values())))
+    per_env = sum(a[0].nbytes for a in arrays.values())
+    if envs * per_env > DUMP_BYTES_MAX:
+        keep = DUMP_BYTES_MAX // (per_env + 8)
+        idx = np.sort(np.random.default_rng(SEED).choice(envs, size=keep, replace=False))
+        arrays = {name: a[idx] for name, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -528,6 +548,8 @@ def run_ours(args):
     total_plies = int(red[0])
     elapsed_s = float(tmax[0].item()) * 1e-3
     value = total_plies / elapsed_s
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"returns": rets, "lengths": lens}, "_rank%d" % rank if world > 1 else "")
 
     # ---- e2e: the same workload through the C ABI with HOST buffers -------------
     ids_host = torch.arange(rank * E, (rank + 1) * E, dtype=torch.int64).pin_memory()
@@ -650,7 +672,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-kernels", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip configs c1_n8 / c3_n12 and adapter_latency_us")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's returns and lengths to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

@@ -21,6 +21,14 @@ Needs /root/reference (authoring container only):
 The tests never read /root/reference; they read these files.
 
     python tests/golden/make_golden.py
+
+  * ref_digests.json      (`python tests/golden/make_golden.py digests`, needs no reference tree) SHA-256 digests
+        of everything the tests that compare live with the compiled reference check -- the crossing table, the
+        seeded random games at every board size, ToString and ActionToString, the CUDA path's lock-step games and
+        fused playouts, the golden playthrough -- so those comparisons also run where oracle/_ref is absent.
+        Computed with the oracle, the host renderer and the adapter, whose outputs on exactly these inputs those
+        same tests found equal to the compiled reference; where oracle/_ref is present the tests still compare
+        with it live, so a digest that disagreed with the reference would fail there.
 """
 import json
 import os
@@ -246,5 +254,44 @@ def main():
         print(name, os.path.getsize(os.path.join(HERE, name)))
 
 
+def gen_digests():
+    import test_gpu_round2
+    import test_oracle_vs_reference as ovr
+    import test_render
+    import ref_gpu_worker
+    from twixt_for_open_spiel_b200.render import board_to_string
+    from twixt_for_open_spiel_b200.spiel import TwixTState
+    from helpers import Digest
+
+    out = {"generator": "tests/golden/make_golden.py digests", "crossing": {}, "random_games": {}, "render": {},
+           "action_strings": {}, "cuda_reference": {}}
+    for n in (5, 6, 8, 24):
+        out["crossing"][str(n)] = ovr.crossing_digest(ovr.oracle_blocker_sets(pyoracle.OracleGame(n), n))
+    for n in range(5, 25):
+        out["random_games"][str(n)] = ovr.random_games_digest(pyoracle.OracleGame(n), n)
+        out["cuda_reference"][str(n)] = ref_gpu_worker.oracle_digests(n, *test_gpu_round2.ref_worker_games(n))
+    for n, ansi in test_render.RENDER_CASES:
+        out["render"]["%d,%d" % (n, ansi)] = test_render.render_digest(
+            pyoracle.OracleGame(n), n, ansi, lambda os_: board_to_string(os_.export_record(), n, ansi))
+    for n in test_render.ACTION_STRING_SIZES:
+
+        class _G:
+            def board_size(self):
+                return n
+        fake = TwixTState.__new__(TwixTState)
+        fake._game = _G()
+        out["action_strings"][str(n)] = Digest().add(
+            test_render.action_strings(n, lambda p, a: TwixTState.action_to_string(fake, p, a))).hex()
+        fake._game = None
+    out["playthrough"] = test_gpu_round2.playthrough_ply_digests(
+        pyoracle.OracleGame(8).new_initial_state, lambda st: board_to_string(st.export_record(), 8, True))
+    with open(os.path.join(HERE, "ref_digests.json"), "w") as f:
+        json.dump(out, f, indent=0)
+    print("ref_digests.json", os.path.getsize(os.path.join(HERE, "ref_digests.json")))
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["digests"]:
+        gen_digests()
+    else:
+        main()

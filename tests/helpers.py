@@ -1,4 +1,7 @@
 """Shared helpers of the test-suite (test infrastructure)."""
+import hashlib
+import json
+import os
 import random
 from typing import List
 
@@ -43,3 +46,38 @@ def pad_games(games: List[List[int]], fill: int = -1) -> np.ndarray:
     for i, g in enumerate(games):
         out[i, :len(g)] = g
     return out
+
+
+# ---- digests of the reference's outputs (tests/golden/ref_digests.json) --------------------------------------
+# A test that compares with the compiled reference feeds the same observables, in the same order, into a Digest
+# whichever implementation produced them; the stored digest is what the reference produced on those inputs.
+GOLDEN_DIGESTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_digests.json")
+
+
+def golden_digests() -> dict:
+    with open(GOLDEN_DIGESTS) as f:
+        return json.load(f)
+
+
+class Digest:
+    def __init__(self):
+        self.h = hashlib.sha256()
+
+    def add(self, *items) -> "Digest":
+        """Integer sequences, float sequences (as float64), arrays (flattened, with their dtype kept by the
+        caller), strings, ints, floats and bools; numpy scalars count as the Python value they hold."""
+        for it in items:
+            if isinstance(it, np.ndarray):
+                self.h.update(b"A" + str(it.dtype).encode() + np.ascontiguousarray(it).reshape(-1).tobytes())
+            elif isinstance(it, str):
+                self.h.update(b"S" + it.encode("utf-8") + b"\0")
+            elif isinstance(it, (bool, np.bool_)):
+                self.h.update(b"B1" if it else b"B0")
+            elif isinstance(it, (list, tuple)):
+                self.h.update(b"L" + repr([v.item() if isinstance(v, np.generic) else v for v in it]).encode())
+            else:
+                self.h.update(b"V" + repr(it.item() if isinstance(it, np.generic) else it).encode())
+        return self
+
+    def hex(self) -> str:
+        return self.h.hexdigest()

@@ -13,7 +13,7 @@ import zlib
 import numpy as np
 import pytest
 
-from helpers import SEED, pad_games, random_game_actions
+from helpers import SEED, Digest, golden_digests, pad_games, random_game_actions
 
 pytestmark = pytest.mark.gpu
 
@@ -55,6 +55,10 @@ def test_fused_playout_every_board_size(oracle_mod, n):
 
 
 # ------------------------------------------------------------ CUDA vs the compiled reference ---
+def ref_worker_games(n):  # (lock-step games, fused playouts) per board size
+    return (24, 256) if n <= 12 else (8, 128)
+
+
 def _ref_worker(n, lock_games, fused):
     res = subprocess.run([sys.executable, os.path.join(HERE, "ref_gpu_worker.py"), str(n), str(lock_games), str(fused)],
                          capture_output=True, text=True, timeout=1500)
@@ -65,20 +69,39 @@ def _ref_worker(n, lock_games, fused):
 def test_cuda_against_compiled_reference(oracle_mod, n):
     """The parity chain closed on ONE machine: CUDA <-> oracle/_ref/libtwixt_ref.so (the unmodified reference,
     compiled in the authoring container, shipped to this box), lock-step and fused playouts, one process per
-    board size because of the reference's static BlockerMap (twixtboard.cc:148-165,211)."""
-    if not oracle_mod.have_reference():
-        pytest.skip("oracle/_ref/libtwixt_ref.so not present")
-    _ref_worker(n, 24 if n <= 12 else 8, 256 if n <= 12 else 128)
+    board size because of the reference's static BlockerMap (twixtboard.cc:148-165,211).  Without oracle/_ref the
+    worker compares with the stored digests of the reference's outputs on the same games."""
+    _ref_worker(n, *ref_worker_games(n))
+
+
+def playthrough_ply_digests(new_state, to_string):
+    """Per ply of the golden playthrough (n = 8): a digest of every observable and the ToString picture."""
+    with open(os.path.join(HERE, "golden", "playthrough_n8.json")) as f:
+        actions = json.load(f)["actions"]
+    st = new_state()
+    out = []
+    for ply in range(36):
+        out.append(Digest().add(st.legal_actions(), st.current_player(), st.is_terminal(), st.returns(),
+                                np.asarray(st.observation_tensor(0), dtype=np.float32),
+                                np.asarray(st.export_record(), dtype=np.uint32), to_string(st)).hex())
+        if ply < 35:
+            st.apply_action(actions[ply])
+    return out
 
 
 def test_cuda_playthrough_against_compiled_reference_in_process(oracle_mod):
     """The golden playthrough (n = 8) with the CUDA adapter and the compiled reference side by side in THIS
-    process: every ply, every observable, and the ToString picture of the CUDA-exported record."""
-    if not oracle_mod.have_reference():
-        pytest.skip("oracle/_ref/libtwixt_ref.so not present")
+    process: every ply, every observable, and the ToString picture of the CUDA-exported record.  Without
+    oracle/_ref, every ply is compared with the stored digest of the reference's observables there."""
     from twixt_for_open_spiel_b200 import load_game
     with open(os.path.join(HERE, "golden", "playthrough_n8.json")) as f:
         pt = json.load(f)
+    got = playthrough_ply_digests(load_game("twixt").new_initial_state, lambda st: st.to_string())
+    want = golden_digests()["playthrough"]
+    for ply in range(36):
+        assert got[ply] == want[ply], ply
+    if not oracle_mod.have_reference():
+        return
     rg = oracle_mod.RefGame(8, True)
     rs = rg.new_initial_state()
     st = load_game("twixt").new_initial_state()

@@ -3,7 +3,9 @@
 1. against the reference's own known-answer tests (twixt_test.cc) and its golden
    playthrough (playthrough.txt), both restated as committed fixtures;
 2. against the unmodified reference compiled into oracle/_ref, move by move, on
-   seeded random games at every board size (skipped only if oracle/_ref is absent).
+   seeded random games at every board size -- and, whether or not oracle/_ref is
+   present, against digests of what the reference produced on the same inputs
+   (tests/golden/ref_digests.json).
 """
 import json
 import os
@@ -13,7 +15,7 @@ import zlib
 import numpy as np
 import pytest
 
-from helpers import draw_seeking_actions, random_game_actions
+from helpers import Digest, draw_seeking_actions, golden_digests, random_game_actions
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -133,36 +135,87 @@ def test_golden_playthrough(oracle_mod, have_ref):
         del st, g
 
 
+DX = [1, 2, 2, 1, -1, -2, -2, -1]
+DY = [2, 1, -1, -2, -2, -1, 1, 2]
+
+
+def oracle_blocker_sets(og, n):
+    """{(x, y, d): the links that block link (x, y, d)}, each blocker named from both of its ends as the
+    reference's BlockerMap holds it."""
+    out = {}
+    for x in range(n):
+        for y in range(n):
+            for d in range(8):
+                both = set()
+                for bx, by, bd in og.blockers(x, y, d):
+                    both.add((bx, by, bd))
+                    both.add((bx + DX[bd], by + DY[bd], (bd + 4) % 8))
+                out[(x, y, d)] = both
+    return out
+
+
+def crossing_digest(sets):
+    dg = Digest()
+    for key in sorted(sets):
+        dg.add(list(key), sorted(sets[key]))
+    return {"entries": sum(len(v) for v in sets.values()), "digest": dg.hex()}
+
+
 def test_crossing_relation_equals_reference_table(oracle_mod, have_ref):
     """The geometric blocker relation == BlockerMap built from kLinkDescriptorTable
-    (twixtboard.cc:38-144, 176-190), link by link; entry totals as in SURVEY 8(a)."""
-    if not have_ref:
-        pytest.skip("oracle/_ref not built")
-    dx = [1, 2, 2, 1, -1, -2, -2, -1]
-    dy = [2, 1, -1, -2, -2, -1, 1, 2]
+    (twixtboard.cc:38-144, 176-190), link by link; entry totals as in SURVEY 8(a).  Against the compiled
+    reference where it is present, and always against the reference's stored table (tests/golden/ref_digests.json)."""
+    want = golden_digests()["crossing"]
     for n, want_entries in ((5, 992), (6, None), (8, 4928), (24, 69696)):
-        rg = oracle_mod.RefGame(n)
-        keep = rg.new_initial_state()  # builds the process-global map for this size
         og = oracle_mod.OracleGame(n)
-        entries = 0
-        for x in range(n):
-            for y in range(n):
-                for d in range(8):
-                    both = set()
-                    for bx, by, bd in og.blockers(x, y, d):
-                        both.add((bx, by, bd))
-                        both.add((bx + dx[bd], by + dy[bd], (bd + 4) % 8))
-                    assert set(rg.blockers(x, y, d)) == both, (n, x, y, d)
-                    entries += len(both)
+        sets = oracle_blocker_sets(og, n)
+        assert crossing_digest(sets) == want[str(n)], n
         if want_entries is not None:
-            assert entries == want_entries
-        del keep, rg
+            assert want[str(n)]["entries"] == want_entries
+        if have_ref:
+            rg = oracle_mod.RefGame(n)
+            keep = rg.new_initial_state()  # builds the process-global map for this size
+            for (x, y, d), both in sets.items():
+                assert set(rg.blockers(x, y, d)) == both, (n, x, y, d)
+            del keep, rg
+
+
+def random_games_digest(game, n):
+    """Seeded random games (forced swap in 1/3) on `game`, every observable the live comparison below checks, in
+    its order, and five Philox playouts."""
+    proto = game.new_initial_state()
+    rng = random.Random(n)
+    dg = Digest()
+    for gi in range(20 if n <= 12 else 6):
+        st = proto.clone()
+        ply, first = 0, None
+        while True:
+            la = st.legal_actions()
+            dg.add(la, st.current_player(), st.is_terminal(), st.returns())
+            if ply % 6 == 0 or st.is_terminal():
+                dg.add(st.observation_tensor(0), st.export_cells(), st.board_header()[:3],
+                       st.legal_list_of(0), st.legal_list_of(1))
+            if st.is_terminal():
+                break
+            a = first if (ply == 1 and gi % 3 == 0 and first in la) else rng.choice(la)
+            if ply == 0:
+                first = a
+            st.apply_action(a)
+            ply += 1
+        del st
+    for s in range(5):
+        dg.add(proto.clone().playout_philox(99, s))
+    del proto
+    return dg.hex()
 
 
 @pytest.mark.parametrize("n", list(range(5, 25)))
 def test_oracle_equals_reference_on_random_games(oracle_mod, have_ref, n):
+    """Move by move against the compiled reference where it is present; always against the digest of what the
+    reference produced on the same games (tests/golden/ref_digests.json)."""
+    assert random_games_digest(oracle_mod.OracleGame(n), n) == golden_digests()["random_games"][str(n)]
     if not have_ref:
-        pytest.skip("oracle/_ref not built")
+        return
     rg = oracle_mod.RefGame(n)
     og = oracle_mod.OracleGame(n)
     proto = rg.new_initial_state()

@@ -1,12 +1,13 @@
 """ToString parity (SURVEY 8f row 1): the host renderer over an exported record reproduces the reference's
-board picture byte for byte -- against the golden playthrough strings and against the compiled reference."""
+board picture byte for byte -- against the golden playthrough strings, stored digests of the reference's pictures
+and, where it is present, the compiled reference itself."""
 import json
 import os
 import random
 
 import pytest
 
-from helpers import random_game_actions
+from helpers import Digest, golden_digests, random_game_actions
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -29,13 +30,37 @@ def test_playthrough_strings(oracle_mod):
     assert board_to_string(st.export_record(), 8, True).endswith("[x has won]")
 
 
-@pytest.mark.parametrize("n,ansi", [(5, True), (6, False), (8, True), (11, False), (12, True), (24, True), (24, False)])
+RENDER_CASES = [(5, True), (6, False), (8, True), (11, False), (12, True), (24, True), (24, False)]
+ACTION_STRING_SIZES = (5, 8, 12, 24)
+
+
+def render_digest(og, n, ansi, to_string):
+    """ToString every 4 plies and at the end of seeded random games (forced swap in every other one);
+    `to_string(oracle_state)` gives the picture to digest."""
+    rng = random.Random(n)
+    dg = Digest()
+    for gi in range(6 if n <= 12 else 2):
+        acts = random_game_actions(og, rng, force_swap=(gi % 2 == 0))
+        os_ = og.new_initial_state()
+        for ply, a in enumerate(acts):
+            if ply % 4 == 0:
+                dg.add(to_string(os_))
+            os_.apply_action(a)
+        dg.add(to_string(os_))
+    return dg.hex()
+
+
+@pytest.mark.parametrize("n,ansi", RENDER_CASES)
 def test_matches_compiled_reference(oracle_mod, have_ref, n, ansi):
-    if not have_ref:
-        pytest.skip("oracle/_ref not built")
+    """The host renderer against the stored digest of the reference's ToString on these games
+    (tests/golden/ref_digests.json), and against the compiled reference itself where it is present."""
     from twixt_for_open_spiel_b200.render import board_to_string
-    rg = oracle_mod.RefGame(n, ansi)
     og = oracle_mod.OracleGame(n)
+    got = render_digest(og, n, ansi, lambda os_: board_to_string(os_.export_record(), n, ansi))
+    assert got == golden_digests()["render"]["%d,%d" % (n, ansi)]
+    if not have_ref:
+        return
+    rg = oracle_mod.RefGame(n, ansi)
     proto = rg.new_initial_state()
     rng = random.Random(n)
     for gi in range(6 if n <= 12 else 2):
@@ -51,25 +76,30 @@ def test_matches_compiled_reference(oracle_mod, have_ref, n, ansi):
     del proto, rg
 
 
+def action_strings(n, action_to_string):
+    return [action_to_string(p, a) for a in range(n * n) for p in (0, 1)]
+
+
 def test_action_to_string_matches_reference(oracle_mod, have_ref):
-    """twixt.cc:67-74; also pinned by StringLegalActions in the playthrough (GPU test)."""
-    if not have_ref:
-        pytest.skip("oracle/_ref not built")
+    """twixt.cc:67-74; also pinned by StringLegalActions in the playthrough (GPU test).  Against the stored
+    digest of the reference's strings (tests/golden/ref_digests.json) and the compiled reference where present."""
     from twixt_for_open_spiel_b200.spiel import TwixTState
-    for n in (5, 8, 12, 24):
-        rg = oracle_mod.RefGame(n)
-        rs = rg.new_initial_state()
+    want = golden_digests()["action_strings"]
+    for n in ACTION_STRING_SIZES:
 
         class _G:
             def board_size(self):
                 return n
         fake = TwixTState.__new__(TwixTState)
         fake._game = _G()
-        for a in range(n * n):
-            for p in (0, 1):
-                assert TwixTState.action_to_string(fake, p, a) == rs.action_to_string(p, a)
+        ours = action_strings(n, lambda p, a: TwixTState.action_to_string(fake, p, a))
         fake._game = None
-        del rs, rg
+        assert Digest().add(ours).hex() == want[str(n)], n
+        if have_ref:
+            rg = oracle_mod.RefGame(n)
+            rs = rg.new_initial_state()
+            assert ours == action_strings(n, rs.action_to_string), n
+            del rs, rg
 
 
 def test_reference_generated_strings(oracle_mod):
