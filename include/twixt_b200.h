@@ -243,6 +243,47 @@ int twixt_set_validation(twixt_batch* b, int enabled);
 int twixt_get_stats(twixt_batch* b, twixt_stats* out);
 int twixt_stats_reset(twixt_batch* b);
 
+/* Batched MCTS: `num_trees` independent searches on the device, each open_spiel's MCTSBot with
+ * RandomRolloutEvaluator(n_rollouts), solve = false and no Dirichlet noise, made deterministic:
+ *  - twixt_mcts_begin: the root of tree t is a COPY of env root_first + t (later changes to that env do not
+ *    affect the tree); its stream id is T = stream_base + root_first + t (twixt_set_stream_base, so results do
+ *    not depend on sharding), which must be below 2^32.  The batch's seed at begin keys every draw.
+ *  - simulation k (k = 0, 1, .. since begin) descends from the root: it stops at a terminal node or at a node
+ *    with N(s) == 0 (the leaf); a node is expanded on its second visit (one edge per legal action, ascending,
+ *    the swap offer included at ply 1); if U > 0 edges are unvisited it takes the j-th of them in ascending
+ *    order, j = (w*U) >> 32 with w = word 0 of Philox4x32-10(key = seed, counter = (T lo, T hi, k, 1)), and
+ *    creates its child; otherwise it takes the edge of largest W/N + c*sqrt(ln N(s) / N) (IEEE double, no
+ *    contraction, ln from the host's libm; ties to the lowest action).
+ *  - the leaf value v: Returns() for a terminal leaf; else the mean of R fused playouts from the leaf
+ *    (rollout r on stream (T << 32) | (k*R + r), as twixt_playout), or in the stepwise form the caller's
+ *    float value.  Every node on the path gets N += 1, every edge N += 1 and W += v[player to move at its
+ *    parent].
+ * twixt_mcts_run(k) queues k simulations (three kernel launches each: select, playout, backup; no host
+ * synchronisation).  Stepwise form: twixt_mcts_select writes each tree's leaf record into batch envs
+ * [leaf_first, leaf_first + count) and out_leaf_status [count] int32 (nullable: 0 needs a value, 1 terminal:
+ * its value is Returns()); the caller evaluates them (e.g. twixt_observation_and_mask + a value network) and
+ * hands twixt_mcts_backup [count, 2] float32 values (entries of terminal leaves are ignored).  run and the
+ * stepwise pair share the same kernels and may be mixed.  twixt_mcts_root_stats: out_visits [count, n*n]
+ * int32 and out_value_sums [count, n*n] double are N(a) / W(a) of the root edges (0 for other actions),
+ * out_best [count] int32 is open_spiel's BestChild (most visits, then larger W, then lowest action), -1 while
+ * the root is terminal or unexpanded; each pointer is nullable.
+ * Errors (TWIXT_EINVAL, trees unchanged): ranges outside the batch, count > num_trees, more than
+ * max_simulations simulations since begin, select twice in a row, backup without select, run while a select
+ * is pending, uct_c not finite or negative, stream ids out of range (T >= 2^32, max_simulations *
+ * n_rollouts >= 2^32).  twixt_mcts_create computes the arena size (per tree: (max_simulations + 1) node slots
+ * of record + 18 bytes per legal action, twixt_mcts.cuh) and fails with TWIXT_ENOMEM, naming it, when the
+ * device has less free memory.  The rollouts count in the batch's twixt_stats like any twixt_playout call.
+ * A search uses its batch's stream and must be destroyed before the batch. */
+typedef struct twixt_mcts twixt_mcts;
+int twixt_mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                      double uct_c, twixt_mcts** out);
+void twixt_mcts_destroy(twixt_mcts* m);
+int twixt_mcts_begin(twixt_mcts* m, int64_t root_first, int64_t count);
+int twixt_mcts_run(twixt_mcts* m, int32_t num_simulations);
+int twixt_mcts_select(twixt_mcts* m, int64_t leaf_first, int32_t* out_leaf_status);
+int twixt_mcts_backup(twixt_mcts* m, const float* values);
+int twixt_mcts_root_stats(twixt_mcts* m, int32_t* out_visits, double* out_value_sums, int32_t* out_best);
+
 /* Multi-GPU plumbing for hosts that are not Python (SURVEY 8e: envs shard by contiguous global id ranges,
  * no data-path collective, one reduction of the counters).  twixt_shard_range: rank's share [first,
  * first+count) of global_envs envs over `world` ranks (shares differ by at most one env); create the rank's

@@ -91,6 +91,13 @@ SYMBOLS = [
     ("twixt_stats_accumulate", C.c_int, [C.POINTER(Stats), C.POINTER(Stats)]),
     ("twixt_get_stats", C.c_int, [_P, C.POINTER(Stats)]),
     ("twixt_stats_reset", C.c_int, [_P]),
+    ("twixt_mcts_create", C.c_int, [_P, _I64, C.c_int32, C.c_int32, C.c_double, C.POINTER(_P)]),
+    ("twixt_mcts_destroy", None, [_P]),
+    ("twixt_mcts_begin", C.c_int, [_P, _I64, _I64]),
+    ("twixt_mcts_run", C.c_int, [_P, C.c_int32]),
+    ("twixt_mcts_select", C.c_int, [_P, _I64, _P]),
+    ("twixt_mcts_backup", C.c_int, [_P, _P]),
+    ("twixt_mcts_root_stats", C.c_int, [_P, _P, _P, _P]),
 ]
 
 OK, EINVAL, ECUDA, EILLEGAL, ENOMEM = 0, -1, -2, -3, -4

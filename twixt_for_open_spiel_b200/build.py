@@ -17,7 +17,8 @@ INCLUDE = os.path.join(os.path.dirname(PKG), "include")
 LIB = os.path.join(PKG, "libtwixt_b200.so")
 OBJ_DIR = os.path.join(PKG, "build")
 # (source, extra flags, object): the playout kernel is compiled once per size group (see its last section)
-SOURCES = [("twixt_kernels_api.cu", [], "twixt_kernels_api.o"), ("twixt_batch.cu", [], "twixt_batch.o")] + [
+SOURCES = [("twixt_kernels_api.cu", [], "twixt_kernels_api.o"), ("twixt_batch.cu", [], "twixt_batch.o"),
+           ("twixt_mcts.cu", [], "twixt_mcts.o")] + [
     ("twixt_kernel_playout.cu", ["-DTW_PLAYOUT_GROUP=%d" % g], "twixt_kernel_playout_g%d.o" % g) for g in range(5)]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

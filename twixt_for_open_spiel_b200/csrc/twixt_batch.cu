@@ -9,15 +9,18 @@
 // There is no CPU implementation behind any of these calls.
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <new>
 #include <string>
+#include <vector>
 
 #include "../../include/twixt_b200.h"
 #include "twixt_engine.cuh"
 #include "twixt_kernels.cuh"
+#include "twixt_mcts.cuh"
 
 namespace twixt {
 
@@ -531,6 +534,7 @@ class TwixTBatch {
   }
 
  private:
+  friend class TwixTMCTS;  // searches run on the batch's stream, staging, counters and Philox key
   uint32_t* rec(int64_t env) const { return records_ + env * rw_; }
 
   // ---- device staging for host-side buffers: a few grow-only slots ------
@@ -658,10 +662,238 @@ class TwixTBatch {
   int64_t launches_ = 0;
 };
 
+// Batched MCTS over the envs of one batch (twixt_mcts_* in the header; kernels in twixt_mcts.cu, storage
+// formula in twixt_mcts.cuh).  Every call is queued on the batch's stream; the rollouts are twixt_playout's
+// kernel on the search's own rollout slots and count in the batch's twixt_stats.
+class TwixTMCTS {
+ public:
+  TwixTMCTS() = default;
+  ~TwixTMCTS() {
+    if (arena_mem_ == nullptr) return;
+    DeviceGuard g(b_->device_);
+    cudaStreamSynchronize(b_->stream_);
+    cudaFree(arena_mem_);
+  }
+
+  int Init(TwixTBatch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c) {
+    if (num_trees <= 0) return fail(TWIXT_EINVAL, "num_trees must be positive: %lld", static_cast<long long>(num_trees));
+    if (max_simulations <= 0) return fail(TWIXT_EINVAL, "max_simulations must be positive: %d", max_simulations);
+    if (n_rollouts <= 0) return fail(TWIXT_EINVAL, "n_rollouts must be positive: %d", n_rollouts);
+    if (!std::isfinite(uct_c) || uct_c < 0.0) return fail(TWIXT_EINVAL, "uct_c must be finite and >= 0: %g", uct_c);
+    if (static_cast<uint64_t>(max_simulations) * static_cast<uint64_t>(n_rollouts) >= (1ull << 32))
+      return fail(TWIXT_EINVAL, "max_simulations * n_rollouts = %llu must be below 2^32 (rollout stream ids)",
+                  static_cast<unsigned long long>(max_simulations) * static_cast<unsigned long long>(n_rollouts));
+    b_ = b;
+    num_trees_ = num_trees;
+    max_sims_ = max_simulations;
+    c_ = uct_c;
+    const int n = b->n_;
+    const MctsSizes s = mcts_sizes(n, max_simulations, n_rollouts);
+    const int64_t per_tree = mcts_bytes_per_tree(s);
+    // carve one allocation; each array starts on a 256-byte boundary
+    const int64_t T = num_trees, nodes = T * s.slots, edges = nodes * s.edges, rolls = T * s.rollouts;
+    const int64_t sizes[13] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
+                               T * 16, T * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8};
+    int64_t offs[13], total = 0;
+    for (int i = 0; i < 13; ++i) {
+      offs[i] = total;
+      total += (sizes[i] + 255) & ~static_cast<int64_t>(255);
+    }
+    DeviceGuard g(b->device_);
+    size_t free_bytes = 0, total_bytes = 0;
+    TW_CUDA(cudaMemGetInfo(&free_bytes, &total_bytes));
+    if (static_cast<uint64_t>(total) > free_bytes)
+      return fail(TWIXT_ENOMEM,
+                  "MCTS arena of %lld bytes (%lld trees x %lld bytes per tree at n = %d, %d simulations, %d rollouts) "
+                  "exceeds the %zu bytes free on device %d",
+                  static_cast<long long>(total), static_cast<long long>(T), static_cast<long long>(per_tree), n,
+                  max_simulations, n_rollouts, free_bytes, b->device_);
+    cudaError_t e = cudaMalloc(&arena_mem_, static_cast<size_t>(total));
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      arena_mem_ = nullptr;
+      return fail(TWIXT_ENOMEM, "cudaMalloc of %lld bytes for the MCTS arena failed: %s", static_cast<long long>(total),
+                  cudaGetErrorString(e));
+    }
+    char* base = static_cast<char*>(arena_mem_);
+    a_.n = n;
+    a_.rw = static_cast<int>(s.rw);
+    a_.M = static_cast<int>(s.edges);
+    a_.S = static_cast<int>(s.slots);
+    a_.P = static_cast<int>(s.path);
+    a_.R = n_rollouts;
+    a_.node_rec = reinterpret_cast<uint32_t*>(base + offs[0]);
+    a_.node_legal = reinterpret_cast<int32_t*>(base + offs[1]);
+    a_.node_n = reinterpret_cast<uint32_t*>(base + offs[2]);
+    a_.edge_action = reinterpret_cast<uint16_t*>(base + offs[3]);
+    a_.edge_n = reinterpret_cast<uint32_t*>(base + offs[4]);
+    a_.edge_w = reinterpret_cast<double*>(base + offs[5]);
+    a_.edge_child = reinterpret_cast<int32_t*>(base + offs[6]);
+    a_.tree = reinterpret_cast<int4*>(base + offs[7]);
+    a_.path = reinterpret_cast<int2*>(base + offs[8]);
+    a_.roll_rec = reinterpret_cast<uint32_t*>(base + offs[9]);
+    a_.roll_ids = reinterpret_cast<uint64_t*>(base + offs[10]);
+    a_.roll_ret = reinterpret_cast<float*>(base + offs[11]);
+    double* table = reinterpret_cast<double*>(base + offs[12]);
+    a_.log_table = table;
+    // ln N(s) from the host's libm, so that a CPU restatement of the search computes the same scores
+    std::vector<double> logs(static_cast<size_t>(s.slots));
+    for (size_t i = 0; i < logs.size(); ++i) logs[i] = std::log(static_cast<double>(i));
+    TW_CUDA(cudaMemcpyAsync(table, logs.data(), logs.size() * sizeof(double), cudaMemcpyHostToDevice, b->stream_));
+    TW_CUDA(cudaStreamSynchronize(b->stream_));
+    return TWIXT_OK;
+  }
+
+  int Begin(int64_t root_first, int64_t count) {
+    TW_TRY(b_->CheckRange(root_first, count));
+    if (count > num_trees_)
+      return fail(TWIXT_EINVAL, "count %lld > num_trees %lld", static_cast<long long>(count),
+                  static_cast<long long>(num_trees_));
+    const uint64_t base = b_->stream_base_;
+    if (count > 0 && (base >= (1ull << 32) || static_cast<uint64_t>(root_first + count - 1) >= (1ull << 32) - base))
+      return fail(TWIXT_EINVAL, "tree stream ids stream_base + root_first + t must be below 2^32: base %llu, roots [%lld, %lld)",
+                  static_cast<unsigned long long>(base), static_cast<long long>(root_first),
+                  static_cast<long long>(root_first + count));
+    DeviceGuard g(b_->device_);
+    TW_CUDA(launch_mcts_begin(a_, b_->rec(root_first), count, b_->stream_));
+    b_->launches_ += count > 0;
+    count_ = count;
+    key_ = b_->seed_;
+    stream0_ = static_cast<uint32_t>(base + static_cast<uint64_t>(root_first));
+    sims_ = 0;
+    pending_ = false;
+    begun_ = true;
+    return TWIXT_OK;
+  }
+
+  int Run(int32_t num_simulations) {
+    TW_TRY(CheckSimulations(num_simulations, "run"));
+    if (count_ == 0 || num_simulations == 0) return TWIXT_OK;
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    PlayoutArgs p;
+    p.records = a_.roll_rec;
+    p.count = count_ * a_.R;
+    p.n = a_.n;
+    p.max_plies = a_.n * a_.n;  // above max_game_length: every rollout plays to the end
+    p.seed = key_;
+    p.stream_base = 0;
+    p.stream_ids = a_.roll_ids;
+    p.out_returns = a_.roll_ret;
+    p.out_lengths = nullptr;
+    p.out_actions = nullptr;
+    p.trace_plies = 0;
+    p.stats = b.d_stats_;
+    p.tickets = &b.d_stats_->tickets;
+    for (int32_t i = 0; i < num_simulations; ++i) {
+      const uint32_t k = static_cast<uint32_t>(sims_);
+      TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, k, c_, nullptr, nullptr, b.stream_));
+      TW_CUDA(cudaMemsetAsync(&b.d_stats_->tickets, 0, sizeof(unsigned long long), b.stream_));
+      TW_CUDA(launch_playout(p, b.stream_));
+      TW_CUDA(launch_mcts_backup(a_, count_, nullptr, b.stream_));
+      b.launches_ += 3;
+      sims_ += 1;
+    }
+    return TWIXT_OK;
+  }
+
+  int Select(int64_t leaf_first, int32_t* out_leaf_status) {
+    TW_TRY(CheckSimulations(1, "select"));
+    TW_TRY(b_->CheckRange(leaf_first, count_));
+    if (count_ == 0) {
+      pending_ = true;
+      return TWIXT_OK;
+    }
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    b.ScratchReset();
+    Staged st;
+    TW_TRY(b.StageOut(out_leaf_status, static_cast<size_t>(count_) * sizeof(int32_t), &st, false));
+    TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, static_cast<uint32_t>(sims_), c_, b.rec(leaf_first),
+                               static_cast<int32_t*>(st.dev), b.stream_));
+    b.launches_ += 1;
+    pending_ = true;
+    TW_TRY(b.Finish(&st));
+    if (st.host) TW_TRY(b.Sync());
+    return TWIXT_OK;
+  }
+
+  int Backup(const float* values) {
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_backup: no search begun");
+    if (!pending_) return fail(TWIXT_EINVAL, "twixt_mcts_backup without a pending twixt_mcts_select");
+    if (values == nullptr && count_ > 0) return fail(TWIXT_EINVAL, "null values pointer");
+    if (count_ > 0) {
+      DeviceGuard g(b_->device_);
+      TwixTBatch& b = *b_;
+      b.ScratchReset();
+      Staged in;
+      TW_TRY(b.StageIn(values, static_cast<size_t>(count_) * 2 * sizeof(float), &in));
+      TW_CUDA(launch_mcts_backup(a_, count_, static_cast<const float*>(in.dev), b.stream_));
+      b.launches_ += 1;
+      if (in.host) TW_TRY(b.Sync());  // the staged copy of the values is reused by the next call
+    }
+    pending_ = false;
+    sims_ += 1;
+    return TWIXT_OK;
+  }
+
+  int RootStats(int32_t* out_visits, double* out_value_sums, int32_t* out_best) {
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_root_stats: no search begun");
+    if (count_ == 0) return TWIXT_OK;
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    b.ScratchReset();
+    const size_t cells = static_cast<size_t>(a_.n) * a_.n;
+    Staged v, w, best;
+    TW_TRY(b.StageOut(out_visits, static_cast<size_t>(count_) * cells * sizeof(int32_t), &v, false));
+    TW_TRY(b.StageOut(out_value_sums, static_cast<size_t>(count_) * cells * sizeof(double), &w, false));
+    TW_TRY(b.StageOut(out_best, static_cast<size_t>(count_) * sizeof(int32_t), &best, false));
+    TW_CUDA(launch_mcts_root_stats(a_, count_, static_cast<int32_t*>(v.dev), static_cast<double*>(w.dev),
+                                   static_cast<int32_t*>(best.dev), b.stream_));
+    b.launches_ += 1;
+    TW_TRY(b.Finish(&v));
+    TW_TRY(b.Finish(&w));
+    TW_TRY(b.Finish(&best));
+    if (v.host || w.host || best.host) TW_TRY(b.Sync());
+    return TWIXT_OK;
+  }
+
+  int64_t count() const { return count_; }
+  int64_t simulations() const { return sims_; }
+
+ private:
+  int CheckSimulations(int32_t num, const char* what) const {
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_%s: no search begun", what);
+    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_%s while a twixt_mcts_select awaits its backup", what);
+    if (num < 0) return fail(TWIXT_EINVAL, "num_simulations must be >= 0: %d", num);
+    if (sims_ + num > max_sims_)
+      return fail(TWIXT_EINVAL, "%lld simulations since begin would exceed max_simulations %d",
+                  static_cast<long long>(sims_ + num), max_sims_);
+    return TWIXT_OK;
+  }
+
+  TwixTBatch* b_ = nullptr;
+  void* arena_mem_ = nullptr;
+  MctsArena a_{};
+  int64_t num_trees_ = 0;
+  int32_t max_sims_ = 0;
+  double c_ = 0.0;
+  int64_t count_ = 0;
+  uint64_t key_ = 0;
+  uint32_t stream0_ = 0;
+  int64_t sims_ = 0;
+  bool pending_ = false;
+  bool begun_ = false;
+};
+
 }  // namespace twixt
 
 struct twixt_batch {
   twixt::TwixTBatch impl;
+};
+
+struct twixt_mcts {
+  twixt::TwixTMCTS impl;
 };
 
 using twixt::fail;
@@ -818,6 +1050,49 @@ int twixt_stats_accumulate(twixt_stats* acc, const twixt_stats* part) {
   acc->kernel_launches += part->kernel_launches;
   if (part->max_length > acc->max_length) acc->max_length = part->max_length;
   return TWIXT_OK;
+}
+
+// ---- batched MCTS (class TwixTMCTS above, kernels in twixt_mcts.cu) ----
+#define TW_NEED_MCTS(m) \
+  if ((m) == nullptr) return fail(TWIXT_EINVAL, "null mcts handle")
+
+int twixt_mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c,
+                      twixt_mcts** out) {
+  TW_NEED(b);
+  if (out == nullptr) return fail(TWIXT_EINVAL, "null output pointer");
+  *out = nullptr;
+  twixt_mcts* m = new (std::nothrow) twixt_mcts();
+  if (m == nullptr) return fail(TWIXT_ENOMEM, "out of host memory");
+  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, uct_c);
+  if (rc != TWIXT_OK) {
+    std::string keep = twixt::g_last_error;
+    delete m;
+    twixt::g_last_error = keep;
+    return rc;
+  }
+  *out = m;
+  return TWIXT_OK;
+}
+void twixt_mcts_destroy(twixt_mcts* m) { delete m; }
+int twixt_mcts_begin(twixt_mcts* m, int64_t root_first, int64_t count) {
+  TW_NEED_MCTS(m);
+  return m->impl.Begin(root_first, count);
+}
+int twixt_mcts_run(twixt_mcts* m, int32_t num_simulations) {
+  TW_NEED_MCTS(m);
+  return m->impl.Run(num_simulations);
+}
+int twixt_mcts_select(twixt_mcts* m, int64_t leaf_first, int32_t* out_leaf_status) {
+  TW_NEED_MCTS(m);
+  return m->impl.Select(leaf_first, out_leaf_status);
+}
+int twixt_mcts_backup(twixt_mcts* m, const float* values) {
+  TW_NEED_MCTS(m);
+  return m->impl.Backup(values);
+}
+int twixt_mcts_root_stats(twixt_mcts* m, int32_t* out_visits, double* out_value_sums, int32_t* out_best) {
+  TW_NEED_MCTS(m);
+  return m->impl.RootStats(out_visits, out_value_sums, out_best);
 }
 
 int twixt_get_stats(twixt_batch* b, twixt_stats* out) {

@@ -51,6 +51,35 @@ struct PlayoutArgs {
   unsigned long long* tickets;  // &stats->tickets
 };
 
+// Device arena of a batched MCTS search (twixt_mcts.cu; sizes and byte formula in twixt_mcts.cuh).  Tree t owns
+// node slots [t*S, (t+1)*S) (slot 0 of a tree is its root), path entries [t*P, (t+1)*P) and rollout slots
+// [t*R, (t+1)*R); the edges of global node slot g are [g*M, (g+1)*M).
+struct MctsArena {
+  int n, rw, M, S, P, R;
+  uint32_t* node_rec;       // [trees*S*rw] state record of each node
+  int32_t* node_legal;      // [trees*S] number of edges, -1 while the node is not expanded
+  uint32_t* node_n;         // [trees*S] N(s)
+  uint16_t* edge_action;    // [trees*S*M] ascending legal actions
+  uint32_t* edge_n;         // [trees*S*M] N(a)
+  double* edge_w;           // [trees*S*M] W(a)
+  int32_t* edge_child;      // [trees*S*M] child slot within the tree, -1 = none yet
+  int4* tree;               // [trees] node count, leaf slot, path length, leaf status
+  int2* path;               // [trees*P] (node slot, edge << 1 | player to move at that node)
+  uint32_t* roll_rec;       // [trees*R*rw] rollout slots
+  uint64_t* roll_ids;       // [trees*R] their Philox stream ids
+  float* roll_ret;          // [trees*R*2] their returns
+  const double* log_table;  // [S] log(i)
+};
+
+cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s);
+// leaf_dst == nullptr: leaves go to the rollout slots (built-in evaluator), else to records leaf_dst + t*rw
+cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed, uint32_t stream0, uint32_t k,
+                               double uct_c, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s);
+// values == nullptr: the mean of the R rollout returns, else the caller's [count, 2] float32
+cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, cudaStream_t s);
+cudaError_t launch_mcts_root_stats(const MctsArena& a, int64_t count, int32_t* out_visits, double* out_value_sums,
+                                   int32_t* out_best, cudaStream_t s);
+
 cudaError_t launch_reset(uint32_t* records, int64_t count, int n, cudaStream_t s);
 cudaError_t launch_clone(uint32_t* dst, const uint32_t* src, const int64_t* src_ids, int64_t count, int n,
                          int64_t num_envs, int64_t dst_first, DeviceStats* stats, cudaStream_t s);

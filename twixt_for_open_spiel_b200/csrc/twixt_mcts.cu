@@ -1,0 +1,303 @@
+// twixt_mcts.cu -- kernels of the batched MCTS search (twixt_mcts_* in include/twixt_b200.h).
+//
+// One warp per tree in every kernel.  A simulation is three launches:
+//   mcts_select_kernel   descend from the root (warp-wide argmax over a node's edges, ballot/popc for the
+//                        unvisited-edge draw), expand a node on its second visit, create the child that a
+//                        simulation first reaches, and write the leaf record to its evaluator: R rollout slots
+//                        (built-in evaluator) or a batch env (stepwise form)
+//   launch_playout       the EXISTING fused playout kernel over the rollout slots, with the stream ids the
+//                        select kernel wrote (twixt_kernel_playout.cu, unchanged)
+//   mcts_backup_kernel   the leaf value (mean rollout return, caller's value or terminal Returns()) added to
+//                        every edge on the path, lanes over the path
+// The scalar arithmetic (score, draw, stream ids, best child) is in twixt_mcts.cuh, shared with the host
+// harness that checks it without a GPU.
+#include <cuda_runtime.h>
+#include <stdint.h>
+
+#include "../../include/twixt_b200.h"
+#include "twixt_engine.cuh"
+#include "twixt_kernels.cuh"
+#include "twixt_mcts.cuh"
+
+namespace twixt {
+
+namespace {
+
+constexpr unsigned kFullMask = 0xFFFFFFFFu;
+constexpr int kMctsFloodStack = 48;  // as the apply kernel
+constexpr int kMctsWarps = 4;        // trees per block
+
+__device__ __forceinline__ int64_t mcts_slot(const MctsArena& a, int64_t t, int local) {
+  return t * a.S + local;
+}
+
+// copy one record (rw is a multiple of 4 words) with 16-byte loads and stores, lanes over the quads
+__device__ __forceinline__ void warp_copy_record(uint32_t* dst, const uint32_t* src, int rw, int lane) {
+  for (int q = lane; q < rw / 4; q += 32)
+    reinterpret_cast<uint4*>(dst)[q] = reinterpret_cast<const uint4*>(src)[q];
+}
+
+// ----------------------------------------------------------------- begin ---
+// The root of tree t is a COPY of env roots + t; every tree is cleared to its root alone.
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a, const uint32_t* __restrict__ roots,
+                                                                     int64_t count) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int64_t root = mcts_slot(a, t, 0);
+  warp_copy_record(a.node_rec + root * a.rw, roots + t * a.rw, a.rw, lane);
+  if (lane == 0) {
+    a.node_legal[root] = -1;
+    a.node_n[root] = 0u;
+    a.tree[t] = make_int4(1, 0, 0, kLeafNeedsValue);
+  }
+}
+
+// ---------------------------------------------------------------- select ---
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena a, int64_t count, uint64_t seed,
+                                                                      uint32_t stream0, uint32_t k, double uct_c,
+                                                                      uint32_t* __restrict__ leaf_dst,
+                                                                      int32_t* __restrict__ out_status) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int n = a.n, rw = a.rw;
+  const uint32_t T = stream0 + static_cast<uint32_t>(t);
+  int node = 0, depth = 0, nodes = a.tree[t].x;
+  int2* path = a.path + t * a.P;
+  bool terminal;
+  for (;;) {
+    const int64_t g = mcts_slot(a, t, node);
+    uint32_t* rec = a.node_rec + g * rw;
+    const uint4 hw = *reinterpret_cast<const uint4*>(rec);
+    Header h;
+    unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+    terminal = h.result != kOpen;
+    const uint32_t visits = a.node_n[g];
+    if (terminal || visits == 0u) break;
+    const int64_t e0 = g * a.M;
+    int legal = a.node_legal[g];
+    if (legal < 0) {
+      // expand: the ascending legal list from the column words (lane = column), all edges N = 0, W = 0
+      RecordRef<1> b{rec, n};
+      const uint32_t w = lane < n ? legal_word(b, h, lane) : 0u;
+      const int c = __popc(w);
+      int incl = c;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const int o = __shfl_up_sync(kFullMask, incl, d);
+        if (lane >= d) incl += o;
+      }
+      legal = __shfl_sync(kFullMask, incl, 31);
+      uint32_t rest = w;
+      for (int i = incl - c; rest != 0u; ++i) {
+        const int y = __ffs(static_cast<int>(rest)) - 1;
+        rest &= rest - 1u;
+        a.edge_action[e0 + i] = static_cast<uint16_t>(lane * n + y);
+      }
+      for (int i = lane; i < legal; i += 32) {
+        a.edge_n[e0 + i] = 0u;
+        a.edge_w[e0 + i] = 0.0;
+        a.edge_child[e0 + i] = -1;
+      }
+      if (lane == 0) a.node_legal[g] = legal;
+      __syncwarp();
+    }
+    // unvisited edges
+    int unvisited = 0;
+    for (int i = lane; i < legal; i += 32) unvisited += a.edge_n[e0 + i] == 0u ? 1 : 0;
+    unvisited = __reduce_add_sync(kFullMask, unvisited);
+    int edge;
+    if (unvisited > 0) {
+      int j = static_cast<int>(mcts_draw(seed, T, k, static_cast<uint32_t>(unvisited)));
+      edge = -1;
+      for (int base = 0; edge < 0; base += 32) {
+        const int i = base + lane;
+        const uint32_t m = __ballot_sync(kFullMask, i < legal && a.edge_n[e0 + i] == 0u);
+        const int c = __popc(m);
+        if (j < c) edge = base + select_bit(m, j);
+        else j -= c;
+      }
+    } else {
+      const double log_parent = a.log_table[visits];
+      double best = 0.0;
+      int bi = 0x7FFFFFFF;
+      for (int i = lane; i < legal; i += 32) {
+        const double s = mcts_uct_score(a.edge_w[e0 + i], a.edge_n[e0 + i], log_parent, uct_c);
+        if (bi == 0x7FFFFFFF || mcts_score_beats(s, i, best, bi)) {
+          best = s;
+          bi = i;
+        }
+      }
+#pragma unroll
+      for (int d = 16; d > 0; d >>= 1) {
+        const double os = __shfl_xor_sync(kFullMask, best, d);
+        const int oi = __shfl_xor_sync(kFullMask, bi, d);
+        if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_score_beats(os, oi, best, bi))) {
+          best = os;
+          bi = oi;
+        }
+      }
+      edge = bi;
+    }
+    if (lane == 0) path[depth] = make_int2(node, (edge << 1) | static_cast<int>(h.ply & 1u));
+    ++depth;
+    int child = a.edge_child[e0 + edge];
+    if (child < 0) {
+      // the first visit of this edge: its child is the parent record with the move applied
+      child = nodes++;
+      const int64_t gc = mcts_slot(a, t, child);
+      uint32_t* crec = a.node_rec + gc * rw;
+      warp_copy_record(crec, rec, rw, lane);
+      __syncwarp();
+      if (lane == 0) {
+        RecordRef<1> cb{crec, n};
+        Header ch = h;
+        const int action = a.edge_action[e0 + edge];
+        const int x = action / n;
+        apply_legal_cell<kMctsFloodStack>(cb, ch, x, action - x * n);
+        uint4 o;
+        pack_header(ch, o.x, o.y, o.z, o.w);
+        *reinterpret_cast<uint4*>(crec) = o;
+        a.node_legal[gc] = -1;
+        a.node_n[gc] = 0u;
+        a.edge_child[e0 + edge] = child;
+      }
+      __syncwarp();
+    }
+    node = child;
+  }
+  const uint32_t* leaf = a.node_rec + mcts_slot(a, t, node) * rw;
+  if (leaf_dst != nullptr) {
+    warp_copy_record(leaf_dst + t * rw, leaf, rw, lane);
+  } else {
+    for (int r = 0; r < a.R; ++r) warp_copy_record(a.roll_rec + (t * a.R + r) * rw, leaf, rw, lane);
+    for (int r = lane; r < a.R; r += 32)
+      a.roll_ids[t * a.R + r] = mcts_rollout_stream(T, k, static_cast<uint32_t>(a.R), static_cast<uint32_t>(r));
+  }
+  const int status = terminal ? kLeafTerminal : kLeafNeedsValue;
+  if (lane == 0) {
+    a.tree[t] = make_int4(nodes, node, depth, status);
+    if (out_status != nullptr) out_status[t] = status;
+  }
+}
+
+// ---------------------------------------------------------------- backup ---
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena a, int64_t count,
+                                                                      const float* __restrict__ values) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int4 info = a.tree[t];
+  const int leaf = info.y, depth = info.z;
+  double v[2];
+  if (info.w == kLeafTerminal) {
+    const uint4 hw = *reinterpret_cast<const uint4*>(a.node_rec + mcts_slot(a, t, leaf) * a.rw);
+    Header h;
+    unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+    mcts_terminal_value(h, v);
+  } else if (values != nullptr) {
+    v[0] = static_cast<double>(values[2 * t]);
+    v[1] = static_cast<double>(values[2 * t + 1]);
+  } else {
+    // (double) sum_r ret_r[p] / R, r ascending
+    double s0 = 0.0, s1 = 0.0;
+    const float* ret = a.roll_ret + t * a.R * 2;
+    for (int r = 0; r < a.R; ++r) {
+      s0 = __dadd_rn(s0, static_cast<double>(ret[2 * r]));
+      s1 = __dadd_rn(s1, static_cast<double>(ret[2 * r + 1]));
+    }
+    v[0] = __ddiv_rn(s0, static_cast<double>(a.R));
+    v[1] = __ddiv_rn(s1, static_cast<double>(a.R));
+  }
+  const int2* path = a.path + t * a.P;
+  for (int i = lane; i < depth; i += 32) {
+    const int2 p = path[i];
+    const int64_t g = mcts_slot(a, t, p.x);
+    const int64_t e = g * a.M + (p.y >> 1);
+    a.node_n[g] += 1u;
+    a.edge_n[e] += 1u;
+    a.edge_w[e] = __dadd_rn(a.edge_w[e], v[p.y & 1]);
+  }
+  if (lane == 0) a.node_n[mcts_slot(a, t, leaf)] += 1u;
+}
+
+// ------------------------------------------------------------ root stats ---
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_root_stats_kernel(MctsArena a, int64_t count,
+                                                                          int32_t* __restrict__ out_visits,
+                                                                          double* __restrict__ out_value_sums,
+                                                                          int32_t* __restrict__ out_best) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int cells = a.n * a.n;
+  const int64_t g = mcts_slot(a, t, 0), e0 = g * a.M;
+  const int legal = a.node_legal[g];
+  for (int c = lane; c < cells; c += 32) {
+    if (out_visits != nullptr) out_visits[t * cells + c] = 0;
+    if (out_value_sums != nullptr) out_value_sums[t * cells + c] = 0.0;
+  }
+  __syncwarp();
+  uint32_t bn = 0u;
+  double bw = 0.0;
+  int bi = 0x7FFFFFFF;
+  for (int i = lane; i < legal; i += 32) {
+    const int action = a.edge_action[e0 + i];
+    const uint32_t en = a.edge_n[e0 + i];
+    const double ew = a.edge_w[e0 + i];
+    if (out_visits != nullptr) out_visits[t * cells + action] = static_cast<int32_t>(en);
+    if (out_value_sums != nullptr) out_value_sums[t * cells + action] = ew;
+    if (bi == 0x7FFFFFFF || mcts_best_beats(en, ew, i, bn, bw, bi)) {
+      bn = en;
+      bw = ew;
+      bi = i;
+    }
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) {
+    const uint32_t on = __shfl_xor_sync(kFullMask, bn, d);
+    const double ow = __shfl_xor_sync(kFullMask, bw, d);
+    const int oi = __shfl_xor_sync(kFullMask, bi, d);
+    if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_best_beats(on, ow, oi, bn, bw, bi))) {
+      bn = on;
+      bw = ow;
+      bi = oi;
+    }
+  }
+  if (out_best != nullptr && lane == 0)
+    out_best[t] = (legal > 0 && bi != 0x7FFFFFFF) ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
+}
+
+unsigned mcts_blocks(int64_t count) { return static_cast<unsigned>((count + kMctsWarps - 1) / kMctsWarps); }
+
+}  // namespace
+
+cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_begin_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed, uint32_t stream0, uint32_t k,
+                               double uct_c, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_select_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c, leaf_dst,
+                                                                     out_status);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_backup_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_root_stats(const MctsArena& a, int64_t count, int32_t* out_visits, double* out_value_sums,
+                                   int32_t* out_best, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_root_stats_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_visits, out_value_sums,
+                                                                         out_best);
+  return cudaGetLastError();
+}
+
+}  // namespace twixt

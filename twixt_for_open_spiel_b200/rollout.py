@@ -6,7 +6,8 @@ moves to the end; Returns() } and averages; its prior is uniform over
 LegalActions().  Here B leaves are evaluated at once: their records are copied
 R times inside a scratch batch (device-side clone) and all B*R games are played
 by ONE launch of the fused playout kernel; the host only sees [B, 2] mean
-returns.  The tree itself stays on the host, as in open_spiel.
+returns.  The tree itself stays on the host, as in open_spiel; `mcts.py` runs whole searches with the
+trees on the device.
 """
 from __future__ import annotations
 
