@@ -2,11 +2,13 @@
 """A/B timing of playout-kernel VARIANT builds on the GPU box (development tool).
 
     python tools/ab_playout.py build  name=-DFLAG=1,-DOTHER=0 ...   # here (CPU): builds tests/_build/variants/<name>.so
-    python tools/ab_playout.py run [n] [envs] [reps]                # on the GPU box: times every variant found
+    python tools/ab_playout.py run [n[,n..]] [envs] [reps] [rounds]  # on the GPU box: times every variant found
 
 Each variant runs in its own process (the library is chosen once per process through TWIXT_B200_LIB), is first
 checked against the oracle on 96 complete games, then timed with CUDA events on the launching stream: `reps`
-launches of reset + playout of `envs` fresh games, each with its own seed; prints min / median ms per launch."""
+launches of reset + playout of `envs` fresh games, each with its own seed; prints min / median ms per launch.
+A list of board sizes is timed size by size in each process; the variants alternate for `rounds` rounds
+(default 2)."""
 import os
 import subprocess
 import sys
@@ -26,7 +28,12 @@ def build(specs):
         print("built", out)
 
 
-def child(n, envs, reps):
+def child(sizes, envs, reps):
+    for n in sizes:
+        child_one(n, envs, reps)
+
+
+def child_one(n, envs, reps):
     import numpy as np
     import torch
     from oracle import pyoracle
@@ -59,8 +66,8 @@ def child(n, envs, reps):
             ms.append(e0.elapsed_time(e1))
             plies = b.stats()["plies"]
     ms.sort()
-    print("RESULT mismatches=%d min=%.3f ms median=%.3f ms  plies/launch=%d  %.2f G steps/s (median)" % (
-        bad, ms[0], ms[len(ms) // 2], plies, plies / ms[len(ms) // 2] / 1e6))
+    print("RESULT n=%d mismatches=%d min=%.3f ms median=%.3f ms  plies/launch=%d  %.2f G steps/s (median)" % (
+        n, bad, ms[0], ms[len(ms) // 2], plies, plies / ms[len(ms) // 2] / 1e6))
 
 
 def child_kernels():
@@ -87,19 +94,22 @@ def run_kernels():
             print("%-24s round %d  %s" % (name, rnd, line[0] if line else "FAILED: " + res.stderr[-600:]), flush=True)
 
 
-def run(n, envs, reps):
+def run(sizes, envs, reps, rounds):
     names = sorted(f for f in os.listdir(VDIR) if f.endswith(".so"))
-    for rnd in range(2):  # two rounds, so that a drifting clock shows up as a difference between rounds
+    for rnd in range(rounds):  # several rounds, so that a drifting clock shows up as a difference between rounds
         for name in names:
             env = dict(os.environ, TWIXT_B200_LIB=os.path.join(VDIR, name))
             try:
-                res = subprocess.run([sys.executable, os.path.abspath(__file__), "child", str(n), str(envs), str(reps)],
-                                     capture_output=True, text=True, env=env, timeout=150)
+                res = subprocess.run([sys.executable, os.path.abspath(__file__), "child", sizes, str(envs), str(reps)],
+                                     capture_output=True, text=True, env=env, timeout=150 * len(sizes.split(",")))
             except subprocess.TimeoutExpired:
                 print("%-28s round %d  TIMEOUT (hung kernel?)" % (name, rnd), flush=True)
                 return
-            line = [l for l in res.stdout.splitlines() if l.startswith("RESULT")]
-            print("%-28s round %d  %s" % (name, rnd, line[0] if line else "FAILED: " + res.stderr[-400:]), flush=True)
+            lines = [l for l in res.stdout.splitlines() if l.startswith("RESULT")]
+            for line in lines or ["FAILED: " + res.stderr[-400:]]:
+                print("%-28s round %d  %s" % (name, rnd, line), flush=True)
+            if res.returncode != 0 and lines:
+                print("%-28s round %d  FAILED: %s" % (name, rnd, res.stderr[-400:]), flush=True)
 
 
 if __name__ == "__main__":
@@ -110,7 +120,8 @@ if __name__ == "__main__":
     elif sys.argv[1] == "kernels":
         run_kernels()
     elif sys.argv[1] == "child":
-        child(int(sys.argv[2]), int(sys.argv[3]), int(sys.argv[4]))
+        child([int(x) for x in sys.argv[2].split(",")], int(sys.argv[3]), int(sys.argv[4]))
     else:
         a = sys.argv[2:]
-        run(int(a[0]) if a else 24, int(a[1]) if len(a) > 1 else 1 << 20, int(a[2]) if len(a) > 2 else 5)
+        run(a[0] if a else "24", int(a[1]) if len(a) > 1 else 1 << 20, int(a[2]) if len(a) > 2 else 5,
+            int(a[3]) if len(a) > 3 else 2)

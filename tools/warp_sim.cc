@@ -12,6 +12,8 @@
 //   policy 4  policy 1 + the FLOOD region only runs every T-th iteration (visits are batched)
 //   policy 6  policy 1 + a second FLOOD pass, only for lanes whose next move is blocked by the flood, when >= T are
 //   policy 5  policy 1 + the FLOOD region only runs when at least T lanes owe a visit, or one has waited 3 iterations
+// Work lists (compile time): the entry stack of flood_visit_entry (default), -DSIM_FRONTIER (one frontier word per
+// column) or -DSIM_COLUMNS (the kernel's: a set of columns, flood_visit_columns; "stack depth" = columns in the set).
 // Build: g++ -O2 -std=c++17 -I twixt_for_open_spiel_b200/csrc -o /tmp/warp_sim tools/warp_sim.cc
 #include <cstdint>
 #include <cstdio>
@@ -64,7 +66,15 @@ struct FrontierStack {
     sp = __builtin_popcount(dirty);
   }
 };
-#ifdef SIM_FRONTIER
+// The set of columns still to expand (flood_visit_columns): no entries at all, so the visits are made below.
+struct ColumnSet {
+  uint32_t todo = 0;
+  int sp = 0;
+  bool empty() const { return todo == 0u; }
+};
+#if defined(SIM_COLUMNS)
+using SimStack = ColumnSet;
+#elif defined(SIM_FRONTIER)
 using SimStack = FrontierStack;
 #else
 using SimStack = LocalStack<64>;
@@ -220,7 +230,7 @@ int main(int argc, char** argv) {
           }
           ++nf;
           ++visits;
-          uint32_t e;
+          uint32_t e = 0;
           if (a.stk.empty()) {
             // begin the flood that blocks the sooner move: the colour to move next first
             const int mover = static_cast<int>(a.h.ply & 1u);
@@ -230,11 +240,21 @@ int main(int argc, char** argv) {
             a.pendc[col] &= start ? ~kFloodStart : ~kFloodEnd;
             a.run_colour = col;
             e = a.originc[col];
+#if defined(SIM_COLUMNS)
+            a.stk.todo = 1u << (e >> 24);
+#endif
           } else {
+#if !defined(SIM_COLUMNS)
             e = a.stk.top();
             a.stk.pop();
+#endif
           }
+#if defined(SIM_COLUMNS)
+          flood_visit_columns(a.b, a.run_colour == kRed ? P_RED : P_BLUE, a.fplane, a.stk.todo);
+          a.stk.sp = __builtin_popcount(a.stk.todo);
+#else
           flood_visit_entry(a.b, a.fplane, a.stk, e);
+#endif
           depth_hist[a.stk.sp]++;
           ++cur_visits[l];
           if (a.stk.empty()) {

@@ -59,8 +59,9 @@ def needs_build() -> bool:
 
 
 def build(force: bool = False, verbose: bool = False, out: str = None, extra_flags=()) -> str:
-    """Build the library.  `out` / `extra_flags` build a VARIANT elsewhere (tests use it to shrink the
-    playout kernel's flood stack so that its overflow path runs); the default build is the product."""
+    """Build the library.  `out` / `extra_flags` build a VARIANT elsewhere (tests use it for the playout
+    kernel's bounds-checking build, tools/ab_playout.py for timing experiments); the default build is the
+    product."""
     variant = out is not None
     lib = out if variant else LIB
     obj_dir = (os.path.splitext(out)[0] + "_obj") if variant else OBJ_DIR

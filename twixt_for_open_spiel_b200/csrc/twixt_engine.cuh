@@ -56,6 +56,14 @@ TW_HD int tw_ctz(uint32_t v) {
   return __builtin_ctz(v);
 #endif
 }
+// index of the highest set bit, v != 0 (one FLO on the device; tw_ctz needs a BREV in front of it)
+TW_HD int tw_msb(uint32_t v) {
+#if defined(__CUDA_ARCH__)
+  return 31 - __clz(static_cast<int>(v));
+#else
+  return 31 - __builtin_clz(v);
+#endif
+}
 
 TW_HD int tw_min(int a, int b) { return a < b ? a : b; }
 TW_HD int tw_max(int a, int b) { return a > b ? a : b; }
@@ -328,10 +336,11 @@ TW_HD uint32_t links_of(const B& b, int x, int y) {
 // shifted off the board meets no link bit.  (Eight data-dependent branches per
 // visit cost more than they skipped, and the per-direction formulation was
 // 40 % more instructions.)
-template <class B, class Stack>
-TW_HD void flood_visit_entry(B& b, int flag_plane, Stack& stk, uint32_t e) {
-  const uint32_t rows = e & 0x00FFFFFFu;
-  const int cx = static_cast<int>(e >> 24);
+//
+// flood_flag_neighbours is that step for the cells `rows` of column cx: it flags their linked neighbours and
+// returns the newly flagged rows of the columns cx+1, cx+2, cx-1, cx-2 in fresh[0..3].
+template <class B>
+TW_HD void flood_flag_neighbours(B& b, int flag_plane, int cx, uint32_t rows, uint32_t fresh[4]) {
   // links stored at these cells (they are their west endpoints): NNE, ENE, ESE, SSE
   const uint32_t own0 = b.ld(P_LINK0 + 0, cx) & rows, own1 = b.ld(P_LINK0 + 1, cx) & rows;
   const uint32_t own2 = b.ld(P_LINK0 + 2, cx) & rows, own3 = b.ld(P_LINK0 + 3, cx) & rows;
@@ -350,10 +359,43 @@ TW_HD void flood_visit_entry(B& b, int flag_plane, Stack& stk, uint32_t e) {
   b.st_if(n_e2 != 0u, flag_plane, cx + 2, f_e2 | n_e2);
   b.st_if(n_w1 != 0u, flag_plane, cx - 1, f_w1 | n_w1);
   b.st_if(n_w2 != 0u, flag_plane, cx - 2, f_w2 | n_w2);
-  const bool found[4] = {n_e1 != 0u, n_e2 != 0u, n_w1 != 0u, n_w2 != 0u};
-  const uint32_t entries[4] = {flood_entry(cx + 1, n_e1), flood_entry(cx + 2, n_e2), flood_entry(cx - 1, n_w1),
-                               flood_entry(cx - 2, n_w2)};
+  fresh[0] = n_e1;
+  fresh[1] = n_e2;
+  fresh[2] = n_w1;
+  fresh[3] = n_w2;
+}
+
+template <class B, class Stack>
+TW_HD void flood_visit_entry(B& b, int flag_plane, Stack& stk, uint32_t e) {
+  const int cx = static_cast<int>(e >> 24);
+  uint32_t fresh[4];
+  flood_flag_neighbours(b, flag_plane, cx, e & 0x00FFFFFFu, fresh);
+  const bool found[4] = {fresh[0] != 0u, fresh[1] != 0u, fresh[2] != 0u, fresh[3] != 0u};
+  const uint32_t entries[4] = {flood_entry(cx + 1, fresh[0]), flood_entry(cx + 2, fresh[1]),
+                               flood_entry(cx - 1, fresh[2]), flood_entry(cx - 2, fresh[3])};
   stk.push4_if(found, entries);
+}
+
+// A flood whose work list is a SET OF COLUMNS (the fused playout kernel): bit c of `todo` = column c holds
+// cells that got the flag and may not have been expanded yet.  A visit takes the highest such column and
+// expands ALL of the flooding colour's flagged cells in it (`own_plane`), not just the new ones: re-expanding
+// a cell adds nothing unless its component still owes this flood, and then it only does that flood's work
+// early.  That rests on the flags being uniform over every component of a colour except the one whose flood
+// is running or owed, which holds for the flooding colour even after the game ends.  (It does not hold for the
+// OPPONENT: a winning move that joins a START and an END component without a neutral link owes no flood, so its
+// component keeps mixed flags; expanding all flagged cells of the column regardless of colour would spread them.)
+// A flood starts with todo = the bit of the new peg's column and ends when todo is 0; the work list needs
+// no memory and cannot overflow.
+template <class B>
+TW_HD void flood_visit_columns(B& b, int own_plane, int flag_plane, uint32_t& todo) {
+  const int cx = tw_msb(todo);
+  todo ^= 1u << cx;  // a visit flags cells of other columns only
+  uint32_t fresh[4];
+  flood_flag_neighbours(b, flag_plane, cx, b.ld(flag_plane, cx) & b.ld_pegs(own_plane, cx), fresh);
+  // bit j of `m` = column cx + j - 2 (a column off the board never gets a flag, so its bit stays clear)
+  const uint32_t m = (fresh[3] != 0u ? 1u : 0u) | (fresh[2] != 0u ? 2u : 0u) | (fresh[0] != 0u ? 8u : 0u) |
+                     (fresh[1] != 0u ? 16u : 0u);
+  todo |= (m << cx) >> 2;
 }
 
 // ... of the entry on top of the stack

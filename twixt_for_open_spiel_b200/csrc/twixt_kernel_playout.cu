@@ -18,9 +18,10 @@
 //    are interleaved with the other lanes' moves: every loop iteration runs
 //    one MOVE for the lanes without flood work and one flood VISIT for the
 //    lanes with it, instead of 31 lanes idling through one lane's whole flood;
-//    the flood stack lives in shared memory next to the planes;
+//    its work list is one register, the set of columns still to expand
+//    (flood_visit_columns);
 //  * candidate links are handled direction-major and branch-free (link_move),
-//    a flood visit handles a whole stack entry (all its cells of one column);
+//    a flood visit handles a whole column at once;
 //  * lanes are PERSISTENT: games end at different plies (250..573 at n=24), so
 //    a lane whose game is over writes its env back and takes the next env of
 //    the range from a ticket counter instead of idling until the slowest game
@@ -33,7 +34,8 @@
 // warp-uniform Philox refresh / loop-exit vote every fourth iteration.
 // Shared memory per env: the planes BLUE, RED, links x4, START, END (this
 // order puts an always-zero word in front of every link plane, so the link
-// window of a move is loaded without bounds tests) + the flood stack; the
+// window of a move is loaded without bounds tests) + 4 pad words (8n + 4 words,
+// 784 B at n = 24: nine warps fit on an SM); the
 // per-column count cache that replaces the 24-word legal scan by 6 bytewise
 // words (twixt_engine.cuh, count_cache_*) lives in registers.  The "blocked
 // neighbour" plane is write-only for the rules, so it stays in HBM and is
@@ -66,26 +68,26 @@ namespace {
 #endif
 constexpr int kPlayoutThreads = TW_PLAYOUT_THREADS;  // 4 warps per block (the default; see playout_threads)
 constexpr int kSmemPlanes = 8;        // P_RED .. P_END
-#ifndef TW_PLAYOUT_STACK_WORDS
-#define TW_PLAYOUT_STACK_WORDS 24
-#endif
-constexpr int kStackWords = TW_PLAYOUT_STACK_WORDS;  // flood stack entries (one per word; tests build with 4)
+// Words behind the END plane.  The rules' unguarded flag loads (ld_any in link_move and the flood visit) read
+// END at columns n and n+1, which land here instead of leaving the lane's column; and while an env is being
+// loaded its header is parked here (the loads' values are ignored, so whatever they find is harmless).
+constexpr int kPadWords = 4;
 constexpr int kCacheWords = 6;        // per-column count cache, four columns per word
 constexpr int kSelectLutBytes = 8 * 256;  // select_bit_lut: [rank 0..7][byte]
 constexpr unsigned kFullMask = 0xFFFFFFFFu;
 
-// words of shared memory per env: the planes and the flood stack; the run-time-size form (never instantiated,
+// words of shared memory per env: the planes and the pad words; the run-time-size form (never instantiated,
 // see PlayoutRef) would keep its count cache there too
 __host__ __device__ constexpr int playout_words(int n, bool cache_in_smem = false) {
-  return kSmemPlanes * n + kStackWords + (cache_in_smem ? kCacheWords : 0);
+  return kSmemPlanes * n + kPadWords + (cache_in_smem ? kCacheWords : 0);
 }
 
 // -DTW_PLAYOUT_BOUNDS_CHECK=1 builds the INSTRUMENTED variant used by tests/ (never the product build): every
-// shared-memory access of the rules and of the flood stack is tested against the lane's own column,
+// shared-memory access of the rules is tested against the lane's own column,
 // [0, playout_words) words, and every blocked-plane reduction against [0, n); a violation is counted in
 // DeviceStats::bounds_violations (twixt_stats.debug_violations) and the access is redirected to word 0 /
 // column 0, so a broken invariant shows up as a number instead of a fault.  The unguarded link-window and
-// flag loads are ALLOWED to leave the board (they land in this env's neighbouring planes or stack words,
+// flag loads are ALLOWED to leave the board (they land in this env's neighbouring planes or pad words,
 // see ld_link / ld_any below) but never the lane's column: that is what this variant proves.
 #ifndef TW_PLAYOUT_BOUNDS_CHECK
 #define TW_PLAYOUT_BOUNDS_CHECK 0
@@ -128,7 +130,7 @@ struct PlayoutRef {
   // first).  With it the word in front of every link plane is always zero -- red never stands in column
   // n-1 (blue's end line), and a link plane holds links at their WEST endpoint, so its column n-1 is
   // empty -- which is what ld_link needs: the rules' link-window loads carry no bounds test at all.  Words
-  // read further off the board belong to this env's neighbouring planes or its stack words.
+  // read further off the board belong to this env's neighbouring planes or its pad words.
   __device__ __forceinline__ uint32_t ld(int plane, int col) const { return p[chk(plane * n() + col) * 32]; }
   __device__ __forceinline__ void st(int plane, int col, uint32_t v) { p[chk(plane * n() + col) * 32] = v; }
   __device__ __forceinline__ uint32_t ld_link(int plane, int col) const { return ld(plane, col); }
@@ -165,14 +167,14 @@ struct PlayoutRef {
   // per-column count cache (twixt_engine.cuh, count_cache_*).  With a compile-time board size every index
   // into it is static after unrolling, so the six words live in REGISTERS (no load before a selection, no
   // store->load round trip after a move); the run-time-size instantiation keeps them in shared memory
-  // after the planes and the stack.
+  // after the planes and the pad words.
   static constexpr bool kCountCache = true;
   static constexpr bool kSelectLut = true;
   const uint8_t* lut;  // shared memory: select_bit_lut's table, filled once per block
   __device__ __forceinline__ const uint8_t* select_lut() const { return lut; }
   static constexpr bool kCacheInRegs = NT > 0;
   uint32_t cw[kCacheWords];
-  __device__ __forceinline__ uint32_t* cache_word(int i) const { return p + (kSmemPlanes * n() + kStackWords + i) * 32; }
+  __device__ __forceinline__ uint32_t* cache_word(int i) const { return p + (kSmemPlanes * n() + kPadWords + i) * 32; }
   __device__ __forceinline__ uint32_t cache_ld(int i) const { return kCacheInRegs ? cw[i] : *cache_word(i); }
   __device__ __forceinline__ void cache_st(int i, uint32_t v) {
     if (kCacheInRegs) cw[i] = v;
@@ -191,69 +193,14 @@ struct PlayoutRef {
   }
 };
 
-// The flood stack in the lane's shared-memory column.  The stack pointer is kept as a shared-space byte
-// address (no index -> address arithmetic per access), pushes are predicated stores (inline PTX: the
-// compiler would make a branch region of each), and the room test is made once per visit for all four
-// possible pushes: if four entries might not fit, none is pushed and the visit counts as overflowed (the
-// closure pass recovers whatever was dropped).
-struct SmemStack {
-  uint32_t* base;      // generic pointer to the lane's first stack word (the header is parked here while loading)
-  uint32_t base_addr;  // ... as a shared-space address
-  uint32_t top_addr;   // address one entry past the top; entries are 32 words = 128 bytes apart
-  bool overflow;
-#if TW_PLAYOUT_BOUNDS_CHECK
-  unsigned long long* viol;
-  __device__ __forceinline__ uint32_t chk(uint32_t addr) const {
-    if (addr < base_addr || addr >= base_addr + kStackWords * 128u) {
-      atomicAdd(viol, 1ull);
-      return base_addr;
-    }
-    return addr;
-  }
-#else
-  __device__ __forceinline__ uint32_t chk(uint32_t addr) const { return addr; }
-#endif
-  __device__ __forceinline__ void init(uint32_t* first_word) {
-    base = first_word;
-    base_addr = static_cast<uint32_t>(__cvta_generic_to_shared(first_word));
-    top_addr = base_addr;
-    overflow = false;
-  }
-  __device__ __forceinline__ void reset() {
-    top_addr = base_addr;
-    overflow = false;
-  }
-  __device__ __forceinline__ bool empty() const { return top_addr == base_addr; }
-  __device__ __forceinline__ void push4_if(const bool c[4], const uint32_t e[4]) {
-    const bool room = top_addr <= base_addr + (kStackWords - 4) * 128u;
-    overflow |= !room && (c[0] || c[1] || c[2] || c[3]);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const bool doit = c[i] && room;
-      asm volatile(
-          "{\n\t.reg .pred pp;\n\tsetp.ne.u32 pp, %0, 0;\n\t@pp st.shared.u32 [%1], %2;\n\t}"
-          :: "r"(static_cast<uint32_t>(doit)), "r"(doit ? chk(top_addr) : top_addr), "r"(e[i]) : "memory");
-      top_addr += doit ? 128u : 0u;
-    }
-  }
-  // pop the top entry, or take `otherwise` if there is none (branch-free: the load address is clamped)
-  __device__ __forceinline__ uint32_t top_or(uint32_t otherwise) {
-    const bool have = top_addr != base_addr;
-    top_addr -= have ? 128u : 0u;
-    uint32_t t;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(t) : "r"(chk(top_addr)) : "memory");
-    return have ? t : otherwise;
-  }
-};
-static_assert(kStackWords >= 4, "a flood visit pushes up to four entries");
-
-// resident blocks per SM the register allocation should allow: what shared memory allows for that size
 // Block geometry per board size.  The resident warps per SM are what this latency-bound kernel lives on
 // (profiles/r2_playout_occupancy_scaling.txt), and they are capped by shared memory: blocks of 128 threads
 // (with 1 KB reserved per block) leave room unused at the sizes where two of them fit but three do not.  For
 // those sizes ONE block of 9 or 10 warps is used instead (10 is what 195 registers per thread allow):
-// measured at n = 16, 28.8 -> 30.6 G steps/s.  n >= 22 fits 8 warps either way, n <= 14 fits three or four
-// blocks of 128 threads.
+// measured at n = 16, 28.8 -> 30.6 G steps/s.  With 8n + 4 words per env that gives 9 warps at n = 22..24,
+// 10 at n = 18..21, 12 (three blocks of 128, 170 registers) at n = 13..17 and 16 (four blocks, 128 registers)
+// at n <= 12.  ptxas fits every size into its register cap without spilling, and each of these counts was
+// measured faster than the previous layout's smaller one (profiles/r3_playout_flood_columns_ab.txt).
 constexpr int kBlockOverhead = 1024 + 8 * 256;  // reserved by CUDA + the select table
 __host__ __device__ constexpr int playout_blocks_of_128(int nt) { return (227 * 1024) / (128 * playout_words(nt) * 4 + kBlockOverhead); }
 __host__ __device__ constexpr int playout_one_block_warps(int nt) {
@@ -302,11 +249,9 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
   }
 #pragma unroll
   for (int i = 0; i < kCacheWords; ++i) b.cw[i] = 0u;
-  SmemStack stk;
-  stk.init(mine + kSmemPlanes * n * 32);
+  uint32_t* const pad = mine + kSmemPlanes * n * 32;  // the pad words (see kPadWords)
 #if TW_PLAYOUT_BOUNDS_CHECK
   b.viol = &a.stats->bounds_violations;
-  stk.viol = &a.stats->bounds_violations;
 #endif
   uint32_t s_lo = 0, s_hi = 0;
   // Random words: block `rq` (moves 4rq..4rq+3) in ra[], block rq+1 in rb[].  Lanes of a warp are at
@@ -329,12 +274,13 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
   uint32_t spegs[2] = {0u, 0u};
   int step = 0;
   // Border-flag floods owed: bits (2c, 2c+1) of `pend` = colour c still has to flood the START / END flag from
-  // its newest peg `origin_of[c]`; `fcol` is the colour of the flood whose entries are on the stack.  A flood of
+  // its newest peg, whose column bit is origin_r / origin_b; `todo` is the work list of the running flood (the
+  // columns still to visit, flood_visit_columns) and `fcol` its colour.  A flood of
   // colour c only ever sets flag bits of c's pegs and walks c's links, and a move of the OTHER colour only
   // reads the flags of its own pegs (link_move masks them with its candidates), so the opponent moves while
   // c's flood is still running; only c's own next move has to wait for it (TW_FLOOD_OVERLAP, modelled with
   // tools/warp_sim.cc before it was built: 4 - 5 % fewer loop iterations at n = 24).
-  uint32_t pend = 0, origin_r = 0, origin_b = 0, swapped_before = 0, fcol = 0;
+  uint32_t pend = 0, todo = 0, origin_r = 0, origin_b = 0, swapped_before = 0, fcol = 0;
   int fplane = P_START;
   bool playing = false, open_at_start = false;
   // the chosen cell is the swap (blue repeats red's first action): its first half -- taking the red peg
@@ -346,7 +292,7 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
 
   // Taking env `e` of the range is split in two so that its HBM latency overlaps the other lanes' work:
   // begin_take issues asynchronous global->shared copies (cp.async, 4 bytes each: the destination is this
-  // lane's strided column) of the header (parked in the idle flood-stack words) and the planes;
+  // lane's strided column) of the header (parked in the pad words) and the planes;
   // finish_take runs at the top of the next loop iteration, when the data has normally arrived.
   bool loading = false;
   bool have = false;  // this lane holds an env (idx >= 0; a flag, because the 64-bit compare sat in every iteration's top)
@@ -354,17 +300,17 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
     idx = e;
     have = true;
     grec = a.records + e * rw;
-    for (int w = 0; w < kHeaderWords; ++w) __pipeline_memcpy_async(stk.base + w * 32, grec + w, 4);
+    for (int w = 0; w < kHeaderWords; ++w) __pipeline_memcpy_async(pad + w * 32, grec + w, 4);
     for (int w = 0; w < kSmemPlanes * n; ++w) __pipeline_memcpy_async(mine + b.smem_word(w) * 32, grec + kHeaderWords + w, 4);
     __pipeline_commit();
     loading = true;
     playing = false;
     pend = 0;
-    stk.reset();
+    todo = 0;
   };
   auto finish_take = [&]() {
     __pipeline_wait_prior(0);
-    unpack_header(stk.base[0], stk.base[32], stk.base[64], stk.base[96], h);
+    unpack_header(pad[0], pad[32], pad[64], pad[96], h);
     b.gblk = grec + kHeaderWords + P_BLOCKED * n;
     const uint64_t stream = a.stream_ids != nullptr ? a.stream_ids[idx] : a.stream_base + static_cast<uint64_t>(idx);
     s_lo = static_cast<uint32_t>(stream);
@@ -443,7 +389,7 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
     // ---- RARE (one branch region): an env whose copy was started an iteration ago is unpacked; a finished
     // env goes back to HBM and the lane starts copying the next one
     {
-      const bool done = have && !loading && !playing && pend == 0u && stk.empty();
+      const bool done = have && !loading && !playing && pend == 0u && todo == 0u;
       if (loading || done || swap_next) {
         if (loading) {
           finish_take();
@@ -476,9 +422,9 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
     // ---- MOVE: lanes whose colour to move owes no flood make their next move -----------
 #if TW_FLOOD_OVERLAP
     const uint32_t mover = h.ply & 1u;
-    const bool flood_blocks = ((pend >> (2u * mover)) & 3u) != 0u || (!stk.empty() && fcol == mover);
+    const bool flood_blocks = ((pend >> (2u * mover)) & 3u) != 0u || (todo != 0u && fcol == mover);
 #else
-    const bool flood_blocks = pend != 0u || !stk.empty();
+    const bool flood_blocks = pend != 0u || todo != 0u;
 #endif
     if (playing && !flood_blocks) {
       if (kTrace && step < a.trace_plies)
@@ -495,9 +441,9 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
       const bool win = link_move</*kAlways=*/true>(b, pl, owed);
       finish_move(h, pl, win);
       pend |= owed << (2 * pl.player);
-      const uint32_t peg = flood_entry(pl.x, 1u << pl.y);
-      origin_r = pl.player == kRed ? peg : origin_r;
-      origin_b = pl.player == kRed ? origin_b : peg;
+      const uint32_t peg_col = 1u << pl.x;
+      origin_r = pl.player == kRed ? peg_col : origin_r;
+      origin_b = pl.player == kRed ? origin_b : peg_col;
       ++step;
       playing = h.result == kOpen && step < a.max_plies;
       sx = nx;
@@ -506,11 +452,10 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
       swap_next = playing && is_swap(h, static_cast<uint32_t>(sact));
     }
     // ---- FLOOD: one visit for the lanes that owe border-flag propagation -----
-    // One branch for "start the next pending flood" and "continue the running one": a lane whose stack is
-    // empty but which owes a flood visits the new peg itself (`origin`, no trip through the stack), the
-    // others visit the entry on top of their stack.
-    if (!stk.empty() || pend != 0u) {
-      const bool begin = stk.empty();
+    // One branch for "start the next pending flood" and "continue the running one": a lane with no running
+    // flood that owes one starts it from the new peg's column, the others visit the next column of theirs.
+    if (todo != 0u || pend != 0u) {
+      const bool begin = todo == 0u;
       // the next flood to start: the lowest owed one (red START, red END, blue START, blue END) -- any order
       // gives the same planes, and this one is three instructions (the "colour that moves next first" rule it
       // replaces cost a dozen with its variable shifts, for 0.1 % fewer iterations in tools/warp_sim.cc)
@@ -519,12 +464,8 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
       fplane = begin ? ((lsb & 5u) != 0u ? P_START : P_END) : fplane;
       fcol = begin ? (blue ? 1u : 0u) : fcol;
       pend ^= begin ? lsb : 0u;
-      const uint32_t e = stk.top_or(blue ? origin_b : origin_r);
-      flood_visit_entry(b, fplane, stk, e);
-      if (stk.empty() && stk.overflow) {
-        flood_closure(b, fcol == kRed ? P_RED : P_BLUE, fplane);
-        stk.overflow = false;
-      }
+      todo = begin ? (blue ? origin_b : origin_r) : todo;
+      flood_visit_columns(b, fcol == kRed ? P_RED : P_BLUE, fplane, todo);
     }
   }
 
