@@ -284,6 +284,40 @@ int twixt_mcts_select(twixt_mcts* m, int64_t leaf_first, int32_t* out_leaf_statu
 int twixt_mcts_backup(twixt_mcts* m, const float* values);
 int twixt_mcts_root_stats(twixt_mcts* m, int32_t* out_visits, double* out_value_sums, int32_t* out_best);
 
+/* PUCT search with policy priors (AlphaZero): open_spiel's MCTSBot with child_selection_fn = puct_value and
+ * solve = false (open_spiel python/algorithms/mcts.py: SearchNode.puct_value, SearchNode.sort_key,
+ * _apply_tree_policy, mcts_search), made deterministic.  As above: the root is a copy of an env, the tree
+ * stream id is T, a simulation descends until a terminal node or a node with N(s) == 0, the backup adds
+ * v[player to move at the parent] to every edge on the path, nodes are numbered in creation order.  What differs:
+ *  - every edge carries a prior P(a) (float32).  A non-terminal leaf is EXPANDED AT ITS BACKUP: one edge per
+ *    legal action, ascending (swap offer at ply 1), N = 0, W = 0, P(a) = priors[t, a] from the caller
+ *    (open_spiel expands on the second visit from evaluator.prior, which AlphaZeroEvaluator answers from the
+ *    network call that valued the leaf).  Without priors (twixt_mcts_run, twixt_mcts_backup, or a null
+ *    pointer) P(a) = float32(1.0 / L), RandomRolloutEvaluator.prior.  Prior entries of illegal actions, and all
+ *    entries of terminal leaves, are ignored.
+ *  - edge a under node s scores, in IEEE double without contraction, q = N(a) > 0 ? W(a)/N(a) : 0,
+ *    u = ((c * (double)P(a)) * sqrt((double)N(s))) / (double)(N(a) + 1), q + u.  Unvisited edges are scored
+ *    like any other (there is no unvisited-edge draw).  An edge whose child exists and is terminal scores
+ *    Returns()[player to move at s] (-1, 0 or +1), with no exploration term.
+ *  - ties reproduce open_spiel's shuffle of the children at expansion: edge i of node slot s has the tie key
+ *    word 0 of Philox4x32-10(key = seed, counter = (T, s, i, 2)); among equal scores the smaller key wins,
+ *    then the lower edge.
+ *  - out_best of twixt_mcts_root_stats is sort_key's maximum: (terminal child ? Returns()[root player] : 0),
+ *    then N(a), then W(a), then the tie rule; -1 while every root edge has N = 0.
+ *  - Dirichlet noise is the caller's: simulation 0's leaf is always the root, so mixing (1-eps)*p +
+ *    eps*Dir(alpha) over each row's legal actions into the priors of the FIRST backup after begin gives
+ *    open_spiel's root noise (mcts.py add_dirichlet_noise does this in float32, where open_spiel mixes in
+ *    double).
+ * twixt_mcts_backup_priors: priors [count, n*n] float32 on the host or the device, or NULL (= twixt_mcts_backup).
+ * Host priors must be finite and >= 0 everywhere, else TWIXT_EINVAL before anything is launched (trees
+ * unchanged); device priors are the caller's responsibility (no input makes the search take an edge outside
+ * the node's legal list).  Priors given to a UCT search: TWIXT_EINVAL.  run, select, backup, root_stats and
+ * destroy work on both kinds with the same errors and launch counts.  The arena adds 9 bytes per edge (prior,
+ * tie key, outcome byte; twixt_mcts.cuh). */
+int twixt_mcts_create_puct(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                           double uct_c, twixt_mcts** out);
+int twixt_mcts_backup_priors(twixt_mcts* m, const float* values, const float* priors);
+
 /* Multi-GPU plumbing for hosts that are not Python (SURVEY 8e: envs shard by contiguous global id ranges,
  * no data-path collective, one reduction of the counters).  twixt_shard_range: rank's share [first,
  * first+count) of global_envs envs over `world` ranks (shares differ by at most one env); create the rank's

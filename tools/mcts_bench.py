@@ -10,6 +10,12 @@ search timed with CUDA events, and the ms per simulation step spent in select / 
 from torch.profiler over a separate run of the same search.  BatchedRolloutEvaluator.evaluate_slots leaves/s
 at n = 12 (8192 leaves x R = 4) is on the same line as the reference point.  The device name and power limit
 are read in the same process.
+
+`puct`: the stepwise PUCT search (selection="puct", select -> backup(values, priors)) with a fixed
+device-resident prior tensor (seeded uniform random, so score ties are as rare as with a network) and zero
+values, so that the search itself is measured and no network:
+  n = 12: 8192 trees x 400 simulations;  n = 24: 1024 trees x 200
+with simulations/s and the select / backup kernel ms per step, next to the UCT configurations above.
 """
 from __future__ import annotations
 
@@ -99,6 +105,60 @@ def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int) -> di
     }
 
 
+def bench_puct(n: int, trees: int, sims: int, profile_sims: int) -> dict:
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+
+    from twixt_for_open_spiel_b200.mcts import BatchedMCTS
+    b = make_roots(n, 2 * trees, 0x70756374)  # envs [trees, 2*trees) take the leaves
+    m = BatchedMCTS(b, trees, sims, selection="puct")
+    gen = torch.Generator(device="cuda").manual_seed(1)
+    priors = torch.rand((trees, n * n), generator=gen, device="cuda", dtype=torch.float32)
+    values = torch.zeros((trees, 2), device="cuda", dtype=torch.float32)
+    status = torch.zeros(trees, dtype=torch.int32, device="cuda")
+
+    def search(k):
+        for _ in range(k):
+            m.select(trees, status)
+            m.backup(values, priors)
+
+    m.begin(0, trees)
+    search(min(sims, 20))
+    b.synchronize()
+    start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    m.begin(0, trees)
+    start.record()
+    search(sims)
+    stop.record()
+    stop.synchronize()
+    ms = start.elapsed_time(stop)
+    m.begin(0, trees)
+    b.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        search(profile_sims)
+        b.synchronize()
+    split = {"select": 0.0, "backup": 0.0}
+    for ev in prof.key_averages():
+        t = getattr(ev, "device_time_total", None)
+        if t is None:
+            t = ev.cuda_time_total
+        if "mcts_select_kernel" in ev.key:
+            split["select"] += t
+        elif "mcts_backup_kernel" in ev.key:
+            split["backup"] += t
+    best = m.best()
+    m.close()
+    b.close()
+    return {
+        "board_size": n, "trees": trees, "simulations": sims,
+        "search_ms": round(ms, 3),
+        "simulations_per_s": round(trees * sims / (ms / 1e3), 1),
+        "ms_per_simulation_step": round(ms / sims, 4),
+        "kernel_ms_per_simulation_step": {k: round(v / 1e3 / profile_sims, 4) for k, v in split.items()},
+        "roots_with_a_best_move": int((best >= 0).sum()),
+    }
+
+
 def bench_evaluator(n: int, leaves: int, R: int, reps: int) -> dict:
     from twixt_for_open_spiel_b200.rollout import BatchedRolloutEvaluator
     ev = BatchedRolloutEvaluator(n, n_rollouts=R, max_leaves=leaves, seed=1)
@@ -123,13 +183,16 @@ def main() -> None:
     info = device_info()
     if args.quick:
         configs = [(12, 256, 40, 4, 10), (24, 64, 20, 4, 5)]
+        puct = [(12, 256, 40, 10), (24, 64, 20, 5)]
         ev = (12, 256, 4, 5)
     else:
         configs = [(12, 8192, 400, 4, 50), (24, 1024, 200, 4, 50)]
+        puct = [(12, 8192, 400, 50), (24, 1024, 200, 50)]
         ev = (12, 8192, 4, 50)
     out = dict(info)
     out["configs"] = [bench_config(*c) for c in configs]
     out["evaluate_slots"] = bench_evaluator(*ev)
+    out["puct"] = [bench_puct(*c) for c in puct]
     print(json.dumps(out))
 
 

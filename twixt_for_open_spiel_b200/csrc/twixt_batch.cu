@@ -675,7 +675,7 @@ class TwixTMCTS {
     cudaFree(arena_mem_);
   }
 
-  int Init(TwixTBatch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c) {
+  int Init(TwixTBatch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c, bool puct) {
     if (num_trees <= 0) return fail(TWIXT_EINVAL, "num_trees must be positive: %lld", static_cast<long long>(num_trees));
     if (max_simulations <= 0) return fail(TWIXT_EINVAL, "max_simulations must be positive: %d", max_simulations);
     if (n_rollouts <= 0) return fail(TWIXT_EINVAL, "n_rollouts must be positive: %d", n_rollouts);
@@ -689,13 +689,15 @@ class TwixTMCTS {
     c_ = uct_c;
     const int n = b->n_;
     const MctsSizes s = mcts_sizes(n, max_simulations, n_rollouts);
-    const int64_t per_tree = mcts_bytes_per_tree(s);
-    // carve one allocation; each array starts on a 256-byte boundary
+    const int64_t per_tree = puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s);
+    // carve one allocation; each array starts on a 256-byte boundary (the last three are PUCT's, empty in UCT)
     const int64_t T = num_trees, nodes = T * s.slots, edges = nodes * s.edges, rolls = T * s.rollouts;
-    const int64_t sizes[13] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
-                               T * 16, T * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8};
-    int64_t offs[13], total = 0;
-    for (int i = 0; i < 13; ++i) {
+    const int64_t pe = puct ? edges : 0;
+    const int64_t sizes[16] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
+                               T * 16, T * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8,
+                               pe * 4, pe * 4, pe};
+    int64_t offs[16], total = 0;
+    for (int i = 0; i < 16; ++i) {
       offs[i] = total;
       total += (sizes[i] + 255) & ~static_cast<int64_t>(255);
     }
@@ -736,6 +738,9 @@ class TwixTMCTS {
     a_.roll_ret = reinterpret_cast<float*>(base + offs[11]);
     double* table = reinterpret_cast<double*>(base + offs[12]);
     a_.log_table = table;
+    a_.edge_p = puct ? reinterpret_cast<float*>(base + offs[13]) : nullptr;
+    a_.edge_key = puct ? reinterpret_cast<uint32_t*>(base + offs[14]) : nullptr;
+    a_.edge_out = puct ? reinterpret_cast<uint8_t*>(base + offs[15]) : nullptr;
     // ln N(s) from the host's libm, so that a CPU restatement of the search computes the same scores
     std::vector<double> logs(static_cast<size_t>(s.slots));
     for (size_t i = 0; i < logs.size(); ++i) logs[i] = std::log(static_cast<double>(i));
@@ -790,7 +795,7 @@ class TwixTMCTS {
       TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, k, c_, nullptr, nullptr, b.stream_));
       TW_CUDA(cudaMemsetAsync(&b.d_stats_->tickets, 0, sizeof(unsigned long long), b.stream_));
       TW_CUDA(launch_playout(p, b.stream_));
-      TW_CUDA(launch_mcts_backup(a_, count_, nullptr, b.stream_));
+      TW_CUDA(launch_mcts_backup(a_, count_, nullptr, nullptr, key_, stream0_, b.stream_));
       b.launches_ += 3;
       sims_ += 1;
     }
@@ -818,19 +823,33 @@ class TwixTMCTS {
     return TWIXT_OK;
   }
 
-  int Backup(const float* values) {
+  // priors: [count, n*n] float32 or nullptr (uniform); host priors are checked before anything is launched
+  int Backup(const float* values, const float* priors) {
     if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_backup: no search begun");
     if (!pending_) return fail(TWIXT_EINVAL, "twixt_mcts_backup without a pending twixt_mcts_select");
     if (values == nullptr && count_ > 0) return fail(TWIXT_EINVAL, "null values pointer");
+    if (priors != nullptr && a_.edge_p == nullptr)
+      return fail(TWIXT_EINVAL, "twixt_mcts_backup_priors: priors given to a UCT search (use twixt_mcts_create_puct)");
+    const size_t cells = static_cast<size_t>(a_.n) * a_.n;
+    if (priors != nullptr && count_ > 0 && !is_device_pointer(priors)) {
+      const size_t total = static_cast<size_t>(count_) * cells;
+      for (size_t i = 0; i < total; ++i)
+        if (!std::isfinite(priors[i]) || priors[i] < 0.0f)
+          return fail(TWIXT_EINVAL, "prior [%lld, %lld] = %g: priors must be finite and >= 0",
+                      static_cast<long long>(i / cells), static_cast<long long>(i % cells),
+                      static_cast<double>(priors[i]));
+    }
     if (count_ > 0) {
       DeviceGuard g(b_->device_);
       TwixTBatch& b = *b_;
       b.ScratchReset();
-      Staged in;
+      Staged in, pin;
       TW_TRY(b.StageIn(values, static_cast<size_t>(count_) * 2 * sizeof(float), &in));
-      TW_CUDA(launch_mcts_backup(a_, count_, static_cast<const float*>(in.dev), b.stream_));
+      TW_TRY(b.StageIn(priors, priors != nullptr ? static_cast<size_t>(count_) * cells * sizeof(float) : 0, &pin));
+      TW_CUDA(launch_mcts_backup(a_, count_, static_cast<const float*>(in.dev), static_cast<const float*>(pin.dev),
+                                 key_, stream0_, b.stream_));
       b.launches_ += 1;
-      if (in.host) TW_TRY(b.Sync());  // the staged copy of the values is reused by the next call
+      if (in.host || pin.host) TW_TRY(b.Sync());  // the staged copies are reused by the next call
     }
     pending_ = false;
     sims_ += 1;
@@ -1056,14 +1075,14 @@ int twixt_stats_accumulate(twixt_stats* acc, const twixt_stats* part) {
 #define TW_NEED_MCTS(m) \
   if ((m) == nullptr) return fail(TWIXT_EINVAL, "null mcts handle")
 
-int twixt_mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c,
-                      twixt_mcts** out) {
+static int mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                       double uct_c, bool puct, twixt_mcts** out) {
   TW_NEED(b);
   if (out == nullptr) return fail(TWIXT_EINVAL, "null output pointer");
   *out = nullptr;
   twixt_mcts* m = new (std::nothrow) twixt_mcts();
   if (m == nullptr) return fail(TWIXT_ENOMEM, "out of host memory");
-  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, uct_c);
+  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, uct_c, puct);
   if (rc != TWIXT_OK) {
     std::string keep = twixt::g_last_error;
     delete m;
@@ -1072,6 +1091,14 @@ int twixt_mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations
   }
   *out = m;
   return TWIXT_OK;
+}
+int twixt_mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c,
+                      twixt_mcts** out) {
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, false, out);
+}
+int twixt_mcts_create_puct(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                           double uct_c, twixt_mcts** out) {
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, true, out);
 }
 void twixt_mcts_destroy(twixt_mcts* m) { delete m; }
 int twixt_mcts_begin(twixt_mcts* m, int64_t root_first, int64_t count) {
@@ -1088,7 +1115,11 @@ int twixt_mcts_select(twixt_mcts* m, int64_t leaf_first, int32_t* out_leaf_statu
 }
 int twixt_mcts_backup(twixt_mcts* m, const float* values) {
   TW_NEED_MCTS(m);
-  return m->impl.Backup(values);
+  return m->impl.Backup(values, nullptr);
+}
+int twixt_mcts_backup_priors(twixt_mcts* m, const float* values, const float* priors) {
+  TW_NEED_MCTS(m);
+  return m->impl.Backup(values, priors);
 }
 int twixt_mcts_root_stats(twixt_mcts* m, int32_t* out_visits, double* out_value_sums, int32_t* out_best) {
   TW_NEED_MCTS(m);

@@ -69,14 +69,20 @@ struct MctsArena {
   uint64_t* roll_ids;       // [trees*R] their Philox stream ids
   float* roll_ret;          // [trees*R*2] their returns
   const double* log_table;  // [S] log(i)
+  // PUCT searches only (nullptr in a UCT search, which selects on that)
+  float* edge_p;            // [trees*S*M] prior P(a), written when the node is expanded at its backup
+  uint32_t* edge_key;       // [trees*S*M] tie key (mcts_tie_key)
+  uint8_t* edge_out;        // [trees*S*M] terminal outcome of the child (mcts_outcome_code), 0 = none
 };
 
 cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s);
 // leaf_dst == nullptr: leaves go to the rollout slots (built-in evaluator), else to records leaf_dst + t*rw
 cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed, uint32_t stream0, uint32_t k,
                                double uct_c, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s);
-// values == nullptr: the mean of the R rollout returns, else the caller's [count, 2] float32
-cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, cudaStream_t s);
+// values == nullptr: the mean of the R rollout returns, else the caller's [count, 2] float32.  A PUCT search
+// expands each non-terminal leaf with priors [count, n*n] float32 (nullptr: uniform over the legal actions).
+cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, const float* priors,
+                               uint64_t seed, uint32_t stream0, cudaStream_t s);
 cudaError_t launch_mcts_root_stats(const MctsArena& a, int64_t count, int32_t* out_visits, double* out_value_sums,
                                    int32_t* out_best, cudaStream_t s);
 

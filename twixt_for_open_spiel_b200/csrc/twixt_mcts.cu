@@ -8,9 +8,11 @@
 //   launch_playout       the EXISTING fused playout kernel over the rollout slots, with the stream ids the
 //                        select kernel wrote (twixt_kernel_playout.cu, unchanged)
 //   mcts_backup_kernel   the leaf value (mean rollout return, caller's value or terminal Returns()) added to
-//                        every edge on the path, lanes over the path
-// The scalar arithmetic (score, draw, stream ids, best child) is in twixt_mcts.cuh, shared with the host
-// harness that checks it without a GPU.
+//                        every edge on the path, lanes over the path; a PUCT search expands the leaf here
+// A PUCT search (a.edge_p != nullptr) scores every edge with its prior from the first visit on (no unvisited-edge
+// draw) and expands a non-terminal leaf in the backup kernel, where the caller's priors for it are known.
+// The scalar arithmetic (scores, draw, tie keys, stream ids, best child) is in twixt_mcts.cuh, shared with the
+// host harnesses that check it without a GPU.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -37,6 +39,37 @@ __device__ __forceinline__ void warp_copy_record(uint32_t* dst, const uint32_t* 
     reinterpret_cast<uint4*>(dst)[q] = reinterpret_cast<const uint4*>(src)[q];
 }
 
+// Expands node slot g (record rec, header h): the ascending legal list from the column words (lane = column),
+// every edge N = 0, W = 0, no child.  Returns the edge count L, also stored as the node's.
+__device__ __forceinline__ int warp_expand(const MctsArena& a, int64_t g, const uint32_t* rec, const Header& h, int lane) {
+  const int n = a.n;
+  const int64_t e0 = g * a.M;
+  RecordRef<1> b{const_cast<uint32_t*>(rec), n};
+  const uint32_t w = lane < n ? legal_word(b, h, lane) : 0u;
+  const int c = __popc(w);
+  int incl = c;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int o = __shfl_up_sync(kFullMask, incl, d);
+    if (lane >= d) incl += o;
+  }
+  const int legal = __shfl_sync(kFullMask, incl, 31);
+  uint32_t rest = w;
+  for (int i = incl - c; rest != 0u; ++i) {
+    const int y = __ffs(static_cast<int>(rest)) - 1;
+    rest &= rest - 1u;
+    a.edge_action[e0 + i] = static_cast<uint16_t>(lane * n + y);
+  }
+  for (int i = lane; i < legal; i += 32) {
+    a.edge_n[e0 + i] = 0u;
+    a.edge_w[e0 + i] = 0.0;
+    a.edge_child[e0 + i] = -1;
+  }
+  if (lane == 0) a.node_legal[g] = legal;
+  __syncwarp();
+  return legal;
+}
+
 // ----------------------------------------------------------------- begin ---
 // The root of tree t is a COPY of env roots + t; every tree is cleared to its root alone.
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a, const uint32_t* __restrict__ roots,
@@ -54,6 +87,8 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a
 }
 
 // ---------------------------------------------------------------- select ---
+// kPuct = (a.edge_p != nullptr): one instantiation per search kind, so the UCT kernel carries no PUCT code
+template <bool kPuct>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena a, int64_t count, uint64_t seed,
                                                                       uint32_t stream0, uint32_t k, double uct_c,
                                                                       uint32_t* __restrict__ leaf_dst,
@@ -77,68 +112,74 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
     if (terminal || visits == 0u) break;
     const int64_t e0 = g * a.M;
     int legal = a.node_legal[g];
-    if (legal < 0) {
-      // expand: the ascending legal list from the column words (lane = column), all edges N = 0, W = 0
-      RecordRef<1> b{rec, n};
-      const uint32_t w = lane < n ? legal_word(b, h, lane) : 0u;
-      const int c = __popc(w);
-      int incl = c;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const int o = __shfl_up_sync(kFullMask, incl, d);
-        if (lane >= d) incl += o;
-      }
-      legal = __shfl_sync(kFullMask, incl, 31);
-      uint32_t rest = w;
-      for (int i = incl - c; rest != 0u; ++i) {
-        const int y = __ffs(static_cast<int>(rest)) - 1;
-        rest &= rest - 1u;
-        a.edge_action[e0 + i] = static_cast<uint16_t>(lane * n + y);
-      }
-      for (int i = lane; i < legal; i += 32) {
-        a.edge_n[e0 + i] = 0u;
-        a.edge_w[e0 + i] = 0.0;
-        a.edge_child[e0 + i] = -1;
-      }
-      if (lane == 0) a.node_legal[g] = legal;
-      __syncwarp();
-    }
-    // unvisited edges
-    int unvisited = 0;
-    for (int i = lane; i < legal; i += 32) unvisited += a.edge_n[e0 + i] == 0u ? 1 : 0;
-    unvisited = __reduce_add_sync(kFullMask, unvisited);
     int edge;
-    if (unvisited > 0) {
-      int j = static_cast<int>(mcts_draw(seed, T, k, static_cast<uint32_t>(unvisited)));
-      edge = -1;
-      for (int base = 0; edge < 0; base += 32) {
-        const int i = base + lane;
-        const uint32_t m = __ballot_sync(kFullMask, i < legal && a.edge_n[e0 + i] == 0u);
-        const int c = __popc(m);
-        if (j < c) edge = base + select_bit(m, j);
-        else j -= c;
-      }
-    } else {
-      const double log_parent = a.log_table[visits];
+    if constexpr (kPuct) {
+      // PUCT: the node was expanded at its first backup; warp argmax of (score, smaller key, lower edge)
+      const double sq = mcts_sqrt_visits(visits);
       double best = 0.0;
+      uint32_t bk = 0u;
       int bi = 0x7FFFFFFF;
       for (int i = lane; i < legal; i += 32) {
-        const double s = mcts_uct_score(a.edge_w[e0 + i], a.edge_n[e0 + i], log_parent, uct_c);
-        if (bi == 0x7FFFFFFF || mcts_score_beats(s, i, best, bi)) {
-          best = s;
+        const uint8_t o = a.edge_out[e0 + i];
+        const double sc = o != 0 ? static_cast<double>(mcts_outcome_value(o))
+                                 : mcts_puct_score(a.edge_w[e0 + i], a.edge_n[e0 + i], a.edge_p[e0 + i], sq, uct_c);
+        const uint32_t key = a.edge_key[e0 + i];
+        if (bi == 0x7FFFFFFF || mcts_puct_beats(sc, key, i, best, bk, bi)) {
+          best = sc;
+          bk = key;
           bi = i;
         }
       }
 #pragma unroll
       for (int d = 16; d > 0; d >>= 1) {
         const double os = __shfl_xor_sync(kFullMask, best, d);
+        const uint32_t ok = __shfl_xor_sync(kFullMask, bk, d);
         const int oi = __shfl_xor_sync(kFullMask, bi, d);
-        if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_score_beats(os, oi, best, bi))) {
+        if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_puct_beats(os, ok, oi, best, bk, bi))) {
           best = os;
+          bk = ok;
           bi = oi;
         }
       }
       edge = bi;
+    } else {
+      if (legal < 0) legal = warp_expand(a, g, rec, h, lane);
+      // unvisited edges
+      int unvisited = 0;
+      for (int i = lane; i < legal; i += 32) unvisited += a.edge_n[e0 + i] == 0u ? 1 : 0;
+      unvisited = __reduce_add_sync(kFullMask, unvisited);
+      if (unvisited > 0) {
+        int j = static_cast<int>(mcts_draw(seed, T, k, static_cast<uint32_t>(unvisited)));
+        edge = -1;
+        for (int base = 0; edge < 0; base += 32) {
+          const int i = base + lane;
+          const uint32_t m = __ballot_sync(kFullMask, i < legal && a.edge_n[e0 + i] == 0u);
+          const int c = __popc(m);
+          if (j < c) edge = base + select_bit(m, j);
+          else j -= c;
+        }
+      } else {
+        const double log_parent = a.log_table[visits];
+        double best = 0.0;
+        int bi = 0x7FFFFFFF;
+        for (int i = lane; i < legal; i += 32) {
+          const double s = mcts_uct_score(a.edge_w[e0 + i], a.edge_n[e0 + i], log_parent, uct_c);
+          if (bi == 0x7FFFFFFF || mcts_score_beats(s, i, best, bi)) {
+            best = s;
+            bi = i;
+          }
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+          const double os = __shfl_xor_sync(kFullMask, best, d);
+          const int oi = __shfl_xor_sync(kFullMask, bi, d);
+          if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_score_beats(os, oi, best, bi))) {
+            best = os;
+            bi = oi;
+          }
+        }
+        edge = bi;
+      }
     }
     if (lane == 0) path[depth] = make_int2(node, (edge << 1) | static_cast<int>(h.ply & 1u));
     ++depth;
@@ -162,6 +203,8 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
         a.node_legal[gc] = -1;
         a.node_n[gc] = 0u;
         a.edge_child[e0 + edge] = child;
+        if (kPuct && ch.result != kOpen)
+          a.edge_out[e0 + edge] = mcts_outcome_code(ch, static_cast<int>(h.ply & 1u));
       }
       __syncwarp();
     }
@@ -184,7 +227,9 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
 
 // ---------------------------------------------------------------- backup ---
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena a, int64_t count,
-                                                                      const float* __restrict__ values) {
+                                                                      const float* __restrict__ values,
+                                                                      const float* __restrict__ priors,
+                                                                      uint64_t seed, uint32_t stream0) {
   const int lane = threadIdx.x & 31;
   const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
   if (t >= count) return;
@@ -220,6 +265,24 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
     a.edge_w[e] = __dadd_rn(a.edge_w[e], v[p.y & 1]);
   }
   if (lane == 0) a.node_n[mcts_slot(a, t, leaf)] += 1u;
+  if (a.edge_p != nullptr && info.w != kLeafTerminal) {
+    // PUCT: expand the leaf with its priors (open_spiel expands on the second visit from evaluator.prior, which
+    // AlphaZeroEvaluator answers from the network call that valued the leaf)
+    const int64_t g = mcts_slot(a, t, leaf), e0 = g * a.M;
+    const uint32_t* rec = a.node_rec + g * a.rw;
+    const uint4 hw = *reinterpret_cast<const uint4*>(rec);
+    Header h;
+    unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+    const int legal = warp_expand(a, g, rec, h, lane);
+    const float uniform = mcts_uniform_prior(legal);
+    const float* row = priors != nullptr ? priors + t * a.n * a.n : nullptr;
+    const uint32_t T = stream0 + static_cast<uint32_t>(t);
+    for (int i = lane; i < legal; i += 32) {
+      a.edge_p[e0 + i] = row != nullptr ? row[a.edge_action[e0 + i]] : uniform;
+      a.edge_key[e0 + i] = mcts_tie_key(seed, T, static_cast<uint32_t>(leaf), static_cast<uint32_t>(i));
+      a.edge_out[e0 + i] = 0;
+    }
+  }
 }
 
 // ------------------------------------------------------------ root stats ---
@@ -238,6 +301,49 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_root_stats_kernel(MctsAr
     if (out_value_sums != nullptr) out_value_sums[t * cells + c] = 0.0;
   }
   __syncwarp();
+  if (a.edge_p != nullptr) {
+    // PUCT BestChild: (terminal outcome, N, W), then the tie key, then the lower edge; -1 while no N > 0
+    int bo = 0;
+    uint32_t bn = 0u, bk = 0u, nmax = 0u;
+    double bw = 0.0;
+    int bi = 0x7FFFFFFF;
+    for (int i = lane; i < legal; i += 32) {
+      const int action = a.edge_action[e0 + i];
+      const uint32_t en = a.edge_n[e0 + i];
+      const double ew = a.edge_w[e0 + i];
+      const int eo = mcts_outcome_value(a.edge_out[e0 + i]);
+      const uint32_t ek = a.edge_key[e0 + i];
+      if (out_visits != nullptr) out_visits[t * cells + action] = static_cast<int32_t>(en);
+      if (out_value_sums != nullptr) out_value_sums[t * cells + action] = ew;
+      nmax = en > nmax ? en : nmax;
+      if (bi == 0x7FFFFFFF || mcts_puct_best_beats(eo, en, ew, ek, i, bo, bn, bw, bk, bi)) {
+        bo = eo;
+        bn = en;
+        bw = ew;
+        bk = ek;
+        bi = i;
+      }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+      const int oo = __shfl_xor_sync(kFullMask, bo, d);
+      const uint32_t on = __shfl_xor_sync(kFullMask, bn, d);
+      const double ow = __shfl_xor_sync(kFullMask, bw, d);
+      const uint32_t ok = __shfl_xor_sync(kFullMask, bk, d);
+      const int oi = __shfl_xor_sync(kFullMask, bi, d);
+      if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_puct_best_beats(oo, on, ow, ok, oi, bo, bn, bw, bk, bi))) {
+        bo = oo;
+        bn = on;
+        bw = ow;
+        bk = ok;
+        bi = oi;
+      }
+    }
+    nmax = __reduce_max_sync(kFullMask, nmax);
+    if (out_best != nullptr && lane == 0)
+      out_best[t] = nmax > 0u ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
+    return;
+  }
   uint32_t bn = 0u;
   double bw = 0.0;
   int bi = 0x7FFFFFFF;
@@ -281,14 +387,19 @@ cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t
 cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed, uint32_t stream0, uint32_t k,
                                double uct_c, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  mcts_select_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c, leaf_dst,
-                                                                     out_status);
+  if (a.edge_p != nullptr)
+    mcts_select_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c,
+                                                                           leaf_dst, out_status);
+  else
+    mcts_select_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c,
+                                                                            leaf_dst, out_status);
   return cudaGetLastError();
 }
 
-cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, cudaStream_t s) {
+cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, const float* priors,
+                               uint64_t seed, uint32_t stream0, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  mcts_backup_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values);
+  mcts_backup_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
   return cudaGetLastError();
 }
 

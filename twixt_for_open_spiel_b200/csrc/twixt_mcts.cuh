@@ -8,6 +8,12 @@
 //   unvisited-edge draw  word 0 of Philox4x32-10(key = seed, counter = (T lo, T hi, k, 1)), index (w*U) >> 32
 //   rollout stream id    (T << 32) | (k*R + r)
 //   best child           most visits, then larger W, then lowest action
+// and, for a PUCT search (twixt_mcts_create_puct):
+//   puct score           q = N(a) > 0 ? W/N(a) : 0, u = ((c * P) * sqrt(N(s))) / (N(a) + 1), q + u in IEEE
+//                        double, no contraction; an edge whose child is terminal scores Returns()[player at s]
+//   tie key              word 0 of Philox4x32-10(key = seed, counter = (T, node slot, edge, 2)); among equal
+//                        scores the smaller key wins, then the lower edge
+//   best child           (terminal outcome or 0, N, W), then the tie key, then the lower edge
 //
 // Storage of one tree (S = max_simulations + 1 node slots, M = max_legal_actions = n(n-2),
 // rw = record_words(n), P = min(max_simulations, max_game_length) + 1 path entries, R = n_rollouts):
@@ -17,6 +23,8 @@
 //              + R * (rw*4 + 8 + 8) (rollout slot records, stream ids, float returns)
 //   bytes per tree = S * (rw*4 + 8 + 18*M) + 16 + 8*P + R * (rw*4 + 16)
 // plus one table of (max_simulations + 1) doubles per search.  At n = 12 a node is 2 616 bytes.
+// A PUCT search adds per edge 4 (prior P f32) + 4 (tie key u32) + 1 (terminal outcome u8):
+//   PUCT bytes per tree = S * (rw*4 + 8 + 27*M) + 16 + 8*P + R * (rw*4 + 16)
 #pragma once
 #include <stdint.h>
 
@@ -55,6 +63,9 @@ TW_HD int64_t mcts_bytes_per_tree(const MctsSizes& s) {
   return s.slots * (s.rw * 4 + 8 + 18 * s.edges) + 16 + 8 * s.path + s.rollouts * (s.rw * 4 + 16);
 }
 
+// the PUCT formula of the header comment above
+TW_HD int64_t mcts_puct_bytes_per_tree(const MctsSizes& s) { return mcts_bytes_per_tree(s) + s.slots * 9 * s.edges; }
+
 // UCT score of an edge with N(a) = n > 0 visits and value sum w, under a parent whose ln N(s) is log_parent.
 // Bit-identical on the device and on a host compiled with -ffp-contract=off.
 TW_HD double mcts_uct_score(double w, uint32_t n, double log_parent, double c) {
@@ -77,6 +88,74 @@ TW_HD bool mcts_score_beats(double a, int ia, double b, int ib) { return a > b |
 TW_HD bool mcts_best_beats(uint32_t na, double wa, int ia, uint32_t nb, double wb, int ib) {
   if (na != nb) return na > nb;
   if (wa != wb) return wa > wb;
+  return ia < ib;
+}
+
+// sqrt(N(s)) of the PUCT score, once per node
+TW_HD double mcts_sqrt_visits(uint32_t parent_visits) {
+#if defined(__CUDA_ARCH__)
+  return __dsqrt_rn(static_cast<double>(parent_visits));
+#else
+  return std::sqrt(static_cast<double>(parent_visits));
+#endif
+}
+
+// PUCT score of an edge with N(a) = n visits, value sum w and prior p under a parent with sqrt(N(s)) =
+// sqrt_parent, in open_spiel's evaluation order (SearchNode.puct_value).  Bit-identical on the device and on a
+// host compiled with -ffp-contract=off.
+TW_HD double mcts_puct_score(double w, uint32_t n, float p, double sqrt_parent, double c) {
+  const double nd = static_cast<double>(n), n1 = static_cast<double>(n) + 1.0;
+#if defined(__CUDA_ARCH__)
+  const double q = n > 0u ? __ddiv_rn(w, nd) : 0.0;
+  const double u = __ddiv_rn(__dmul_rn(__dmul_rn(c, static_cast<double>(p)), sqrt_parent), n1);
+  return __dadd_rn(q, u);
+#else
+  const double q = n > 0u ? w / nd : 0.0;
+  const double u = ((c * static_cast<double>(p)) * sqrt_parent) / n1;
+  return q + u;
+#endif
+}
+
+// P(a) when no priors are given: float32(1.0 / L), RandomRolloutEvaluator.prior
+TW_HD float mcts_uniform_prior(int legal) {
+#if defined(__CUDA_ARCH__)
+  return __double2float_rn(__ddiv_rn(1.0, static_cast<double>(legal)));
+#else
+  return static_cast<float>(1.0 / static_cast<double>(legal));
+#endif
+}
+
+// the tie key of edge `edge` of node slot `slot` (its place in open_spiel's shuffled child list)
+TW_HD uint32_t mcts_tie_key(uint64_t seed, uint32_t tree_stream, uint32_t slot, uint32_t edge) {
+  uint32_t r[4];
+  philox4x32_10(tree_stream, slot, edge, 2u, static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), r);
+  return r[0];
+}
+
+// PUCT selection: (score a, key ka, edge ia) beats (b, kb, ib): the larger score, then the smaller key, then
+// the lower edge
+TW_HD bool mcts_puct_beats(double a, uint32_t ka, int ia, double b, uint32_t kb, int ib) {
+  if (a != b) return a > b;
+  if (ka != kb) return ka < kb;
+  return ia < ib;
+}
+
+// terminal outcome byte of an edge: 0 while its child does not exist or is not terminal, else
+// 2 + Returns()[player to move at the parent]
+TW_HD uint8_t mcts_outcome_code(const Header& child, int player) {
+  const int red = child.result == kRedWin ? 1 : (child.result == kBlueWin ? -1 : 0);
+  return static_cast<uint8_t>(2 + (player == 0 ? red : -red));
+}
+TW_HD int mcts_outcome_value(uint8_t code) { return code == 0 ? 0 : static_cast<int>(code) - 2; }
+
+// PUCT BestChild (open_spiel SearchNode.sort_key): (outcome value, N, W), then the smaller key, then the
+// lower edge
+TW_HD bool mcts_puct_best_beats(int oa, uint32_t na, double wa, uint32_t ka, int ia, int ob, uint32_t nb, double wb,
+                                uint32_t kb, int ib) {
+  if (oa != ob) return oa > ob;
+  if (na != nb) return na > nb;
+  if (wa != wb) return wa > wb;
+  if (ka != kb) return ka < kb;
   return ia < ib;
 }
 

@@ -11,6 +11,11 @@ Two ways to evaluate leaves:
     the caller evaluates them (e.g. `observation_and_mask` + a value network) and hands the values to
     `backup(values)`.
 
+`selection="puct"` makes every tree open_spiel's AlphaZero search instead (MCTSBot with
+child_selection_fn = puct_value): `backup(values, priors)` hands the policy head's priors [count, n*n] with
+the values, and the leaf is expanded with them.  `add_dirichlet_noise` mixes open_spiel's root noise into the
+priors of the first backup after `begin` (simulation 0's leaf is always the root).
+
 `MCTSBot` is the open_spiel-shaped bot over one tree for adapter `TwixTState`s.
 
 Arrays may be numpy (synchronous) or torch CUDA tensors (asynchronous on the batch's stream), as for
@@ -31,12 +36,16 @@ LEAF_NEEDS_VALUE, LEAF_TERMINAL = 0, 1
 
 class BatchedMCTS:
     def __init__(self, batch: TwixTBatch, num_trees: int, max_simulations: int, n_rollouts: int = 1,
-                 uct_c: float = 2.0):
+                 uct_c: float = 2.0, selection: str = "uct"):
+        if selection not in ("uct", "puct"):
+            raise ValueError("selection must be 'uct' or 'puct', got %r" % (selection,))
         self._lib = _lib.load()
         self.batch = batch  # the search runs on the batch's envs and stream: keep it alive
         self._h = C.c_void_p()
-        self._check(self._lib.twixt_mcts_create(batch._h, int(num_trees), int(max_simulations), int(n_rollouts),
-                                                float(uct_c), C.byref(self._h)))
+        create = self._lib.twixt_mcts_create_puct if selection == "puct" else self._lib.twixt_mcts_create
+        self._check(create(batch._h, int(num_trees), int(max_simulations), int(n_rollouts), float(uct_c),
+                           C.byref(self._h)))
+        self.selection = selection
         self.num_trees = int(num_trees)
         self.max_simulations = int(max_simulations)
         self.n_rollouts = int(n_rollouts)
@@ -80,15 +89,21 @@ class BatchedMCTS:
                                                 _ptr(out_status, _dt(np.int32, "int32"), self.count)))
         return out_status
 
-    def backup(self, values):
-        """Stepwise form, second half: values [count, 2] float32 of the leaves select() wrote."""
+    def backup(self, values, priors=None):
+        """Stepwise form, second half: values [count, 2] float32 of the leaves select() wrote.  A PUCT search
+        also takes priors [count, n*n] float32 (None: uniform over the legal actions); entries of illegal
+        actions and rows of terminal leaves are ignored."""
         if not _is_torch(values):
             values = np.ascontiguousarray(values, dtype=np.float32)
-        self._check(self._lib.twixt_mcts_backup(self._h, _ptr(values, _dt(np.float32, "float32"), 2 * self.count)))
+        if priors is not None and not _is_torch(priors):
+            priors = np.ascontiguousarray(priors, dtype=np.float32)
+        self._check(self._lib.twixt_mcts_backup_priors(
+            self._h, _ptr(values, _dt(np.float32, "float32"), 2 * self.count),
+            _ptr(priors, _dt(np.float32, "float32"), self.count * self._cells)))
 
     def root_stats(self, out_visits=None, out_value_sums=None, out_best=None):
         """(visits [count, n*n] int32, value_sums [count, n*n] float64, best [count] int32) of the root edges;
-        best is -1 where the root is terminal or not yet expanded."""
+        best is -1 where the root is terminal or not yet expanded (PUCT: while no root edge has a visit)."""
         if out_visits is None:
             out_visits = np.zeros((self.count, self._cells), dtype=np.int32)
         if out_value_sums is None:
@@ -103,6 +118,26 @@ class BatchedMCTS:
 
     def best(self) -> np.ndarray:
         return self.root_stats()[2]
+
+
+def add_dirichlet_noise(priors, legal_mask, epsilon: float, alpha: float):
+    """open_spiel's root noise: (1 - epsilon) * p + epsilon * Dir(alpha) over each row's legal actions.
+
+    priors [B, A] float32 and legal_mask [B, A] (bool or 0/1) are torch tensors on the CPU or a GPU; returns a
+    new float32 tensor on the same device.  Gamma(alpha) is drawn for every entry with torch's generator (so the
+    result is reproducible under torch.manual_seed), in float64, zeroed where illegal and normalised per row;
+    the mix is done in float32 (open_spiel mixes in double).  Entries of illegal actions are returned
+    unchanged.  A row whose legal draws all underflow to 0 gets uniform noise over its legal actions."""
+    import torch
+    legal = legal_mask.to(device=priors.device, dtype=torch.bool)
+    conc = torch.full(priors.shape, float(alpha), dtype=torch.float64, device=priors.device)
+    g = torch.where(legal, torch.distributions.Gamma(conc, torch.ones_like(conc)).sample(),
+                    torch.zeros_like(conc))
+    total = g.sum(dim=1, keepdim=True)
+    uniform = legal.to(torch.float64) / legal.sum(dim=1, keepdim=True).clamp_min(1)
+    noise = torch.where(total > 0, g / torch.where(total > 0, total, torch.ones_like(total)), uniform)
+    mixed = (1.0 - float(epsilon)) * priors.float() + float(epsilon) * noise.float()
+    return torch.where(legal, mixed, priors.float())
 
 
 class MCTSBot:
