@@ -244,7 +244,8 @@ int twixt_get_stats(twixt_batch* b, twixt_stats* out);
 int twixt_stats_reset(twixt_batch* b);
 
 /* Batched MCTS: `num_trees` independent searches on the device, each open_spiel's MCTSBot with
- * RandomRolloutEvaluator(n_rollouts), solve = false and no Dirichlet noise, made deterministic:
+ * RandomRolloutEvaluator(n_rollouts), solve = false (the solver is TWIXT_MCTS_SOLVE, below) and no Dirichlet
+ * noise, made deterministic:
  *  - twixt_mcts_begin: the root of tree t is a COPY of env root_first + t (later changes to that env do not
  *    affect the tree); its stream id is T = stream_base + root_first + t (twixt_set_stream_base, so results do
  *    not depend on sharding), which must be below 2^32.  The batch's seed at begin keys every draw.
@@ -317,6 +318,42 @@ int twixt_mcts_root_stats(twixt_mcts* m, int32_t* out_visits, double* out_value_
 int twixt_mcts_create_puct(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
                            double uct_c, twixt_mcts** out);
 int twixt_mcts_backup_priors(twixt_mcts* m, const float* values, const float* priors);
+
+/* MCTS-Solver (open_spiel MCTSBot(..., solve=True), its default; python/algorithms/mcts.py mcts_search).
+ * twixt_mcts_create_ex takes flags: TWIXT_MCTS_PUCT selects PUCT (flags 0 and TWIXT_MCTS_PUCT are exactly
+ * twixt_mcts_create and twixt_mcts_create_puct), TWIXT_MCTS_SOLVE adds the solver to either kind; other bits are
+ * TWIXT_EINVAL.  Everything above holds, plus:
+ *  - every edge has an outcome code: 0 unknown, else 2 + the child's value for the player to move at the parent
+ *    (1 loss, 2 draw, 3 win).  It is set when a terminal child is created and when a child becomes proven.
+ *  - proof pass: in the backup of a simulation whose leaf is terminal, and only then, walking up the path from
+ *    the leaf's parent: node c (player to move p) is proven when some edge of c has code 3 (a win for p) or
+ *    all of its edges have non-zero codes; its value is v = max(code) - 2 and the parent's edge into c gets
+ *    code 2 - v (zero-sum, players alternate by ply: the swap is blue's move at ply 1).  The walk stops at the
+ *    first node that is not proven.  A proven root, or a terminal root at its first simulation (with
+ *    Returns()), makes the tree FINISHED.
+ *  - a finished tree does nothing in later simulations: select takes no path and reports leaf status 2
+ *    (TWIXT_MCTS_LEAF_SOLVED), the stepwise form leaves env leaf_first + t untouched, backup ignores that
+ *    row's values and priors, and its rollout slots add no plies and no games to twixt_stats.  The
+ *    simulation counter and the max_simulations check do not change.
+ *  - UCT + solve: a visited edge with a non-zero code scores its value (-1, 0, +1) instead of the UCT term
+ *    (open_spiel uct_value); the unvisited-edge draw comes first as before.  out_best of twixt_mcts_root_stats is
+ *    open_spiel's sort_key: (outcome value, N, W), then the lowest action; -1 while the root is terminal or
+ *    unexpanded.  PUCT + solve: selection and out_best read the codes as PUCT does for terminal children.
+ *  - arena: 1 byte per tree more, and a UCT search 1 byte per edge (twixt_mcts.cuh).
+ * twixt_mcts_solver_stats: out_proven [count] u8 (1 once the root is proven), out_returns [count, 2] float32
+ * (open_spiel's root.outcome: Returns() of the proven result, (0, 0) while unproven), out_edge_values
+ * [count, n*n] int8 (-1, 0 or +1 for a proven root move, from the view of the player to move at the root;
+ * TWIXT_MCTS_UNPROVEN elsewhere), out_simulations [count] int32 (N(root): the simulations the tree ran since
+ * begin).  Each pointer is nullable, host or device; one launch.  TWIXT_EINVAL on a search created without
+ * TWIXT_MCTS_SOLVE, before begin, or while a select awaits its backup. */
+#define TWIXT_MCTS_PUCT 1u
+#define TWIXT_MCTS_SOLVE 2u
+#define TWIXT_MCTS_LEAF_SOLVED 2
+#define TWIXT_MCTS_UNPROVEN (-128)
+int twixt_mcts_create_ex(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                         double uct_c, uint32_t flags, twixt_mcts** out);
+int twixt_mcts_solver_stats(twixt_mcts* m, uint8_t* out_proven, float* out_returns, int8_t* out_edge_values,
+                            int32_t* out_simulations);
 
 /* Multi-GPU plumbing for hosts that are not Python (SURVEY 8e: envs shard by contiguous global id ranges,
  * no data-path collective, one reduction of the counters).  twixt_shard_range: rank's share [first,

@@ -16,6 +16,12 @@ device-resident prior tensor (seeded uniform random, so score ties are as rare a
 values, so that the search itself is measured and no network:
   n = 12: 8192 trees x 400 simulations;  n = 24: 1024 trees x 200
 with simulations/s and the select / backup kernel ms per step, next to the UCT configurations above.
+
+`solve`: the MCTS-Solver (solve=True, UCT with rollouts):
+  n = 12: the first UCT configuration above with solve=True: the solver's overhead where little gets proven;
+  n = 8 endgames: 8192 roots 2..6 plies before the end of seeded games x 400 simulations x R = 4, where most
+  trees finish early; simulations/s counts every tree's simulations (finished ones too), next to the fraction of
+  roots proven, the mean N(root) and the backup kernel ms per step.
 """
 from __future__ import annotations
 
@@ -53,13 +59,27 @@ def make_roots(n: int, trees: int, seed: int):
     return b
 
 
-def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int) -> dict:
+def endgame_roots(n: int, trees: int, seed: int):
+    from twixt_for_open_spiel_b200 import TwixTBatch
+    sys.path.insert(0, os.path.join(ROOT, "examples"))
+    try:
+        from mcts_solver import endgame_roots as make
+    finally:
+        sys.path.pop(0)
+    b = TwixTBatch(n, trees, 0, seed)
+    make(b, 0, trees)
+    b.use_torch_stream()
+    return b
+
+
+def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int, solve: bool = False,
+                 endgame: bool = False) -> dict:
     import torch
     from torch.profiler import ProfilerActivity, profile
 
     from twixt_for_open_spiel_b200.mcts import BatchedMCTS
-    b = make_roots(n, trees, 0x6D637473)
-    m = BatchedMCTS(b, trees, sims, R)
+    b = endgame_roots(n, trees, 0x736F6C76) if endgame else make_roots(n, trees, 0x6D637473)
+    m = BatchedMCTS(b, trees, sims, R, solve=solve)
     # warm-up: every kernel of a simulation, at this size
     m.begin(0, trees)
     m.run(min(sims, 20))
@@ -73,6 +93,7 @@ def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int) -> di
     stop.synchronize()
     ms = start.elapsed_time(stop)
     plies = b.stats()["plies"] - p0
+    solved = m.solver_stats() if solve else None
     # the split, from the kernels' device time in a separate profiled run
     m.begin(0, trees)
     b.synchronize()
@@ -94,7 +115,7 @@ def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int) -> di
     best = m.best()
     m.close()
     b.close()
-    return {
+    out = {
         "board_size": n, "trees": trees, "simulations": sims, "n_rollouts": R,
         "search_ms": round(ms, 3),
         "simulations_per_s": round(trees * sims / (ms / 1e3), 1),
@@ -103,6 +124,12 @@ def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int) -> di
         "kernel_ms_per_simulation_step": {k: round(v / 1e3 / profile_sims, 4) for k, v in split.items()},
         "roots_with_a_best_move": int((best >= 0).sum()),
     }
+    if solve:
+        proven, _, _, simulations = solved
+        out.update({"solve": True, "roots": "endgame" if endgame else "opening",
+                    "fraction_proven": round(float(proven.mean()), 4),
+                    "mean_root_visits": round(float(simulations.mean()), 2)})
+    return out
 
 
 def bench_puct(n: int, trees: int, sims: int, profile_sims: int) -> dict:
@@ -176,6 +203,7 @@ def bench_evaluator(n: int, leaves: int, R: int, reps: int) -> dict:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--quick", action="store_true", help="small sizes (a functional check, not a measurement)")
+    ap.add_argument("--no-solve", action="store_true", help="skip the solver entries")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -185,14 +213,18 @@ def main() -> None:
         configs = [(12, 256, 40, 4, 10), (24, 64, 20, 4, 5)]
         puct = [(12, 256, 40, 10), (24, 64, 20, 5)]
         ev = (12, 256, 4, 5)
+        solve = [(12, 256, 40, 4, 10, True, False), (8, 256, 40, 4, 10, True, True)]
     else:
         configs = [(12, 8192, 400, 4, 50), (24, 1024, 200, 4, 50)]
         puct = [(12, 8192, 400, 50), (24, 1024, 200, 50)]
         ev = (12, 8192, 4, 50)
+        solve = [(12, 8192, 400, 4, 50, True, False), (8, 8192, 400, 4, 50, True, True)]
     out = dict(info)
     out["configs"] = [bench_config(*c) for c in configs]
     out["evaluate_slots"] = bench_evaluator(*ev)
     out["puct"] = [bench_puct(*c) for c in puct]
+    if not args.no_solve:
+        out["solve"] = [bench_config(*c) for c in solve]
     print(json.dumps(out))
 
 

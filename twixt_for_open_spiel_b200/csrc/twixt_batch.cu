@@ -675,7 +675,8 @@ class TwixTMCTS {
     cudaFree(arena_mem_);
   }
 
-  int Init(TwixTBatch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c, bool puct) {
+  int Init(TwixTBatch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c, bool puct,
+           bool solve) {
     if (num_trees <= 0) return fail(TWIXT_EINVAL, "num_trees must be positive: %lld", static_cast<long long>(num_trees));
     if (max_simulations <= 0) return fail(TWIXT_EINVAL, "max_simulations must be positive: %d", max_simulations);
     if (n_rollouts <= 0) return fail(TWIXT_EINVAL, "n_rollouts must be positive: %d", n_rollouts);
@@ -689,15 +690,17 @@ class TwixTMCTS {
     c_ = uct_c;
     const int n = b->n_;
     const MctsSizes s = mcts_sizes(n, max_simulations, n_rollouts);
-    const int64_t per_tree = puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s);
-    // carve one allocation; each array starts on a 256-byte boundary (the last three are PUCT's, empty in UCT)
+    const int64_t per_tree = solve ? mcts_solve_bytes_per_tree(s, puct)
+                                   : (puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s));
+    // carve one allocation; each array starts on a 256-byte boundary (priors and tie keys are PUCT's, the outcome
+    // bytes PUCT's and the solver's, the root codes the solver's: empty otherwise)
     const int64_t T = num_trees, nodes = T * s.slots, edges = nodes * s.edges, rolls = T * s.rollouts;
-    const int64_t pe = puct ? edges : 0;
-    const int64_t sizes[16] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
+    const int64_t pe = puct ? edges : 0, oe = (puct || solve) ? edges : 0, rt = solve ? T : 0;
+    const int64_t sizes[17] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
                                T * 16, T * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8,
-                               pe * 4, pe * 4, pe};
-    int64_t offs[16], total = 0;
-    for (int i = 0; i < 16; ++i) {
+                               pe * 4, pe * 4, oe, rt};
+    int64_t offs[17], total = 0;
+    for (int i = 0; i < 17; ++i) {
       offs[i] = total;
       total += (sizes[i] + 255) & ~static_cast<int64_t>(255);
     }
@@ -740,7 +743,8 @@ class TwixTMCTS {
     a_.log_table = table;
     a_.edge_p = puct ? reinterpret_cast<float*>(base + offs[13]) : nullptr;
     a_.edge_key = puct ? reinterpret_cast<uint32_t*>(base + offs[14]) : nullptr;
-    a_.edge_out = puct ? reinterpret_cast<uint8_t*>(base + offs[15]) : nullptr;
+    a_.edge_out = (puct || solve) ? reinterpret_cast<uint8_t*>(base + offs[15]) : nullptr;
+    a_.root_out = solve ? reinterpret_cast<uint8_t*>(base + offs[16]) : nullptr;
     // ln N(s) from the host's libm, so that a CPU restatement of the search computes the same scores
     std::vector<double> logs(static_cast<size_t>(s.slots));
     for (size_t i = 0; i < logs.size(); ++i) logs[i] = std::log(static_cast<double>(i));
@@ -874,6 +878,33 @@ class TwixTMCTS {
     TW_TRY(b.Finish(&w));
     TW_TRY(b.Finish(&best));
     if (v.host || w.host || best.host) TW_TRY(b.Sync());
+    return TWIXT_OK;
+  }
+
+  // MCTS-Solver results of a solver search; every output nullable, host or device
+  int SolverStats(uint8_t* out_proven, float* out_returns, int8_t* out_edge_values, int32_t* out_simulations) {
+    if (a_.root_out == nullptr)
+      return fail(TWIXT_EINVAL, "twixt_mcts_solver_stats: the search was not created with TWIXT_MCTS_SOLVE");
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_solver_stats: no search begun");
+    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_solver_stats while a twixt_mcts_select awaits its backup");
+    if (count_ == 0) return TWIXT_OK;
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    b.ScratchReset();
+    const size_t cells = static_cast<size_t>(a_.n) * a_.n, cnt = static_cast<size_t>(count_);
+    Staged pr, re, ev, sm;
+    TW_TRY(b.StageOut(out_proven, cnt, &pr, false));
+    TW_TRY(b.StageOut(out_returns, cnt * 2 * sizeof(float), &re, false));
+    TW_TRY(b.StageOut(out_edge_values, cnt * cells, &ev, false));
+    TW_TRY(b.StageOut(out_simulations, cnt * sizeof(int32_t), &sm, false));
+    TW_CUDA(launch_mcts_solver_stats(a_, count_, static_cast<uint8_t*>(pr.dev), static_cast<float*>(re.dev),
+                                     static_cast<int8_t*>(ev.dev), static_cast<int32_t*>(sm.dev), b.stream_));
+    b.launches_ += 1;
+    TW_TRY(b.Finish(&pr));
+    TW_TRY(b.Finish(&re));
+    TW_TRY(b.Finish(&ev));
+    TW_TRY(b.Finish(&sm));
+    if (pr.host || re.host || ev.host || sm.host) TW_TRY(b.Sync());
     return TWIXT_OK;
   }
 
@@ -1076,13 +1107,16 @@ int twixt_stats_accumulate(twixt_stats* acc, const twixt_stats* part) {
   if ((m) == nullptr) return fail(TWIXT_EINVAL, "null mcts handle")
 
 static int mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
-                       double uct_c, bool puct, twixt_mcts** out) {
+                       double uct_c, uint32_t flags, twixt_mcts** out) {
   TW_NEED(b);
   if (out == nullptr) return fail(TWIXT_EINVAL, "null output pointer");
   *out = nullptr;
+  if ((flags & ~static_cast<uint32_t>(TWIXT_MCTS_PUCT | TWIXT_MCTS_SOLVE)) != 0u)
+    return fail(TWIXT_EINVAL, "unknown twixt_mcts_create_ex flags 0x%x", flags);
+  const bool puct = (flags & TWIXT_MCTS_PUCT) != 0u, solve = (flags & TWIXT_MCTS_SOLVE) != 0u;
   twixt_mcts* m = new (std::nothrow) twixt_mcts();
   if (m == nullptr) return fail(TWIXT_ENOMEM, "out of host memory");
-  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, uct_c, puct);
+  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, uct_c, puct, solve);
   if (rc != TWIXT_OK) {
     std::string keep = twixt::g_last_error;
     delete m;
@@ -1094,11 +1128,15 @@ static int mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulation
 }
 int twixt_mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c,
                       twixt_mcts** out) {
-  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, false, out);
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, 0u, out);
 }
 int twixt_mcts_create_puct(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
                            double uct_c, twixt_mcts** out) {
-  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, true, out);
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, TWIXT_MCTS_PUCT, out);
+}
+int twixt_mcts_create_ex(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                         double uct_c, uint32_t flags, twixt_mcts** out) {
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, flags, out);
 }
 void twixt_mcts_destroy(twixt_mcts* m) { delete m; }
 int twixt_mcts_begin(twixt_mcts* m, int64_t root_first, int64_t count) {
@@ -1124,6 +1162,11 @@ int twixt_mcts_backup_priors(twixt_mcts* m, const float* values, const float* pr
 int twixt_mcts_root_stats(twixt_mcts* m, int32_t* out_visits, double* out_value_sums, int32_t* out_best) {
   TW_NEED_MCTS(m);
   return m->impl.RootStats(out_visits, out_value_sums, out_best);
+}
+int twixt_mcts_solver_stats(twixt_mcts* m, uint8_t* out_proven, float* out_returns, int8_t* out_edge_values,
+                            int32_t* out_simulations) {
+  TW_NEED_MCTS(m);
+  return m->impl.SolverStats(out_proven, out_returns, out_edge_values, out_simulations);
 }
 
 int twixt_get_stats(twixt_batch* b, twixt_stats* out) {

@@ -72,7 +72,10 @@ struct MctsArena {
   // PUCT searches only (nullptr in a UCT search, which selects on that)
   float* edge_p;            // [trees*S*M] prior P(a), written when the node is expanded at its backup
   uint32_t* edge_key;       // [trees*S*M] tie key (mcts_tie_key)
-  uint8_t* edge_out;        // [trees*S*M] terminal outcome of the child (mcts_outcome_code), 0 = none
+  uint8_t* edge_out;        // [trees*S*M] terminal outcome of the child (mcts_outcome_code), 0 = none; a solver
+                            // search (UCT ones too) also writes the code of a proven child here
+  // solver searches only (nullptr otherwise, which selects on that)
+  uint8_t* root_out;        // [trees] outcome code of the root (twixt_mcts.cuh), 0 = unproven; cleared by begin
 };
 
 cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s);
@@ -85,6 +88,9 @@ cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* v
                                uint64_t seed, uint32_t stream0, cudaStream_t s);
 cudaError_t launch_mcts_root_stats(const MctsArena& a, int64_t count, int32_t* out_visits, double* out_value_sums,
                                    int32_t* out_best, cudaStream_t s);
+// solver searches: proven [count] u8, returns [count, 2] f32, edge values [count, n*n] i8, N(root) [count] i32
+cudaError_t launch_mcts_solver_stats(const MctsArena& a, int64_t count, uint8_t* out_proven, float* out_returns,
+                                     int8_t* out_edge_values, int32_t* out_simulations, cudaStream_t s);
 
 cudaError_t launch_reset(uint32_t* records, int64_t count, int n, cudaStream_t s);
 cudaError_t launch_clone(uint32_t* dst, const uint32_t* src, const int64_t* src_ids, int64_t count, int n,

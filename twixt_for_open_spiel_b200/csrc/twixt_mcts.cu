@@ -8,9 +8,12 @@
 //   launch_playout       the EXISTING fused playout kernel over the rollout slots, with the stream ids the
 //                        select kernel wrote (twixt_kernel_playout.cu, unchanged)
 //   mcts_backup_kernel   the leaf value (mean rollout return, caller's value or terminal Returns()) added to
-//                        every edge on the path, lanes over the path; a PUCT search expands the leaf here
+//                        every edge on the path, lanes over the path; a PUCT search expands the leaf here, a
+//                        solver search proves nodes up the path from a terminal leaf
 // A PUCT search (a.edge_p != nullptr) scores every edge with its prior from the first visit on (no unvisited-edge
 // draw) and expands a non-terminal leaf in the backup kernel, where the caller's priors for it are known.
+// A solver search (a.root_out != nullptr, MCTS-Solver) keeps an outcome code per edge and per root: a proven child
+// is scored by its outcome, and a tree whose root is proven is finished and takes no further part.
 // The scalar arithmetic (scores, draw, tie keys, stream ids, best child) is in twixt_mcts.cuh, shared with the
 // host harnesses that check it without a GPU.
 #include <cuda_runtime.h>
@@ -71,7 +74,9 @@ __device__ __forceinline__ int warp_expand(const MctsArena& a, int64_t g, const 
 }
 
 // ----------------------------------------------------------------- begin ---
-// The root of tree t is a COPY of env roots + t; every tree is cleared to its root alone.
+// The root of tree t is a COPY of env roots + t; every tree is cleared to its root alone (a solver search: and its
+// root code to unproven).
+template <bool kSolve>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a, const uint32_t* __restrict__ roots,
                                                                      int64_t count) {
   const int lane = threadIdx.x & 31;
@@ -83,12 +88,16 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a
     a.node_legal[root] = -1;
     a.node_n[root] = 0u;
     a.tree[t] = make_int4(1, 0, 0, kLeafNeedsValue);
+    if constexpr (kSolve) a.root_out[t] = 0;
   }
 }
 
 // ---------------------------------------------------------------- select ---
-// kPuct = (a.edge_p != nullptr): one instantiation per search kind, so the UCT kernel carries no PUCT code
-template <bool kPuct>
+// kPuct = (a.edge_p != nullptr), kSolve = (a.root_out != nullptr): one instantiation per search kind, so the UCT
+// kernel carries no PUCT code and neither carries solver code.  A solver search's finished tree (proven root) takes
+// no path: status kLeafSolved, its leaf env is not written, and in run mode its rollout slots get a copy of the
+// root marked drawn, which the playout kernel counts as neither a ply nor a game.
+template <bool kPuct, bool kSolve>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena a, int64_t count, uint64_t seed,
                                                                       uint32_t stream0, uint32_t k, double uct_c,
                                                                       uint32_t* __restrict__ leaf_dst,
@@ -99,6 +108,30 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
   const int n = a.n, rw = a.rw;
   const uint32_t T = stream0 + static_cast<uint32_t>(t);
   int node = 0, depth = 0, nodes = a.tree[t].x;
+  if constexpr (kSolve) {
+    if (a.root_out[t] != 0) {
+      if (leaf_dst == nullptr) {
+        const uint4* root = reinterpret_cast<const uint4*>(a.node_rec + mcts_slot(a, t, 0) * rw);
+        const uint4 hw = root[0];
+        Header h;
+        unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+        h.result = kDraw;
+        uint4 o;
+        pack_header(h, o.x, o.y, o.z, o.w);
+        for (int r = 0; r < a.R; ++r) {
+          uint4* dst = reinterpret_cast<uint4*>(a.roll_rec + (t * a.R + r) * rw);
+          for (int q = lane; q < rw / 4; q += 32) dst[q] = q == 0 ? o : root[q];
+        }
+        for (int r = lane; r < a.R; r += 32)
+          a.roll_ids[t * a.R + r] = mcts_rollout_stream(T, k, static_cast<uint32_t>(a.R), static_cast<uint32_t>(r));
+      }
+      if (lane == 0) {
+        a.tree[t] = make_int4(nodes, 0, 0, kLeafSolved);
+        if (out_status != nullptr) out_status[t] = kLeafSolved;
+      }
+      return;
+    }
+  }
   int2* path = a.path + t * a.P;
   bool terminal;
   for (;;) {
@@ -143,7 +176,13 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
       }
       edge = bi;
     } else {
-      if (legal < 0) legal = warp_expand(a, g, rec, h, lane);
+      if (legal < 0) {
+        legal = warp_expand(a, g, rec, h, lane);
+        if constexpr (kSolve) {
+          for (int i = lane; i < legal; i += 32) a.edge_out[e0 + i] = 0;
+          __syncwarp();
+        }
+      }
       // unvisited edges
       int unvisited = 0;
       for (int i = lane; i < legal; i += 32) unvisited += a.edge_n[e0 + i] == 0u ? 1 : 0;
@@ -163,7 +202,15 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
         double best = 0.0;
         int bi = 0x7FFFFFFF;
         for (int i = lane; i < legal; i += 32) {
-          const double s = mcts_uct_score(a.edge_w[e0 + i], a.edge_n[e0 + i], log_parent, uct_c);
+          double s;
+          if constexpr (kSolve) {
+            // MCTS-Solver: a proven child scores its outcome (open_spiel uct_value)
+            const uint8_t o = a.edge_out[e0 + i];
+            s = o != 0 ? static_cast<double>(mcts_outcome_value(o))
+                       : mcts_uct_score(a.edge_w[e0 + i], a.edge_n[e0 + i], log_parent, uct_c);
+          } else {
+            s = mcts_uct_score(a.edge_w[e0 + i], a.edge_n[e0 + i], log_parent, uct_c);
+          }
           if (bi == 0x7FFFFFFF || mcts_score_beats(s, i, best, bi)) {
             best = s;
             bi = i;
@@ -203,7 +250,7 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
         a.node_legal[gc] = -1;
         a.node_n[gc] = 0u;
         a.edge_child[e0 + edge] = child;
-        if (kPuct && ch.result != kOpen)
+        if ((kPuct || kSolve) && ch.result != kOpen)
           a.edge_out[e0 + edge] = mcts_outcome_code(ch, static_cast<int>(h.ply & 1u));
       }
       __syncwarp();
@@ -226,6 +273,8 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
 }
 
 // ---------------------------------------------------------------- backup ---
+// kSolve: a finished tree's row is ignored, and a terminal leaf starts the MCTS-Solver proof pass up its path
+template <bool kSolve>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena a, int64_t count,
                                                                       const float* __restrict__ values,
                                                                       const float* __restrict__ priors,
@@ -234,6 +283,9 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
   const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
   if (t >= count) return;
   const int4 info = a.tree[t];
+  if constexpr (kSolve) {
+    if (info.w == kLeafSolved) return;
+  }
   const int leaf = info.y, depth = info.z;
   double v[2];
   if (info.w == kLeafTerminal) {
@@ -283,9 +335,51 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
       a.edge_out[e0 + i] = 0;
     }
   }
+  if constexpr (kSolve) {
+    if (info.w == kLeafTerminal) {
+      if (depth == 0) {
+        // a terminal root is proven with its Returns()
+        if (lane == 0) {
+          const uint4 hw = *reinterpret_cast<const uint4*>(a.node_rec + mcts_slot(a, t, 0) * a.rw);
+          Header h;
+          unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+          a.root_out[t] = mcts_outcome_code(h, static_cast<int>(h.ply & 1u));
+        }
+        return;
+      }
+      // proof pass from the leaf's parent up: level i is path node i, whose edges' codes decide it; a proven node
+      // writes its parent's edge (or the root code), which the next level reads
+      for (int i = depth - 1; i >= 0; --i) {
+        const int64_t g = mcts_slot(a, t, path[i].x), e0 = g * a.M;
+        const int legal = a.node_legal[g];
+        int mx = 0;
+        bool all = true;
+        for (int j = lane; j < legal; j += 32) {
+          const int c = a.edge_out[e0 + j];
+          mx = c > mx ? c : mx;
+          all = all && c != 0;
+        }
+        mx = __reduce_max_sync(kFullMask, mx);
+        all = __all_sync(kFullMask, all);
+        const int pv = mcts_proven_value(mx, all);
+        if (pv == kUnproven) break;
+        if (lane == 0) {
+          if (i > 0) {
+            const int2 q = path[i - 1];
+            a.edge_out[mcts_slot(a, t, q.x) * a.M + (q.y >> 1)] = mcts_parent_code(pv);
+          } else {
+            a.root_out[t] = static_cast<uint8_t>(2 + pv);
+          }
+        }
+        __syncwarp();
+      }
+    }
+  }
 }
 
 // ------------------------------------------------------------ root stats ---
+// kSolve: a UCT solver search ranks by open_spiel's sort_key (outcome value, N, W), then the lower edge
+template <bool kSolve>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_root_stats_kernel(MctsArena a, int64_t count,
                                                                           int32_t* __restrict__ out_visits,
                                                                           double* __restrict__ out_value_sums,
@@ -344,6 +438,42 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_root_stats_kernel(MctsAr
       out_best[t] = nmax > 0u ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
     return;
   }
+  if constexpr (kSolve) {
+    int bo = 0;
+    uint32_t bn = 0u;
+    double bw = 0.0;
+    int bi = 0x7FFFFFFF;
+    for (int i = lane; i < legal; i += 32) {
+      const int action = a.edge_action[e0 + i];
+      const uint32_t en = a.edge_n[e0 + i];
+      const double ew = a.edge_w[e0 + i];
+      const int eo = mcts_outcome_value(a.edge_out[e0 + i]);
+      if (out_visits != nullptr) out_visits[t * cells + action] = static_cast<int32_t>(en);
+      if (out_value_sums != nullptr) out_value_sums[t * cells + action] = ew;
+      if (bi == 0x7FFFFFFF || mcts_puct_best_beats(eo, en, ew, 0u, i, bo, bn, bw, 0u, bi)) {
+        bo = eo;
+        bn = en;
+        bw = ew;
+        bi = i;
+      }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+      const int oo = __shfl_xor_sync(kFullMask, bo, d);
+      const uint32_t on = __shfl_xor_sync(kFullMask, bn, d);
+      const double ow = __shfl_xor_sync(kFullMask, bw, d);
+      const int oi = __shfl_xor_sync(kFullMask, bi, d);
+      if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_puct_best_beats(oo, on, ow, 0u, oi, bo, bn, bw, 0u, bi))) {
+        bo = oo;
+        bn = on;
+        bw = ow;
+        bi = oi;
+      }
+    }
+    if (out_best != nullptr && lane == 0)
+      out_best[t] = (legal > 0 && bi != 0x7FFFFFFF) ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
+    return;
+  }
   uint32_t bn = 0u;
   double bw = 0.0;
   int bi = 0x7FFFFFFF;
@@ -374,40 +504,92 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_root_stats_kernel(MctsAr
     out_best[t] = (legal > 0 && bi != 0x7FFFFFFF) ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
 }
 
+// ---------------------------------------------------------- solver stats ---
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_solver_stats_kernel(MctsArena a, int64_t count,
+                                                                            uint8_t* __restrict__ out_proven,
+                                                                            float* __restrict__ out_returns,
+                                                                            int8_t* __restrict__ out_edge_values,
+                                                                            int32_t* __restrict__ out_simulations) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int cells = a.n * a.n;
+  const int64_t g = mcts_slot(a, t, 0), e0 = g * a.M;
+  if (out_edge_values != nullptr) {
+    for (int c = lane; c < cells; c += 32) out_edge_values[t * cells + c] = static_cast<int8_t>(kUnproven);
+    __syncwarp();
+    const int legal = a.node_legal[g];
+    for (int i = lane; i < legal; i += 32) {
+      const uint8_t o = a.edge_out[e0 + i];
+      if (o != 0) out_edge_values[t * cells + a.edge_action[e0 + i]] = static_cast<int8_t>(mcts_outcome_value(o));
+    }
+  }
+  if (lane == 0) {
+    const uint8_t rc = a.root_out[t];
+    if (out_proven != nullptr) out_proven[t] = rc != 0 ? 1 : 0;
+    if (out_returns != nullptr) {
+      // root.outcome: the code is for the root's player to move by ply parity
+      const uint4 hw = *reinterpret_cast<const uint4*>(a.node_rec + g * a.rw);
+      Header h;
+      unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+      const int p = static_cast<int>(h.ply & 1u), v = mcts_outcome_value(rc);
+      out_returns[2 * t + p] = static_cast<float>(v);
+      out_returns[2 * t + 1 - p] = static_cast<float>(-v);
+    }
+    if (out_simulations != nullptr) out_simulations[t] = static_cast<int32_t>(a.node_n[g]);
+  }
+}
+
 unsigned mcts_blocks(int64_t count) { return static_cast<unsigned>((count + kMctsWarps - 1) / kMctsWarps); }
 
 }  // namespace
 
 cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  mcts_begin_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
+  if (a.root_out != nullptr)
+    mcts_begin_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
+  else
+    mcts_begin_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
   return cudaGetLastError();
 }
 
 cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed, uint32_t stream0, uint32_t k,
                                double uct_c, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  if (a.edge_p != nullptr)
-    mcts_select_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c,
-                                                                           leaf_dst, out_status);
-  else
-    mcts_select_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c,
-                                                                            leaf_dst, out_status);
+  const bool puct = a.edge_p != nullptr, solve = a.root_out != nullptr;
+  auto kernel = puct ? (solve ? mcts_select_kernel<true, true> : mcts_select_kernel<true, false>)
+                     : (solve ? mcts_select_kernel<false, true> : mcts_select_kernel<false, false>);
+  kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c, leaf_dst, out_status);
   return cudaGetLastError();
 }
 
 cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, const float* priors,
                                uint64_t seed, uint32_t stream0, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  mcts_backup_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
+  if (a.root_out != nullptr)
+    mcts_backup_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
+  else
+    mcts_backup_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
   return cudaGetLastError();
 }
 
 cudaError_t launch_mcts_root_stats(const MctsArena& a, int64_t count, int32_t* out_visits, double* out_value_sums,
                                    int32_t* out_best, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  mcts_root_stats_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_visits, out_value_sums,
-                                                                         out_best);
+  if (a.root_out != nullptr)
+    mcts_root_stats_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_visits, out_value_sums,
+                                                                                out_best);
+  else
+    mcts_root_stats_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_visits,
+                                                                                 out_value_sums, out_best);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_solver_stats(const MctsArena& a, int64_t count, uint8_t* out_proven, float* out_returns,
+                                     int8_t* out_edge_values, int32_t* out_simulations, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_solver_stats_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_proven, out_returns,
+                                                                           out_edge_values, out_simulations);
   return cudaGetLastError();
 }
 

@@ -25,6 +25,13 @@
 // plus one table of (max_simulations + 1) doubles per search.  At n = 12 a node is 2 616 bytes.
 // A PUCT search adds per edge 4 (prior P f32) + 4 (tie key u32) + 1 (terminal outcome u8):
 //   PUCT bytes per tree = S * (rw*4 + 8 + 27*M) + 16 + 8*P + R * (rw*4 + 16)
+// A solver search (TWIXT_MCTS_SOLVE, MCTS-Solver) adds 1 per tree (root outcome code u8); a UCT one also the
+// outcome byte per edge, which PUCT already has:
+//   UCT + solve bytes per tree  = S * (rw*4 + 8 + 19*M) + 17 + 8*P + R * (rw*4 + 16)
+//   PUCT + solve bytes per tree = S * (rw*4 + 8 + 27*M) + 17 + 8*P + R * (rw*4 + 16)
+// The outcome code of an edge is 0 while its child is unproven, else 2 + the child's value for the player to move
+// at the parent (1 = loss, 2 = draw, 3 = win); the root code is 2 + the root's value for its own player to move
+// (ply parity, also for a terminal root).
 #pragma once
 #include <stdint.h>
 
@@ -37,7 +44,7 @@
 
 namespace twixt {
 
-enum : int { kLeafNeedsValue = 0, kLeafTerminal = 1 };
+enum : int { kLeafNeedsValue = 0, kLeafTerminal = 1, kLeafSolved = 2 };
 
 struct MctsSizes {
   int64_t slots;      // node slots per tree (max_simulations + 1)
@@ -65,6 +72,11 @@ TW_HD int64_t mcts_bytes_per_tree(const MctsSizes& s) {
 
 // the PUCT formula of the header comment above
 TW_HD int64_t mcts_puct_bytes_per_tree(const MctsSizes& s) { return mcts_bytes_per_tree(s) + s.slots * 9 * s.edges; }
+
+// the solver formulas of the header comment above
+TW_HD int64_t mcts_solve_bytes_per_tree(const MctsSizes& s, bool puct) {
+  return (puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s) + s.slots * s.edges) + 1;
+}
 
 // UCT score of an edge with N(a) = n > 0 visits and value sum w, under a parent whose ln N(s) is log_parent.
 // Bit-identical on the device and on a host compiled with -ffp-contract=off.
@@ -147,6 +159,16 @@ TW_HD uint8_t mcts_outcome_code(const Header& child, int player) {
   return static_cast<uint8_t>(2 + (player == 0 ? red : -red));
 }
 TW_HD int mcts_outcome_value(uint8_t code) { return code == 0 ? 0 : static_cast<int>(code) - 2; }
+
+// MCTS-Solver proof step of an expanded node from its L > 0 edge codes, given their maximum and whether every one
+// is non-zero: the node is proven when some edge is a win for its player to move (code 3) or every edge is
+// proven.  Returns its value v for that player, or kUnproven.
+enum : int { kUnproven = -128 };
+TW_HD int mcts_proven_value(int max_code, bool all_proven) {
+  return (max_code == 3 || all_proven) ? max_code - 2 : static_cast<int>(kUnproven);
+}
+// the code of the parent's edge into a node proven with value v (zero-sum, players alternate by ply)
+TW_HD uint8_t mcts_parent_code(int v) { return static_cast<uint8_t>(2 - v); }
 
 // PUCT BestChild (open_spiel SearchNode.sort_key): (outcome value, N, W), then the smaller key, then the
 // lower edge

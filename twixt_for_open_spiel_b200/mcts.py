@@ -16,6 +16,11 @@ child_selection_fn = puct_value): `backup(values, priors)` hands the policy head
 the values, and the leaf is expanded with them.  `add_dirichlet_noise` mixes open_spiel's root noise into the
 priors of the first backup after `begin` (simulation 0's leaf is always the root).
 
+`solve=True` adds open_spiel's MCTS-Solver to either kind (MCTSBot(..., solve=True), open_spiel's default):
+a terminal leaf proves nodes up its path, a proven child is scored by its outcome, and a tree whose root is
+proven is finished: later simulations do nothing for it (`select` reports LEAF_SOLVED and leaves its env
+alone).  `solver_stats()` returns the proven root and move values.
+
 `MCTSBot` is the open_spiel-shaped bot over one tree for adapter `TwixTState`s.
 
 Arrays may be numpy (synchronous) or torch CUDA tensors (asynchronous on the batch's stream), as for
@@ -31,21 +36,24 @@ import numpy as np
 from . import _lib
 from .batch import TwixTBatch, _dt, _is_torch, _ptr
 
-LEAF_NEEDS_VALUE, LEAF_TERMINAL = 0, 1
+LEAF_NEEDS_VALUE, LEAF_TERMINAL, LEAF_SOLVED = 0, 1, 2
+UNPROVEN = -128  # solver_stats' edge value of a root move that is not proven
+_PUCT, _SOLVE = 1, 2  # TWIXT_MCTS_PUCT, TWIXT_MCTS_SOLVE
 
 
 class BatchedMCTS:
     def __init__(self, batch: TwixTBatch, num_trees: int, max_simulations: int, n_rollouts: int = 1,
-                 uct_c: float = 2.0, selection: str = "uct"):
+                 uct_c: float = 2.0, selection: str = "uct", solve: bool = False):
         if selection not in ("uct", "puct"):
             raise ValueError("selection must be 'uct' or 'puct', got %r" % (selection,))
         self._lib = _lib.load()
         self.batch = batch  # the search runs on the batch's envs and stream: keep it alive
         self._h = C.c_void_p()
-        create = self._lib.twixt_mcts_create_puct if selection == "puct" else self._lib.twixt_mcts_create
-        self._check(create(batch._h, int(num_trees), int(max_simulations), int(n_rollouts), float(uct_c),
-                           C.byref(self._h)))
+        flags = (_PUCT if selection == "puct" else 0) | (_SOLVE if solve else 0)
+        self._check(self._lib.twixt_mcts_create_ex(batch._h, int(num_trees), int(max_simulations), int(n_rollouts),
+                                                   float(uct_c), flags, C.byref(self._h)))
         self.selection = selection
+        self.solve = bool(solve)
         self.num_trees = int(num_trees)
         self.max_simulations = int(max_simulations)
         self.n_rollouts = int(n_rollouts)
@@ -82,7 +90,8 @@ class BatchedMCTS:
     def select(self, leaf_first: int, out_status=None):
         """Stepwise form, first half: leaf of tree t -> batch env leaf_first + t.  Returns the statuses
         [count] int32 (LEAF_NEEDS_VALUE, or LEAF_TERMINAL: its value is Returns() and backup ignores the
-        caller's)."""
+        caller's, or with solve=True LEAF_SOLVED: the tree is finished, its env was not written and backup
+        ignores its row)."""
         if out_status is None:
             out_status = np.zeros(self.count, dtype=np.int32)
         self._check(self._lib.twixt_mcts_select(self._h, int(leaf_first),
@@ -119,6 +128,27 @@ class BatchedMCTS:
     def best(self) -> np.ndarray:
         return self.root_stats()[2]
 
+    def solver_stats(self, out_proven=None, out_returns=None, out_edge_values=None, out_simulations=None):
+        """solve=True only: (proven [count] uint8, returns [count, 2] float32, edge_values [count, n*n] int8,
+        simulations [count] int32).  proven is 1 once the root is proven; returns is open_spiel's root.outcome
+        ((0, 0) while unproven); edge_values is -1, 0 or +1 for a proven root move from the view of the player to
+        move at the root, UNPROVEN elsewhere; simulations is N(root), the simulations the tree ran since begin
+        (a finished tree stops counting)."""
+        if out_proven is None:
+            out_proven = np.zeros(self.count, dtype=np.uint8)
+        if out_returns is None:
+            out_returns = np.zeros((self.count, 2), dtype=np.float32)
+        if out_edge_values is None:
+            out_edge_values = np.zeros((self.count, self._cells), dtype=np.int8)
+        if out_simulations is None:
+            out_simulations = np.zeros(self.count, dtype=np.int32)
+        self._check(self._lib.twixt_mcts_solver_stats(
+            self._h, _ptr(out_proven, _dt(np.uint8, "uint8"), self.count),
+            _ptr(out_returns, _dt(np.float32, "float32"), 2 * self.count),
+            _ptr(out_edge_values, _dt(np.int8, "int8"), self.count * self._cells),
+            _ptr(out_simulations, _dt(np.int32, "int32"), self.count)))
+        return out_proven, out_returns, out_edge_values, out_simulations
+
 
 def add_dirichlet_noise(priors, legal_mask, epsilon: float, alpha: float):
     """open_spiel's root noise: (1 - epsilon) * p + epsilon * Dir(alpha) over each row's legal actions.
@@ -141,18 +171,22 @@ def add_dirichlet_noise(priors, legal_mask, epsilon: float, alpha: float):
 
 
 class MCTSBot:
-    """open_spiel's MCTSBot with RandomRolloutEvaluator(n_rollouts), solve = false, for adapter states:
-    what `mcts_example --player1=mcts --rollout_count=4` plays, without the solver.  Each step copies the
-    state's record into a private one-tree batch and runs max_simulations simulations on the device."""
+    """open_spiel's MCTSBot with RandomRolloutEvaluator(n_rollouts), for adapter states: what
+    `mcts_example --player1=mcts --rollout_count=4` plays.  Each step copies the state's record into a private
+    one-tree batch and runs max_simulations simulations on the device.
+
+    solve defaults to False here, so existing callers keep the search they had; open_spiel's MCTSBot and
+    mcts_example default to solve=True, which is `MCTSBot(..., solve=True)`: a proven win is played at once and
+    the search of a step ends when its root is proven."""
 
     def __init__(self, game, uct_c: float = 2.0, max_simulations: int = 1000, n_rollouts: int = 4, seed: int = 0,
-                 device: int = 0):
+                 device: int = 0, solve: bool = False):
         if max_simulations < 2:
             raise ValueError("MCTSBot needs max_simulations >= 2: the first simulation only evaluates the root")
         self._game = game
         self._batch = TwixTBatch(game.board_size(), 1, device, seed)
         self._batch.set_validation(False)  # records come from the adapter's own exports
-        self._mcts = BatchedMCTS(self._batch, 1, max_simulations, n_rollouts, uct_c)
+        self._mcts = BatchedMCTS(self._batch, 1, max_simulations, n_rollouts, uct_c, solve=solve)
         self.max_simulations = int(max_simulations)
 
     def step(self, state) -> int:
