@@ -14,7 +14,12 @@ Everything stays on the device; per move only the count of running games, which 
 bus.  The trajectories (obs, mask, policy target, player, action per move) and the final returns are copied to
 the host at the end.
 
-    python examples/alphazero_selfplay.py [board_size] [games] [simulations]
+leaves_per_step=K > 1 searches K leaves per tree in each step with virtual loss (BatchedMCTS): the leaf envs are
+[B, B + B*K), row g*K + j being descent j of game g, so each network call evaluates B*K leaves and a move takes
+sims / K calls.  Every descent of the first step stops at the root, which takes the priors of row g*K + 0: the
+Dirichlet noise goes into those rows.
+
+    python examples/alphazero_selfplay.py [board_size] [games] [simulations] [leaves_per_step]
 """
 import os
 import sys
@@ -49,18 +54,24 @@ def masked_softmax(logits, legal):
 
 
 def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_c=2.0, dirichlet_epsilon=0.25,
-              dirichlet_alpha=1.0, seed=0, net=None, verbose=True):
+              dirichlet_alpha=1.0, seed=0, net=None, verbose=True, leaves_per_step=1, virtual_loss=1.0):
     """Plays `games` games to the end.  Returns (trajectories, returns [games, 2]); trajectories[g] is a list of
-    per-move dicts with obs [12, n, n-2], mask [n*n], policy [n*n], player and action."""
+    per-move dicts with obs [12, n, n-2], mask [n*n], policy [n*n], player and action.  sims must be a multiple
+    of leaves_per_step."""
+    K = int(leaves_per_step)
+    if sims % K:
+        raise ValueError("sims = %d is not a multiple of leaves_per_step = %d" % (sims, K))
     torch.manual_seed(seed)
     dev = torch.device("cuda:0")
-    batch = TwixTBatch(n, 2 * games, 0, seed)  # envs [0, games) are the games, [games, 2*games) the leaves
+    rows = games * K
+    batch = TwixTBatch(n, games + rows, 0, seed)  # envs [0, games) are the games, [games, games + games*K) the leaves
     batch.use_torch_stream()
-    producer = ObservationMaskProducer(batch, max_count=games)
+    producer = ObservationMaskProducer(batch, max_count=rows)
     if net is None:
         net = PolicyValueNet(n).to(dev).eval()
-    search = BatchedMCTS(batch, games, sims, uct_c=uct_c, selection="puct")
-    player = torch.zeros(games, dtype=torch.int8, device=dev)
+    search = BatchedMCTS(batch, games, sims, uct_c=uct_c, selection="puct", leaves_per_step=K,
+                         virtual_loss=virtual_loss)
+    player = torch.zeros(rows, dtype=torch.int8, device=dev)
     root_player = torch.zeros(games, dtype=torch.int8, device=dev)
     done = torch.zeros(games, dtype=torch.uint8, device=dev)
     visits = torch.zeros((games, n * n), dtype=torch.int32, device=dev)
@@ -80,15 +91,18 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
             root_obs, root_mask = root_obs.clone(), root_mask.clone()
             batch.current_player(0, games, out=root_player)
             search.begin(0, games)
-            for k in range(sims):
+            for k in range(sims // K):
                 search.select(games)
-                obs, mask = producer.produce(games, games)
+                obs, mask = producer.produce(games, rows)
                 legal = mask.bool()
                 logits, v = net(obs)
                 priors = masked_softmax(logits, legal)
                 if k == 0:
-                    priors = add_dirichlet_noise(priors, legal, dirichlet_epsilon, dirichlet_alpha)
-                batch.current_player(games, games, out=player)
+                    if K == 1:
+                        priors = add_dirichlet_noise(priors, legal, dirichlet_epsilon, dirichlet_alpha)
+                    else:  # the root rows g*K + 0
+                        priors[::K] = add_dirichlet_noise(priors[::K], legal[::K], dirichlet_epsilon, dirichlet_alpha)
+                batch.current_player(games, rows, out=player)
                 v = torch.where(player == 1, -v, v).float()
                 search.backup(torch.stack([v, -v], dim=1).contiguous(), priors.contiguous())
             search.root_stats(out_visits=visits, out_best=best)
@@ -119,7 +133,8 @@ def main():
     n = int(sys.argv[1]) if len(sys.argv) > 1 else 8
     games = int(sys.argv[2]) if len(sys.argv) > 2 else 256
     sims = int(sys.argv[3]) if len(sys.argv) > 3 else 100
-    trajectories, returns = self_play(n, games, sims)
+    leaves = int(sys.argv[4]) if len(sys.argv) > 4 else 1
+    trajectories, returns = self_play(n, games, sims, leaves_per_step=leaves)
     lengths = [len(t) for t in trajectories]
     print("%d games at n = %d, %d simulations per move: mean length %.1f, red wins %d, blue wins %d, draws %d" % (
         games, n, sims, float(np.mean(lengths)), int((returns[:, 0] > 0).sum()), int((returns[:, 1] > 0).sum()),

@@ -355,6 +355,40 @@ int twixt_mcts_create_ex(twixt_batch* b, int64_t num_trees, int32_t max_simulati
 int twixt_mcts_solver_stats(twixt_mcts* m, uint8_t* out_proven, float* out_returns, int8_t* out_edge_values,
                             int32_t* out_simulations);
 
+/* Several leaves per step with virtual loss (leaf parallelism, as in AlphaGo, Leela Zero and KataGo): not an
+ * open_spiel behaviour but this search's own, which reduces to the searches above at leaves_per_step = 1.
+ * twixt_mcts_create_parallel takes the flags of twixt_mcts_create_ex, K = leaves_per_step (1 <= K <= 4096 and
+ * K <= max_simulations) and the virtual loss vl (finite, >= 0); K = 1 is exactly twixt_mcts_create_ex with the same
+ * flags.  TWIXT_MCTS_SOLVE with K > 1 is TWIXT_EINVAL.  One STEP is K simulations of every tree:
+ *  - every node has a virtual visit count V(s) and every edge V(a), both 0 between steps.  Descent j = 0 .. K-1 of
+ *    a step is simulation k = (simulations since begin) + j, whose k keys the unvisited-edge draw and the rollout
+ *    streams as above.  The descents of a tree run in order j; each sees the virtual counts of the earlier ones.
+ *  - the leaf rule is unchanged: a descent stops at a terminal node or at a node with N(s) == 0 (real visits).
+ *    UCT still expands a node on its second real visit, in select; PUCT in backup.  A descent may end at a leaf
+ *    that an earlier descent of the step already took (a repeated leaf): it is an ordinary row with its own env,
+ *    rollouts or caller value.
+ *  - scores use n_eff = N(a) + V(a), N_eff(s) = N(s) + V(s) and w_eff = (V(a) > 0 ? W(a) - vl*V(a) : W(a)) in IEEE
+ *    double without contraction: UCT's unvisited-edge draw counts the edges with n_eff == 0, otherwise edges score
+ *    q + c*sqrt(ln N_eff(s) / n_eff) with q = w_eff / n_eff; PUCT scores (w_eff / n_eff or 0) +
+ *    ((c*P)*sqrt(N_eff(s))) / (n_eff + 1), and an edge whose child is terminal still scores its outcome.  Ties as
+ *    before.
+ *  - after descent j picks its path, V += 1 on every edge and every node of the path and on the leaf.
+ *  - backup takes rows j = 0 .. K-1 of each tree in order: row j removes its virtual visits and adds its value
+ *    as above (W only ever receives real values).  A PUCT leaf is expanded by the LOWEST row whose leaf it is,
+ *    with that row's priors; the priors of repeated leaves are ignored.
+ *  - step 0: N(root) = 0, so every descent stops at the root; a PUCT root is expanded with the priors of row
+ *    t*K + 0 of the first backup, which is where root Dirichlet noise goes.
+ * Shapes: twixt_mcts_select writes descent j of tree t to env leaf_first + t*K + j (the range check covers count*K
+ * envs) and out_leaf_status [count*K]; twixt_mcts_backup / _backup_priors take values [count*K, 2] and priors
+ * [count*K, n*n] (host priors are checked on every row).  twixt_mcts_run(s) needs s to be a multiple of K and
+ * queues s / K steps of three launches, the playout launch running K*R rollouts per tree.  max_simulations counts
+ * simulations: each step, or select/backup pair, counts K.  root_stats and destroy are unchanged.  The arena
+ * holds K paths, K leaf entries and K*R rollout slots per tree and a u16 V per node and per edge
+ * (twixt_mcts.cuh); K = 1 allocates nothing more. */
+int twixt_mcts_create_parallel(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                               double uct_c, uint32_t flags, int32_t leaves_per_step, double virtual_loss,
+                               twixt_mcts** out);
+
 /* Multi-GPU plumbing for hosts that are not Python (SURVEY 8e: envs shard by contiguous global id ranges,
  * no data-path collective, one reduction of the counters).  twixt_shard_range: rank's share [first,
  * first+count) of global_envs envs over `world` ranks (shares differ by at most one env); create the rank's

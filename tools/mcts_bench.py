@@ -22,6 +22,13 @@ with simulations/s and the select / backup kernel ms per step, next to the UCT c
   n = 8 endgames: 8192 roots 2..6 plies before the end of seeded games x 400 simulations x R = 4, where most
   trees finish early; simulations/s counts every tree's simulations (finished ones too), next to the fraction of
   roots proven, the mean N(root) and the backup kernel ms per step.
+
+`parallel`: several leaves per step with virtual loss (leaves_per_step = K, virtual_loss = 1):
+  one tree at n = 12 x 1000 simulations x R = 4 (an MCTSBot.step-sized search) at K = 1, 8 and 32 (992
+  simulations there, whole steps): wall time per search (begin + run, ending in a device synchronise), mean of 5
+  after a warm-up;
+  64 trees x 400 simulations at n = 12, UCT x R = 4 (run) and the stepwise PUCT search above, at K = 1 and 8:
+  simulations/s and the select / playout / backup kernel ms per step (a step is K simulations of every tree).
 """
 from __future__ import annotations
 
@@ -73,16 +80,17 @@ def endgame_roots(n: int, trees: int, seed: int):
 
 
 def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int, solve: bool = False,
-                 endgame: bool = False) -> dict:
+                 endgame: bool = False, leaves_per_step: int = 1) -> dict:
     import torch
     from torch.profiler import ProfilerActivity, profile
 
     from twixt_for_open_spiel_b200.mcts import BatchedMCTS
+    K = leaves_per_step
     b = endgame_roots(n, trees, 0x736F6C76) if endgame else make_roots(n, trees, 0x6D637473)
-    m = BatchedMCTS(b, trees, sims, R, solve=solve)
+    m = BatchedMCTS(b, trees, sims, R, solve=solve, leaves_per_step=K)
     # warm-up: every kernel of a simulation, at this size
     m.begin(0, trees)
-    m.run(min(sims, 20))
+    m.run(max(K, min(sims, 20) // K * K))
     b.synchronize()
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     p0 = b.stats()["plies"]
@@ -120,10 +128,12 @@ def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int, solve
         "search_ms": round(ms, 3),
         "simulations_per_s": round(trees * sims / (ms / 1e3), 1),
         "rollout_plies_per_s": round(plies / (ms / 1e3), 1),
-        "ms_per_simulation_step": round(ms / sims, 4),
-        "kernel_ms_per_simulation_step": {k: round(v / 1e3 / profile_sims, 4) for k, v in split.items()},
+        "ms_per_simulation_step": round(ms / (sims // K), 4),
+        "kernel_ms_per_simulation_step": {k: round(v / 1e3 / (profile_sims // K), 4) for k, v in split.items()},
         "roots_with_a_best_move": int((best >= 0).sum()),
     }
+    if K > 1:
+        out["leaves_per_step"] = K
     if solve:
         proven, _, _, simulations = solved
         out.update({"solve": True, "roots": "endgame" if endgame else "opening",
@@ -132,25 +142,27 @@ def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int, solve
     return out
 
 
-def bench_puct(n: int, trees: int, sims: int, profile_sims: int) -> dict:
+def bench_puct(n: int, trees: int, sims: int, profile_sims: int, leaves_per_step: int = 1) -> dict:
     import torch
     from torch.profiler import ProfilerActivity, profile
 
     from twixt_for_open_spiel_b200.mcts import BatchedMCTS
-    b = make_roots(n, 2 * trees, 0x70756374)  # envs [trees, 2*trees) take the leaves
-    m = BatchedMCTS(b, trees, sims, selection="puct")
+    K = leaves_per_step
+    rows = trees * K
+    b = make_roots(n, trees + rows, 0x70756374)  # envs [trees, trees + trees*K) take the leaves
+    m = BatchedMCTS(b, trees, sims, selection="puct", leaves_per_step=K)
     gen = torch.Generator(device="cuda").manual_seed(1)
-    priors = torch.rand((trees, n * n), generator=gen, device="cuda", dtype=torch.float32)
-    values = torch.zeros((trees, 2), device="cuda", dtype=torch.float32)
-    status = torch.zeros(trees, dtype=torch.int32, device="cuda")
+    priors = torch.rand((rows, n * n), generator=gen, device="cuda", dtype=torch.float32)
+    values = torch.zeros((rows, 2), device="cuda", dtype=torch.float32)
+    status = torch.zeros(rows, dtype=torch.int32, device="cuda")
 
-    def search(k):
-        for _ in range(k):
+    def search(k):  # k simulations of every tree: k / K steps
+        for _ in range(k // K):
             m.select(trees, status)
             m.backup(values, priors)
 
     m.begin(0, trees)
-    search(min(sims, 20))
+    search(max(K, min(sims, 20) // K * K))
     b.synchronize()
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     m.begin(0, trees)
@@ -176,14 +188,41 @@ def bench_puct(n: int, trees: int, sims: int, profile_sims: int) -> dict:
     best = m.best()
     m.close()
     b.close()
-    return {
+    out = {
         "board_size": n, "trees": trees, "simulations": sims,
         "search_ms": round(ms, 3),
         "simulations_per_s": round(trees * sims / (ms / 1e3), 1),
-        "ms_per_simulation_step": round(ms / sims, 4),
-        "kernel_ms_per_simulation_step": {k: round(v / 1e3 / profile_sims, 4) for k, v in split.items()},
+        "ms_per_simulation_step": round(ms / (sims // K), 4),
+        "kernel_ms_per_simulation_step": {k: round(v / 1e3 / (profile_sims // K), 4) for k, v in split.items()},
         "roots_with_a_best_move": int((best >= 0).sum()),
     }
+    if K > 1:
+        out["leaves_per_step"] = K
+    return out
+
+
+def bench_single_tree(n: int, sims: int, R: int, K: int, reps: int) -> dict:
+    """One tree, the search of one MCTSBot.step: wall time of begin + run(sims), ending in a synchronise.  sims is
+    rounded down to a multiple of K (run takes whole steps): 992 at K = 32 for 1000."""
+    from twixt_for_open_spiel_b200.mcts import BatchedMCTS
+    sims -= sims % K
+    b = make_roots(n, 1, 0x626F7473)
+    m = BatchedMCTS(b, 1, sims, R, leaves_per_step=K)
+    m.begin(0, 1)
+    m.run(sims)
+    b.synchronize()
+    times = []
+    for _ in range(reps):
+        t0 = time.perf_counter()
+        m.begin(0, 1)
+        m.run(sims)
+        b.synchronize()
+        times.append(time.perf_counter() - t0)
+    m.close()
+    b.close()
+    return {"board_size": n, "trees": 1, "simulations": sims, "n_rollouts": R, "leaves_per_step": K,
+            "steps": sims // K, "ms_per_search": round(1e3 * sum(times) / reps, 3),
+            "ms_per_search_min": round(1e3 * min(times), 3)}
 
 
 def bench_evaluator(n: int, leaves: int, R: int, reps: int) -> dict:
@@ -204,6 +243,7 @@ def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--quick", action="store_true", help="small sizes (a functional check, not a measurement)")
     ap.add_argument("--no-solve", action="store_true", help="skip the solver entries")
+    ap.add_argument("--no-parallel", action="store_true", help="skip the leaves_per_step entries")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -214,17 +254,27 @@ def main() -> None:
         puct = [(12, 256, 40, 10), (24, 64, 20, 5)]
         ev = (12, 256, 4, 5)
         solve = [(12, 256, 40, 4, 10, True, False), (8, 256, 40, 4, 10, True, True)]
+        single = [(12, 96, 4, K, 2) for K in (1, 8, 32)]
+        many = [(12, 16, 48, 4, 16, K) for K in (1, 8)]
     else:
         configs = [(12, 8192, 400, 4, 50), (24, 1024, 200, 4, 50)]
         puct = [(12, 8192, 400, 50), (24, 1024, 200, 50)]
         ev = (12, 8192, 4, 50)
         solve = [(12, 8192, 400, 4, 50, True, False), (8, 8192, 400, 4, 50, True, True)]
+        single = [(12, 1000, 4, K, 5) for K in (1, 8, 32)]
+        many = [(12, 64, 400, 4, 80, K) for K in (1, 8)]
     out = dict(info)
     out["configs"] = [bench_config(*c) for c in configs]
     out["evaluate_slots"] = bench_evaluator(*ev)
     out["puct"] = [bench_puct(*c) for c in puct]
     if not args.no_solve:
         out["solve"] = [bench_config(*c) for c in solve]
+    if not args.no_parallel:
+        out["parallel"] = {
+            "single_tree": [bench_single_tree(*c) for c in single],
+            "uct": [bench_config(n, t, s, R, p, leaves_per_step=K) for n, t, s, R, p, K in many],
+            "puct": [bench_puct(n, t, s, p, leaves_per_step=K) for n, t, s, _, p, K in many],
+        }
     print(json.dumps(out))
 
 

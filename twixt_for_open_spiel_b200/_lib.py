@@ -102,6 +102,8 @@ SYMBOLS = [
     ("twixt_mcts_backup_priors", C.c_int, [_P, _P, _P]),
     ("twixt_mcts_create_ex", C.c_int, [_P, _I64, C.c_int32, C.c_int32, C.c_double, C.c_uint32, C.POINTER(_P)]),
     ("twixt_mcts_solver_stats", C.c_int, [_P, _P, _P, _P, _P]),
+    ("twixt_mcts_create_parallel", C.c_int, [_P, _I64, C.c_int32, C.c_int32, C.c_double, C.c_uint32, C.c_int32,
+                                             C.c_double, C.POINTER(_P)]),
 ]
 
 OK, EINVAL, ECUDA, EILLEGAL, ENOMEM = 0, -1, -2, -3, -4

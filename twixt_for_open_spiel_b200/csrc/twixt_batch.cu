@@ -675,8 +675,9 @@ class TwixTMCTS {
     cudaFree(arena_mem_);
   }
 
+  // leaves_per_step K > 1: K descents per step with virtual loss vl (checked by the caller, twixt_mcts_create_parallel)
   int Init(TwixTBatch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c, bool puct,
-           bool solve) {
+           bool solve, int32_t leaves_per_step, double virtual_loss) {
     if (num_trees <= 0) return fail(TWIXT_EINVAL, "num_trees must be positive: %lld", static_cast<long long>(num_trees));
     if (max_simulations <= 0) return fail(TWIXT_EINVAL, "max_simulations must be positive: %d", max_simulations);
     if (n_rollouts <= 0) return fail(TWIXT_EINVAL, "n_rollouts must be positive: %d", n_rollouts);
@@ -689,18 +690,22 @@ class TwixTMCTS {
     max_sims_ = max_simulations;
     c_ = uct_c;
     const int n = b->n_;
+    const int K = leaves_per_step;
     const MctsSizes s = mcts_sizes(n, max_simulations, n_rollouts);
-    const int64_t per_tree = solve ? mcts_solve_bytes_per_tree(s, puct)
-                                   : (puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s));
+    const int64_t per_tree = mcts_parallel_bytes_per_tree(
+        s, solve ? mcts_solve_bytes_per_tree(s, puct) : (puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s)),
+        K);
     // carve one allocation; each array starts on a 256-byte boundary (priors and tie keys are PUCT's, the outcome
-    // bytes PUCT's and the solver's, the root codes the solver's: empty otherwise)
-    const int64_t T = num_trees, nodes = T * s.slots, edges = nodes * s.edges, rolls = T * s.rollouts;
+    // bytes PUCT's and the solver's, the root codes the solver's, the virtual counts those of K > 1: empty
+    // otherwise).  Tree entries, paths and rollout slots are per leaf row: K per tree.
+    const int64_t T = num_trees, nodes = T * s.slots, edges = nodes * s.edges, rows = T * K, rolls = rows * s.rollouts;
     const int64_t pe = puct ? edges : 0, oe = (puct || solve) ? edges : 0, rt = solve ? T : 0;
-    const int64_t sizes[17] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
-                               T * 16, T * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8,
-                               pe * 4, pe * 4, oe, rt};
-    int64_t offs[17], total = 0;
-    for (int i = 0; i < 17; ++i) {
+    const int64_t vn = K > 1 ? nodes : 0, ve = K > 1 ? edges : 0;
+    const int64_t sizes[19] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
+                               rows * 16, rows * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8,
+                               pe * 4, pe * 4, oe, rt, vn * 2, ve * 2};
+    int64_t offs[19], total = 0;
+    for (int i = 0; i < 19; ++i) {
       offs[i] = total;
       total += (sizes[i] + 255) & ~static_cast<int64_t>(255);
     }
@@ -709,10 +714,10 @@ class TwixTMCTS {
     TW_CUDA(cudaMemGetInfo(&free_bytes, &total_bytes));
     if (static_cast<uint64_t>(total) > free_bytes)
       return fail(TWIXT_ENOMEM,
-                  "MCTS arena of %lld bytes (%lld trees x %lld bytes per tree at n = %d, %d simulations, %d rollouts) "
-                  "exceeds the %zu bytes free on device %d",
+                  "MCTS arena of %lld bytes (%lld trees x %lld bytes per tree at n = %d, %d simulations, %d rollouts, "
+                  "%d leaves per step) exceeds the %zu bytes free on device %d",
                   static_cast<long long>(total), static_cast<long long>(T), static_cast<long long>(per_tree), n,
-                  max_simulations, n_rollouts, free_bytes, b->device_);
+                  max_simulations, n_rollouts, K, free_bytes, b->device_);
     cudaError_t e = cudaMalloc(&arena_mem_, static_cast<size_t>(total));
     if (e != cudaSuccess) {
       cudaGetLastError();
@@ -745,6 +750,11 @@ class TwixTMCTS {
     a_.edge_key = puct ? reinterpret_cast<uint32_t*>(base + offs[14]) : nullptr;
     a_.edge_out = (puct || solve) ? reinterpret_cast<uint8_t*>(base + offs[15]) : nullptr;
     a_.root_out = solve ? reinterpret_cast<uint8_t*>(base + offs[16]) : nullptr;
+    a_.node_v = K > 1 ? reinterpret_cast<uint16_t*>(base + offs[17]) : nullptr;
+    a_.edge_v = K > 1 ? reinterpret_cast<uint16_t*>(base + offs[18]) : nullptr;
+    a_.K = K;
+    a_.vl = virtual_loss;
+    K_ = K;
     // ln N(s) from the host's libm, so that a CPU restatement of the search computes the same scores
     std::vector<double> logs(static_cast<size_t>(s.slots));
     for (size_t i = 0; i < logs.size(); ++i) logs[i] = std::log(static_cast<double>(i));
@@ -777,12 +787,15 @@ class TwixTMCTS {
 
   int Run(int32_t num_simulations) {
     TW_TRY(CheckSimulations(num_simulations, "run"));
+    if (num_simulations % K_ != 0)
+      return fail(TWIXT_EINVAL, "twixt_mcts_run: %d simulations is not a multiple of leaves_per_step %d",
+                  num_simulations, K_);
     if (count_ == 0 || num_simulations == 0) return TWIXT_OK;
     DeviceGuard g(b_->device_);
     TwixTBatch& b = *b_;
     PlayoutArgs p;
     p.records = a_.roll_rec;
-    p.count = count_ * a_.R;
+    p.count = count_ * K_ * a_.R;
     p.n = a_.n;
     p.max_plies = a_.n * a_.n;  // above max_game_length: every rollout plays to the end
     p.seed = key_;
@@ -794,21 +807,22 @@ class TwixTMCTS {
     p.trace_plies = 0;
     p.stats = b.d_stats_;
     p.tickets = &b.d_stats_->tickets;
-    for (int32_t i = 0; i < num_simulations; ++i) {
+    for (int32_t i = 0; i < num_simulations; i += K_) {  // one step: K simulations of every tree
       const uint32_t k = static_cast<uint32_t>(sims_);
       TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, k, c_, nullptr, nullptr, b.stream_));
       TW_CUDA(cudaMemsetAsync(&b.d_stats_->tickets, 0, sizeof(unsigned long long), b.stream_));
       TW_CUDA(launch_playout(p, b.stream_));
       TW_CUDA(launch_mcts_backup(a_, count_, nullptr, nullptr, key_, stream0_, b.stream_));
       b.launches_ += 3;
-      sims_ += 1;
+      sims_ += K_;
     }
     return TWIXT_OK;
   }
 
+  // K leaf rows per tree: row t*K + j goes to env leaf_first + t*K + j
   int Select(int64_t leaf_first, int32_t* out_leaf_status) {
-    TW_TRY(CheckSimulations(1, "select"));
-    TW_TRY(b_->CheckRange(leaf_first, count_));
+    TW_TRY(CheckSimulations(K_, "select"));
+    TW_TRY(b_->CheckRange(leaf_first, count_ * K_));
     if (count_ == 0) {
       pending_ = true;
       return TWIXT_OK;
@@ -817,7 +831,7 @@ class TwixTMCTS {
     TwixTBatch& b = *b_;
     b.ScratchReset();
     Staged st;
-    TW_TRY(b.StageOut(out_leaf_status, static_cast<size_t>(count_) * sizeof(int32_t), &st, false));
+    TW_TRY(b.StageOut(out_leaf_status, static_cast<size_t>(count_ * K_) * sizeof(int32_t), &st, false));
     TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, static_cast<uint32_t>(sims_), c_, b.rec(leaf_first),
                                static_cast<int32_t*>(st.dev), b.stream_));
     b.launches_ += 1;
@@ -827,7 +841,8 @@ class TwixTMCTS {
     return TWIXT_OK;
   }
 
-  // priors: [count, n*n] float32 or nullptr (uniform); host priors are checked before anything is launched
+  // values [count*K, 2], priors: [count*K, n*n] float32 or nullptr (uniform); host priors are checked before anything
+  // is launched
   int Backup(const float* values, const float* priors) {
     if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_backup: no search begun");
     if (!pending_) return fail(TWIXT_EINVAL, "twixt_mcts_backup without a pending twixt_mcts_select");
@@ -836,7 +851,7 @@ class TwixTMCTS {
       return fail(TWIXT_EINVAL, "twixt_mcts_backup_priors: priors given to a UCT search (use twixt_mcts_create_puct)");
     const size_t cells = static_cast<size_t>(a_.n) * a_.n;
     if (priors != nullptr && count_ > 0 && !is_device_pointer(priors)) {
-      const size_t total = static_cast<size_t>(count_) * cells;
+      const size_t total = static_cast<size_t>(count_ * K_) * cells;
       for (size_t i = 0; i < total; ++i)
         if (!std::isfinite(priors[i]) || priors[i] < 0.0f)
           return fail(TWIXT_EINVAL, "prior [%lld, %lld] = %g: priors must be finite and >= 0",
@@ -848,15 +863,16 @@ class TwixTMCTS {
       TwixTBatch& b = *b_;
       b.ScratchReset();
       Staged in, pin;
-      TW_TRY(b.StageIn(values, static_cast<size_t>(count_) * 2 * sizeof(float), &in));
-      TW_TRY(b.StageIn(priors, priors != nullptr ? static_cast<size_t>(count_) * cells * sizeof(float) : 0, &pin));
+      const size_t rows = static_cast<size_t>(count_ * K_);
+      TW_TRY(b.StageIn(values, rows * 2 * sizeof(float), &in));
+      TW_TRY(b.StageIn(priors, priors != nullptr ? rows * cells * sizeof(float) : 0, &pin));
       TW_CUDA(launch_mcts_backup(a_, count_, static_cast<const float*>(in.dev), static_cast<const float*>(pin.dev),
                                  key_, stream0_, b.stream_));
       b.launches_ += 1;
       if (in.host || pin.host) TW_TRY(b.Sync());  // the staged copies are reused by the next call
     }
     pending_ = false;
-    sims_ += 1;
+    sims_ += K_;
     return TWIXT_OK;
   }
 
@@ -927,6 +943,7 @@ class TwixTMCTS {
   MctsArena a_{};
   int64_t num_trees_ = 0;
   int32_t max_sims_ = 0;
+  int32_t K_ = 1;  // leaves per step
   double c_ = 0.0;
   int64_t count_ = 0;
   uint64_t key_ = 0;
@@ -1107,16 +1124,25 @@ int twixt_stats_accumulate(twixt_stats* acc, const twixt_stats* part) {
   if ((m) == nullptr) return fail(TWIXT_EINVAL, "null mcts handle")
 
 static int mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
-                       double uct_c, uint32_t flags, twixt_mcts** out) {
+                       double uct_c, uint32_t flags, int32_t leaves_per_step, double virtual_loss, twixt_mcts** out) {
   TW_NEED(b);
   if (out == nullptr) return fail(TWIXT_EINVAL, "null output pointer");
   *out = nullptr;
   if ((flags & ~static_cast<uint32_t>(TWIXT_MCTS_PUCT | TWIXT_MCTS_SOLVE)) != 0u)
     return fail(TWIXT_EINVAL, "unknown twixt_mcts_create_ex flags 0x%x", flags);
   const bool puct = (flags & TWIXT_MCTS_PUCT) != 0u, solve = (flags & TWIXT_MCTS_SOLVE) != 0u;
+  if (leaves_per_step < 1 || leaves_per_step > 4096)
+    return fail(TWIXT_EINVAL, "leaves_per_step must be in [1, 4096]: %d", leaves_per_step);
+  if (leaves_per_step > 1 && leaves_per_step > max_simulations)
+    return fail(TWIXT_EINVAL, "leaves_per_step %d exceeds max_simulations %d", leaves_per_step, max_simulations);
+  if (!std::isfinite(virtual_loss) || virtual_loss < 0.0)
+    return fail(TWIXT_EINVAL, "virtual_loss must be finite and >= 0: %g", virtual_loss);
+  if (solve && leaves_per_step > 1)
+    return fail(TWIXT_EINVAL, "TWIXT_MCTS_SOLVE runs one leaf per step: leaves_per_step %d", leaves_per_step);
   twixt_mcts* m = new (std::nothrow) twixt_mcts();
   if (m == nullptr) return fail(TWIXT_ENOMEM, "out of host memory");
-  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, uct_c, puct, solve);
+  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, uct_c, puct, solve, leaves_per_step,
+                        virtual_loss);
   if (rc != TWIXT_OK) {
     std::string keep = twixt::g_last_error;
     delete m;
@@ -1128,15 +1154,20 @@ static int mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulation
 }
 int twixt_mcts_create(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c,
                       twixt_mcts** out) {
-  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, 0u, out);
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, 0u, 1, 0.0, out);
 }
 int twixt_mcts_create_puct(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
                            double uct_c, twixt_mcts** out) {
-  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, TWIXT_MCTS_PUCT, out);
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, TWIXT_MCTS_PUCT, 1, 0.0, out);
 }
 int twixt_mcts_create_ex(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
                          double uct_c, uint32_t flags, twixt_mcts** out) {
-  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, flags, out);
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, flags, 1, 0.0, out);
+}
+int twixt_mcts_create_parallel(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                               double uct_c, uint32_t flags, int32_t leaves_per_step, double virtual_loss,
+                               twixt_mcts** out) {
+  return mcts_create(b, num_trees, max_simulations, n_rollouts, uct_c, flags, leaves_per_step, virtual_loss, out);
 }
 void twixt_mcts_destroy(twixt_mcts* m) { delete m; }
 int twixt_mcts_begin(twixt_mcts* m, int64_t root_first, int64_t count) {

@@ -76,6 +76,13 @@ struct MctsArena {
                             // search (UCT ones too) also writes the code of a proven child here
   // solver searches only (nullptr otherwise, which selects on that)
   uint8_t* root_out;        // [trees] outcome code of the root (twixt_mcts.cuh), 0 = unproven; cleared by begin
+  // searches with K > 1 leaves per step only (nullptr otherwise, which selects on that).  Their tree entries, paths
+  // and rollout slots are per leaf row t*K + j: tree [trees*K], path [trees*K*P], rollout slots [trees*K*R]; the
+  // node count of tree t is in tree[t*K].x
+  uint16_t* node_v;         // [trees*S] virtual visits V(s), 0 between steps
+  uint16_t* edge_v;         // [trees*S*M] virtual visits V(a), 0 between steps
+  int K;                    // leaves per step (1 without node_v)
+  double vl;                // virtual loss
 };
 
 cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s);

@@ -75,8 +75,8 @@ __device__ __forceinline__ int warp_expand(const MctsArena& a, int64_t g, const 
 
 // ----------------------------------------------------------------- begin ---
 // The root of tree t is a COPY of env roots + t; every tree is cleared to its root alone (a solver search: and its
-// root code to unproven).
-template <bool kSolve>
+// root code to unproven; kVirtual: its V(s) to 0, and the node count goes to tree entry t*K).
+template <bool kSolve, bool kVirtual>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a, const uint32_t* __restrict__ roots,
                                                                      int64_t count) {
   const int lane = threadIdx.x & 31;
@@ -87,9 +87,174 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a
   if (lane == 0) {
     a.node_legal[root] = -1;
     a.node_n[root] = 0u;
-    a.tree[t] = make_int4(1, 0, 0, kLeafNeedsValue);
+    if constexpr (kVirtual) {
+      a.node_v[root] = 0;
+      a.tree[t * a.K] = make_int4(1, 0, 0, kLeafNeedsValue);
+    } else {
+      a.tree[t] = make_int4(1, 0, 0, kLeafNeedsValue);
+    }
     if constexpr (kSolve) a.root_out[t] = 0;
   }
+}
+
+// ------------------------------------------------------- select, K > 1 ---
+// The K descents of tree t in a search with K = a.K > 1 leaves per step (the kVirtual select kernels): descent j
+// is simulation k + j, scores with the virtual counts of descents 0 .. j-1 (n_eff, N_eff(s), w_eff: twixt_mcts.cuh),
+// writes leaf row t*K + j (tree entry, status, leaf env or its R rollout slots), then adds V += 1 along its path
+// (lanes over the path) and on its leaf.  The descent itself is the one of the kernel below.
+template <bool kPuct>
+__device__ __forceinline__ void select_descents(const MctsArena& a, int64_t t, int lane, uint64_t seed, uint32_t T,
+                                                uint32_t k, double uct_c, uint32_t* __restrict__ leaf_dst,
+                                                int32_t* __restrict__ out_status) {
+  const int n = a.n, rw = a.rw, K = a.K;
+  int nodes = a.tree[t * K].x;
+  for (int j = 0; j < K; ++j) {
+    const int64_t row = t * K + j;
+    int2* path = a.path + row * a.P;
+    int node = 0, depth = 0;
+    bool terminal;
+    for (;;) {
+      const int64_t g = mcts_slot(a, t, node);
+      uint32_t* rec = a.node_rec + g * rw;
+      const uint4 hw = *reinterpret_cast<const uint4*>(rec);
+      Header h;
+      unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+      terminal = h.result != kOpen;
+      const uint32_t visits = a.node_n[g];
+      if (terminal || visits == 0u) break;
+      const uint32_t visits_eff = visits + a.node_v[g];
+      const int64_t e0 = g * a.M;
+      int legal = a.node_legal[g];
+      int edge;
+      if constexpr (kPuct) {
+        const double sq = mcts_sqrt_visits(visits_eff);
+        double best = 0.0;
+        uint32_t bk = 0u;
+        int bi = 0x7FFFFFFF;
+        for (int i = lane; i < legal; i += 32) {
+          const uint8_t o = a.edge_out[e0 + i];
+          const uint32_t v = a.edge_v[e0 + i];
+          const double sc = o != 0 ? static_cast<double>(mcts_outcome_value(o))
+                                   : mcts_puct_score(mcts_virtual_w(a.edge_w[e0 + i], v, a.vl), a.edge_n[e0 + i] + v,
+                                                     a.edge_p[e0 + i], sq, uct_c);
+          const uint32_t key = a.edge_key[e0 + i];
+          if (bi == 0x7FFFFFFF || mcts_puct_beats(sc, key, i, best, bk, bi)) {
+            best = sc;
+            bk = key;
+            bi = i;
+          }
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+          const double os = __shfl_xor_sync(kFullMask, best, d);
+          const uint32_t ok = __shfl_xor_sync(kFullMask, bk, d);
+          const int oi = __shfl_xor_sync(kFullMask, bi, d);
+          if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_puct_beats(os, ok, oi, best, bk, bi))) {
+            best = os;
+            bk = ok;
+            bi = oi;
+          }
+        }
+        edge = bi;
+      } else {
+        if (legal < 0) {
+          legal = warp_expand(a, g, rec, h, lane);
+          for (int i = lane; i < legal; i += 32) a.edge_v[e0 + i] = 0;
+          __syncwarp();
+        }
+        // edges with n_eff == 0
+        int unvisited = 0;
+        for (int i = lane; i < legal; i += 32) unvisited += a.edge_n[e0 + i] + a.edge_v[e0 + i] == 0u ? 1 : 0;
+        unvisited = __reduce_add_sync(kFullMask, unvisited);
+        if (unvisited > 0) {
+          int pick = static_cast<int>(mcts_draw(seed, T, k + static_cast<uint32_t>(j), static_cast<uint32_t>(unvisited)));
+          edge = -1;
+          for (int base = 0; edge < 0; base += 32) {
+            const int i = base + lane;
+            const uint32_t m = __ballot_sync(kFullMask, i < legal && a.edge_n[e0 + i] + a.edge_v[e0 + i] == 0u);
+            const int c = __popc(m);
+            if (pick < c) edge = base + select_bit(m, pick);
+            else pick -= c;
+          }
+        } else {
+          const double log_parent = a.log_table[visits_eff];
+          double best = 0.0;
+          int bi = 0x7FFFFFFF;
+          for (int i = lane; i < legal; i += 32) {
+            const uint32_t v = a.edge_v[e0 + i];
+            const double sc = mcts_uct_score(mcts_virtual_w(a.edge_w[e0 + i], v, a.vl), a.edge_n[e0 + i] + v,
+                                             log_parent, uct_c);
+            if (bi == 0x7FFFFFFF || mcts_score_beats(sc, i, best, bi)) {
+              best = sc;
+              bi = i;
+            }
+          }
+#pragma unroll
+          for (int d = 16; d > 0; d >>= 1) {
+            const double os = __shfl_xor_sync(kFullMask, best, d);
+            const int oi = __shfl_xor_sync(kFullMask, bi, d);
+            if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_score_beats(os, oi, best, bi))) {
+              best = os;
+              bi = oi;
+            }
+          }
+          edge = bi;
+        }
+      }
+      if (lane == 0) path[depth] = make_int2(node, (edge << 1) | static_cast<int>(h.ply & 1u));
+      ++depth;
+      int child = a.edge_child[e0 + edge];
+      if (child < 0) {
+        child = nodes++;
+        const int64_t gc = mcts_slot(a, t, child);
+        uint32_t* crec = a.node_rec + gc * rw;
+        warp_copy_record(crec, rec, rw, lane);
+        __syncwarp();
+        if (lane == 0) {
+          RecordRef<1> cb{crec, n};
+          Header ch = h;
+          const int action = a.edge_action[e0 + edge];
+          const int x = action / n;
+          apply_legal_cell<kMctsFloodStack>(cb, ch, x, action - x * n);
+          uint4 o;
+          pack_header(ch, o.x, o.y, o.z, o.w);
+          *reinterpret_cast<uint4*>(crec) = o;
+          a.node_legal[gc] = -1;
+          a.node_n[gc] = 0u;
+          a.node_v[gc] = 0;
+          a.edge_child[e0 + edge] = child;
+          if (kPuct && ch.result != kOpen) a.edge_out[e0 + edge] = mcts_outcome_code(ch, static_cast<int>(h.ply & 1u));
+        }
+        __syncwarp();
+      }
+      node = child;
+    }
+    const uint32_t* leaf = a.node_rec + mcts_slot(a, t, node) * rw;
+    if (leaf_dst != nullptr) {
+      warp_copy_record(leaf_dst + row * rw, leaf, rw, lane);
+    } else {
+      for (int r = 0; r < a.R; ++r) warp_copy_record(a.roll_rec + (row * a.R + r) * rw, leaf, rw, lane);
+      for (int r = lane; r < a.R; r += 32)
+        a.roll_ids[row * a.R + r] = mcts_rollout_stream(T, k + static_cast<uint32_t>(j), static_cast<uint32_t>(a.R),
+                                                        static_cast<uint32_t>(r));
+    }
+    const int status = terminal ? kLeafTerminal : kLeafNeedsValue;
+    if (lane == 0) {
+      a.tree[row] = make_int4(nodes, node, depth, status);
+      if (out_status != nullptr) out_status[row] = status;
+    }
+    // V += 1 along the path and on the leaf, seen by the next descent
+    __syncwarp();
+    for (int i = lane; i < depth; i += 32) {
+      const int2 p = path[i];
+      const int64_t g = mcts_slot(a, t, p.x);
+      a.node_v[g] += 1;
+      a.edge_v[g * a.M + (p.y >> 1)] += 1;
+    }
+    if (lane == 0) a.node_v[mcts_slot(a, t, node)] += 1;
+    __syncwarp();
+  }
+  if (lane == 0) a.tree[t * K].x = nodes;  // the node count of the tree
 }
 
 // ---------------------------------------------------------------- select ---
@@ -97,14 +262,22 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a
 // kernel carries no PUCT code and neither carries solver code.  A solver search's finished tree (proven root) takes
 // no path: status kLeafSolved, its leaf env is not written, and in run mode its rollout slots get a copy of the
 // root marked drawn, which the playout kernel counts as neither a ply nor a game.
-template <bool kPuct, bool kSolve>
+// kVirtual (a.node_v != nullptr, K = a.K > 1 leaves per step; never with kSolve): the warp runs descents
+// j = 0 .. K-1 in order, descent j as simulation k + j on the virtual counts of the earlier ones, writes leaf row
+// t*K + j, and adds its virtual visits along its path (lanes over the path) before the next descent.
+template <bool kPuct, bool kSolve, bool kVirtual>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena a, int64_t count, uint64_t seed,
                                                                       uint32_t stream0, uint32_t k, double uct_c,
                                                                       uint32_t* __restrict__ leaf_dst,
                                                                       int32_t* __restrict__ out_status) {
+  static_assert(!(kSolve && kVirtual), "the solver runs one leaf per step");
   const int lane = threadIdx.x & 31;
   const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
   if (t >= count) return;
+  if constexpr (kVirtual) {
+    select_descents<kPuct>(a, t, lane, seed, stream0 + static_cast<uint32_t>(t), k, uct_c, leaf_dst, out_status);
+    return;
+  }
   const int n = a.n, rw = a.rw;
   const uint32_t T = stream0 + static_cast<uint32_t>(t);
   int node = 0, depth = 0, nodes = a.tree[t].x;
@@ -273,16 +446,22 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_select_kernel(MctsArena 
 }
 
 // ---------------------------------------------------------------- backup ---
-// kSolve: a finished tree's row is ignored, and a terminal leaf starts the MCTS-Solver proof pass up its path
-template <bool kSolve>
+// kSolve: a finished tree's row is ignored, and a terminal leaf starts the MCTS-Solver proof pass up its path.
+// kVirtual: rows j = 0 .. K-1 of the tree in order, each removing its virtual visits; a PUCT leaf is expanded by
+// the lowest row whose leaf it is (later rows find it expanded and their priors are ignored).
+template <bool kSolve, bool kVirtual>
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena a, int64_t count,
                                                                       const float* __restrict__ values,
                                                                       const float* __restrict__ priors,
                                                                       uint64_t seed, uint32_t stream0) {
+  static_assert(!(kSolve && kVirtual), "the solver runs one leaf per step");
   const int lane = threadIdx.x & 31;
   const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
   if (t >= count) return;
-  const int4 info = a.tree[t];
+  const int K = kVirtual ? a.K : 1;
+  for (int j = 0; j < K; ++j) {  // K == 1 unless kVirtual
+  const int64_t row = t * K + j;
+  const int4 info = a.tree[row];
   if constexpr (kSolve) {
     if (info.w == kLeafSolved) return;
   }
@@ -294,12 +473,12 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
     unpack_header(hw.x, hw.y, hw.z, hw.w, h);
     mcts_terminal_value(h, v);
   } else if (values != nullptr) {
-    v[0] = static_cast<double>(values[2 * t]);
-    v[1] = static_cast<double>(values[2 * t + 1]);
+    v[0] = static_cast<double>(values[2 * row]);
+    v[1] = static_cast<double>(values[2 * row + 1]);
   } else {
     // (double) sum_r ret_r[p] / R, r ascending
     double s0 = 0.0, s1 = 0.0;
-    const float* ret = a.roll_ret + t * a.R * 2;
+    const float* ret = a.roll_ret + row * a.R * 2;
     for (int r = 0; r < a.R; ++r) {
       s0 = __dadd_rn(s0, static_cast<double>(ret[2 * r]));
       s1 = __dadd_rn(s1, static_cast<double>(ret[2 * r + 1]));
@@ -307,7 +486,7 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
     v[0] = __ddiv_rn(s0, static_cast<double>(a.R));
     v[1] = __ddiv_rn(s1, static_cast<double>(a.R));
   }
-  const int2* path = a.path + t * a.P;
+  const int2* path = a.path + row * a.P;
   for (int i = lane; i < depth; i += 32) {
     const int2 p = path[i];
     const int64_t g = mcts_slot(a, t, p.x);
@@ -315,9 +494,17 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
     a.node_n[g] += 1u;
     a.edge_n[e] += 1u;
     a.edge_w[e] = __dadd_rn(a.edge_w[e], v[p.y & 1]);
+    if constexpr (kVirtual) {
+      a.node_v[g] -= 1;
+      a.edge_v[e] -= 1;
+    }
   }
-  if (lane == 0) a.node_n[mcts_slot(a, t, leaf)] += 1u;
-  if (a.edge_p != nullptr && info.w != kLeafTerminal) {
+  if (lane == 0) {
+    a.node_n[mcts_slot(a, t, leaf)] += 1u;
+    if constexpr (kVirtual) a.node_v[mcts_slot(a, t, leaf)] -= 1;
+  }
+  if (a.edge_p != nullptr && info.w != kLeafTerminal &&
+      (!kVirtual || a.node_legal[mcts_slot(a, t, leaf)] < 0)) {
     // PUCT: expand the leaf with its priors (open_spiel expands on the second visit from evaluator.prior, which
     // AlphaZeroEvaluator answers from the network call that valued the leaf)
     const int64_t g = mcts_slot(a, t, leaf), e0 = g * a.M;
@@ -327,14 +514,16 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
     unpack_header(hw.x, hw.y, hw.z, hw.w, h);
     const int legal = warp_expand(a, g, rec, h, lane);
     const float uniform = mcts_uniform_prior(legal);
-    const float* row = priors != nullptr ? priors + t * a.n * a.n : nullptr;
+    const float* prow = priors != nullptr ? priors + row * a.n * a.n : nullptr;
     const uint32_t T = stream0 + static_cast<uint32_t>(t);
     for (int i = lane; i < legal; i += 32) {
-      a.edge_p[e0 + i] = row != nullptr ? row[a.edge_action[e0 + i]] : uniform;
+      a.edge_p[e0 + i] = prow != nullptr ? prow[a.edge_action[e0 + i]] : uniform;
       a.edge_key[e0 + i] = mcts_tie_key(seed, T, static_cast<uint32_t>(leaf), static_cast<uint32_t>(i));
       a.edge_out[e0 + i] = 0;
+      if constexpr (kVirtual) a.edge_v[e0 + i] = 0;
     }
   }
+  if constexpr (kVirtual) __syncwarp();  // the next row may update the same nodes and edges
   if constexpr (kSolve) {
     if (info.w == kLeafTerminal) {
       if (depth == 0) {
@@ -374,6 +563,7 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
         __syncwarp();
       }
     }
+  }
   }
 }
 
@@ -546,10 +736,10 @@ unsigned mcts_blocks(int64_t count) { return static_cast<unsigned>((count + kMct
 
 cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  if (a.root_out != nullptr)
-    mcts_begin_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
-  else
-    mcts_begin_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
+  auto kernel = a.node_v != nullptr ? mcts_begin_kernel<false, true>
+                                    : (a.root_out != nullptr ? mcts_begin_kernel<true, false>
+                                                             : mcts_begin_kernel<false, false>);
+  kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
   return cudaGetLastError();
 }
 
@@ -557,8 +747,10 @@ cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed,
                                double uct_c, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
   const bool puct = a.edge_p != nullptr, solve = a.root_out != nullptr;
-  auto kernel = puct ? (solve ? mcts_select_kernel<true, true> : mcts_select_kernel<true, false>)
-                     : (solve ? mcts_select_kernel<false, true> : mcts_select_kernel<false, false>);
+  auto kernel = a.node_v != nullptr
+                    ? (puct ? mcts_select_kernel<true, false, true> : mcts_select_kernel<false, false, true>)
+                : puct ? (solve ? mcts_select_kernel<true, true, false> : mcts_select_kernel<true, false, false>)
+                       : (solve ? mcts_select_kernel<false, true, false> : mcts_select_kernel<false, false, false>);
   kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c, leaf_dst, out_status);
   return cudaGetLastError();
 }
@@ -566,10 +758,10 @@ cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed,
 cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, const float* priors,
                                uint64_t seed, uint32_t stream0, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
-  if (a.root_out != nullptr)
-    mcts_backup_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
-  else
-    mcts_backup_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
+  auto kernel = a.node_v != nullptr ? mcts_backup_kernel<false, true>
+                                    : (a.root_out != nullptr ? mcts_backup_kernel<true, false>
+                                                             : mcts_backup_kernel<false, false>);
+  kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
   return cudaGetLastError();
 }
 

@@ -32,6 +32,25 @@
 // The outcome code of an edge is 0 while its child is unproven, else 2 + the child's value for the player to move
 // at the parent (1 = loss, 2 = draw, 3 = win); the root code is 2 + the root's value for its own player to move
 // (ply parity, also for a terminal root).
+//
+// Several leaves per step (twixt_mcts_create_parallel, K = leaves_per_step > 1, virtual loss vl): one step is K
+// descents j = 0 .. K-1 of every tree, descent j being simulation k = sims_since_begin + j (draw and rollout
+// streams as above).  Every node has a virtual visit count V(s) and every edge V(a), both 0 between steps; after
+// descent j picks its path, V += 1 on every edge and node of the path and on the leaf, so later descents of the
+// step see it:
+//   effective counts     n_eff = N(a) + V(a), N_eff(s) = N(s) + V(s)
+//   effective value sum  w_eff = V(a) > 0 ? W(a) - vl * V(a) : W(a), IEEE double, no contraction
+//   uct                  the unvisited-edge draw counts edges with n_eff == 0, else uct score(w_eff, n_eff, L[N_eff(s)])
+//   puct                 puct score(w_eff, n_eff, P, sqrt(N_eff(s))); a terminal child still scores its outcome
+// The leaf rule is unchanged (a terminal node or N(s) == 0, real visits only), so every descent of step 0 stops
+// at the root, and a descent may end at a leaf an earlier descent of the step already took (a repeated leaf, an
+// ordinary row).  Backup takes rows j = 0 .. K-1 in order: row j removes its V and adds its value as before; a
+// PUCT leaf is expanded by the lowest row whose leaf it is.  W only ever receives real values.
+// Storage for K > 1: K paths, K (leaf slot, depth, status) entries and K*R rollout slots per tree, and a u16 V per
+// node and per edge:
+//   K-leaf bytes per tree = (bytes per tree of the kind above) + (K - 1) * (16 + 8*P + R * (rw*4 + 16))
+//                           + S * 2 * (1 + M)
+// K = 1 is exactly the search above and allocates nothing more.
 #pragma once
 #include <stdint.h>
 
@@ -76,6 +95,24 @@ TW_HD int64_t mcts_puct_bytes_per_tree(const MctsSizes& s) { return mcts_bytes_p
 // the solver formulas of the header comment above
 TW_HD int64_t mcts_solve_bytes_per_tree(const MctsSizes& s, bool puct) {
   return (puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s) + s.slots * s.edges) + 1;
+}
+
+// the K-leaf formula of the header comment above, from the bytes per tree of the search kind at K = 1
+TW_HD int64_t mcts_parallel_bytes_per_tree(const MctsSizes& s, int64_t kind_bytes, int leaves_per_step) {
+  if (leaves_per_step <= 1) return kind_bytes;
+  return kind_bytes + static_cast<int64_t>(leaves_per_step - 1) * (16 + 8 * s.path + s.rollouts * (s.rw * 4 + 16)) +
+         s.slots * 2 * (1 + s.edges);
+}
+
+// w_eff of an edge with value sum w and V(a) = v virtual visits under virtual loss vl.  Bit-identical on the
+// device and on a host compiled with -ffp-contract=off; w itself when v == 0.
+TW_HD double mcts_virtual_w(double w, uint32_t v, double vl) {
+  if (v == 0u) return w;
+#if defined(__CUDA_ARCH__)
+  return __dsub_rn(w, __dmul_rn(vl, static_cast<double>(v)));
+#else
+  return w - vl * static_cast<double>(v);
+#endif
 }
 
 // UCT score of an edge with N(a) = n > 0 visits and value sum w, under a parent whose ln N(s) is log_parent.

@@ -14,12 +14,19 @@ Two ways to evaluate leaves:
 `selection="puct"` makes every tree open_spiel's AlphaZero search instead (MCTSBot with
 child_selection_fn = puct_value): `backup(values, priors)` hands the policy head's priors [count, n*n] with
 the values, and the leaf is expanded with them.  `add_dirichlet_noise` mixes open_spiel's root noise into the
-priors of the first backup after `begin` (simulation 0's leaf is always the root).
+priors of the first backup after `begin` (simulation 0's leaf is always the root; with leaves_per_step = K, row
+t*K + 0 of that backup).
 
 `solve=True` adds open_spiel's MCTS-Solver to either kind (MCTSBot(..., solve=True), open_spiel's default):
 a terminal leaf proves nodes up its path, a proven child is scored by its outcome, and a tree whose root is
 proven is finished: later simulations do nothing for it (`select` reports LEAF_SOLVED and leaves its env
 alone).  `solver_stats()` returns the proven root and move values.
+
+`leaves_per_step=K` (K > 1) descends K times per tree in one step, with virtual loss steering the later descents
+of a step away from the earlier ones (leaf parallelism, as in AlphaGo, Leela Zero and KataGo; not an open_spiel
+behaviour, and exactly the search above at K = 1).  All K leaves of every tree are evaluated together: `run`
+plays K*R rollouts per tree in one playout launch, and the stepwise form hands the caller K rows per tree, so a
+search needs max_simulations / K steps instead of max_simulations.  Row t*K + j is descent j of tree t.
 
 `MCTSBot` is the open_spiel-shaped bot over one tree for adapter `TwixTState`s.
 
@@ -43,15 +50,23 @@ _PUCT, _SOLVE = 1, 2  # TWIXT_MCTS_PUCT, TWIXT_MCTS_SOLVE
 
 class BatchedMCTS:
     def __init__(self, batch: TwixTBatch, num_trees: int, max_simulations: int, n_rollouts: int = 1,
-                 uct_c: float = 2.0, selection: str = "uct", solve: bool = False):
+                 uct_c: float = 2.0, selection: str = "uct", solve: bool = False, leaves_per_step: int = 1,
+                 virtual_loss: float = 1.0):
         if selection not in ("uct", "puct"):
             raise ValueError("selection must be 'uct' or 'puct', got %r" % (selection,))
         self._lib = _lib.load()
         self.batch = batch  # the search runs on the batch's envs and stream: keep it alive
         self._h = C.c_void_p()
         flags = (_PUCT if selection == "puct" else 0) | (_SOLVE if solve else 0)
-        self._check(self._lib.twixt_mcts_create_ex(batch._h, int(num_trees), int(max_simulations), int(n_rollouts),
-                                                   float(uct_c), flags, C.byref(self._h)))
+        if int(leaves_per_step) == 1:
+            self._check(self._lib.twixt_mcts_create_ex(batch._h, int(num_trees), int(max_simulations),
+                                                       int(n_rollouts), float(uct_c), flags, C.byref(self._h)))
+        else:
+            self._check(self._lib.twixt_mcts_create_parallel(
+                batch._h, int(num_trees), int(max_simulations), int(n_rollouts), float(uct_c), flags,
+                int(leaves_per_step), float(virtual_loss), C.byref(self._h)))
+        self.leaves_per_step = int(leaves_per_step)
+        self.virtual_loss = float(virtual_loss)
         self.selection = selection
         self.solve = bool(solve)
         self.num_trees = int(num_trees)
@@ -84,31 +99,34 @@ class BatchedMCTS:
         self.count = int(count)
 
     def run(self, num_simulations: int):
-        """num_simulations simulations of every tree with the built-in rollout evaluator (asynchronous)."""
+        """num_simulations simulations of every tree with the built-in rollout evaluator (asynchronous); a
+        multiple of leaves_per_step."""
         self._check(self._lib.twixt_mcts_run(self._h, int(num_simulations)))
 
     def select(self, leaf_first: int, out_status=None):
-        """Stepwise form, first half: leaf of tree t -> batch env leaf_first + t.  Returns the statuses
-        [count] int32 (LEAF_NEEDS_VALUE, or LEAF_TERMINAL: its value is Returns() and backup ignores the
-        caller's, or with solve=True LEAF_SOLVED: the tree is finished, its env was not written and backup
-        ignores its row)."""
+        """Stepwise form, first half: leaf of descent j of tree t -> batch env leaf_first + t*K + j (K =
+        leaves_per_step; t with K = 1).  Returns the statuses [count*K] int32 (LEAF_NEEDS_VALUE, or LEAF_TERMINAL:
+        its value is Returns() and backup ignores the caller's, or with solve=True LEAF_SOLVED: the tree is
+        finished, its env was not written and backup ignores its row)."""
+        rows = self.count * self.leaves_per_step
         if out_status is None:
-            out_status = np.zeros(self.count, dtype=np.int32)
+            out_status = np.zeros(rows, dtype=np.int32)
         self._check(self._lib.twixt_mcts_select(self._h, int(leaf_first),
-                                                _ptr(out_status, _dt(np.int32, "int32"), self.count)))
+                                                _ptr(out_status, _dt(np.int32, "int32"), rows)))
         return out_status
 
     def backup(self, values, priors=None):
-        """Stepwise form, second half: values [count, 2] float32 of the leaves select() wrote.  A PUCT search
-        also takes priors [count, n*n] float32 (None: uniform over the legal actions); entries of illegal
-        actions and rows of terminal leaves are ignored."""
+        """Stepwise form, second half: values [count*K, 2] float32 of the leaves select() wrote.  A PUCT search
+        also takes priors [count*K, n*n] float32 (None: uniform over the legal actions); entries of illegal
+        actions, rows of terminal leaves and (K > 1) the rows of repeated leaves after the first are ignored."""
+        rows = self.count * self.leaves_per_step
         if not _is_torch(values):
             values = np.ascontiguousarray(values, dtype=np.float32)
         if priors is not None and not _is_torch(priors):
             priors = np.ascontiguousarray(priors, dtype=np.float32)
         self._check(self._lib.twixt_mcts_backup_priors(
-            self._h, _ptr(values, _dt(np.float32, "float32"), 2 * self.count),
-            _ptr(priors, _dt(np.float32, "float32"), self.count * self._cells)))
+            self._h, _ptr(values, _dt(np.float32, "float32"), 2 * rows),
+            _ptr(priors, _dt(np.float32, "float32"), rows * self._cells)))
 
     def root_stats(self, out_visits=None, out_value_sums=None, out_best=None):
         """(visits [count, n*n] int32, value_sums [count, n*n] float64, best [count] int32) of the root edges;
@@ -153,6 +171,10 @@ class BatchedMCTS:
 def add_dirichlet_noise(priors, legal_mask, epsilon: float, alpha: float):
     """open_spiel's root noise: (1 - epsilon) * p + epsilon * Dir(alpha) over each row's legal actions.
 
+    It goes into the priors of the first backup after `begin`, whose rows are the roots.  With leaves_per_step =
+    K > 1 every descent of that first step stops at the root and the root takes the priors of row t*K + 0, so
+    noise belongs in the rows t*K + 0 (the other rows' priors for the root are ignored).
+
     priors [B, A] float32 and legal_mask [B, A] (bool or 0/1) are torch tensors on the CPU or a GPU; returns a
     new float32 tensor on the same device.  Gamma(alpha) is drawn for every entry with torch's generator (so the
     result is reproducible under torch.manual_seed), in float64, zeroed where illegal and normalised per row;
@@ -177,16 +199,24 @@ class MCTSBot:
 
     solve defaults to False here, so existing callers keep the search they had; open_spiel's MCTSBot and
     mcts_example default to solve=True, which is `MCTSBot(..., solve=True)`: a proven win is played at once and
-    the search of a step ends when its root is proven."""
+    the search of a step ends when its root is proven.
+
+    leaves_per_step=K > 1 searches the one tree K leaves at a time with virtual loss (BatchedMCTS above), in
+    max_simulations / K steps per move; max_simulations must then be a multiple of K and at least 2*K (step 0
+    only evaluates the root).  The default K = 1 is the bot above."""
 
     def __init__(self, game, uct_c: float = 2.0, max_simulations: int = 1000, n_rollouts: int = 4, seed: int = 0,
-                 device: int = 0, solve: bool = False):
+                 device: int = 0, solve: bool = False, leaves_per_step: int = 1, virtual_loss: float = 1.0):
         if max_simulations < 2:
             raise ValueError("MCTSBot needs max_simulations >= 2: the first simulation only evaluates the root")
+        if leaves_per_step > 1 and (max_simulations % leaves_per_step or max_simulations < 2 * leaves_per_step):
+            raise ValueError("MCTSBot with leaves_per_step = %d needs max_simulations to be a multiple of it and at "
+                             "least twice it, got %d" % (leaves_per_step, max_simulations))
         self._game = game
         self._batch = TwixTBatch(game.board_size(), 1, device, seed)
         self._batch.set_validation(False)  # records come from the adapter's own exports
-        self._mcts = BatchedMCTS(self._batch, 1, max_simulations, n_rollouts, uct_c, solve=solve)
+        self._mcts = BatchedMCTS(self._batch, 1, max_simulations, n_rollouts, uct_c, solve=solve,
+                                 leaves_per_step=leaves_per_step, virtual_loss=virtual_loss)
         self.max_simulations = int(max_simulations)
 
     def step(self, state) -> int:
