@@ -19,7 +19,14 @@ leaves_per_step=K > 1 searches K leaves per tree in each step with virtual loss 
 sims / K calls.  Every descent of the first step stops at the root, which takes the priors of row g*K + 0: the
 Dirichlet noise goes into those rows.
 
-    python examples/alphazero_selfplay.py [board_size] [games] [simulations] [leaves_per_step]
+reuse_tree=True keeps each game's tree between moves (BatchedMCTS.advance): `begin` runs once, and after each
+`apply` the played move's subtree becomes the new root with its statistics (at most sims + 1 nodes of a search
+holding 2*sims), so every move still runs sims new simulations on top of what the last search spent there.  The
+root Dirichlet noise then reaches a kept root through `set_root_priors`; a root the advance left without
+statistics (ROOT_FRESH) is expanded by the first backup as after `begin`, so the noise goes into its row g*K + 0
+there, masked on the device.
+
+    python examples/alphazero_selfplay.py [board_size] [games] [simulations] [leaves_per_step] [reuse_tree]
 """
 import os
 import sys
@@ -29,7 +36,7 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from twixt_for_open_spiel_b200 import TwixTBatch  # noqa: E402
-from twixt_for_open_spiel_b200.mcts import BatchedMCTS, add_dirichlet_noise  # noqa: E402
+from twixt_for_open_spiel_b200.mcts import ROOT_FRESH, BatchedMCTS, add_dirichlet_noise  # noqa: E402
 from twixt_for_open_spiel_b200.producer import ObservationMaskProducer  # noqa: E402
 
 
@@ -54,10 +61,11 @@ def masked_softmax(logits, legal):
 
 
 def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_c=2.0, dirichlet_epsilon=0.25,
-              dirichlet_alpha=1.0, seed=0, net=None, verbose=True, leaves_per_step=1, virtual_loss=1.0):
+              dirichlet_alpha=1.0, seed=0, net=None, verbose=True, leaves_per_step=1, virtual_loss=1.0,
+              reuse_tree=False):
     """Plays `games` games to the end.  Returns (trajectories, returns [games, 2]); trajectories[g] is a list of
     per-move dicts with obs [12, n, n-2], mask [n*n], policy [n*n], player and action.  sims must be a multiple
-    of leaves_per_step."""
+    of leaves_per_step.  reuse_tree=True keeps the played move's subtree between moves (see the module text)."""
     K = int(leaves_per_step)
     if sims % K:
         raise ValueError("sims = %d is not a multiple of leaves_per_step = %d" % (sims, K))
@@ -69,8 +77,11 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
     producer = ObservationMaskProducer(batch, max_count=rows)
     if net is None:
         net = PolicyValueNet(n).to(dev).eval()
-    search = BatchedMCTS(batch, games, sims, uct_c=uct_c, selection="puct", leaves_per_step=K,
+    capacity = 2 * sims if reuse_tree else sims
+    search = BatchedMCTS(batch, games, capacity, uct_c=uct_c, selection="puct", leaves_per_step=K,
                          virtual_loss=virtual_loss)
+    fresh = torch.ones(games, dtype=torch.bool, device=dev)  # roots without statistics (all of them at begin)
+    status = torch.zeros(games, dtype=torch.int32, device=dev)
     player = torch.zeros(rows, dtype=torch.int8, device=dev)
     root_player = torch.zeros(games, dtype=torch.int8, device=dev)
     done = torch.zeros(games, dtype=torch.uint8, device=dev)
@@ -90,7 +101,15 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
             root_obs, root_mask = producer.produce(0, games)
             root_obs, root_mask = root_obs.clone(), root_mask.clone()
             batch.current_player(0, games, out=root_player)
-            search.begin(0, games)
+            if not reuse_tree:
+                search.begin(0, games)
+            elif move == 0:
+                search.begin(0, games)
+            else:  # kept roots take their noise now; fresh ones at the first backup below
+                root_legal = root_mask.bool()
+                root_priors = masked_softmax(net(root_obs)[0], root_legal)
+                search.set_root_priors(add_dirichlet_noise(root_priors, root_legal, dirichlet_epsilon,
+                                                           dirichlet_alpha).contiguous())
             for k in range(sims // K):
                 search.select(games)
                 obs, mask = producer.produce(games, rows)
@@ -98,10 +117,11 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
                 logits, v = net(obs)
                 priors = masked_softmax(logits, legal)
                 if k == 0:
-                    if K == 1:
+                    if K == 1 and not reuse_tree:
                         priors = add_dirichlet_noise(priors, legal, dirichlet_epsilon, dirichlet_alpha)
-                    else:  # the root rows g*K + 0
-                        priors[::K] = add_dirichlet_noise(priors[::K], legal[::K], dirichlet_epsilon, dirichlet_alpha)
+                    else:  # the root rows g*K + 0, and with reuse_tree only where the root is fresh
+                        noisy = add_dirichlet_noise(priors[::K], legal[::K], dirichlet_epsilon, dirichlet_alpha)
+                        priors[::K] = torch.where(fresh[:, None], noisy, priors[::K])
                 batch.current_player(games, rows, out=player)
                 v = torch.where(player == 1, -v, v).float()
                 search.backup(torch.stack([v, -v], dim=1).contiguous(), priors.contiguous())
@@ -116,6 +136,9 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
             action = torch.where(live, action, torch.full_like(action, -1)).contiguous()
             history.append((root_obs, root_mask, policy, root_player.clone(), action, live))
             batch.apply(action, 0)
+            if reuse_tree:
+                search.advance(action, sims + 1, out_status=status)
+                fresh = status == ROOT_FRESH
             move += 1
     returns = batch.returns(0, games)
     trajectories = [[] for _ in range(games)]
@@ -134,7 +157,8 @@ def main():
     games = int(sys.argv[2]) if len(sys.argv) > 2 else 256
     sims = int(sys.argv[3]) if len(sys.argv) > 3 else 100
     leaves = int(sys.argv[4]) if len(sys.argv) > 4 else 1
-    trajectories, returns = self_play(n, games, sims, leaves_per_step=leaves)
+    reuse = len(sys.argv) > 5 and sys.argv[5] not in ("0", "false", "False")
+    trajectories, returns = self_play(n, games, sims, leaves_per_step=leaves, reuse_tree=reuse)
     lengths = [len(t) for t in trajectories]
     print("%d games at n = %d, %d simulations per move: mean length %.1f, red wins %d, blue wins %d, draws %d" % (
         games, n, sims, float(np.mean(lengths)), int((returns[:, 0] > 0).sum()), int((returns[:, 1] > 0).sum()),

@@ -389,6 +389,48 @@ int twixt_mcts_create_parallel(twixt_batch* b, int64_t num_trees, int32_t max_si
                                double uct_c, uint32_t flags, int32_t leaves_per_step, double virtual_loss,
                                twixt_mcts** out);
 
+/* Tree reuse across moves (as AlphaGo Zero, Leela Zero and KataGo do; open_spiel's MCTSBot has none, so this is
+ * the search's own behaviour).  A caller that never calls twixt_mcts_advance gets exactly the searches above.
+ * twixt_mcts_advance(m, actions, keep_nodes, out_status): actions [count] int32 on the host or the device,
+ * 1 <= keep_nodes <= S = max_simulations + 1, out_status [count] int32 (nullable).  For tree t:
+ *  - a legal action whose root edge has a child: that child becomes the new root.  The kept nodes are its
+ *    subtree, renumbered by their rank in old slot order (the new root is slot 0, children stay above their
+ *    parents), each with all its data: record, N(s), legal count and its edges' action, N, W, child (remapped),
+ *    prior, tie key and outcome code.  The node count becomes the number of kept nodes.
+ *  - the cap: only the first keep_nodes nodes of that order are kept (still a rooted tree).  An edge whose child
+ *    the cap drops is unvisited again (N = 0, W = 0, no child; prior, tie key and outcome code stay); its parent's
+ *    N(s) is unchanged, and a later simulation that takes it creates the child afresh.
+ *  - a legal action without a child (the edge was never taken, or the root is not expanded): the tree is cleared
+ *    to the root with the move applied, as twixt_mcts_begin would from that state.
+ *  - action -1: the tree keeps its root and is only cut to keep_nodes (finished self-play games).
+ *  - an illegal action, which includes anything but -1 at a terminal root: the tree is unchanged and gets status
+ *    1, and the call fails with TWIXT_EILLEGAL "Not a legal action: %d" exactly as twixt_apply reports it (with a
+ *    device out_status the call returns at once and the statuses are the report; begin such a tree again before
+ *    it runs more simulations, since the host's node bound below assumes every tree was cut to keep_nodes).
+ *  - statuses: TWIXT_MCTS_ROOT_KEPT (0) the new root has statistics (N(root) > 0), TWIXT_MCTS_ROOT_ILLEGAL (1),
+ *    TWIXT_MCTS_ROOT_FRESH (2) the new root has none (N(root) = 0): the next simulation evaluates it.
+ *  - solver searches: the new root's code is 4 - c from the chosen edge's code c != 0 (the child's value for its
+ *    own player to move), else 0; a tree advanced into a proven child stays finished.
+ *  - the stream id T and the simulation counter k, which key the unvisited-edge draw and the rollout streams,
+ *    carry on across advances, so a tree never repeats a Philox counter.
+ * It is TWIXT_EINVAL before begin and while a select is pending, and works with every kind and with K > 1.  One
+ * launch; the first call allocates an int32 slot map of count x S entries (not part of the create-time arena).
+ * Budget, without host synchronisation: the host bounds the node count (1 after begin, min(keep_nodes, bound)
+ * after an advance, +K per step) and run(s) / select fail with TWIXT_EINVAL when bound + s > S; without an
+ * advance this is the "more than max_simulations simulations since begin" check.  k*R + r must stay below 2^32.
+ * Size the arena for reuse: max_simulations = the capacity, e.g. 2*sims with keep_nodes = sims + 1 runs sims new
+ * simulations every move.
+ * twixt_mcts_set_root_priors(m, priors [count, n*n] float32, host or device), PUCT only: replaces P(a) on every
+ * root edge of each tree whose root is expanded; other trees are left alone (their first backup still takes the
+ * priors of row t*K + 0).  This is how root Dirichlet noise reaches a kept root.  Host priors are checked as
+ * twixt_mcts_backup_priors checks them.  TWIXT_EINVAL on a UCT search, before begin or while a select is pending.
+ * One launch. */
+#define TWIXT_MCTS_ROOT_KEPT 0
+#define TWIXT_MCTS_ROOT_ILLEGAL 1
+#define TWIXT_MCTS_ROOT_FRESH 2
+int twixt_mcts_advance(twixt_mcts* m, const int32_t* actions, int32_t keep_nodes, int32_t* out_status);
+int twixt_mcts_set_root_priors(twixt_mcts* m, const float* priors);
+
 /* Multi-GPU plumbing for hosts that are not Python (SURVEY 8e: envs shard by contiguous global id ranges,
  * no data-path collective, one reduction of the counters).  twixt_shard_range: rank's share [first,
  * first+count) of global_envs envs over `world` ranks (shares differ by at most one env); create the rank's

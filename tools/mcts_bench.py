@@ -29,6 +29,17 @@ with simulations/s and the select / backup kernel ms per step, next to the UCT c
   after a warm-up;
   64 trees x 400 simulations at n = 12, UCT x R = 4 (run) and the stepwise PUCT search above, at K = 1 and 8:
   simulations/s and the select / playout / backup kernel ms per step (a step is K simulations of every tree).
+
+`reuse`: tree reuse across moves (BatchedMCTS.advance):
+  the advance kernel alone at n = 12 for 8192 stepwise PUCT trees after a 400-simulation search (capacity 800,
+  keep 401), along each tree's best move: device ms (torch.profiler, mean of 3 searches) and an estimate of the
+  bytes it moves (each kept node's record, counts and L edges read and written once, L the root's legal count, the
+  kept nodes N(new root)), as GB/s and a fraction of the 7.7 TB/s HBM3e peak of one HGX B200 GPU (data sheet);
+  a multi-move loop of the stepwise PUCT search above (1024 trees at n = 12, 100 new simulations per move, 12
+  moves along the best move) with begin every move and with advance(best, 101) on a capacity of 200: moves/s and
+  the mean N(root) at the start of each move's search (sum of the root's N(a) + 1 for an expanded root).
+  Both use seeded uniform random priors raised to the 8th power, so that a few moves carry most of a node's prior
+  as with a trained policy (flat priors spread the visits over all moves and leave little to keep), and zero values.
 """
 from __future__ import annotations
 
@@ -225,6 +236,104 @@ def bench_single_tree(n: int, sims: int, R: int, K: int, reps: int) -> dict:
             "ms_per_search_min": round(1e3 * min(times), 3)}
 
 
+def _puct_steps(m, trees, sims, values, priors, status):
+    for _ in range(sims):
+        m.select(trees, status)
+        m.backup(values, priors)
+
+
+def bench_advance(n: int, trees: int, sims: int, reps: int) -> dict:
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+
+    from twixt_for_open_spiel_b200.mcts import BatchedMCTS
+    b = make_roots(n, 2 * trees, 0x72757365)
+    m = BatchedMCTS(b, trees, 2 * sims, selection="puct")
+    gen = torch.Generator(device="cuda").manual_seed(2)
+    priors = torch.rand((trees, n * n), generator=gen, device="cuda", dtype=torch.float32) ** 8  # peaked
+    values = torch.zeros((trees, 2), device="cuda", dtype=torch.float32)
+    status = torch.zeros(trees, dtype=torch.int32, device="cuda")
+    visits = torch.zeros((trees, n * n), dtype=torch.int32, device="cuda")
+    best = torch.zeros(trees, dtype=torch.int32, device="cuda")
+    rw = b.record_words
+    kernel_us, kept_total, edge_bytes = [], 0, 0
+    for rep in range(reps + 1):  # the first is a warm-up
+        m.begin(0, trees)
+        _puct_steps(m, trees, sims, values, priors, status)
+        m.root_stats(out_visits=visits, out_best=best)
+        b.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            m.advance(best, sims + 1, out_status=status)
+            b.synchronize()
+        if rep == 0:
+            continue
+        kernel_us.append(sum(getattr(ev, "device_time_total", None) or ev.cuda_time_total
+                             for ev in prof.key_averages() if "mcts_advance_kernel" in ev.key))
+        kept = visits.gather(1, best.clamp_min(0).long()[:, None])[:, 0].long()  # N(a) of the move = kept nodes
+        _, cnt = b.legal_actions(0, trees)  # the old roots' legal counts
+        L = torch.as_tensor(cnt, device="cuda").long()
+        kept_total = int(kept.sum())
+        # per kept node: record + legal count + N(s) + L edges (action 2, N 4, W 8, child 4, prior 4, key 4,
+        # outcome 1) read and written, and the slot map written and read
+        edge_bytes = int((kept * (2 * (rw * 4 + 8 + 27 * L) + 8)).sum())
+    ms = sum(kernel_us) / len(kernel_us) / 1e3
+    m.close()
+    b.close()
+    gbs = edge_bytes / (ms / 1e3) / 1e9
+    return {"board_size": n, "trees": trees, "simulations": sims, "capacity": 2 * sims, "keep_nodes": sims + 1,
+            "advance_kernel_ms": round(ms, 4), "kept_nodes": kept_total, "estimated_bytes_moved": edge_bytes,
+            "estimated_gb_per_s": round(gbs, 1), "fraction_of_hbm_peak": round(gbs / 7700.0, 4)}
+
+
+def bench_moves(n: int, trees: int, sims: int, moves: int, reuse: bool) -> dict:
+    import torch
+
+    from twixt_for_open_spiel_b200.mcts import BatchedMCTS
+    b = make_roots(n, 2 * trees, 0x6D6F7665)
+    start_records = b.export_state(0, trees)
+    m = BatchedMCTS(b, trees, 2 * sims, selection="puct")
+    gen = torch.Generator(device="cuda").manual_seed(3)
+    priors = torch.rand((trees, n * n), generator=gen, device="cuda", dtype=torch.float32) ** 8  # peaked
+    values = torch.zeros((trees, 2), device="cuda", dtype=torch.float32)
+    status = torch.zeros(trees, dtype=torch.int32, device="cuda")
+    visits = torch.zeros((trees, n * n), dtype=torch.int32, device="cuda")
+    best = torch.zeros(trees, dtype=torch.int32, device="cuda")
+    root_n = torch.zeros(moves, dtype=torch.float64, device="cuda")
+
+    def play(record_n):
+        m.begin(0, trees)
+        for mv in range(moves):
+            if mv > 0 and not reuse:
+                m.begin(0, trees)
+            if record_n:
+                m.root_stats(out_visits=visits)
+                total = visits.sum(1)
+                root_n[mv] = (total + (total > 0).int()).double().mean()
+            _puct_steps(m, trees, sims, values, priors, status)
+            m.root_stats(out_best=best)
+            b.apply(best, 0)
+            if reuse:
+                m.advance(best, sims + 1, out_status=status)
+
+    play(False)  # warm-up
+    b.import_state(start_records, 0)
+    b.synchronize()
+    t0 = time.perf_counter()
+    play(False)
+    b.synchronize()
+    dt = time.perf_counter() - t0
+    b.import_state(start_records, 0)
+    play(True)
+    b.synchronize()
+    per_move = root_n.cpu().tolist()
+    m.close()
+    b.close()
+    return {"board_size": n, "trees": trees, "new_simulations_per_move": sims, "moves": moves, "reuse_tree": reuse,
+            "moves_per_s": round(moves / dt, 2), "simulations_per_s": round(trees * sims * moves / dt, 1),
+            "mean_root_visits_at_search_start": round(sum(per_move) / moves, 2),
+            "mean_root_visits_by_move": [round(x, 1) for x in per_move]}
+
+
 def bench_evaluator(n: int, leaves: int, R: int, reps: int) -> dict:
     from twixt_for_open_spiel_b200.rollout import BatchedRolloutEvaluator
     ev = BatchedRolloutEvaluator(n, n_rollouts=R, max_leaves=leaves, seed=1)
@@ -244,6 +353,7 @@ def main() -> None:
     ap.add_argument("--quick", action="store_true", help="small sizes (a functional check, not a measurement)")
     ap.add_argument("--no-solve", action="store_true", help="skip the solver entries")
     ap.add_argument("--no-parallel", action="store_true", help="skip the leaves_per_step entries")
+    ap.add_argument("--no-reuse", action="store_true", help="skip the tree reuse entries")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -256,6 +366,8 @@ def main() -> None:
         solve = [(12, 256, 40, 4, 10, True, False), (8, 256, 40, 4, 10, True, True)]
         single = [(12, 96, 4, K, 2) for K in (1, 8, 32)]
         many = [(12, 16, 48, 4, 16, K) for K in (1, 8)]
+        adv = (12, 256, 40, 2)
+        moves = (12, 64, 20, 4)
     else:
         configs = [(12, 8192, 400, 4, 50), (24, 1024, 200, 4, 50)]
         puct = [(12, 8192, 400, 50), (24, 1024, 200, 50)]
@@ -263,6 +375,8 @@ def main() -> None:
         solve = [(12, 8192, 400, 4, 50, True, False), (8, 8192, 400, 4, 50, True, True)]
         single = [(12, 1000, 4, K, 5) for K in (1, 8, 32)]
         many = [(12, 64, 400, 4, 80, K) for K in (1, 8)]
+        adv = (12, 8192, 400, 3)
+        moves = (12, 1024, 100, 12)
     out = dict(info)
     out["configs"] = [bench_config(*c) for c in configs]
     out["evaluate_slots"] = bench_evaluator(*ev)
@@ -275,6 +389,9 @@ def main() -> None:
             "uct": [bench_config(n, t, s, R, p, leaves_per_step=K) for n, t, s, R, p, K in many],
             "puct": [bench_puct(n, t, s, p, leaves_per_step=K) for n, t, s, _, p, K in many],
         }
+    if not args.no_reuse:
+        out["reuse"] = {"advance": bench_advance(*adv),
+                        "moves": [bench_moves(*moves, reuse=r) for r in (False, True)]}
     print(json.dumps(out))
 
 

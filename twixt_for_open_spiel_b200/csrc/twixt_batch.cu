@@ -671,8 +671,10 @@ class TwixTMCTS {
   ~TwixTMCTS() {
     if (arena_mem_ == nullptr) return;
     DeviceGuard g(b_->device_);
+    if (log_grown_ != nullptr) cudaFreeAsync(log_grown_, b_->stream_);
     cudaStreamSynchronize(b_->stream_);
     cudaFree(arena_mem_);
+    if (map_ != nullptr) cudaFree(map_);
   }
 
   // leaves_per_step K > 1: K descents per step with virtual loss vl (checked by the caller, twixt_mcts_create_parallel)
@@ -755,6 +757,7 @@ class TwixTMCTS {
     a_.K = K;
     a_.vl = virtual_loss;
     K_ = K;
+    log_size_ = s.slots;
     // ln N(s) from the host's libm, so that a CPU restatement of the search computes the same scores
     std::vector<double> logs(static_cast<size_t>(s.slots));
     for (size_t i = 0; i < logs.size(); ++i) logs[i] = std::log(static_cast<double>(i));
@@ -780,6 +783,8 @@ class TwixTMCTS {
     key_ = b_->seed_;
     stream0_ = static_cast<uint32_t>(base + static_cast<uint64_t>(root_first));
     sims_ = 0;
+    node_bound_ = 1;
+    advanced_ = false;
     pending_ = false;
     begun_ = true;
     return TWIXT_OK;
@@ -792,6 +797,7 @@ class TwixTMCTS {
                   num_simulations, K_);
     if (count_ == 0 || num_simulations == 0) return TWIXT_OK;
     DeviceGuard g(b_->device_);
+    TW_TRY(GrowLogTable(num_simulations));
     TwixTBatch& b = *b_;
     PlayoutArgs p;
     p.records = a_.roll_rec;
@@ -815,6 +821,7 @@ class TwixTMCTS {
       TW_CUDA(launch_mcts_backup(a_, count_, nullptr, nullptr, key_, stream0_, b.stream_));
       b.launches_ += 3;
       sims_ += K_;
+      node_bound_ += K_;
     }
     return TWIXT_OK;
   }
@@ -828,6 +835,7 @@ class TwixTMCTS {
       return TWIXT_OK;
     }
     DeviceGuard g(b_->device_);
+    TW_TRY(GrowLogTable(K_));
     TwixTBatch& b = *b_;
     b.ScratchReset();
     Staged st;
@@ -836,6 +844,7 @@ class TwixTMCTS {
                                static_cast<int32_t*>(st.dev), b.stream_));
     b.launches_ += 1;
     pending_ = true;
+    node_bound_ += K_;
     TW_TRY(b.Finish(&st));
     if (st.host) TW_TRY(b.Sync());
     return TWIXT_OK;
@@ -924,17 +933,150 @@ class TwixTMCTS {
     return TWIXT_OK;
   }
 
+  // Tree reuse: actions [count] int32 (host or device), 1 <= keep_nodes <= S, out_status [count] int32 or nullptr.
+  // Illegal actions are reported as twixt_apply reports them: TWIXT_EILLEGAL naming the first one, except with
+  // device statuses, where the call returns at once and the caller reads the statuses.
+  int Advance(const int32_t* actions, int32_t keep_nodes, int32_t* out_status) {
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_advance: no search begun");
+    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_advance while a twixt_mcts_select awaits its backup");
+    if (keep_nodes < 1 || keep_nodes > a_.S)
+      return fail(TWIXT_EINVAL, "keep_nodes must be in [1, max_simulations + 1 = %d]: %d", a_.S, keep_nodes);
+    if (count_ == 0) return TWIXT_OK;
+    if (actions == nullptr) return fail(TWIXT_EINVAL, "null actions pointer");
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    if (map_ == nullptr) {  // old -> new slot map, [num_trees, S] int32, allocated at the first advance
+      const size_t bytes = static_cast<size_t>(num_trees_) * a_.S * sizeof(int32_t);
+      cudaError_t e = cudaMalloc(&map_, bytes);
+      if (e != cudaSuccess) {
+        cudaGetLastError();
+        map_ = nullptr;
+        return fail(TWIXT_ENOMEM, "cudaMalloc of %zu bytes for the twixt_mcts_advance slot map failed: %s", bytes,
+                    cudaGetErrorString(e));
+      }
+    }
+    b.ScratchReset();
+    Staged in, st;
+    TW_TRY(b.StageIn(actions, static_cast<size_t>(count_) * sizeof(int32_t), &in));
+    const size_t status_bytes = static_cast<size_t>(count_) * sizeof(int32_t);
+    if (out_status == nullptr) b.PinAlloc(status_bytes, &st);  // as twixt_apply: statuses read below
+    else TW_TRY(b.StageOut(out_status, status_bytes, &st, false));
+    const bool scan_host = st.pin != nullptr;
+    if (!scan_host) TW_CUDA(cudaMemsetAsync(&b.d_stats_->illegal_index, 0xFF, sizeof(unsigned int), b.stream_));
+    TW_CUDA(launch_mcts_advance(a_, count_, static_cast<const int32_t*>(in.dev), keep_nodes, map_,
+                                static_cast<int32_t*>(st.dev), &b.d_stats_->illegal_index, b.stream_));
+    b.launches_ += 1;
+    advanced_ = true;
+    TW_TRY(b.Finish(&st));
+    // every tree now holds at most min(keep_nodes, bound) nodes, except one whose action was illegal (unchanged);
+    // device statuses are the caller's to read, who must begin again after an illegal one
+    const int64_t truncated = keep_nodes < node_bound_ ? keep_nodes : node_bound_;
+    if (out_status != nullptr && !st.host) {
+      node_bound_ = truncated;
+      if (in.host) TW_TRY(b.Sync());  // the staged actions are reused by the next call
+      return TWIXT_OK;
+    }
+    int64_t bad = -1;
+    if (scan_host) {
+      TW_TRY(b.Sync());
+      const int32_t* seen = static_cast<const int32_t*>(st.pin);
+      for (int64_t i = 0; i < count_ && bad < 0; ++i)
+        if (seen[i] == kRootIllegal) bad = i;
+    } else {
+      unsigned int flag = 0xFFFFFFFFu;
+      TW_CUDA(cudaMemcpyAsync(&flag, &b.d_stats_->illegal_index, sizeof(flag), cudaMemcpyDeviceToHost, b.stream_));
+      TW_TRY(b.Sync());
+      if (flag != 0xFFFFFFFFu) bad = flag;
+    }
+    if (bad >= 0) {
+      int32_t act = 0;
+      if (in.host) act = actions[bad];
+      else TW_CUDA(cudaMemcpy(&act, actions + bad, sizeof(act), cudaMemcpyDeviceToHost));
+      return fail(TWIXT_EILLEGAL, "Not a legal action: %d", act);  // twixt.h:96, as twixt_apply
+    }
+    node_bound_ = truncated;
+    return TWIXT_OK;
+  }
+
+  // PUCT searches: P(a) of every root edge of the trees whose root is expanded, from priors [count, n*n]
+  int SetRootPriors(const float* priors) {
+    if (a_.edge_p == nullptr)
+      return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors: the search is not a PUCT search");
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors: no search begun");
+    if (pending_)
+      return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors while a twixt_mcts_select awaits its backup");
+    if (count_ == 0) return TWIXT_OK;
+    if (priors == nullptr) return fail(TWIXT_EINVAL, "null priors pointer");
+    const size_t cells = static_cast<size_t>(a_.n) * a_.n;
+    if (!is_device_pointer(priors)) {
+      const size_t total = static_cast<size_t>(count_) * cells;
+      for (size_t i = 0; i < total; ++i)
+        if (!std::isfinite(priors[i]) || priors[i] < 0.0f)
+          return fail(TWIXT_EINVAL, "prior [%lld, %lld] = %g: priors must be finite and >= 0",
+                      static_cast<long long>(i / cells), static_cast<long long>(i % cells),
+                      static_cast<double>(priors[i]));
+    }
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    b.ScratchReset();
+    Staged pin;
+    TW_TRY(b.StageIn(priors, static_cast<size_t>(count_) * cells * sizeof(float), &pin));
+    TW_CUDA(launch_mcts_set_root_priors(a_, count_, static_cast<const float*>(pin.dev), b.stream_));
+    b.launches_ += 1;
+    if (pin.host) TW_TRY(b.Sync());  // the staged copy is reused by the next call
+    return TWIXT_OK;
+  }
+
   int64_t count() const { return count_; }
   int64_t simulations() const { return sims_; }
 
  private:
+  // The host's bound on a tree's node count (node_bound_: 1 after begin, min(keep_nodes, bound) after an advance,
+  // +K per step) keeps every step inside the S node slots without reading the trees back.  Without an advance this
+  // is "at most max_simulations simulations since begin".
   int CheckSimulations(int32_t num, const char* what) const {
     if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_%s: no search begun", what);
     if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_%s while a twixt_mcts_select awaits its backup", what);
     if (num < 0) return fail(TWIXT_EINVAL, "num_simulations must be >= 0: %d", num);
-    if (sims_ + num > max_sims_)
+    if (!advanced_ && sims_ + num > max_sims_)
       return fail(TWIXT_EINVAL, "%lld simulations since begin would exceed max_simulations %d",
                   static_cast<long long>(sims_ + num), max_sims_);
+    if (advanced_ && node_bound_ + num > a_.S)
+      return fail(TWIXT_EINVAL,
+                  "twixt_mcts_%s: %d simulations on trees of up to %lld nodes since twixt_mcts_advance would exceed "
+                  "the max_simulations + 1 = %d node slots of a tree (advance with a smaller keep_nodes)",
+                  what, num, static_cast<long long>(node_bound_), a_.S);
+    // the simulation counter k carries on across advances: k*R + r keys the rollout streams and must stay 32-bit
+    if (static_cast<uint64_t>(sims_ + num) * static_cast<uint64_t>(a_.R) > (1ull << 32))
+      return fail(TWIXT_EINVAL,
+                  "twixt_mcts_%s: simulation counter %lld + %d times n_rollouts %d would reach 2^32 (rollout stream "
+                  "ids); begin the search again",
+                  what, static_cast<long long>(sims_), num, a_.R);
+    return TWIXT_OK;
+  }
+
+  // ln N(s) for N(s) < sims_ + num: N(s) <= the simulations since begin, which outgrow the S entries of the arena's
+  // table once advances keep trees.  A larger table is filled from the host's libm as at create, and the old one is
+  // freed in stream order.
+  int GrowLogTable(int32_t num) {
+    const int64_t need = sims_ + num;
+    if (need <= log_size_) return TWIXT_OK;
+    const int64_t size = need > 2 * log_size_ ? need : 2 * log_size_;
+    std::vector<double> logs(static_cast<size_t>(size));
+    for (size_t i = 0; i < logs.size(); ++i) logs[i] = std::log(static_cast<double>(i));
+    void* table = nullptr;
+    cudaError_t e = cudaMallocAsync(&table, logs.size() * sizeof(double), b_->stream_);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(TWIXT_ENOMEM, "cudaMallocAsync of %zu bytes for the ln N(s) table failed: %s",
+                  logs.size() * sizeof(double), cudaGetErrorString(e));
+    }
+    // pageable source: the copy has taken the data when it returns
+    TW_CUDA(cudaMemcpyAsync(table, logs.data(), logs.size() * sizeof(double), cudaMemcpyHostToDevice, b_->stream_));
+    if (log_grown_ != nullptr) TW_CUDA(cudaFreeAsync(log_grown_, b_->stream_));
+    log_grown_ = static_cast<double*>(table);
+    a_.log_table = log_grown_;
+    log_size_ = size;
     return TWIXT_OK;
   }
 
@@ -949,6 +1091,11 @@ class TwixTMCTS {
   uint64_t key_ = 0;
   uint32_t stream0_ = 0;
   int64_t sims_ = 0;
+  int64_t node_bound_ = 1;     // bound on every tree's node count (CheckSimulations)
+  bool advanced_ = false;      // an advance since begin
+  int32_t* map_ = nullptr;     // [num_trees, S] old -> new slots of twixt_mcts_advance
+  double* log_grown_ = nullptr;  // the ln table once it outgrew the arena's
+  int64_t log_size_ = 0;       // its entries
   bool pending_ = false;
   bool begun_ = false;
 };
@@ -1198,6 +1345,14 @@ int twixt_mcts_solver_stats(twixt_mcts* m, uint8_t* out_proven, float* out_retur
                             int32_t* out_simulations) {
   TW_NEED_MCTS(m);
   return m->impl.SolverStats(out_proven, out_returns, out_edge_values, out_simulations);
+}
+int twixt_mcts_advance(twixt_mcts* m, const int32_t* actions, int32_t keep_nodes, int32_t* out_status) {
+  TW_NEED_MCTS(m);
+  return m->impl.Advance(actions, keep_nodes, out_status);
+}
+int twixt_mcts_set_root_priors(twixt_mcts* m, const float* priors) {
+  TW_NEED_MCTS(m);
+  return m->impl.SetRootPriors(priors);
 }
 
 int twixt_get_stats(twixt_batch* b, twixt_stats* out) {

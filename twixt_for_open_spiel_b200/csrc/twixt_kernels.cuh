@@ -98,6 +98,12 @@ cudaError_t launch_mcts_root_stats(const MctsArena& a, int64_t count, int32_t* o
 // solver searches: proven [count] u8, returns [count, 2] f32, edge values [count, n*n] i8, N(root) [count] i32
 cudaError_t launch_mcts_solver_stats(const MctsArena& a, int64_t count, uint8_t* out_proven, float* out_returns,
                                      int8_t* out_edge_values, int32_t* out_simulations, cudaStream_t s);
+// tree reuse: actions [count] (device), map [count*S] int32 scratch, out_status [count] or nullptr; an illegal action
+// lowers *illegal_index to its tree
+cudaError_t launch_mcts_advance(const MctsArena& a, int64_t count, const int32_t* actions, int keep_nodes,
+                                int32_t* map, int32_t* out_status, unsigned int* illegal_index, cudaStream_t s);
+// PUCT searches: P(a) of the root edges of every expanded root from priors [count, n*n] (device)
+cudaError_t launch_mcts_set_root_priors(const MctsArena& a, int64_t count, const float* priors, cudaStream_t s);
 
 cudaError_t launch_reset(uint32_t* records, int64_t count, int n, cudaStream_t s);
 cudaError_t launch_clone(uint32_t* dst, const uint32_t* src, const int64_t* src_ids, int64_t count, int n,

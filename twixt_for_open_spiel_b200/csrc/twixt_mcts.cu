@@ -730,6 +730,179 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_solver_stats_kernel(Mcts
   }
 }
 
+// --------------------------------------------------------------- advance ---
+// Tree reuse (twixt_mcts_advance; semantics in twixt_mcts.cuh).  One warp per tree, three phases:
+//   1. legality: the action's bit in the root's legal_word (lane = column); the root edge of the action by a
+//      ballot over edge_action.  An edge without a child (or an unexpanded root) makes a fresh root: one lane
+//      applies the move to slot 0's record, as select creates a child.
+//   2. mark and rank, sequential in slot order from the new root s0: a slot is in the subtree when it is s0 or its
+//      parent (a lower slot) kept it; kept slots get their rank in map[] until keep_nodes are ranked, the others
+//      stay negative.  Lanes over a kept node's edges mark its children; a ballot over a window of 32 map entries
+//      skips the slots that are not in the subtree.
+//   3. move: each kept node, in ascending old slot order, goes to its rank r: the record with 16-byte stores and its
+//      L edges' SoA entries (not M), children remapped through map[] and dropped children reset.
+// The move is in place.  It is safe because r <= s - s0 <= s for every kept slot s, and slots are moved in
+// ascending s: the destination r is either s itself (each lane rewrites the entries it has just read) or a lower
+// slot, which is outside the subtree or was already moved.  So every source is read before its slot can be
+// overwritten.  map[] is per-tree scratch, not part of the tree.  The V counts (K > 1) are 0 between steps and are
+// written as 0 at the destinations.
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_advance_kernel(MctsArena a, int64_t count,
+                                                                       const int32_t* __restrict__ actions,
+                                                                       int keep_nodes, int32_t* map_all,
+                                                                       int32_t* __restrict__ out_status,
+                                                                       unsigned int* __restrict__ illegal_index) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int n = a.n, rw = a.rw, M = a.M;
+  int4* entry = a.tree + t * a.K;
+  const int nodes = entry->x;
+  const int action = actions[t];
+  const int64_t root = mcts_slot(a, t, 0), r0 = root * M;
+  uint32_t* rrec = a.node_rec + root * rw;
+  const uint4 hw = *reinterpret_cast<const uint4*>(rrec);
+  Header h;
+  unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+
+  // 1. legality and the root edge
+  int s0 = 0;        // old slot of the new root, -1: a fresh root
+  uint8_t code = 0;  // outcome code of the chosen edge
+  if (action != -1) {
+    bool legal = false;
+    if (h.result == kOpen && action >= 0 && action < n * n) {
+      RecordRef<1> b{rrec, n};
+      const int x = action / n;
+      const uint32_t w = lane < n ? legal_word(b, h, lane) : 0u;
+      legal = ((__shfl_sync(kFullMask, w, x) >> (action - x * n)) & 1u) != 0u;
+    }
+    if (!legal) {
+      if (lane == 0) {
+        if (out_status != nullptr) out_status[t] = kRootIllegal;
+        atomicMin(illegal_index, static_cast<unsigned int>(t));  // the host names this action in its message
+      }
+      return;
+    }
+    s0 = -1;
+    const int L = a.node_legal[root];
+    for (int base = 0; base < L; base += 32) {
+      const int i = base + lane;
+      const unsigned m = __ballot_sync(kFullMask, i < L && a.edge_action[r0 + i] == action);
+      if (m != 0u) {
+        const int e = base + __ffs(static_cast<int>(m)) - 1;
+        s0 = a.edge_child[r0 + e];
+        if (a.edge_out != nullptr) code = a.edge_out[r0 + e];
+        break;
+      }
+    }
+    if (s0 < 0) {
+      // no child: the root with the move applied, cleared as begin clears a tree
+      if (lane == 0) {
+        RecordRef<1> b{rrec, n};
+        const int x = action / n;
+        apply_legal_cell<kMctsFloodStack>(b, h, x, action - x * n);
+        uint4 o;
+        pack_header(h, o.x, o.y, o.z, o.w);
+        *reinterpret_cast<uint4*>(rrec) = o;
+        a.node_legal[root] = -1;
+        a.node_n[root] = 0u;
+        if (a.node_v != nullptr) a.node_v[root] = 0;
+        if (a.root_out != nullptr) a.root_out[t] = mcts_advanced_root_code(code);
+        entry->x = 1;
+        if (out_status != nullptr) out_status[t] = kRootFresh;
+      }
+      return;
+    }
+  }
+
+  // 2. mark and rank: map = -1 outside the subtree, -2 marked (a kept parent's child), >= 0 the rank
+  int32_t* map = map_all + t * a.S;
+  for (int s = s0 + 1 + lane; s < nodes; s += 32) map[s] = -1;
+  if (lane == 0) map[s0] = -2;
+  __syncwarp();
+  int kept = 0;
+  for (int s = s0; s < nodes && kept < keep_nodes;) {
+    const int q = s + lane;
+    const unsigned m = __ballot_sync(kFullMask, q < nodes && map[q] != -1);
+    if (m == 0u) {
+      s += 32;
+      continue;
+    }
+    s += __ffs(static_cast<int>(m)) - 1;  // the next slot in the subtree
+    const int64_t g = mcts_slot(a, t, s), e0 = g * M;
+    const int L = a.node_legal[g];
+    for (int i = lane; i < L; i += 32) {
+      const int c = a.edge_child[e0 + i];
+      if (c >= 0) map[c] = -2;
+    }
+    if (lane == 0) map[s] = kept;
+    ++kept;
+    ++s;
+    __syncwarp();
+  }
+
+  // 3. move the kept nodes down to their ranks
+  uint32_t root_visits = 0u;
+  for (int s = s0, moved = 0; moved < kept;) {
+    const int q = s + lane;
+    const unsigned m = __ballot_sync(kFullMask, q < nodes && map[q] >= 0);
+    if (m == 0u) {
+      s += 32;
+      continue;
+    }
+    s += __ffs(static_cast<int>(m)) - 1;
+    const int r = moved++;
+    const int64_t gs = mcts_slot(a, t, s), gr = mcts_slot(a, t, r), es = gs * M, er = gr * M;
+    const int L = a.node_legal[gs];
+    const uint32_t visits = a.node_n[gs];
+    if (r == 0) root_visits = visits;
+    if (r != s) warp_copy_record(a.node_rec + gr * rw, a.node_rec + gs * rw, rw, lane);
+    for (int i = lane; i < L; i += 32) {
+      const int c = a.edge_child[es + i];
+      const int mc = c >= 0 ? map[c] : -1;
+      const bool dropped = c >= 0 && mc < 0;  // cut by keep_nodes: unvisited again
+      const uint32_t en = dropped ? 0u : a.edge_n[es + i];
+      const double ew = dropped ? 0.0 : a.edge_w[es + i];
+      if (r != s) {
+        a.edge_action[er + i] = a.edge_action[es + i];
+        if (a.edge_p != nullptr) {
+          a.edge_p[er + i] = a.edge_p[es + i];
+          a.edge_key[er + i] = a.edge_key[es + i];
+        }
+        if (a.edge_out != nullptr) a.edge_out[er + i] = a.edge_out[es + i];
+      }
+      a.edge_n[er + i] = en;
+      a.edge_w[er + i] = ew;
+      a.edge_child[er + i] = c >= 0 ? (mc >= 0 ? mc : -1) : -1;
+      if (a.edge_v != nullptr) a.edge_v[er + i] = 0;
+    }
+    __syncwarp();  // every lane has read slot s before lane 0 writes slot r
+    if (lane == 0) {
+      a.node_legal[gr] = L;
+      a.node_n[gr] = visits;
+      if (a.node_v != nullptr) a.node_v[gr] = 0;
+    }
+    ++s;
+  }
+  if (lane == 0) {
+    entry->x = kept;
+    if (action != -1 && a.root_out != nullptr) a.root_out[t] = mcts_advanced_root_code(code);
+    if (out_status != nullptr) out_status[t] = root_visits > 0u ? kRootKept : kRootFresh;
+  }
+}
+
+// ------------------------------------------------------ set root priors ---
+// P(a) of every root edge of each expanded root from priors [count, n*n]; unexpanded roots are left alone
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_set_root_priors_kernel(MctsArena a, int64_t count,
+                                                                               const float* __restrict__ priors) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int64_t g = mcts_slot(a, t, 0), e0 = g * a.M;
+  const int legal = a.node_legal[g];
+  const float* row = priors + t * a.n * a.n;
+  for (int i = lane; i < legal; i += 32) a.edge_p[e0 + i] = row[a.edge_action[e0 + i]];
+}
+
 unsigned mcts_blocks(int64_t count) { return static_cast<unsigned>((count + kMctsWarps - 1) / kMctsWarps); }
 
 }  // namespace
@@ -782,6 +955,20 @@ cudaError_t launch_mcts_solver_stats(const MctsArena& a, int64_t count, uint8_t*
   if (count <= 0) return cudaSuccess;
   mcts_solver_stats_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_proven, out_returns,
                                                                            out_edge_values, out_simulations);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_advance(const MctsArena& a, int64_t count, const int32_t* actions, int keep_nodes,
+                                int32_t* map, int32_t* out_status, unsigned int* illegal_index, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_advance_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, actions, keep_nodes, map, out_status,
+                                                                      illegal_index);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_set_root_priors(const MctsArena& a, int64_t count, const float* priors, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_set_root_priors_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, priors);
   return cudaGetLastError();
 }
 

@@ -51,6 +51,17 @@
 //   K-leaf bytes per tree = (bytes per tree of the kind above) + (K - 1) * (16 + 8*P + R * (rw*4 + 16))
 //                           + S * 2 * (1 + M)
 // K = 1 is exactly the search above and allocates nothing more.
+//
+// Tree reuse (twixt_mcts_advance(actions, keep_nodes)): the child of the root along actions[t] becomes the new
+// root.  The kept nodes are that child's subtree, renumbered by their rank in old slot order (the new root is slot
+// 0, children stay above their parents), and only the first keep_nodes of that order are kept; an edge whose child
+// the cap drops goes back to N = 0, W = 0, child -1 (prior, tie key and outcome code stay).  Every kept node keeps
+// its record, N(s), legal count and its edges' action, N, W, prior, tie key and outcome code, children remapped.
+// A legal action without a child clears the tree to the root with the move applied; -1 keeps the root and only
+// applies the cap; an illegal action leaves the tree as it is.  A solver search's new root takes code 4 - c from
+// the chosen edge's code c != 0 (the child's value for its own player to move), else 0.  The draw and rollout
+// streams keep counting k: a tree never repeats a Philox counter.  The kernel needs an int32 old -> new slot map of
+// S entries per tree, allocated at the first advance.
 #pragma once
 #include <stdint.h>
 
@@ -64,6 +75,12 @@
 namespace twixt {
 
 enum : int { kLeafNeedsValue = 0, kLeafTerminal = 1, kLeafSolved = 2 };
+// statuses of twixt_mcts_advance: the new root kept its statistics (N(root) > 0), the action was illegal (tree
+// unchanged), the new root has none (N(root) == 0: the next simulation evaluates it)
+enum : int { kRootKept = 0, kRootIllegal = 1, kRootFresh = 2 };
+
+// the solver root code of a tree advanced along an edge with outcome code c (twixt_mcts_advance)
+TW_HD uint8_t mcts_advanced_root_code(uint8_t c) { return c != 0 ? static_cast<uint8_t>(4 - c) : 0; }
 
 struct MctsSizes {
   int64_t slots;      // node slots per tree (max_simulations + 1)

@@ -28,6 +28,12 @@ behaviour, and exactly the search above at K = 1).  All K leaves of every tree a
 plays K*R rollouts per tree in one playout launch, and the stepwise form hands the caller K rows per tree, so a
 search needs max_simulations / K steps instead of max_simulations.  Row t*K + j is descent j of tree t.
 
+`advance(actions, keep_nodes)` reuses the trees across moves (as AlphaGo Zero, Leela Zero and KataGo do; not an
+open_spiel behaviour): the child of each root along the move played becomes the new root with its subtree and all
+its statistics, up to keep_nodes nodes, so the next search starts from the visits the last one already spent there.
+Size the search for it: max_simulations is the node capacity, e.g. 2*sims with keep_nodes = sims + 1 runs sims new
+simulations every move.  `set_root_priors` puts fresh priors (root Dirichlet noise) on the kept roots.
+
 `MCTSBot` is the open_spiel-shaped bot over one tree for adapter `TwixTState`s.
 
 Arrays may be numpy (synchronous) or torch CUDA tensors (asynchronous on the batch's stream), as for
@@ -44,6 +50,7 @@ from . import _lib
 from .batch import TwixTBatch, _dt, _is_torch, _ptr
 
 LEAF_NEEDS_VALUE, LEAF_TERMINAL, LEAF_SOLVED = 0, 1, 2
+ROOT_KEPT, ROOT_ILLEGAL, ROOT_FRESH = 0, 1, 2  # advance(): statistics kept, illegal action, new root unvisited
 UNPROVEN = -128  # solver_stats' edge value of a root move that is not proven
 _PUCT, _SOLVE = 1, 2  # TWIXT_MCTS_PUCT, TWIXT_MCTS_SOLVE
 
@@ -82,7 +89,11 @@ class BatchedMCTS:
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
-            self._lib.twixt_mcts_destroy(self._h)
+            # a search must be destroyed before its batch; when the garbage collector finalises a cycle that holds
+            # both (a failed test's frame, interpreter exit) the batch may go first, and the search's device memory
+            # is then left to the process's exit rather than freed through the batch's released stream
+            if self.batch._h.value:
+                self._lib.twixt_mcts_destroy(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):
@@ -167,6 +178,34 @@ class BatchedMCTS:
             _ptr(out_simulations, _dt(np.int32, "int32"), self.count)))
         return out_proven, out_returns, out_edge_values, out_simulations
 
+    def advance(self, actions, keep_nodes: Optional[int] = None, out_status=None):
+        """Tree reuse: actions [count] int32 (the move played in each tree's root, -1 to keep the root).  The child
+        along the move becomes the new root with its subtree and all its statistics, at most keep_nodes nodes of it
+        (None: max_simulations + 1, all of them); a move whose edge has no child clears the tree to the new
+        position.  Returns the statuses [count] int32: ROOT_KEPT (the new root has visits), ROOT_FRESH (it has
+        none: the next simulation evaluates it) or ROOT_ILLEGAL.  An illegal move leaves its tree unchanged and
+        raises, as `TwixTBatch.apply` does, unless out_status is a torch CUDA tensor (asynchronous: the statuses
+        are the report).  The simulation counter carries on, so the draws never repeat."""
+        if keep_nodes is None:
+            keep_nodes = self.max_simulations + 1
+        if not _is_torch(actions):
+            actions = np.ascontiguousarray(np.reshape(actions, -1), dtype=np.int32)
+        if out_status is None:
+            out_status = np.zeros(self.count, dtype=np.int32)
+        self._check(self._lib.twixt_mcts_advance(self._h, _ptr(actions, _dt(np.int32, "int32"), self.count),
+                                                 int(keep_nodes), _ptr(out_status, _dt(np.int32, "int32"),
+                                                                       self.count)))
+        return out_status
+
+    def set_root_priors(self, priors):
+        """PUCT only: replaces P(a) of every root edge of each tree whose root is expanded with priors [count, n*n]
+        float32 (e.g. root Dirichlet noise after `advance`).  Trees whose root is not expanded are left alone: their
+        first backup takes the priors of row t*K + 0 as after `begin`."""
+        if not _is_torch(priors):
+            priors = np.ascontiguousarray(priors, dtype=np.float32)
+        self._check(self._lib.twixt_mcts_set_root_priors(
+            self._h, _ptr(priors, _dt(np.float32, "float32"), self.count * self._cells)))
+
 
 def add_dirichlet_noise(priors, legal_mask, epsilon: float, alpha: float):
     """open_spiel's root noise: (1 - epsilon) * p + epsilon * Dir(alpha) over each row's legal actions.
@@ -203,10 +242,16 @@ class MCTSBot:
 
     leaves_per_step=K > 1 searches the one tree K leaves at a time with virtual loss (BatchedMCTS above), in
     max_simulations / K steps per move; max_simulations must then be a multiple of K and at least 2*K (step 0
-    only evaluates the root).  The default K = 1 is the bot above."""
+    only evaluates the root).  The default K = 1 is the bot above.
+
+    reuse_tree=True keeps the tree between steps (BatchedMCTS.advance): the search holds 2*max_simulations nodes,
+    and `step(state)` advances through the actions by which state.history() extends the history it last searched
+    (its own move, then the opponent's), keeping max_simulations + 1 nodes, then runs max_simulations new
+    simulations.  A history that does not extend the last one begins a fresh tree."""
 
     def __init__(self, game, uct_c: float = 2.0, max_simulations: int = 1000, n_rollouts: int = 4, seed: int = 0,
-                 device: int = 0, solve: bool = False, leaves_per_step: int = 1, virtual_loss: float = 1.0):
+                 device: int = 0, solve: bool = False, leaves_per_step: int = 1, virtual_loss: float = 1.0,
+                 reuse_tree: bool = False):
         if max_simulations < 2:
             raise ValueError("MCTSBot needs max_simulations >= 2: the first simulation only evaluates the root")
         if leaves_per_step > 1 and (max_simulations % leaves_per_step or max_simulations < 2 * leaves_per_step):
@@ -215,15 +260,25 @@ class MCTSBot:
         self._game = game
         self._batch = TwixTBatch(game.board_size(), 1, device, seed)
         self._batch.set_validation(False)  # records come from the adapter's own exports
-        self._mcts = BatchedMCTS(self._batch, 1, max_simulations, n_rollouts, uct_c, solve=solve,
+        capacity = (2 if reuse_tree else 1) * int(max_simulations)
+        self._mcts = BatchedMCTS(self._batch, 1, capacity, n_rollouts, uct_c, solve=solve,
                                  leaves_per_step=leaves_per_step, virtual_loss=virtual_loss)
         self.max_simulations = int(max_simulations)
+        self.reuse_tree = bool(reuse_tree)
+        self._searched = None  # the history of the state the tree's root holds (reuse_tree)
 
     def step(self, state) -> int:
         if state.is_terminal():
             raise ValueError("MCTSBot.step on a terminal state")
-        self._batch.import_state(state.export_record(), 0)
-        self._mcts.begin(0, 1)
+        history = list(state.history())
+        last = self._searched
+        if self.reuse_tree and last is not None and history[:len(last)] == last:
+            for a in history[len(last):] or [-1]:
+                self._mcts.advance([a], self.max_simulations + 1)
+        else:
+            self._batch.import_state(state.export_record(), 0)
+            self._mcts.begin(0, 1)
+        self._searched = history
         self._mcts.run(self.max_simulations)
         return int(self._mcts.best()[0])
 
