@@ -26,7 +26,14 @@ root Dirichlet noise then reaches a kept root through `set_root_priors`; a root 
 statistics (ROOT_FRESH) is expanded by the first backup as after `begin`, so the noise goes into its row g*K + 0
 there, masked on the device.
 
-    python examples/alphazero_selfplay.py [board_size] [games] [simulations] [leaves_per_step] [reuse_tree]
+search="gumbel" plays Gumbel AlphaZero instead (BatchedMCTS(selection="gumbel"); Danihelka et al., ICLR 2022),
+the search for small simulation budgets: each move `begin`s the trees, sets fresh root Gumbel noise with
+`set_root_gumbel(gumbel_noise(...))`, and hands the net's logits (not a softmax) to every backup.  There is no
+Dirichlet noise and no temperature: the move played is `gumbel_stats`' action (Sequential Halving over
+max_considered root moves), and the policy target is its improved policy softmax(logits + sigma(completed Q)).  It
+runs one leaf per step and without tree reuse.
+
+    python examples/alphazero_selfplay.py [board_size] [games] [simulations] [leaves_per_step] [reuse_tree] [search]
 """
 import os
 import sys
@@ -36,7 +43,7 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from twixt_for_open_spiel_b200 import TwixTBatch  # noqa: E402
-from twixt_for_open_spiel_b200.mcts import ROOT_FRESH, BatchedMCTS, add_dirichlet_noise  # noqa: E402
+from twixt_for_open_spiel_b200.mcts import ROOT_FRESH, BatchedMCTS, add_dirichlet_noise, gumbel_noise  # noqa: E402
 from twixt_for_open_spiel_b200.producer import ObservationMaskProducer  # noqa: E402
 
 
@@ -62,11 +69,18 @@ def masked_softmax(logits, legal):
 
 def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_c=2.0, dirichlet_epsilon=0.25,
               dirichlet_alpha=1.0, seed=0, net=None, verbose=True, leaves_per_step=1, virtual_loss=1.0,
-              reuse_tree=False):
+              reuse_tree=False, search="puct", max_considered=16):
     """Plays `games` games to the end.  Returns (trajectories, returns [games, 2]); trajectories[g] is a list of
     per-move dicts with obs [12, n, n-2], mask [n*n], policy [n*n], player and action.  sims must be a multiple
-    of leaves_per_step.  reuse_tree=True keeps the played move's subtree between moves (see the module text)."""
+    of leaves_per_step.  reuse_tree=True keeps the played move's subtree between moves (see the module text).
+    search="gumbel" plays Gumbel AlphaZero with max_considered root moves (temperature, the Dirichlet noise,
+    leaves_per_step and reuse_tree do not apply to it)."""
     K = int(leaves_per_step)
+    if search not in ("puct", "gumbel"):
+        raise ValueError("search must be 'puct' or 'gumbel', got %r" % (search,))
+    gumbel = search == "gumbel"
+    if gumbel and (K != 1 or reuse_tree):
+        raise ValueError("search='gumbel' runs one leaf per step and without tree reuse")
     if sims % K:
         raise ValueError("sims = %d is not a multiple of leaves_per_step = %d" % (sims, K))
     torch.manual_seed(seed)
@@ -78,8 +92,11 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
     if net is None:
         net = PolicyValueNet(n).to(dev).eval()
     capacity = 2 * sims if reuse_tree else sims
-    search = BatchedMCTS(batch, games, capacity, uct_c=uct_c, selection="puct", leaves_per_step=K,
-                         virtual_loss=virtual_loss)
+    if gumbel:
+        search = BatchedMCTS(batch, games, sims, selection="gumbel", max_considered=max_considered)
+    else:
+        search = BatchedMCTS(batch, games, capacity, uct_c=uct_c, selection="puct", leaves_per_step=K,
+                             virtual_loss=virtual_loss)
     fresh = torch.ones(games, dtype=torch.bool, device=dev)  # roots without statistics (all of them at begin)
     status = torch.zeros(games, dtype=torch.int32, device=dev)
     player = torch.zeros(rows, dtype=torch.int8, device=dev)
@@ -87,6 +104,7 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
     done = torch.zeros(games, dtype=torch.uint8, device=dev)
     visits = torch.zeros((games, n * n), dtype=torch.int32, device=dev)
     best = torch.zeros(games, dtype=torch.int32, device=dev)
+    improved = torch.zeros((games, n * n), dtype=torch.float32, device=dev)  # search="gumbel"'s policy target
     history = []  # per move: (obs, mask, policy, player, action, live) on the device
     move = 0
     with torch.no_grad():
@@ -101,7 +119,10 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
             root_obs, root_mask = producer.produce(0, games)
             root_obs, root_mask = root_obs.clone(), root_mask.clone()
             batch.current_player(0, games, out=root_player)
-            if not reuse_tree:
+            if gumbel:
+                search.begin(0, games)
+                search.set_root_gumbel(gumbel_noise(games, n * n, device=dev))
+            elif not reuse_tree:
                 search.begin(0, games)
             elif move == 0:
                 search.begin(0, games)
@@ -115,6 +136,12 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
                 obs, mask = producer.produce(games, rows)
                 legal = mask.bool()
                 logits, v = net(obs)
+                batch.current_player(games, rows, out=player)
+                v = torch.where(player == 1, -v, v).float()
+                values = torch.stack([v, -v], dim=1).contiguous()
+                if gumbel:  # the logits themselves; illegal entries are ignored
+                    search.backup(values, logits.float().contiguous())
+                    continue
                 priors = masked_softmax(logits, legal)
                 if k == 0:
                     if K == 1 and not reuse_tree:
@@ -122,17 +149,19 @@ def self_play(n=8, games=64, sims=50, temperature=1.0, temperature_drop=10, uct_
                     else:  # the root rows g*K + 0, and with reuse_tree only where the root is fresh
                         noisy = add_dirichlet_noise(priors[::K], legal[::K], dirichlet_epsilon, dirichlet_alpha)
                         priors[::K] = torch.where(fresh[:, None], noisy, priors[::K])
-                batch.current_player(games, rows, out=player)
-                v = torch.where(player == 1, -v, v).float()
-                search.backup(torch.stack([v, -v], dim=1).contiguous(), priors.contiguous())
-            search.root_stats(out_visits=visits, out_best=best)
-            policy = visits.double() ** (1.0 / temperature)
-            policy = (policy / policy.sum(1, keepdim=True).clamp_min(1e-300)).float()
-            if move < temperature_drop:
-                sampled = torch.multinomial(torch.where(live[:, None], policy, torch.ones_like(policy)), 1)
-                action = sampled.squeeze(1).int()
+                search.backup(values, priors.contiguous())
+            if gumbel:
+                search.gumbel_stats(out_action=best, out_policy=improved)
+                policy, action = improved.clone(), best.clone()
             else:
-                action = best.clone()
+                search.root_stats(out_visits=visits, out_best=best)
+                policy = visits.double() ** (1.0 / temperature)
+                policy = (policy / policy.sum(1, keepdim=True).clamp_min(1e-300)).float()
+                if move < temperature_drop:
+                    sampled = torch.multinomial(torch.where(live[:, None], policy, torch.ones_like(policy)), 1)
+                    action = sampled.squeeze(1).int()
+                else:
+                    action = best.clone()
             action = torch.where(live, action, torch.full_like(action, -1)).contiguous()
             history.append((root_obs, root_mask, policy, root_player.clone(), action, live))
             batch.apply(action, 0)
@@ -158,7 +187,8 @@ def main():
     sims = int(sys.argv[3]) if len(sys.argv) > 3 else 100
     leaves = int(sys.argv[4]) if len(sys.argv) > 4 else 1
     reuse = len(sys.argv) > 5 and sys.argv[5] not in ("0", "false", "False")
-    trajectories, returns = self_play(n, games, sims, leaves_per_step=leaves, reuse_tree=reuse)
+    search = sys.argv[6] if len(sys.argv) > 6 else "puct"
+    trajectories, returns = self_play(n, games, sims, leaves_per_step=leaves, reuse_tree=reuse, search=search)
     lengths = [len(t) for t in trajectories]
     print("%d games at n = %d, %d simulations per move: mean length %.1f, red wins %d, blue wins %d, draws %d" % (
         games, n, sims, float(np.mean(lengths)), int((returns[:, 0] > 0).sum()), int((returns[:, 1] > 0).sum()),

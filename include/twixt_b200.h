@@ -431,6 +431,46 @@ int twixt_mcts_create_parallel(twixt_batch* b, int64_t num_trees, int32_t max_si
 int twixt_mcts_advance(twixt_mcts* m, const int32_t* actions, int32_t keep_nodes, int32_t* out_status);
 int twixt_mcts_set_root_priors(twixt_mcts* m, const float* priors);
 
+/* Gumbel AlphaZero search (Danihelka, Guez, Schrittwieser, Silver, "Policy improvement by planning with Gumbel",
+ * ICLR 2022; mctx gumbel_muzero_policy with qtransform_completed_by_mix_value's defaults), in reproducible IEEE
+ * double instead of float32.  The tree is the PUCT one: one node per simulation in creation order, edges the legal
+ * actions ascending, a leaf at a terminal node or a node with N(s) == 0, expanded at its backup, and the backup adds
+ * v[player to move at the parent] to W(a) along the path.  What differs:
+ *  - every edge carries a float32 logit l(a): the backup's [count, n*n] array (the priors of twixt_mcts_backup_priors
+ *    are read as logits), or 0 for every edge without one (twixt_mcts_run, twixt_mcts_backup, a NULL pointer).
+ *    Entries of illegal actions are ignored; host logits must be finite on the legal actions of every non-terminal
+ *    leaf (checked on the host against the leaf envs select wrote; TWIXT_EINVAL, trees unchanged).
+ *  - every node keeps its raw value v(s): its evaluation for its own player to move (the caller's value, the
+ *    rollout mean, or Returns() of a terminal leaf).
+ *  - the completed Q at a node s: pi = softmax(l) raised to the smallest normal double, q(a) = W(a)/N(a) on visited
+ *    edges, SN = sum N(a), v_mix = (v(s) + SN * sum_{N>0} (pi*q / sum_{N>0} pi)) / (SN + 1), q~ = q on visited
+ *    edges and v_mix elsewhere, q^ = (q~ - min q~) / max(max q~ - min q~, 1e-8), sigma = ((c_visit + max N) *
+ *    c_scale) * q^.
+ *  - interior nodes take argmax of softmax(l + sigma)(a) - N(a) / (1 + SN), ties to the lower edge.
+ *  - the root takes Sequential Halving: m = min(max_considered, L), i = SN (= N(root) - 1); the eligible edges have
+ *    N(a) = table[m][i] with table = mctx's get_table_of_considered_visits(max_considered, max_simulations - 1);
+ *    among them argmax of max(-1e9, (g(a) + (l(a) - max l)) + sigma(a)), ties to the lower edge.
+ *  - g is the root's Gumbel noise per action cell, zeroed by begin (mctx's gumbel_scale = 0) and set by
+ *    twixt_mcts_set_root_gumbel(m, gumbel [count, n*n] float32, host or device; host values must be finite).
+ *  - every exp and every sum over a node's edges is fixed bit for bit (twixt_mcts.cuh: mcts_exp, mcts_lane_sums).
+ * twixt_mcts_create_gumbel: max_considered >= 1 (above n(n-2) it acts as n(n-2)), c_visit (mctx maxvisit_init, 50)
+ * and c_scale (mctx value_scale, 0.1) finite and >= 0, else TWIXT_EINVAL.  A Gumbel search has no solver and one
+ * leaf per step, and twixt_mcts_advance and twixt_mcts_set_root_priors on it are TWIXT_EINVAL (Sequential Halving
+ * assumes a fresh root).  begin, run, select, backup and backup_priors work as above with the same launch counts.
+ * twixt_mcts_root_stats returns visits and value sums as for every kind, and out_best is the Gumbel action (one
+ * more launch).
+ * twixt_mcts_gumbel_stats: out_action [count] int32, the root score above among the edges with N(a) = max N (-1 for
+ * a terminal or unexpanded root), and out_policy [count, n*n] float32, the improved policy softmax(l + sigma) at the
+ * root's action cells, 0 elsewhere (all 0 for a terminal or unexpanded root; mctx's action_weights).  Each pointer
+ * is nullable, host or device; one launch; TWIXT_EINVAL on another kind, before begin or while a select is pending.
+ * Arena per tree: S*(rw*4 + 16 + 22*M) + 16 + 8*P + R*(rw*4 + 16) + 4*n*n bytes (a logit per edge, v per node,
+ * the root noise), plus (min(max_considered, M) + 1) * (max_simulations - 1) int32 of table per search; TWIXT_ENOMEM
+ * names it. */
+int twixt_mcts_create_gumbel(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                             int32_t max_considered, double c_visit, double c_scale, twixt_mcts** out);
+int twixt_mcts_set_root_gumbel(twixt_mcts* m, const float* gumbel);
+int twixt_mcts_gumbel_stats(twixt_mcts* m, int32_t* out_action, float* out_policy);
+
 /* Multi-GPU plumbing for hosts that are not Python (SURVEY 8e: envs shard by contiguous global id ranges,
  * no data-path collective, one reduction of the counters).  twixt_shard_range: rank's share [first,
  * first+count) of global_envs envs over `world` ranks (shares differ by at most one env); create the rank's

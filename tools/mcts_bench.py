@@ -40,6 +40,12 @@ with simulations/s and the select / backup kernel ms per step, next to the UCT c
   the mean N(root) at the start of each move's search (sum of the root's N(a) + 1 for an expanded root).
   Both use seeded uniform random priors raised to the 8th power, so that a few moves carry most of a node's prior
   as with a trained policy (flat priors spread the visits over all moves and leave little to keep), and zero values.
+
+`gumbel`: the stepwise Gumbel AlphaZero search (selection="gumbel", max_considered = 16, select -> backup(values,
+logits)) with fixed device-resident logits (seeded standard normal), zero values and fresh root Gumbel noise per
+search, and next to each entry the stepwise PUCT search above at the same size, in the same process:
+  n = 12: 8192 trees x 16, 64 and 400 simulations;  n = 24: 1024 trees x 200
+with simulations/s and the select / backup kernel ms per step.  `--gumbel-only` runs just these entries.
 """
 from __future__ import annotations
 
@@ -153,54 +159,67 @@ def bench_config(n: int, trees: int, sims: int, R: int, profile_sims: int, solve
     return out
 
 
-def bench_puct(n: int, trees: int, sims: int, profile_sims: int, leaves_per_step: int = 1) -> dict:
+def bench_puct(n: int, trees: int, sims: int, profile_sims: int, leaves_per_step: int = 1,
+               selection: str = "puct") -> dict:
     import torch
     from torch.profiler import ProfilerActivity, profile
 
-    from twixt_for_open_spiel_b200.mcts import BatchedMCTS
+    from twixt_for_open_spiel_b200.mcts import BatchedMCTS, gumbel_noise
     K = leaves_per_step
     rows = trees * K
+    gumbel = selection == "gumbel"
     b = make_roots(n, trees + rows, 0x70756374)  # envs [trees, trees + trees*K) take the leaves
-    m = BatchedMCTS(b, trees, sims, selection="puct", leaves_per_step=K)
+    m = BatchedMCTS(b, trees, sims, selection=selection, leaves_per_step=K)
     gen = torch.Generator(device="cuda").manual_seed(1)
-    priors = torch.rand((rows, n * n), generator=gen, device="cuda", dtype=torch.float32)
+    if gumbel:  # logits
+        priors = torch.randn((rows, n * n), generator=gen, device="cuda", dtype=torch.float32)
+    else:
+        priors = torch.rand((rows, n * n), generator=gen, device="cuda", dtype=torch.float32)
     values = torch.zeros((rows, 2), device="cuda", dtype=torch.float32)
     status = torch.zeros(rows, dtype=torch.int32, device="cuda")
+
+    def begin():
+        m.begin(0, trees)
+        if gumbel:
+            m.set_root_gumbel(gumbel_noise(trees, n * n, generator=gen, device="cuda"))
 
     def search(k):  # k simulations of every tree: k / K steps
         for _ in range(k // K):
             m.select(trees, status)
             m.backup(values, priors)
 
-    m.begin(0, trees)
+    begin()
     search(max(K, min(sims, 20) // K * K))
     b.synchronize()
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    m.begin(0, trees)
+    begin()
     start.record()
     search(sims)
     stop.record()
     stop.synchronize()
     ms = start.elapsed_time(stop)
-    m.begin(0, trees)
+    begin()
     b.synchronize()
+    profile_sims = min(profile_sims, sims)
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         search(profile_sims)
         b.synchronize()
     split = {"select": 0.0, "backup": 0.0}
+    names = ("mcts_gumbel_select_kernel", "mcts_gumbel_backup_kernel") if gumbel else ("mcts_select_kernel",
+                                                                                      "mcts_backup_kernel")
     for ev in prof.key_averages():
         t = getattr(ev, "device_time_total", None)
         if t is None:
             t = ev.cuda_time_total
-        if "mcts_select_kernel" in ev.key:
+        if names[0] in ev.key:
             split["select"] += t
-        elif "mcts_backup_kernel" in ev.key:
+        elif names[1] in ev.key:
             split["backup"] += t
     best = m.best()
     m.close()
     b.close()
     out = {
-        "board_size": n, "trees": trees, "simulations": sims,
+        "selection": selection, "board_size": n, "trees": trees, "simulations": sims,
         "search_ms": round(ms, 3),
         "simulations_per_s": round(trees * sims / (ms / 1e3), 1),
         "ms_per_simulation_step": round(ms / (sims // K), 4),
@@ -354,6 +373,7 @@ def main() -> None:
     ap.add_argument("--no-solve", action="store_true", help="skip the solver entries")
     ap.add_argument("--no-parallel", action="store_true", help="skip the leaves_per_step entries")
     ap.add_argument("--no-reuse", action="store_true", help="skip the tree reuse entries")
+    ap.add_argument("--gumbel-only", action="store_true", help="only the gumbel entries and their puct pairs")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -368,6 +388,7 @@ def main() -> None:
         many = [(12, 16, 48, 4, 16, K) for K in (1, 8)]
         adv = (12, 256, 40, 2)
         moves = (12, 64, 20, 4)
+        gumbel = [(12, 256, 16, 16), (12, 256, 64, 20), (24, 64, 20, 10)]
     else:
         configs = [(12, 8192, 400, 4, 50), (24, 1024, 200, 4, 50)]
         puct = [(12, 8192, 400, 50), (24, 1024, 200, 50)]
@@ -377,7 +398,12 @@ def main() -> None:
         many = [(12, 64, 400, 4, 80, K) for K in (1, 8)]
         adv = (12, 8192, 400, 3)
         moves = (12, 1024, 100, 12)
+        gumbel = [(12, 8192, 16, 16), (12, 8192, 64, 50), (12, 8192, 400, 50), (24, 1024, 200, 50)]
     out = dict(info)
+    if args.gumbel_only:
+        out["gumbel"] = [[bench_puct(*c, selection=k) for k in ("gumbel", "puct")] for c in gumbel]
+        print(json.dumps(out))
+        return
     out["configs"] = [bench_config(*c) for c in configs]
     out["evaluate_slots"] = bench_evaluator(*ev)
     out["puct"] = [bench_puct(*c) for c in puct]
@@ -392,6 +418,7 @@ def main() -> None:
     if not args.no_reuse:
         out["reuse"] = {"advance": bench_advance(*adv),
                         "moves": [bench_moves(*moves, reuse=r) for r in (False, True)]}
+    out["gumbel"] = [[bench_puct(*c, selection=k) for k in ("gumbel", "puct")] for c in gumbel]
     print(json.dumps(out))
 
 

@@ -106,6 +106,10 @@ SYMBOLS = [
                                              C.c_double, C.POINTER(_P)]),
     ("twixt_mcts_advance", C.c_int, [_P, _P, C.c_int32, _P]),
     ("twixt_mcts_set_root_priors", C.c_int, [_P, _P]),
+    ("twixt_mcts_create_gumbel", C.c_int, [_P, _I64, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
+                                           C.POINTER(_P)]),
+    ("twixt_mcts_set_root_gumbel", C.c_int, [_P, _P]),
+    ("twixt_mcts_gumbel_stats", C.c_int, [_P, _P, _P]),
 ]
 
 OK, EINVAL, ECUDA, EILLEGAL, ENOMEM = 0, -1, -2, -3, -4

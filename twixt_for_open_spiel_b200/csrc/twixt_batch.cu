@@ -677,9 +677,12 @@ class TwixTMCTS {
     if (map_ != nullptr) cudaFree(map_);
   }
 
-  // leaves_per_step K > 1: K descents per step with virtual loss vl (checked by the caller, twixt_mcts_create_parallel)
+  // leaves_per_step K > 1: K descents per step with virtual loss vl (checked by the caller, twixt_mcts_create_parallel).
+  // gumbel: a Gumbel AlphaZero search (puct, solve and K > 1 excluded by the caller, twixt_mcts_create_gumbel) with
+  // max_considered >= 1 and c_visit, c_scale finite and >= 0.
   int Init(TwixTBatch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts, double uct_c, bool puct,
-           bool solve, int32_t leaves_per_step, double virtual_loss) {
+           bool solve, int32_t leaves_per_step, double virtual_loss, bool gumbel = false, int32_t max_considered = 0,
+           double c_visit = 0.0, double c_scale = 0.0) {
     if (num_trees <= 0) return fail(TWIXT_EINVAL, "num_trees must be positive: %lld", static_cast<long long>(num_trees));
     if (max_simulations <= 0) return fail(TWIXT_EINVAL, "max_simulations must be positive: %d", max_simulations);
     if (n_rollouts <= 0) return fail(TWIXT_EINVAL, "n_rollouts must be positive: %d", n_rollouts);
@@ -694,26 +697,43 @@ class TwixTMCTS {
     const int n = b->n_;
     const int K = leaves_per_step;
     const MctsSizes s = mcts_sizes(n, max_simulations, n_rollouts);
-    const int64_t per_tree = mcts_parallel_bytes_per_tree(
-        s, solve ? mcts_solve_bytes_per_tree(s, puct) : (puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s)),
-        K);
+    const int64_t cells = static_cast<int64_t>(n) * n;
+    const int64_t per_tree =
+        gumbel ? mcts_gumbel_bytes_per_tree(s, cells)
+               : mcts_parallel_bytes_per_tree(s, solve ? mcts_solve_bytes_per_tree(s, puct)
+                                                       : (puct ? mcts_puct_bytes_per_tree(s) : mcts_bytes_per_tree(s)),
+                                              K);
+    // Gumbel: the considered-visits table, rows m = 0 .. min(max_considered, M), max_simulations - 1 columns
+    const int mc = gumbel ? static_cast<int>(max_considered < s.edges ? max_considered : s.edges) : 0;
+    const int cols = gumbel ? max_simulations - 1 : 0;
+    std::vector<int32_t> considered(gumbel ? static_cast<size_t>(mc + 1) * cols : 0);
+    for (int m = 0; gumbel && m <= mc; ++m) mcts_considered_visits(m, cols, considered.data() + static_cast<size_t>(m) * cols);
     // carve one allocation; each array starts on a 256-byte boundary (priors and tie keys are PUCT's, the outcome
     // bytes PUCT's and the solver's, the root codes the solver's, the virtual counts those of K > 1: empty
     // otherwise).  Tree entries, paths and rollout slots are per leaf row: K per tree.
     const int64_t T = num_trees, nodes = T * s.slots, edges = nodes * s.edges, rows = T * K, rolls = rows * s.rollouts;
     const int64_t pe = puct ? edges : 0, oe = (puct || solve) ? edges : 0, rt = solve ? T : 0;
     const int64_t vn = K > 1 ? nodes : 0, ve = K > 1 ? edges : 0;
-    const int64_t sizes[19] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
+    const int64_t ge = gumbel ? edges : 0, gn = gumbel ? nodes : 0, gt = gumbel ? T * cells : 0;
+    const int64_t sizes[23] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
                                rows * 16, rows * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8,
-                               pe * 4, pe * 4, oe, rt, vn * 2, ve * 2};
-    int64_t offs[19], total = 0;
-    for (int i = 0; i < 19; ++i) {
+                               pe * 4, pe * 4, oe, rt, vn * 2, ve * 2,
+                               ge * 4, gn * 8, gt * 4, static_cast<int64_t>(considered.size()) * 4};
+    int64_t offs[23], total = 0;
+    for (int i = 0; i < 23; ++i) {
       offs[i] = total;
       total += (sizes[i] + 255) & ~static_cast<int64_t>(255);
     }
     DeviceGuard g(b->device_);
     size_t free_bytes = 0, total_bytes = 0;
     TW_CUDA(cudaMemGetInfo(&free_bytes, &total_bytes));
+    if (gumbel && static_cast<uint64_t>(total) > free_bytes)
+      return fail(TWIXT_ENOMEM,
+                  "Gumbel MCTS arena of %lld bytes (%lld trees x %lld bytes per tree = S*(rw*4 + 16 + 22*M) + 16 + 8*P "
+                  "+ R*(rw*4 + 16) + 4*n*n at n = %d, %d simulations, %d rollouts; plus a %lld-byte considered-visits "
+                  "table) exceeds the %zu bytes free on device %d",
+                  static_cast<long long>(total), static_cast<long long>(T), static_cast<long long>(per_tree), n,
+                  max_simulations, n_rollouts, static_cast<long long>(considered.size() * 4), free_bytes, b->device_);
     if (static_cast<uint64_t>(total) > free_bytes)
       return fail(TWIXT_ENOMEM,
                   "MCTS arena of %lld bytes (%lld trees x %lld bytes per tree at n = %d, %d simulations, %d rollouts, "
@@ -757,6 +777,20 @@ class TwixTMCTS {
     a_.K = K;
     a_.vl = virtual_loss;
     K_ = K;
+    gumbel_ = gumbel;
+    if (gumbel) {
+      gm_.edge_logit = reinterpret_cast<float*>(base + offs[19]);
+      gm_.node_value = reinterpret_cast<double*>(base + offs[20]);
+      gm_.root_gumbel = reinterpret_cast<float*>(base + offs[21]);
+      gm_.table = reinterpret_cast<const int32_t*>(base + offs[22]);
+      gm_.max_considered = mc;
+      gm_.cols = cols;
+      gm_.c_visit = c_visit;
+      gm_.c_scale = c_scale;
+      if (!considered.empty())
+        TW_CUDA(cudaMemcpyAsync(base + offs[22], considered.data(), considered.size() * sizeof(int32_t),
+                                cudaMemcpyHostToDevice, b->stream_));
+    }
     log_size_ = s.slots;
     // ln N(s) from the host's libm, so that a CPU restatement of the search computes the same scores
     std::vector<double> logs(static_cast<size_t>(s.slots));
@@ -779,6 +813,9 @@ class TwixTMCTS {
     DeviceGuard g(b_->device_);
     TW_CUDA(launch_mcts_begin(a_, b_->rec(root_first), count, b_->stream_));
     b_->launches_ += count > 0;
+    if (gumbel_ && count > 0)  // g = 0 until twixt_mcts_set_root_gumbel
+      TW_CUDA(cudaMemsetAsync(gm_.root_gumbel, 0, static_cast<size_t>(count) * a_.n * a_.n * sizeof(float),
+                              b_->stream_));
     count_ = count;
     key_ = b_->seed_;
     stream0_ = static_cast<uint32_t>(base + static_cast<uint64_t>(root_first));
@@ -815,10 +852,12 @@ class TwixTMCTS {
     p.tickets = &b.d_stats_->tickets;
     for (int32_t i = 0; i < num_simulations; i += K_) {  // one step: K simulations of every tree
       const uint32_t k = static_cast<uint32_t>(sims_);
-      TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, k, c_, nullptr, nullptr, b.stream_));
+      if (gumbel_) TW_CUDA(launch_mcts_gumbel_select(a_, gm_, count_, stream0_, k, nullptr, nullptr, b.stream_));
+      else TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, k, c_, nullptr, nullptr, b.stream_));
       TW_CUDA(cudaMemsetAsync(&b.d_stats_->tickets, 0, sizeof(unsigned long long), b.stream_));
       TW_CUDA(launch_playout(p, b.stream_));
-      TW_CUDA(launch_mcts_backup(a_, count_, nullptr, nullptr, key_, stream0_, b.stream_));
+      if (gumbel_) TW_CUDA(launch_mcts_gumbel_backup(a_, gm_, count_, nullptr, nullptr, b.stream_));
+      else TW_CUDA(launch_mcts_backup(a_, count_, nullptr, nullptr, key_, stream0_, b.stream_));
       b.launches_ += 3;
       sims_ += K_;
       node_bound_ += K_;
@@ -840,10 +879,15 @@ class TwixTMCTS {
     b.ScratchReset();
     Staged st;
     TW_TRY(b.StageOut(out_leaf_status, static_cast<size_t>(count_ * K_) * sizeof(int32_t), &st, false));
-    TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, static_cast<uint32_t>(sims_), c_, b.rec(leaf_first),
-                               static_cast<int32_t*>(st.dev), b.stream_));
+    if (gumbel_)
+      TW_CUDA(launch_mcts_gumbel_select(a_, gm_, count_, stream0_, static_cast<uint32_t>(sims_), b.rec(leaf_first),
+                                        static_cast<int32_t*>(st.dev), b.stream_));
+    else
+      TW_CUDA(launch_mcts_select(a_, count_, key_, stream0_, static_cast<uint32_t>(sims_), c_, b.rec(leaf_first),
+                                 static_cast<int32_t*>(st.dev), b.stream_));
     b.launches_ += 1;
     pending_ = true;
+    leaf_first_ = leaf_first;
     node_bound_ += K_;
     TW_TRY(b.Finish(&st));
     if (st.host) TW_TRY(b.Sync());
@@ -856,10 +900,12 @@ class TwixTMCTS {
     if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_backup: no search begun");
     if (!pending_) return fail(TWIXT_EINVAL, "twixt_mcts_backup without a pending twixt_mcts_select");
     if (values == nullptr && count_ > 0) return fail(TWIXT_EINVAL, "null values pointer");
-    if (priors != nullptr && a_.edge_p == nullptr)
+    if (priors != nullptr && a_.edge_p == nullptr && !gumbel_)
       return fail(TWIXT_EINVAL, "twixt_mcts_backup_priors: priors given to a UCT search (use twixt_mcts_create_puct)");
     const size_t cells = static_cast<size_t>(a_.n) * a_.n;
-    if (priors != nullptr && count_ > 0 && !is_device_pointer(priors)) {
+    if (gumbel_ && priors != nullptr && count_ > 0 && !is_device_pointer(priors)) {
+      TW_TRY(CheckHostLogits(priors));
+    } else if (priors != nullptr && count_ > 0 && !is_device_pointer(priors)) {
       const size_t total = static_cast<size_t>(count_ * K_) * cells;
       for (size_t i = 0; i < total; ++i)
         if (!std::isfinite(priors[i]) || priors[i] < 0.0f)
@@ -875,8 +921,12 @@ class TwixTMCTS {
       const size_t rows = static_cast<size_t>(count_ * K_);
       TW_TRY(b.StageIn(values, rows * 2 * sizeof(float), &in));
       TW_TRY(b.StageIn(priors, priors != nullptr ? rows * cells * sizeof(float) : 0, &pin));
-      TW_CUDA(launch_mcts_backup(a_, count_, static_cast<const float*>(in.dev), static_cast<const float*>(pin.dev),
-                                 key_, stream0_, b.stream_));
+      if (gumbel_)
+        TW_CUDA(launch_mcts_gumbel_backup(a_, gm_, count_, static_cast<const float*>(in.dev),
+                                          static_cast<const float*>(pin.dev), b.stream_));
+      else
+        TW_CUDA(launch_mcts_backup(a_, count_, static_cast<const float*>(in.dev), static_cast<const float*>(pin.dev),
+                                   key_, stream0_, b.stream_));
       b.launches_ += 1;
       if (in.host || pin.host) TW_TRY(b.Sync());  // the staged copies are reused by the next call
     }
@@ -896,9 +946,21 @@ class TwixTMCTS {
     TW_TRY(b.StageOut(out_visits, static_cast<size_t>(count_) * cells * sizeof(int32_t), &v, false));
     TW_TRY(b.StageOut(out_value_sums, static_cast<size_t>(count_) * cells * sizeof(double), &w, false));
     TW_TRY(b.StageOut(out_best, static_cast<size_t>(count_) * sizeof(int32_t), &best, false));
-    TW_CUDA(launch_mcts_root_stats(a_, count_, static_cast<int32_t*>(v.dev), static_cast<double*>(w.dev),
-                                   static_cast<int32_t*>(best.dev), b.stream_));
-    b.launches_ += 1;
+    if (gumbel_) {  // visits and value sums as for every kind; the best action is the Gumbel action
+      if (v.dev != nullptr || w.dev != nullptr) {
+        TW_CUDA(launch_mcts_root_stats(a_, count_, static_cast<int32_t*>(v.dev), static_cast<double*>(w.dev), nullptr,
+                                       b.stream_));
+        b.launches_ += 1;
+      }
+      if (best.dev != nullptr) {
+        TW_CUDA(launch_mcts_gumbel_stats(a_, gm_, count_, static_cast<int32_t*>(best.dev), nullptr, b.stream_));
+        b.launches_ += 1;
+      }
+    } else {
+      TW_CUDA(launch_mcts_root_stats(a_, count_, static_cast<int32_t*>(v.dev), static_cast<double*>(w.dev),
+                                     static_cast<int32_t*>(best.dev), b.stream_));
+      b.launches_ += 1;
+    }
     TW_TRY(b.Finish(&v));
     TW_TRY(b.Finish(&w));
     TW_TRY(b.Finish(&best));
@@ -937,6 +999,9 @@ class TwixTMCTS {
   // Illegal actions are reported as twixt_apply reports them: TWIXT_EILLEGAL naming the first one, except with
   // device statuses, where the call returns at once and the caller reads the statuses.
   int Advance(const int32_t* actions, int32_t keep_nodes, int32_t* out_status) {
+    if (gumbel_)
+      return fail(TWIXT_EINVAL, "twixt_mcts_advance: a Gumbel search does not reuse trees (Sequential Halving needs a "
+                                "fresh root); begin it again");
     if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_advance: no search begun");
     if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_advance while a twixt_mcts_select awaits its backup");
     if (keep_nodes < 1 || keep_nodes > a_.S)
@@ -1000,6 +1065,9 @@ class TwixTMCTS {
 
   // PUCT searches: P(a) of every root edge of the trees whose root is expanded, from priors [count, n*n]
   int SetRootPriors(const float* priors) {
+    if (gumbel_)
+      return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors: a Gumbel search takes its root logits at its first backup "
+                                "and its root noise from twixt_mcts_set_root_gumbel");
     if (a_.edge_p == nullptr)
       return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors: the search is not a PUCT search");
     if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors: no search begun");
@@ -1027,10 +1095,87 @@ class TwixTMCTS {
     return TWIXT_OK;
   }
 
+  // Gumbel searches: the root noise g [count, n*n] float32 (host or device; host values must be finite)
+  int SetRootGumbel(const float* gumbel) {
+    if (!gumbel_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_gumbel: the search is not a Gumbel search");
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_gumbel: no search begun");
+    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_gumbel while a twixt_mcts_select awaits its backup");
+    if (count_ == 0) return TWIXT_OK;
+    if (gumbel == nullptr) return fail(TWIXT_EINVAL, "null gumbel pointer");
+    const size_t cells = static_cast<size_t>(a_.n) * a_.n, total = static_cast<size_t>(count_) * cells;
+    if (!is_device_pointer(gumbel))
+      for (size_t i = 0; i < total; ++i)
+        if (!std::isfinite(gumbel[i]))
+          return fail(TWIXT_EINVAL, "gumbel [%lld, %lld] = %g: the root noise must be finite",
+                      static_cast<long long>(i / cells), static_cast<long long>(i % cells),
+                      static_cast<double>(gumbel[i]));
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    b.ScratchReset();
+    Staged in;
+    TW_TRY(b.StageIn(gumbel, total * sizeof(float), &in));
+    TW_CUDA(launch_mcts_set_root_gumbel(a_, gm_, count_, static_cast<const float*>(in.dev), b.stream_));
+    b.launches_ += 1;
+    if (in.host) TW_TRY(b.Sync());  // the staged copy is reused by the next call
+    return TWIXT_OK;
+  }
+
+  // Gumbel searches: the action [count] int32 and the improved policy [count, n*n] float32; each nullable, host or
+  // device
+  int GumbelStats(int32_t* out_action, float* out_policy) {
+    if (!gumbel_) return fail(TWIXT_EINVAL, "twixt_mcts_gumbel_stats: the search is not a Gumbel search");
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_gumbel_stats: no search begun");
+    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_gumbel_stats while a twixt_mcts_select awaits its backup");
+    if (count_ == 0) return TWIXT_OK;
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    b.ScratchReset();
+    const size_t cells = static_cast<size_t>(a_.n) * a_.n, cnt = static_cast<size_t>(count_);
+    Staged ac, po;
+    TW_TRY(b.StageOut(out_action, cnt * sizeof(int32_t), &ac, false));
+    TW_TRY(b.StageOut(out_policy, cnt * cells * sizeof(float), &po, false));
+    TW_CUDA(launch_mcts_gumbel_stats(a_, gm_, count_, static_cast<int32_t*>(ac.dev), static_cast<float*>(po.dev),
+                                     b.stream_));
+    b.launches_ += 1;
+    TW_TRY(b.Finish(&ac));
+    TW_TRY(b.Finish(&po));
+    if (ac.host || po.host) TW_TRY(b.Sync());
+    return TWIXT_OK;
+  }
+
   int64_t count() const { return count_; }
   int64_t simulations() const { return sims_; }
 
  private:
+  // Host logits of a Gumbel backup must be finite on the legal actions of every non-terminal leaf: the leaf records
+  // select wrote to envs [leaf_first_, leaf_first_ + count) are read back and their legal lists computed here.
+  int CheckHostLogits(const float* logits) {
+    DeviceGuard g(b_->device_);
+    TwixTBatch& b = *b_;
+    const int n = a_.n, rw = a_.rw;
+    const size_t cells = static_cast<size_t>(n) * n;
+    std::vector<uint32_t> recs(static_cast<size_t>(count_) * rw);
+    TW_CUDA(cudaMemcpyAsync(recs.data(), b.rec(leaf_first_), recs.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                            b.stream_));
+    TW_TRY(b.Sync());
+    for (int64_t t = 0; t < count_; ++t) {
+      uint32_t* rec = recs.data() + t * rw;
+      Header h;
+      unpack_header(rec[0], rec[1], rec[2], rec[3], h);
+      if (h.result != kOpen) continue;
+      RecordRef<1> rb{rec, n};
+      for (int x = 0; x < n; ++x)
+        for (uint32_t w = legal_word(rb, h, x); w != 0u; w &= w - 1u) {
+          const int a = x * n + tw_ctz(w);
+          const float l = logits[t * cells + a];
+          if (!std::isfinite(l))
+            return fail(TWIXT_EINVAL, "logit [%lld, %d] = %g: logits must be finite on the leaf's legal actions",
+                        static_cast<long long>(t), a, static_cast<double>(l));
+        }
+    }
+    return TWIXT_OK;
+  }
+
   // The host's bound on a tree's node count (node_bound_: 1 after begin, min(keep_nodes, bound) after an advance,
   // +K per step) keeps every step inside the S node slots without reading the trees back.  Without an advance this
   // is "at most max_simulations simulations since begin".
@@ -1098,6 +1243,9 @@ class TwixTMCTS {
   int64_t log_size_ = 0;       // its entries
   bool pending_ = false;
   bool begun_ = false;
+  bool gumbel_ = false;        // a Gumbel AlphaZero search (gm_ holds its arrays)
+  MctsGumbel gm_{};
+  int64_t leaf_first_ = 0;     // the leaf envs of the pending select (host logits are checked against them)
 };
 
 }  // namespace twixt
@@ -1353,6 +1501,37 @@ int twixt_mcts_advance(twixt_mcts* m, const int32_t* actions, int32_t keep_nodes
 int twixt_mcts_set_root_priors(twixt_mcts* m, const float* priors) {
   TW_NEED_MCTS(m);
   return m->impl.SetRootPriors(priors);
+}
+int twixt_mcts_create_gumbel(twixt_batch* b, int64_t num_trees, int32_t max_simulations, int32_t n_rollouts,
+                             int32_t max_considered, double c_visit, double c_scale, twixt_mcts** out) {
+  TW_NEED(b);
+  if (out == nullptr) return fail(TWIXT_EINVAL, "null output pointer");
+  *out = nullptr;
+  if (max_considered < 1) return fail(TWIXT_EINVAL, "max_considered must be >= 1: %d", max_considered);
+  if (!std::isfinite(c_visit) || c_visit < 0.0)
+    return fail(TWIXT_EINVAL, "c_visit must be finite and >= 0: %g", c_visit);
+  if (!std::isfinite(c_scale) || c_scale < 0.0)
+    return fail(TWIXT_EINVAL, "c_scale must be finite and >= 0: %g", c_scale);
+  twixt_mcts* m = new (std::nothrow) twixt_mcts();
+  if (m == nullptr) return fail(TWIXT_ENOMEM, "out of host memory");
+  int rc = m->impl.Init(&b->impl, num_trees, max_simulations, n_rollouts, 0.0, false, false, 1, 0.0, true,
+                        max_considered, c_visit, c_scale);
+  if (rc != TWIXT_OK) {
+    std::string keep = twixt::g_last_error;
+    delete m;
+    twixt::g_last_error = keep;
+    return rc;
+  }
+  *out = m;
+  return TWIXT_OK;
+}
+int twixt_mcts_set_root_gumbel(twixt_mcts* m, const float* gumbel) {
+  TW_NEED_MCTS(m);
+  return m->impl.SetRootGumbel(gumbel);
+}
+int twixt_mcts_gumbel_stats(twixt_mcts* m, int32_t* out_action, float* out_policy) {
+  TW_NEED_MCTS(m);
+  return m->impl.GumbelStats(out_action, out_policy);
 }
 
 int twixt_get_stats(twixt_batch* b, twixt_stats* out) {

@@ -85,6 +85,20 @@ struct MctsArena {
   double vl;                // virtual loss
 };
 
+// The Gumbel part of a Gumbel AlphaZero search's arena (twixt_mcts_create_gumbel; semantics in twixt_mcts.cuh).  It is
+// passed to the Gumbel kernels next to the MctsArena, whose priors, tie keys, outcome bytes and virtual counts are
+// all nullptr in such a search.
+struct MctsGumbel {
+  float* edge_logit;     // [trees*S*M] l(a), written when the node is expanded at its backup
+  double* node_value;    // [trees*S] raw value v(s) for the player to move at s, written at the node's backup
+  float* root_gumbel;    // [trees*n*n] root noise g by action cell; zeroed by begin
+  const int32_t* table;  // [(max_considered + 1) * cols] considered visits, row m = mcts_considered_visits(m, cols)
+  int max_considered;    // min(max_considered, M)
+  int cols;              // max_simulations - 1
+  double c_visit;
+  double c_scale;
+};
+
 cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s);
 // leaf_dst == nullptr: leaves go to the rollout slots (built-in evaluator), else to records leaf_dst + t*rw
 cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed, uint32_t stream0, uint32_t k,
@@ -104,6 +118,16 @@ cudaError_t launch_mcts_advance(const MctsArena& a, int64_t count, const int32_t
                                 int32_t* map, int32_t* out_status, unsigned int* illegal_index, cudaStream_t s);
 // PUCT searches: P(a) of the root edges of every expanded root from priors [count, n*n] (device)
 cudaError_t launch_mcts_set_root_priors(const MctsArena& a, int64_t count, const float* priors, cudaStream_t s);
+// Gumbel searches: select (leaf_dst as launch_mcts_select), backup (logits [count, n*n] or nullptr: 0), the root
+// noise [count, n*n] (device) and the stats (action [count], improved policy [count, n*n]; each nullable)
+cudaError_t launch_mcts_gumbel_select(const MctsArena& a, const MctsGumbel& gm, int64_t count, uint32_t stream0,
+                                      uint32_t k, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s);
+cudaError_t launch_mcts_gumbel_backup(const MctsArena& a, const MctsGumbel& gm, int64_t count, const float* values,
+                                      const float* logits, cudaStream_t s);
+cudaError_t launch_mcts_set_root_gumbel(const MctsArena& a, const MctsGumbel& gm, int64_t count, const float* gumbel,
+                                        cudaStream_t s);
+cudaError_t launch_mcts_gumbel_stats(const MctsArena& a, const MctsGumbel& gm, int64_t count, int32_t* out_action,
+                                     float* out_policy, cudaStream_t s);
 
 cudaError_t launch_reset(uint32_t* records, int64_t count, int n, cudaStream_t s);
 cudaError_t launch_clone(uint32_t* dst, const uint32_t* src, const int64_t* src_ids, int64_t count, int n,

@@ -903,6 +903,322 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_set_root_priors_kernel(M
   for (int i = lane; i < legal; i += 32) a.edge_p[e0 + i] = row[a.edge_action[e0 + i]];
 }
 
+// ------------------------------------------------------ Gumbel AlphaZero ---
+// Semantics in twixt_mcts.cuh.  Every reduction over a node's edges is lanes over the edges (lane l takes edges l,
+// l+32, .. in ascending order), then an xor butterfly, so that a sum has the order of mcts_lane_sums in every lane.
+__device__ __forceinline__ double warp_sum(double s) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) s = __dadd_rn(s, __shfl_xor_sync(kFullMask, s, d));
+  return s;
+}
+__device__ __forceinline__ double warp_max(double x) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) x = mcts_max(x, __shfl_xor_sync(kFullMask, x, d));
+  return x;
+}
+__device__ __forceinline__ double warp_min(double x) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) x = mcts_min(x, __shfl_xor_sync(kFullMask, x, d));
+  return x;
+}
+// (score, edge) argmax over the lanes: the larger score, then the lower edge; bi = 0x7FFFFFFF for none
+__device__ __forceinline__ int warp_argmax(double best, int bi) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) {
+    const double os = __shfl_xor_sync(kFullMask, best, d);
+    const int oi = __shfl_xor_sync(kFullMask, bi, d);
+    if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_score_beats(os, oi, best, bi))) {
+      best = os;
+      bi = oi;
+    }
+  }
+  return bi;
+}
+
+// What sigma(a) of a node's edges needs: max l, SN, max N, v_mix and the min / max / scale of q^
+struct GumbelNode {
+  double max_logit, v_mix, q_min, q_max, scale;
+  uint32_t sum_n, max_n;
+};
+
+// The completed-Q transform of the expanded node at global slot g with L = legal edges (every lane gets the same)
+__device__ GumbelNode gumbel_node(const MctsArena& a, const MctsGumbel& gm, int64_t g, int legal, int lane) {
+  const int64_t e0 = g * a.M;
+  GumbelNode s;
+  double mx = -INFINITY;
+  uint32_t sn = 0u, mn = 0u;
+  for (int i = lane; i < legal; i += 32) {
+    mx = mcts_max(mx, static_cast<double>(gm.edge_logit[e0 + i]));
+    const uint32_t n = a.edge_n[e0 + i];
+    sn += n;
+    mn = n > mn ? n : mn;
+  }
+  s.max_logit = warp_max(mx);
+  s.sum_n = __reduce_add_sync(kFullMask, sn);
+  s.max_n = __reduce_max_sync(kFullMask, mn);
+  double weighted_q = 0.0;
+  if (s.sum_n > 0u) {  // with no visited edge both sums below are 0.0
+    double z = 0.0;
+    for (int i = lane; i < legal; i += 32)
+      z = __dadd_rn(z, mcts_exp(__dsub_rn(static_cast<double>(gm.edge_logit[e0 + i]), s.max_logit)));
+    z = warp_sum(z);
+    double sp = 0.0;
+    for (int i = lane; i < legal; i += 32)
+      if (a.edge_n[e0 + i] > 0u)
+        sp = __dadd_rn(sp, mcts_gumbel_prob(mcts_exp(__dsub_rn(static_cast<double>(gm.edge_logit[e0 + i]),
+                                                               s.max_logit)), z));
+    sp = warp_sum(sp);
+    for (int i = lane; i < legal; i += 32) {
+      const uint32_t n = a.edge_n[e0 + i];
+      if (n > 0u) {
+        const double pi = mcts_gumbel_prob(mcts_exp(__dsub_rn(static_cast<double>(gm.edge_logit[e0 + i]), s.max_logit)), z);
+        weighted_q = __dadd_rn(weighted_q, mcts_gumbel_mix_term(pi, a.edge_w[e0 + i], n, sp));
+      }
+    }
+    weighted_q = warp_sum(weighted_q);
+  }
+  s.v_mix = mcts_gumbel_mixed_value(gm.node_value[g], s.sum_n, weighted_q);
+  double qmin = INFINITY, qmax = -INFINITY;
+  for (int i = lane; i < legal; i += 32) {
+    const double q = mcts_gumbel_completed_q(a.edge_w[e0 + i], a.edge_n[e0 + i], s.v_mix);
+    qmin = mcts_min(qmin, q);
+    qmax = mcts_max(qmax, q);
+  }
+  s.q_min = warp_min(qmin);
+  s.q_max = warp_max(qmax);
+  s.scale = mcts_gumbel_scale(gm.c_visit, gm.c_scale, s.max_n);
+  return s;
+}
+
+// sigma(a) of edge e
+__device__ __forceinline__ double gumbel_sigma(const MctsArena& a, const GumbelNode& s, int64_t e) {
+  const double q = mcts_gumbel_completed_q(a.edge_w[e], a.edge_n[e], s.v_mix);
+  return mcts_gumbel_sigma(q, s.q_min, s.q_max, s.scale);
+}
+
+// l(a) + sigma(a) of edge e
+__device__ __forceinline__ double gumbel_completed_logit(const MctsGumbel& gm, const MctsArena& a, const GumbelNode& s,
+                                                         int64_t e) {
+  return __dadd_rn(static_cast<double>(gm.edge_logit[e]), gumbel_sigma(a, s, e));
+}
+
+// max over the edges of l + sigma and the sum of mcts_exp(l + sigma - that max): softmax(l + sigma) = e / z
+__device__ __forceinline__ void gumbel_softmax_norm(const MctsArena& a, const MctsGumbel& gm, const GumbelNode& s,
+                                                    int64_t e0, int legal, int lane, double& mx, double& z) {
+  double m = -INFINITY;
+  for (int i = lane; i < legal; i += 32) m = mcts_max(m, gumbel_completed_logit(gm, a, s, e0 + i));
+  mx = warp_max(m);
+  double sum = 0.0;
+  for (int i = lane; i < legal; i += 32)
+    sum = __dadd_rn(sum, mcts_exp(__dsub_rn(gumbel_completed_logit(gm, a, s, e0 + i), mx)));
+  z = warp_sum(sum);
+}
+
+// the root's edge among those with N(a) = considered (-1: none eligible, the lowest edge), by the root score
+__device__ __forceinline__ int gumbel_root_argmax(const MctsArena& a, const MctsGumbel& gm, const GumbelNode& s,
+                                                  int64_t t, int64_t e0, int legal, int64_t considered, int lane) {
+  const float* noise = gm.root_gumbel + t * a.n * a.n;
+  double best = 0.0;
+  int bi = 0x7FFFFFFF;
+  for (int i = lane; i < legal; i += 32) {
+    if (static_cast<int64_t>(a.edge_n[e0 + i]) != considered) continue;
+    const double sc = mcts_gumbel_root_score(noise[a.edge_action[e0 + i]], gm.edge_logit[e0 + i], s.max_logit,
+                                             gumbel_sigma(a, s, e0 + i));
+    if (bi == 0x7FFFFFFF || mcts_score_beats(sc, i, best, bi)) {
+      best = sc;
+      bi = i;
+    }
+  }
+  bi = warp_argmax(best, bi);
+  return bi == 0x7FFFFFFF ? 0 : bi;
+}
+
+// ------------------------------------------------------------------ Gumbel select ---
+// One warp per tree, one descent (K = 1, no solver): the root takes Sequential Halving's edge, every other node the
+// interior rule; a chosen edge without a child creates it as the PUCT select does.  The leaf goes to leaf_dst + t*rw
+// or to the R rollout slots, as mcts_select_kernel writes it.
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_gumbel_select_kernel(MctsArena a, MctsGumbel gm, int64_t count,
+                                                                             uint32_t stream0, uint32_t k,
+                                                                             uint32_t* __restrict__ leaf_dst,
+                                                                             int32_t* __restrict__ out_status) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int n = a.n, rw = a.rw;
+  const uint32_t T = stream0 + static_cast<uint32_t>(t);
+  int node = 0, depth = 0, nodes = a.tree[t].x;
+  int2* path = a.path + t * a.P;
+  bool terminal;
+  for (;;) {
+    const int64_t g = mcts_slot(a, t, node);
+    uint32_t* rec = a.node_rec + g * rw;
+    const uint4 hw = *reinterpret_cast<const uint4*>(rec);
+    Header h;
+    unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+    terminal = h.result != kOpen;
+    if (terminal || a.node_n[g] == 0u) break;
+    const int64_t e0 = g * a.M;
+    const int legal = a.node_legal[g];
+    const GumbelNode s = gumbel_node(a, gm, g, legal, lane);
+    int edge;
+    if (node == 0) {
+      const int m = gm.max_considered < legal ? gm.max_considered : legal;
+      const int64_t considered =
+          static_cast<int>(s.sum_n) < gm.cols ? gm.table[static_cast<int64_t>(m) * gm.cols + s.sum_n] : -1;
+      edge = gumbel_root_argmax(a, gm, s, t, e0, legal, considered, lane);
+    } else {
+      double mx, z;
+      gumbel_softmax_norm(a, gm, s, e0, legal, lane, mx, z);
+      double best = 0.0;
+      int bi = 0x7FFFFFFF;
+      for (int i = lane; i < legal; i += 32) {
+        const double e = mcts_exp(__dsub_rn(gumbel_completed_logit(gm, a, s, e0 + i), mx));
+        const double sc = mcts_gumbel_interior_score(e, z, a.edge_n[e0 + i], s.sum_n);
+        if (bi == 0x7FFFFFFF || mcts_score_beats(sc, i, best, bi)) {
+          best = sc;
+          bi = i;
+        }
+      }
+      edge = warp_argmax(best, bi);
+    }
+    if (lane == 0) path[depth] = make_int2(node, (edge << 1) | static_cast<int>(h.ply & 1u));
+    ++depth;
+    int child = a.edge_child[e0 + edge];
+    if (child < 0) {
+      child = nodes++;
+      const int64_t gc = mcts_slot(a, t, child);
+      uint32_t* crec = a.node_rec + gc * rw;
+      warp_copy_record(crec, rec, rw, lane);
+      __syncwarp();
+      if (lane == 0) {
+        RecordRef<1> cb{crec, n};
+        Header ch = h;
+        const int action = a.edge_action[e0 + edge];
+        const int x = action / n;
+        apply_legal_cell<kMctsFloodStack>(cb, ch, x, action - x * n);
+        uint4 o;
+        pack_header(ch, o.x, o.y, o.z, o.w);
+        *reinterpret_cast<uint4*>(crec) = o;
+        a.node_legal[gc] = -1;
+        a.node_n[gc] = 0u;
+        a.edge_child[e0 + edge] = child;
+      }
+      __syncwarp();
+    }
+    node = child;
+  }
+  const uint32_t* leaf = a.node_rec + mcts_slot(a, t, node) * rw;
+  if (leaf_dst != nullptr) {
+    warp_copy_record(leaf_dst + t * rw, leaf, rw, lane);
+  } else {
+    for (int r = 0; r < a.R; ++r) warp_copy_record(a.roll_rec + (t * a.R + r) * rw, leaf, rw, lane);
+    for (int r = lane; r < a.R; r += 32)
+      a.roll_ids[t * a.R + r] = mcts_rollout_stream(T, k, static_cast<uint32_t>(a.R), static_cast<uint32_t>(r));
+  }
+  const int status = terminal ? kLeafTerminal : kLeafNeedsValue;
+  if (lane == 0) {
+    a.tree[t] = make_int4(nodes, node, depth, status);
+    if (out_status != nullptr) out_status[t] = status;
+  }
+}
+
+// ------------------------------------------------------------------ Gumbel backup ---
+// The leaf value as mcts_backup_kernel takes it, added along the path; the leaf's raw value v(leaf) is that value for
+// its player to move, and a non-terminal leaf is expanded with l(a) = logits[t, action] (0 without logits).
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_gumbel_backup_kernel(MctsArena a, MctsGumbel gm, int64_t count,
+                                                                             const float* __restrict__ values,
+                                                                             const float* __restrict__ logits) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int4 info = a.tree[t];
+  const int leaf = info.y, depth = info.z;
+  const int64_t gl = mcts_slot(a, t, leaf);
+  const uint32_t* rec = a.node_rec + gl * a.rw;
+  const uint4 hw = *reinterpret_cast<const uint4*>(rec);
+  Header h;
+  unpack_header(hw.x, hw.y, hw.z, hw.w, h);
+  double v[2];
+  if (info.w == kLeafTerminal) {
+    mcts_terminal_value(h, v);
+  } else if (values != nullptr) {
+    v[0] = static_cast<double>(values[2 * t]);
+    v[1] = static_cast<double>(values[2 * t + 1]);
+  } else {
+    double s0 = 0.0, s1 = 0.0;
+    const float* ret = a.roll_ret + t * a.R * 2;
+    for (int r = 0; r < a.R; ++r) {
+      s0 = __dadd_rn(s0, static_cast<double>(ret[2 * r]));
+      s1 = __dadd_rn(s1, static_cast<double>(ret[2 * r + 1]));
+    }
+    v[0] = __ddiv_rn(s0, static_cast<double>(a.R));
+    v[1] = __ddiv_rn(s1, static_cast<double>(a.R));
+  }
+  const int2* path = a.path + t * a.P;
+  for (int i = lane; i < depth; i += 32) {
+    const int2 p = path[i];
+    const int64_t g = mcts_slot(a, t, p.x);
+    const int64_t e = g * a.M + (p.y >> 1);
+    a.node_n[g] += 1u;
+    a.edge_n[e] += 1u;
+    a.edge_w[e] = __dadd_rn(a.edge_w[e], v[p.y & 1]);
+  }
+  if (lane == 0) {
+    a.node_n[gl] += 1u;
+    gm.node_value[gl] = (h.ply & 1u) != 0u ? v[1] : v[0];
+  }
+  if (info.w != kLeafTerminal) {
+    const int64_t e0 = gl * a.M;
+    const int legal = warp_expand(a, gl, rec, h, lane);
+    const float* row = logits != nullptr ? logits + t * a.n * a.n : nullptr;
+    for (int i = lane; i < legal; i += 32) gm.edge_logit[e0 + i] = row != nullptr ? row[a.edge_action[e0 + i]] : 0.0f;
+  }
+}
+
+// -------------------------------------------------------------- set root gumbel ---
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_set_root_gumbel_kernel(MctsArena a, MctsGumbel gm, int64_t count,
+                                                                               const float* __restrict__ gumbel) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int cells = a.n * a.n;
+  for (int c = lane; c < cells; c += 32) gm.root_gumbel[t * cells + c] = gumbel[t * cells + c];
+}
+
+// ------------------------------------------------------------------ Gumbel stats ---
+// The action (the root score among the edges of most visits; -1 for a terminal or unexpanded root) and the improved
+// policy softmax(l + sigma) at the root's action cells (0 elsewhere, all 0 for a terminal or unexpanded root)
+__global__ void __launch_bounds__(kMctsWarps * 32) mcts_gumbel_stats_kernel(MctsArena a, MctsGumbel gm, int64_t count,
+                                                                            int32_t* __restrict__ out_action,
+                                                                            float* __restrict__ out_policy) {
+  const int lane = threadIdx.x & 31;
+  const int64_t t = blockIdx.x * static_cast<int64_t>(kMctsWarps) + (threadIdx.x >> 5);
+  if (t >= count) return;
+  const int cells = a.n * a.n;
+  const int64_t g = mcts_slot(a, t, 0), e0 = g * a.M;
+  const int legal = a.node_legal[g];
+  if (out_policy != nullptr) {
+    for (int c = lane; c < cells; c += 32) out_policy[t * cells + c] = 0.0f;
+    __syncwarp();
+  }
+  if (legal < 0) {
+    if (out_action != nullptr && lane == 0) out_action[t] = -1;
+    return;
+  }
+  const GumbelNode s = gumbel_node(a, gm, g, legal, lane);
+  if (out_action != nullptr) {
+    const int edge = gumbel_root_argmax(a, gm, s, t, e0, legal, s.max_n, lane);
+    if (lane == 0) out_action[t] = a.edge_action[e0 + edge];
+  }
+  if (out_policy != nullptr) {
+    double mx, z;
+    gumbel_softmax_norm(a, gm, s, e0, legal, lane, mx, z);
+    for (int i = lane; i < legal; i += 32)
+      out_policy[t * cells + a.edge_action[e0 + i]] =
+          __double2float_rn(__ddiv_rn(mcts_exp(__dsub_rn(gumbel_completed_logit(gm, a, s, e0 + i), mx)), z));
+  }
+}
+
 unsigned mcts_blocks(int64_t count) { return static_cast<unsigned>((count + kMctsWarps - 1) / kMctsWarps); }
 
 }  // namespace
@@ -969,6 +1285,35 @@ cudaError_t launch_mcts_advance(const MctsArena& a, int64_t count, const int32_t
 cudaError_t launch_mcts_set_root_priors(const MctsArena& a, int64_t count, const float* priors, cudaStream_t s) {
   if (count <= 0) return cudaSuccess;
   mcts_set_root_priors_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, priors);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_gumbel_select(const MctsArena& a, const MctsGumbel& gm, int64_t count, uint32_t stream0,
+                                      uint32_t k, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_gumbel_select_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, stream0, k, leaf_dst,
+                                                                            out_status);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_gumbel_backup(const MctsArena& a, const MctsGumbel& gm, int64_t count, const float* values,
+                                      const float* logits, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_gumbel_backup_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, values, logits);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_set_root_gumbel(const MctsArena& a, const MctsGumbel& gm, int64_t count, const float* gumbel,
+                                        cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_set_root_gumbel_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, gumbel);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mcts_gumbel_stats(const MctsArena& a, const MctsGumbel& gm, int64_t count, int32_t* out_action,
+                                     float* out_policy, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  mcts_gumbel_stats_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, out_action, out_policy);
   return cudaGetLastError();
 }
 

@@ -62,12 +62,34 @@
 // the chosen edge's code c != 0 (the child's value for its own player to move), else 0.  The draw and rollout
 // streams keep counting k: a tree never repeats a Philox counter.  The kernel needs an int32 old -> new slot map of
 // S entries per tree, allocated at the first advance.
+//
+// Gumbel AlphaZero (twixt_mcts_create_gumbel; mctx gumbel_muzero_policy, Danihelka et al., ICLR 2022): the tree
+// above, one node per simulation, leaves expanded at their backup as PUCT does, but every edge carries a float32
+// logit l(a) (the caller's [n*n] row, 0 without one) and every node its raw value v(s) (its evaluation for its own
+// player to move), and the root takes Gumbel noise g(a) per action cell.  Selection (IEEE double, no
+// contraction, the helpers below):
+//   pi(a)      max(softmax(l)(a), smallest normal double)
+//   v_mix      (v + SN * sum_{N(b)>0} (pi(b) * q(b) / sum_{N(b)>0} pi(b))) / (SN + 1),  q = W/N, SN = sum N(b)
+//   q~(a)      q(a) if N(a) > 0, else v_mix;  q^ = (q~ - min q~) / max(max q~ - min q~, 1e-8)
+//   sigma(a)   ((c_visit + max N(b)) * c_scale) * q^(a)
+//   interior   argmax of softmax(l + sigma)(a) - N(a) / (1 + SN), ties to the lower edge
+//   root       Sequential Halving: among edges with N(a) = table[min(max_considered, L)][SN], argmax of
+//              max(-1e9, (g(a) + (l(a) - max l)) + sigma(a)), ties to the lower edge (none eligible: edge 0)
+//   action     the root score among the edges with N(a) = max N;  improved policy softmax(l + sigma) at the root
+// table is mctx's get_table_of_considered_visits(max_considered, max_simulations - 1) (mcts_considered_visits).
+// Every exp is mcts_exp and every sum over a node's edges is in the order of mcts_lane_sums: lane l adds edges
+// l, l+32, .. from 0.0, then an xor butterfly over offsets 16, 8, 4, 2, 1.  A Gumbel search has no priors, tie keys
+// or outcome bytes; it adds 4 (logit f32) per edge, 8 (v f64) per node and 4*n*n (root noise f32) per tree:
+//   Gumbel bytes per tree = S * (rw*4 + 16 + 22*M) + 16 + 8*P + R * (rw*4 + 16) + 4*n*n
+// plus the table, (min(max_considered, M) + 1) * (max_simulations - 1) int32, once per search.
 #pragma once
 #include <stdint.h>
 
 #include "twixt_engine.cuh"
 #include "twixt_philox.cuh"
 
+#include <cstring>
+#include <vector>
 #if !defined(__CUDA_ARCH__)
 #include <cmath>
 #endif
@@ -252,6 +274,162 @@ TW_HD uint64_t mcts_rollout_stream(uint32_t tree_stream, uint32_t k, uint32_t R,
 TW_HD void mcts_terminal_value(const Header& h, double v[2]) {
   v[0] = h.result == kRedWin ? 1.0 : (h.result == kBlueWin ? -1.0 : 0.0);
   v[1] = h.result == kBlueWin ? 1.0 : (h.result == kRedWin ? -1.0 : 0.0);
+}
+
+// ------------------------------------------------------------------------------------ Gumbel AlphaZero ---
+// IEEE double operations, round to nearest, identical on the device and on a host built with -ffp-contract=off
+TW_HD double mcts_add(double a, double b) {
+#if defined(__CUDA_ARCH__)
+  return __dadd_rn(a, b);
+#else
+  return a + b;
+#endif
+}
+TW_HD double mcts_sub(double a, double b) {
+#if defined(__CUDA_ARCH__)
+  return __dsub_rn(a, b);
+#else
+  return a - b;
+#endif
+}
+TW_HD double mcts_mul(double a, double b) {
+#if defined(__CUDA_ARCH__)
+  return __dmul_rn(a, b);
+#else
+  return a * b;
+#endif
+}
+TW_HD double mcts_div(double a, double b) {
+#if defined(__CUDA_ARCH__)
+  return __ddiv_rn(a, b);
+#else
+  return a / b;
+#endif
+}
+TW_HD double mcts_max(double a, double b) { return a > b ? a : b; }
+TW_HD double mcts_min(double a, double b) { return a < b ? a : b; }
+
+// 2^j for -1022 <= j <= 1023, exact
+TW_HD double mcts_pow2(int j) {
+  const uint64_t bits = static_cast<uint64_t>(j + 1023) << 52;
+#if defined(__CUDA_ARCH__)
+  return __longlong_as_double(static_cast<long long>(bits));
+#else
+  double d;
+  std::memcpy(&d, &bits, sizeof(d));
+  return d;
+#endif
+}
+
+// exp(x) for x <= 0 (every softmax argument is max-centred), part of the specification: 0 below -746 (and for NaN);
+// else k = round-half-even(x * log2(e)), r = (x - k*ln2_hi) - k*ln2_lo (Cody-Waite; k*ln2_hi is exact), the
+// degree-13 Taylor polynomial of e^r in Horner form (coefficients float64(1/j!)), scaled by 2^(k >> 1) and then
+// 2^(k - (k >> 1)): only the last product can round (a subnormal result).  Within 1 ulp of a correctly rounded exp.
+TW_HD double mcts_exp_step(double p, double r, double c) { return mcts_add(mcts_mul(p, r), c); }
+TW_HD double mcts_exp(double x) {
+  if (!(x >= -746.0)) return 0.0;
+#if defined(__CUDA_ARCH__)
+  const int k = __double2int_rn(__dmul_rn(x, 0x1.71547652b82fep+0));
+#else
+  const int k = static_cast<int>(std::nearbyint(x * 0x1.71547652b82fep+0));
+#endif
+  const double kd = static_cast<double>(k);
+  const double r = mcts_sub(mcts_sub(x, mcts_mul(kd, 0x1.62e42fee00000p-1)), mcts_mul(kd, 0x1.a39ef35793c76p-33));
+  double p = 0x1.6124613a86d09p-33;             // 1/13!
+  p = mcts_exp_step(p, r, 0x1.1eed8eff8d898p-29);  // 1/12!
+  p = mcts_exp_step(p, r, 0x1.ae64567f544e4p-26);  // 1/11!
+  p = mcts_exp_step(p, r, 0x1.27e4fb7789f5cp-22);  // 1/10!
+  p = mcts_exp_step(p, r, 0x1.71de3a556c734p-19);  // 1/9!
+  p = mcts_exp_step(p, r, 0x1.a01a01a01a01ap-16);  // 1/8!
+  p = mcts_exp_step(p, r, 0x1.a01a01a01a01ap-13);  // 1/7!
+  p = mcts_exp_step(p, r, 0x1.6c16c16c16c17p-10);  // 1/6!
+  p = mcts_exp_step(p, r, 0x1.1111111111111p-7);   // 1/5!
+  p = mcts_exp_step(p, r, 0x1.5555555555555p-5);   // 1/4!
+  p = mcts_exp_step(p, r, 0x1.5555555555555p-3);   // 1/3!
+  p = mcts_exp_step(p, r, 0x1.0p-1);
+  p = mcts_exp_step(p, r, 1.0);
+  p = mcts_exp_step(p, r, 1.0);
+  return mcts_mul(mcts_mul(p, mcts_pow2(k >> 1)), mcts_pow2(k - (k >> 1)));
+}
+
+// pi(a) from e = mcts_exp(l(a) - max l) and Z = the sum of e: raised to the smallest normal double (mctx's
+// jnp.finfo.tiny in _compute_mixed_value)
+TW_HD double mcts_gumbel_prob(double e, double z) { return mcts_max(mcts_div(e, z), 0x1.0p-1022); }
+// one term of the mixed value's weighted Q: pi(b) * q(b) / sum_{N(b)>0} pi(b), q = W/N
+TW_HD double mcts_gumbel_mix_term(double pi, double w, uint32_t n, double sum_probs) {
+  return mcts_div(mcts_mul(pi, mcts_div(w, static_cast<double>(n))), sum_probs);
+}
+// v_mix from the node's raw value, SN = sum N(b) and the weighted Q
+TW_HD double mcts_gumbel_mixed_value(double raw, uint32_t sum_n, double weighted_q) {
+  const double sn = static_cast<double>(sum_n);
+  return mcts_div(mcts_add(raw, mcts_mul(sn, weighted_q)), mcts_add(sn, 1.0));
+}
+// q~(a): W/N for a visited edge, else v_mix
+TW_HD double mcts_gumbel_completed_q(double w, uint32_t n, double v_mix) {
+  return n > 0u ? mcts_div(w, static_cast<double>(n)) : v_mix;
+}
+// (c_visit + max N(b)) * c_scale, the factor of sigma
+TW_HD double mcts_gumbel_scale(double c_visit, double c_scale, uint32_t max_n) {
+  return mcts_mul(mcts_add(c_visit, static_cast<double>(max_n)), c_scale);
+}
+// sigma(a) from q~(a), the node's min and max q~ and its scale
+TW_HD double mcts_gumbel_sigma(double q, double q_min, double q_max, double scale) {
+  return mcts_mul(scale, mcts_div(mcts_sub(q, q_min), mcts_max(mcts_sub(q_max, q_min), 1e-8)));
+}
+// interior score pi'(a) - N(a) / (1 + SN), pi'(a) = e / Z' (e = mcts_exp(l + sigma - max(l + sigma)))
+TW_HD double mcts_gumbel_interior_score(double e, double z, uint32_t n, uint32_t sum_n) {
+  return mcts_sub(mcts_div(e, z), mcts_div(static_cast<double>(n), mcts_add(static_cast<double>(sum_n), 1.0)));
+}
+// root score max(-1e9, (g + (l - max l)) + sigma)
+TW_HD double mcts_gumbel_root_score(float g, float logit, double max_logit, double sigma) {
+  return mcts_max(-1e9, mcts_add(mcts_add(static_cast<double>(g), mcts_sub(static_cast<double>(logit), max_logit)),
+                                 sigma));
+}
+
+// The device's order of a sum over L edges, on the host (host code only): lane l adds terms l, l+32, .. (ascending) from 0.0 where
+// include(i), then partials combine as p[l] + p[l ^ d] for d = 16, 8, 4, 2, 1 (the same in every lane).
+template <class Term, class Include>
+double mcts_lane_sums(int L, Term term, Include include) {
+  double p[32];
+  for (int l = 0; l < 32; ++l) {
+    p[l] = 0.0;
+    for (int i = l; i < L; i += 32)
+      if (include(i)) p[l] = p[l] + term(i);
+  }
+  for (int d = 16; d > 0; d >>= 1) {
+    double q[32];
+    for (int l = 0; l < 32; ++l) q[l] = p[l] + p[l ^ d];
+    std::memcpy(p, q, sizeof(p));
+  }
+  return p[0];
+}
+
+// mctx seq_halving.get_sequence_of_considered_visits(m, num_simulations) in integer arithmetic: out[0 ..
+// num_simulations) (host code only)
+inline void mcts_considered_visits(int m, int num_simulations, int32_t* out) {
+  if (m <= 1) {
+    for (int i = 0; i < num_simulations; ++i) out[i] = i;
+    return;
+  }
+  int log2max = 0;  // ceil(log2(m))
+  while ((1 << log2max) < m) ++log2max;
+  std::vector<int32_t> visits(static_cast<size_t>(m), 0);
+  int num_considered = m, len = 0;
+  while (len < num_simulations) {
+    int extra = num_simulations / (log2max * num_considered);
+    if (extra < 1) extra = 1;
+    for (int e = 0; e < extra; ++e) {
+      for (int i = 0; i < num_considered; ++i, ++len)
+        if (len < num_simulations) out[len] = visits[i];
+      for (int i = 0; i < num_considered; ++i) visits[i] += 1;
+    }
+    num_considered = num_considered / 2 > 2 ? num_considered / 2 : 2;
+  }
+}
+
+// the Gumbel formula of the header comment above; cells = n*n
+TW_HD int64_t mcts_gumbel_bytes_per_tree(const MctsSizes& s, int64_t cells) {
+  return mcts_bytes_per_tree(s) + s.slots * (8 + 4 * s.edges) + 4 * cells;
 }
 
 }  // namespace twixt

@@ -34,6 +34,13 @@ its statistics, up to keep_nodes nodes, so the next search starts from the visit
 Size the search for it: max_simulations is the node capacity, e.g. 2*sims with keep_nodes = sims + 1 runs sims new
 simulations every move.  `set_root_priors` puts fresh priors (root Dirichlet noise) on the kept roots.
 
+`selection="gumbel"` is Gumbel AlphaZero (Danihelka et al., ICLR 2022; DeepMind mctx's gumbel_muzero_policy), the
+search for small simulation budgets: Sequential Halving with Gumbel noise over max_considered root moves, and the
+completed-Q rule below the root.  `backup(values, logits)` hands the policy head's logits instead of priors,
+`set_root_gumbel(gumbel_noise(...))` after `begin` sets the root's noise (zero until then), and `gumbel_stats()`
+returns the move to play and the improved policy softmax(logits + sigma(completed Q)), the training target.  It has
+no solver, one leaf per step and no tree reuse.
+
 `MCTSBot` is the open_spiel-shaped bot over one tree for adapter `TwixTState`s.
 
 Arrays may be numpy (synchronous) or torch CUDA tensors (asynchronous on the batch's stream), as for
@@ -53,19 +60,26 @@ LEAF_NEEDS_VALUE, LEAF_TERMINAL, LEAF_SOLVED = 0, 1, 2
 ROOT_KEPT, ROOT_ILLEGAL, ROOT_FRESH = 0, 1, 2  # advance(): statistics kept, illegal action, new root unvisited
 UNPROVEN = -128  # solver_stats' edge value of a root move that is not proven
 _PUCT, _SOLVE = 1, 2  # TWIXT_MCTS_PUCT, TWIXT_MCTS_SOLVE
+_SELECTIONS = ("uct", "puct", "gumbel")
 
 
 class BatchedMCTS:
     def __init__(self, batch: TwixTBatch, num_trees: int, max_simulations: int, n_rollouts: int = 1,
                  uct_c: float = 2.0, selection: str = "uct", solve: bool = False, leaves_per_step: int = 1,
-                 virtual_loss: float = 1.0):
-        if selection not in ("uct", "puct"):
-            raise ValueError("selection must be 'uct' or 'puct', got %r" % (selection,))
+                 virtual_loss: float = 1.0, max_considered: int = 16, c_visit: float = 50.0, c_scale: float = 0.1):
+        if selection not in _SELECTIONS:
+            raise ValueError("selection must be one of %s, got %r" % (", ".join(map(repr, _SELECTIONS)), selection))
+        if selection == "gumbel" and (solve or int(leaves_per_step) != 1):
+            raise ValueError("selection='gumbel' runs without the solver and with one leaf per step")
         self._lib = _lib.load()
         self.batch = batch  # the search runs on the batch's envs and stream: keep it alive
         self._h = C.c_void_p()
         flags = (_PUCT if selection == "puct" else 0) | (_SOLVE if solve else 0)
-        if int(leaves_per_step) == 1:
+        if selection == "gumbel":
+            self._check(self._lib.twixt_mcts_create_gumbel(batch._h, int(num_trees), int(max_simulations),
+                                                           int(n_rollouts), int(max_considered), float(c_visit),
+                                                           float(c_scale), C.byref(self._h)))
+        elif int(leaves_per_step) == 1:
             self._check(self._lib.twixt_mcts_create_ex(batch._h, int(num_trees), int(max_simulations),
                                                        int(n_rollouts), float(uct_c), flags, C.byref(self._h)))
         else:
@@ -80,6 +94,9 @@ class BatchedMCTS:
         self.max_simulations = int(max_simulations)
         self.n_rollouts = int(n_rollouts)
         self.uct_c = float(uct_c)
+        self.max_considered = int(max_considered)
+        self.c_visit = float(c_visit)
+        self.c_scale = float(c_scale)
         self.count = 0
         self._cells = batch.board_size * batch.board_size
 
@@ -129,7 +146,9 @@ class BatchedMCTS:
     def backup(self, values, priors=None):
         """Stepwise form, second half: values [count*K, 2] float32 of the leaves select() wrote.  A PUCT search
         also takes priors [count*K, n*n] float32 (None: uniform over the legal actions); entries of illegal
-        actions, rows of terminal leaves and (K > 1) the rows of repeated leaves after the first are ignored."""
+        actions, rows of terminal leaves and (K > 1) the rows of repeated leaves after the first are ignored.  A
+        Gumbel search reads priors as the leaves' logits [count, n*n] float32 (None: 0 for every edge); they must
+        be finite on the legal actions."""
         rows = self.count * self.leaves_per_step
         if not _is_torch(values):
             values = np.ascontiguousarray(values, dtype=np.float32)
@@ -141,7 +160,8 @@ class BatchedMCTS:
 
     def root_stats(self, out_visits=None, out_value_sums=None, out_best=None):
         """(visits [count, n*n] int32, value_sums [count, n*n] float64, best [count] int32) of the root edges;
-        best is -1 where the root is terminal or not yet expanded (PUCT: while no root edge has a visit)."""
+        best is -1 where the root is terminal or not yet expanded (PUCT: while no root edge has a visit).  For a
+        Gumbel search best is the Gumbel action of `gumbel_stats`."""
         if out_visits is None:
             out_visits = np.zeros((self.count, self._cells), dtype=np.int32)
         if out_value_sums is None:
@@ -197,6 +217,28 @@ class BatchedMCTS:
                                                                        self.count)))
         return out_status
 
+    def set_root_gumbel(self, gumbel):
+        """Gumbel only: the root noise [count, n*n] float32 by action cell (`gumbel_noise`), after `begin` (which
+        sets it to 0) and before the root's second simulation.  Host values must be finite."""
+        if not _is_torch(gumbel):
+            gumbel = np.ascontiguousarray(gumbel, dtype=np.float32)
+        self._check(self._lib.twixt_mcts_set_root_gumbel(
+            self._h, _ptr(gumbel, _dt(np.float32, "float32"), self.count * self._cells)))
+
+    def gumbel_stats(self, out_action=None, out_policy=None):
+        """Gumbel only: (action [count] int32, policy [count, n*n] float32).  action is the move to play: the
+        Sequential Halving score among the root moves of most visits, -1 for a terminal or unexpanded root.  policy
+        is the improved policy softmax(logits + sigma(completed Q)) over the root's legal moves, 0 elsewhere (all 0
+        for a terminal or unexpanded root): the policy target of Gumbel AlphaZero."""
+        if out_action is None:
+            out_action = np.zeros(self.count, dtype=np.int32)
+        if out_policy is None:
+            out_policy = np.zeros((self.count, self._cells), dtype=np.float32)
+        self._check(self._lib.twixt_mcts_gumbel_stats(
+            self._h, _ptr(out_action, _dt(np.int32, "int32"), self.count),
+            _ptr(out_policy, _dt(np.float32, "float32"), self.count * self._cells)))
+        return out_action, out_policy
+
     def set_root_priors(self, priors):
         """PUCT only: replaces P(a) of every root edge of each tree whose root is expanded with priors [count, n*n]
         float32 (e.g. root Dirichlet noise after `advance`).  Trees whose root is not expanded are left alone: their
@@ -205,6 +247,17 @@ class BatchedMCTS:
             priors = np.ascontiguousarray(priors, dtype=np.float32)
         self._check(self._lib.twixt_mcts_set_root_priors(
             self._h, _ptr(priors, _dt(np.float32, "float32"), self.count * self._cells)))
+
+
+def gumbel_noise(count: int, cells: int, generator=None, device=None):
+    """Gumbel(0, 1) noise [count, cells] float32 for `BatchedMCTS.set_root_gumbel`: -log(-log U) with U uniform
+    in (0, 1), drawn in float64 with torch's generator (reproducible under torch.manual_seed or with `generator`),
+    on `device` (default: the CPU)."""
+    import torch
+    u = torch.rand((int(count), int(cells)), dtype=torch.float64, generator=generator,
+                   device=device if device is not None else "cpu")
+    u = u.clamp_min(torch.finfo(torch.float64).tiny)  # rand is in [0, 1): keep log(0) out
+    return (-torch.log(-torch.log(u))).float()
 
 
 def add_dirichlet_noise(priors, legal_mask, epsilon: float, alpha: float):
