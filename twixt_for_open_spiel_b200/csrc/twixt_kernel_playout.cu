@@ -95,6 +95,12 @@ __host__ __device__ constexpr int playout_words(int n, bool cache_in_smem = fals
 #ifndef TW_FLOOD_OVERLAP
 #define TW_FLOOD_OVERLAP 1
 #endif
+// -DTW_PLAYOUT_MAX_BLOCKS=b (b > 0) caps the persistent grid at b blocks: a TEST variant (never the product
+// build) in which every lane plays many envs in a row through the ticket counter, so the hand-over from one
+// game to the next is exercised ten or more times per lane instead of once or twice.
+#ifndef TW_PLAYOUT_MAX_BLOCKS
+#define TW_PLAYOUT_MAX_BLOCKS 0
+#endif
 
 // The env's planes in shared memory (stride 32 words) + its blocked plane in HBM.
 template <int NT>
@@ -520,6 +526,7 @@ cudaError_t launch_nt(const PlayoutArgs& a, cudaStream_t s) {
   int64_t blocks = (a.count + kEnvsPerBlock - 1) / kEnvsPerBlock;
   const int64_t resident = static_cast<int64_t>(g_num_sms > 0 ? g_num_sms : 148) * per_sm;
   if (blocks > resident) blocks = resident;
+  if (TW_PLAYOUT_MAX_BLOCKS > 0 && blocks > TW_PLAYOUT_MAX_BLOCKS) blocks = TW_PLAYOUT_MAX_BLOCKS;
   if (getenv("TWIXT_B200_DEBUG") != nullptr)
     fprintf(stderr, "[twixt_b200] playout n=%d: %lld blocks x %d threads, %zu B smem, %d blocks/SM resident\n", a.n,
             static_cast<long long>(blocks), kLaunchThreads, smem, per_sm);
