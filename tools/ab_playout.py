@@ -3,12 +3,15 @@
 
     python tools/ab_playout.py build  name=-DFLAG=1,-DOTHER=0 ...   # here (CPU): builds tests/_build/variants/<name>.so
     python tools/ab_playout.py run [n[,n..]] [envs] [reps] [rounds]  # on the GPU box: times every variant found
+    python tools/ab_playout.py records                               # on the GPU box: record digests per variant
 
 Each variant runs in its own process (the library is chosen once per process through TWIXT_B200_LIB), is first
 checked against the oracle on 96 complete games, then timed with CUDA events on the launching stream: `reps`
 launches of reset + playout of `envs` fresh games, each with its own seed; prints min / median ms per launch.
 A list of board sizes is timed size by size in each process; the variants alternate for `rounds` rounds
-(default 2)."""
+(default 2).  `records` prints, per variant and board size 5..24, a digest of every exported record after playouts
+from fresh and from mid-game starting states (and of their returns and lengths): equal digests = bit-identical
+results."""
 import os
 import subprocess
 import sys
@@ -70,6 +73,40 @@ def child_one(n, envs, reps):
         n, bad, ms[0], ms[len(ms) // 2], plies, plies / ms[len(ms) // 2] / 1e6))
 
 
+def child_records():
+    import hashlib
+    import numpy as np
+    from twixt_for_open_spiel_b200 import TwixTBatch
+    for n in range(5, 25):
+        envs = 4096
+        b = TwixTBatch(n, envs, 0, 0x7477697854)
+        h = hashlib.sha256()
+        for rnd in range(3):
+            b.set_seed(0x7477697854 + rnd)
+            b.reset()
+            if rnd > 0:  # mid-game starts: ranges of envs stopped after 1 .. 60 plies, then played to the end
+                for d in range(1, 61):
+                    lo, hi = (d - 1) * envs // 60, d * envs // 60
+                    b.playout(lo, hi - lo, max_plies=d * rnd, want_returns=False, want_lengths=False)
+                b.set_seed(0x7477697854 + 100 + rnd)
+            rets, lens, _ = b.playout()
+            for a in (b.export_state(), rets, lens):
+                h.update(np.ascontiguousarray(a).tobytes())
+        b.close()
+        print("RESULT n=%d records %s" % (n, h.hexdigest()[:32]), flush=True)
+
+
+def run_records():
+    names = sorted(f for f in os.listdir(VDIR) if f.endswith(".so"))
+    for name in names:
+        env = dict(os.environ, TWIXT_B200_LIB=os.path.join(VDIR, name))
+        res = subprocess.run([sys.executable, os.path.abspath(__file__), "child_records"], capture_output=True,
+                             text=True, env=env, timeout=1200)
+        lines = [l for l in res.stdout.splitlines() if l.startswith("RESULT")]
+        for line in lines or ["FAILED: " + res.stderr[-400:]]:
+            print("%-28s %s" % (name, line), flush=True)
+
+
 def child_kernels():
     """the per-call kernels (bench.py's kernel section) with the library of this process"""
     import json
@@ -117,6 +154,10 @@ if __name__ == "__main__":
         build(sys.argv[2:])
     elif sys.argv[1] == "child_kernels":
         child_kernels()
+    elif sys.argv[1] == "child_records":
+        child_records()
+    elif sys.argv[1] == "records":
+        run_records()
     elif sys.argv[1] == "kernels":
         run_kernels()
     elif sys.argv[1] == "child":

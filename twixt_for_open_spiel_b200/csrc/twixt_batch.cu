@@ -115,6 +115,7 @@ class TwixTBatch {
     if (stream_ != nullptr) cudaStreamSynchronize(stream_);
     if (records_ != nullptr) cudaFree(records_);
     if (d_stats_ != nullptr) cudaFree(d_stats_);
+    if (playout_start_ != nullptr) cudaFree(playout_start_);
     if (pinned_ != nullptr) cudaFreeHost(pinned_);
     for (int k = 0; k < kSlots; ++k)
       if (slot_[k] != nullptr) cudaFree(slot_[k]);
@@ -452,9 +453,12 @@ class TwixTBatch {
     a.trace_plies = out_actions ? trace_plies : 0;
     a.stats = d_stats_;
     a.tickets = &d_stats_->tickets;
+    const bool derive = n_ >= kPlayoutDeriveMinN;
+    a.start = nullptr;
+    if (derive) TW_TRY(PlayoutStart(count, &a.start));
     TW_CUDA(cudaMemsetAsync(&d_stats_->tickets, 0, sizeof(unsigned long long), stream_));
-    TW_CUDA(launch_playout(a, stream_));
-    launches_ += 1;
+    TW_CUDA(launch_playout(a, stream_));  // the playout kernel (+ the blocked-plane pass)
+    launches_ += derive ? 2 : 1;
     TW_TRY(Finish(&ret));
     TW_TRY(Finish(&len));
     TW_TRY(Finish(&act));
@@ -566,6 +570,26 @@ class TwixTBatch {
     return TWIXT_OK;
   }
 
+  // the playout's scratch for the blocked-plane pass (PlayoutArgs::start), grown to `count` envs
+  int PlayoutStart(int64_t count, uint32_t** out) {
+    const size_t bytes = static_cast<size_t>(playout_scratch_words(count, n_)) * sizeof(uint32_t);
+    if (bytes > playout_start_cap_) {
+      TW_CUDA(cudaStreamSynchronize(stream_));
+      if (playout_start_ != nullptr) cudaFree(playout_start_);
+      playout_start_ = nullptr;
+      playout_start_cap_ = 0;
+      cudaError_t e = cudaMalloc(&playout_start_, bytes);
+      if (e != cudaSuccess) {
+        cudaGetLastError();
+        playout_start_ = nullptr;
+        return fail(TWIXT_ENOMEM, "cudaMalloc of %zu playout scratch bytes failed: %s", bytes, cudaGetErrorString(e));
+      }
+      playout_start_cap_ = bytes;
+    }
+    *out = playout_start_;
+    return TWIXT_OK;
+  }
+
   int SlotAlloc(size_t bytes, void** out) {
     if (next_slot_ >= kSlots) return fail(TWIXT_ENOMEM, "internal: out of staging slots");
     const int k = next_slot_++;
@@ -640,6 +664,8 @@ class TwixTBatch {
   bool validate_ = true;
   uint32_t* records_ = nullptr;
   DeviceStats* d_stats_ = nullptr;
+  uint32_t* playout_start_ = nullptr;  // see PlayoutStart
+  size_t playout_start_cap_ = 0;
   cudaStream_t stream_ = nullptr;
   bool own_stream_ = false;
   // pinned, device-mapped arena for small host transfers
@@ -850,6 +876,7 @@ class TwixTMCTS {
     p.trace_plies = 0;
     p.stats = b.d_stats_;
     p.tickets = &b.d_stats_->tickets;
+    p.start = nullptr;  // rollout records are discarded after their returns are read: no blocked-plane pass
     for (int32_t i = 0; i < num_simulations; i += K_) {  // one step: K simulations of every tree
       const uint32_t k = static_cast<uint32_t>(sims_);
       if (gumbel_) TW_CUDA(launch_mcts_gumbel_select(a_, gm_, count_, stream0_, k, nullptr, nullptr, b.stream_));

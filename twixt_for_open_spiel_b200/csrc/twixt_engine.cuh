@@ -519,7 +519,9 @@ TW_HD Placement begin_move(B& b, Header& h, int x, int y, uint32_t own_word = 0u
 // directions are handled direction-major with compile-time offsets and crossing
 // masks, all inputs fetched up front by independent loads; kAlways = true drops
 // even the `any candidate?` branch so the whole function is one basic block.
-template <bool kAlways, class B>
+// kBlocked = false leaves the blocked plane alone: the fused playout kernel
+// derives it from the final position instead (derive_blocked_word below).
+template <bool kAlways, bool kBlocked = true, class B>
 TW_HD bool link_move(B& b, const Placement& p, uint32_t& pending) {
   const int n = b.n();
   const int x = p.x, y = p.y;
@@ -602,7 +604,7 @@ TW_HD bool link_move(B& b, const Placement& p, uint32_t& pending) {
     to_start |= hit_s != 0u;
     to_end |= hit_e != 0u;
     neutral = hit_n != 0u;
-    b.or_blocked3(x, blk);
+    if constexpr (kBlocked) b.or_blocked3(x, blk);
     // the new peg's own flag words are fs[2] / fe[2]
     b.st_if(to_start, P_START, x, fs[2] | bit);
     b.st_if(to_end, P_END, x, fe[2] | bit);
@@ -612,6 +614,25 @@ TW_HD bool link_move(B& b, const Placement& p, uint32_t& pending) {
   }
   pending = (new_links && neutral) ? ((to_start ? kFloodStart : 0u) | (to_end ? kFloodEnd : 0u)) : 0u;
   return to_start && to_end;
+}
+
+// The blocked plane from the position, one column word at a time.  Links are only made when a peg is placed
+// and never removed, and when the second peg of an own-colour knight pair is placed the link between them is
+// either made or refused as crossed, which sets the blocked bit on the pair's WEST endpoint (link_move above;
+// the swap at ply 1 comes before any pair exists).  So in a position reached by play the bit of (x, y) is set iff
+// the peg there has an own-colour peg at one of the east knight offsets NNE (+1,+2), ENE (+2,+1), ESE (+2,-1),
+// SSE (+1,-2) and no link is stored at (x, y) in that direction (link plane P_LINK0 + 0..3).
+// pegs0..2: ONE colour's peg words of the columns x, x+1, x+2 (0 off the board); link[d]: the link words of
+// column x; fresh0..2: the pegs of pegs0..2 placed since the plane was last exact.  Only pairs with a fresh peg
+// are counted: a pair that was already on the board was judged by the rules back then (or, in a record built
+// by hand, never), and its bit is whatever the plane already holds.
+TW_HD uint32_t derive_blocked_word(uint32_t pegs0, uint32_t pegs1, uint32_t pegs2, uint32_t fresh0, uint32_t fresh1,
+                                   uint32_t fresh2, const uint32_t link[4]) {
+  const uint32_t nne = (pegs1 >> 2) & ~link[0] & (fresh0 | (fresh1 >> 2));
+  const uint32_t ene = (pegs2 >> 1) & ~link[1] & (fresh0 | (fresh2 >> 1));
+  const uint32_t ese = (pegs2 << 1) & ~link[2] & (fresh0 | (fresh2 << 1));
+  const uint32_t sse = (pegs1 << 2) & ~link[3] & (fresh0 | (fresh1 << 2));
+  return pegs0 & (nne | ene | ese | sse);
 }
 
 TW_HD void finish_move(Header& h, const Placement& p, bool win) {

@@ -38,8 +38,14 @@
 // 784 B at n = 24: nine warps fit on an SM); the
 // per-column count cache that replaces the 24-word legal scan by 6 bytewise
 // words (twixt_engine.cuh, count_cache_*) lives in registers.  The "blocked
-// neighbour" plane is write-only for the rules, so it stays in HBM and is
-// OR-ed in place (RED.OR, fire-and-forget).
+// neighbour" plane is write-only for the rules and follows from the final
+// position (derive_blocked_word).  From n = kPlayoutDeriveMinN on the moves
+// leave it alone in HBM: the kernel only notes each env's starting ply --
+// and, from ply 2 on, its occupied cells -- in PlayoutArgs::start, and
+// derive_blocked_kernel (twixt_kernels_api.cu, launched right after this
+// kernel by launch_playout) ORs in the bits of the pairs this launch formed.
+// On the smaller boards, where games are too short for that pass to pay,
+// every move ORs its bits in place (RED.OR, fire-and-forget).
 //
 // Reference loop reproduced: upstream example.cc / RandomRolloutEvaluator
 // (LegalActions -> uniform pick -> ApplyAction until IsTerminal), with the
@@ -102,11 +108,11 @@ __host__ __device__ constexpr int playout_words(int n, bool cache_in_smem = fals
 #define TW_PLAYOUT_MAX_BLOCKS 0
 #endif
 
-// The env's planes in shared memory (stride 32 words) + its blocked plane in HBM.
+// The env's planes in shared memory (stride 32 words) + below kPlayoutDeriveMinN its blocked plane in HBM.
 template <int NT>
 struct PlayoutRef {
   uint32_t* p;     // smem, this lane's column
-  uint32_t* gblk;  // global: the record's P_BLOCKED words
+  uint32_t* gblk;  // global: the record's P_BLOCKED words (n < kPlayoutDeriveMinN only)
 #if TW_PLAYOUT_BOUNDS_CHECK
   unsigned long long* viol;
   __device__ __forceinline__ int chk(int word) const {
@@ -159,12 +165,10 @@ struct PlayoutRef {
   __device__ __forceinline__ uint32_t ld_pegs(int plane, int col) const { return ld(plane ^ 1, col); }
   __device__ __forceinline__ void st_pegs(int plane, int col, uint32_t v) { st(plane ^ 1, col, v); }
   __device__ __forceinline__ uint32_t ld_pegs_guard(int plane, int col) const { return ld_guard(plane ^ 1, col); }
-  // fire-and-forget reduction (RED.OR): no load to wait for; only this thread touches the word
-  __device__ __forceinline__ void or_blocked(int col, uint32_t bits) { atomicOr(gblk + chk_col(col), bits); }
-  // Three UNCONDITIONAL reductions per move: OR-ing zero bits is harmless (and a column left of the board
-  // only ever gets zero bits: its address is clamped).  ptxas cannot predicate a RED -- every conditional
-  // one becomes its own branch region (three of them cost 9 %), and even one branch around all three
-  // (taken by half of the moves) was 2.5 % slower than always issuing them.
+  // Three UNCONDITIONAL fire-and-forget reductions (RED.OR) per move: OR-ing zero bits is harmless (and a column
+  // left of the board only ever gets zero bits: its address is clamped).  ptxas cannot predicate a RED -- every
+  // conditional one becomes its own branch region (three of them cost 9 %), and even one branch around all
+  // three (taken by half of the moves) was 2.5 % slower than always issuing them.
   __device__ __forceinline__ void or_blocked3(int x, const uint32_t blk[3]) {
     atomicOr(gblk + chk_col(x), blk[0]);
     atomicOr(gblk + chk_col(max(x - 1, 0)), blk[1]);
@@ -228,6 +232,7 @@ __host__ __device__ constexpr int playout_min_blocks(int nt) {
 template <int NT, bool kTrace>
 __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) playout_kernel(const PlayoutArgs a) {
   constexpr int kThreads = playout_threads(NT);
+  constexpr bool kDerive = NT >= kPlayoutDeriveMinN;  // blocked plane by derive_blocked_kernel (a.start is set)
   extern __shared__ uint4 smem_raw[];
   uint32_t* smem = reinterpret_cast<uint32_t*>(smem_raw);
   const int n = NT > 0 ? NT : a.n;
@@ -317,7 +322,8 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
   auto finish_take = [&]() {
     __pipeline_wait_prior(0);
     unpack_header(pad[0], pad[32], pad[64], pad[96], h);
-    b.gblk = grec + kHeaderWords + P_BLOCKED * n;
+    if (!kDerive) b.gblk = grec + kHeaderWords + P_BLOCKED * n;
+    else if (a.start != nullptr) a.start[idx] = min(h.ply, 2u);
     const uint64_t stream = a.stream_ids != nullptr ? a.stream_ids[idx] : a.stream_base + static_cast<uint64_t>(idx);
     s_lo = static_cast<uint32_t>(stream);
     s_hi = static_cast<uint32_t>(stream >> 32);
@@ -341,6 +347,11 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
       spegs[0] = spegs[1] = 0u;  // an empty board
     } else {
       count_cache_build(b);
+      if (kDerive && a.start != nullptr && h.ply >= 2u) {  // the cells whose pairs the rules have already judged
+        uint32_t* occ = a.start + a.count + idx * n;
+#pragma unroll 1
+        for (int x = 0; x < n; ++x) occ[x] = b.ld_pegs(P_RED, x) | b.ld_pegs(P_BLUE, x);
+      }
       if (playing)
         select_legal(b, h, static_cast<int>(playout_index(word_at(0u), static_cast<uint32_t>(legal_count(h, n)))), sx, sy, spegs);
     }
@@ -444,7 +455,7 @@ __global__ void __launch_bounds__(playout_threads(NT), playout_min_blocks(NT)) p
       int nx, ny;
       select_legal(b, hn, static_cast<int>(playout_index(word_at(static_cast<uint32_t>(step) + 1u), static_cast<uint32_t>(ln))), nx, ny, spegs);
       uint32_t owed;
-      const bool win = link_move</*kAlways=*/true>(b, pl, owed);
+      const bool win = link_move</*kAlways=*/true, /*kBlocked=*/!kDerive>(b, pl, owed);
       finish_move(h, pl, win);
       pend |= owed << (2 * pl.player);
       const uint32_t peg_col = 1u << pl.x;

@@ -49,7 +49,21 @@ struct PlayoutArgs {
   int trace_plies;
   DeviceStats* stats;
   unsigned long long* tickets;  // &stats->tickets
+  // From n = kPlayoutDeriveMinN on, the kernel does not maintain P_BLOCKED: launch_playout derives it after the
+  // kernel from the final planes (derive_blocked_word) when this is set, and leaves it stale when it is nullptr
+  // (records nobody reads again, such as MCTS rollouts).  playout_scratch_words(count, n) words; the playout
+  // kernel writes, when it takes env i:
+  //   start[i]                    min(ply, 2) of the starting position
+  //   start[count + i*n + x]      its occupied cells of column x (ply >= 2 only: earlier, no pair exists yet)
+  uint32_t* start;
 };
+
+// The smallest board whose playout derives the blocked plane after the kernel.  Below it games are short and the
+// pass's bytes per env cost more than the three reductions per move it replaces (n = 8: +2.3 % per launch with the
+// pass, n = 12: -5.1 %; profiles/r4_playout_derive_blocked_ab.txt), so those kernels keep the per-move rule.
+constexpr int kPlayoutDeriveMinN = 10;
+
+inline int64_t playout_scratch_words(int64_t count, int n) { return count * (1 + n); }
 
 // Device arena of a batched MCTS search (twixt_mcts.cu; sizes and byte formula in twixt_mcts.cuh).  Tree t owns
 // node slots [t*S, (t+1)*S) (slot 0 of a tree is its root), path entries [t*P, (t+1)*P) and rollout slots

@@ -844,6 +844,82 @@ cudaError_t launch_observation(const uint32_t* records, int64_t count, int n, fl
   return cudaGetLastError();
 }
 
+// ------------------------------------------------------ blocked derivation ---
+// Runs right after the fused playout kernel on the same records: ORs into P_BLOCKED the bits of every knight pair
+// the launch formed (derive_blocked_word), which the kernel's moves no longer write.  The kernel leaves, per env,
+// the starting ply clamped to 2 and -- for ply >= 2 -- the cells occupied at the start (PlayoutArgs::start):
+//   0  the board was empty, so P_BLOCKED was zero: the derived plane is stored as it is
+//   1  one red peg, no pair yet: every pair is new, the derived bits are OR-ed into the plane
+//   2  only pairs with a peg on a cell that was empty at the start are counted (a record built by hand may hold
+//      an unlinked pair without its bit, which the per-move rules never examine and so never set)
+// HBM-bound: one warp per kDeriveEnvs envs reads their peg and link planes (6n words each, the span right after the
+// header) with 16-byte loads into shared memory, then lane = column forms the words; the plane is only read back
+// for envs that did not start empty.
+constexpr int kDeriveWarps = 8, kDeriveEnvs = 4;
+constexpr int kDeriveQuads = (6 * TWIXT_MAX_BOARD_SIZE + 3) / 4;  // per env: RED, BLUE, LINK0..3
+constexpr int kDeriveLoads = (kDeriveEnvs * kDeriveQuads + 31) / 32;
+
+__global__ void __launch_bounds__(kDeriveWarps * 32) derive_blocked_kernel(uint32_t* __restrict__ records,
+                                                                           int64_t count, int n, int rw,
+                                                                           const uint32_t* __restrict__ start) {
+  __shared__ uint4 planes[kDeriveWarps][kDeriveEnvs * kDeriveQuads];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t first = (blockIdx.x * static_cast<int64_t>(kDeriveWarps) + warp) * kDeriveEnvs;
+  if (first >= count) return;  // whole warp leaves together
+  const int envs = count - first < kDeriveEnvs ? static_cast<int>(count - first) : kDeriveEnvs;
+  const int quads = (6 * n + 3) / 4;  // the span may end inside P_START (odd n): those words are not used
+  uint32_t* const rec0 = records + first * rw;
+  // every load of the group first, then the shared-memory stores
+  uint4 v[kDeriveLoads];
+  const uint32_t mode = lane < envs ? start[first + lane] : 0u;
+#pragma unroll
+  for (int j = 0; j < kDeriveLoads; ++j) {
+    const int i = lane + 32 * j, e = i / quads;
+    if (e < envs) v[j] = __ldg(reinterpret_cast<const uint4*>(rec0 + e * rw + kHeaderWords) + (i - e * quads));
+  }
+  // the plane words and start cells of the envs that did not start empty, requested together (one round trip)
+  const int x = lane;
+  const bool on = x < n;
+  uint32_t old[kDeriveEnvs], occ[kDeriveEnvs];
+#pragma unroll
+  for (int e = 0; e < kDeriveEnvs; ++e) {
+    const uint32_t m = __shfl_sync(kFullMask, mode, e);  // warp-uniform
+    old[e] = (e < envs && m != 0u && on) ? rec0[e * rw + kHeaderWords + P_BLOCKED * n + x] : 0u;
+    occ[e] = (e < envs && m == 2u && on) ? start[count + (first + e) * n + x] : 0u;
+  }
+  uint32_t* const sw = reinterpret_cast<uint32_t*>(planes[warp]);
+#pragma unroll
+  for (int j = 0; j < kDeriveLoads; ++j) {
+    const int i = lane + 32 * j, e = i / quads;
+    if (e < envs) reinterpret_cast<uint4*>(sw + e * 4 * quads)[i - e * quads] = v[j];
+  }
+  __syncwarp();
+#pragma unroll
+  for (int e = 0; e < kDeriveEnvs; ++e) {
+    if (e >= envs) break;  // warp-uniform
+    const uint32_t* s = sw + e * 4 * quads;
+    const uint32_t occ1 = __shfl_down_sync(kFullMask, occ[e], 1), occ2 = __shfl_down_sync(kFullMask, occ[e], 2);
+    uint32_t bits = 0u;
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {  // P_RED, P_BLUE
+      const uint32_t p0 = on ? s[c * n + x] : 0u, p1 = x + 1 < n ? s[c * n + x + 1] : 0u;
+      const uint32_t p2 = x + 2 < n ? s[c * n + x + 2] : 0u;
+      const uint32_t link[4] = {on ? s[(P_LINK0 + 0) * n + x] : 0u, on ? s[(P_LINK0 + 1) * n + x] : 0u,
+                                on ? s[(P_LINK0 + 2) * n + x] : 0u, on ? s[(P_LINK0 + 3) * n + x] : 0u};
+      bits |= derive_blocked_word(p0, p1, p2, p0 & ~occ[e], p1 & ~occ1, p2 & ~occ2, link);
+    }
+    if (on) rec0[e * rw + kHeaderWords + P_BLOCKED * n + x] = old[e] | bits;
+  }
+}
+
+cudaError_t launch_derive_blocked(uint32_t* records, int64_t count, int n, const uint32_t* start, cudaStream_t s) {
+  if (count <= 0) return cudaSuccess;
+  const int64_t blocks = (count + kDeriveWarps * kDeriveEnvs - 1) / (kDeriveWarps * kDeriveEnvs);
+  derive_blocked_kernel<<<static_cast<unsigned>(blocks), kDeriveWarps * 32, 0, s>>>(records, count, n,
+                                                                                      record_words(n), start);
+  return cudaGetLastError();
+}
+
 // The fused playout kernel: one compiled form per board size, in five translation units (size groups).
 cudaError_t playout_setup() {
   cudaError_t e;
@@ -856,13 +932,16 @@ cudaError_t playout_setup() {
 
 cudaError_t launch_playout(const PlayoutArgs& a, cudaStream_t s) {
   if (a.n < TWIXT_MIN_BOARD_SIZE || a.n > TWIXT_MAX_BOARD_SIZE) return cudaErrorInvalidValue;
+  cudaError_t e;
   switch ((a.n - TWIXT_MIN_BOARD_SIZE) % 5) {
-    case 0: return launch_playout_g0(a, s);
-    case 1: return launch_playout_g1(a, s);
-    case 2: return launch_playout_g2(a, s);
-    case 3: return launch_playout_g3(a, s);
-    default: return launch_playout_g4(a, s);
+    case 0: e = launch_playout_g0(a, s); break;
+    case 1: e = launch_playout_g1(a, s); break;
+    case 2: e = launch_playout_g2(a, s); break;
+    case 3: e = launch_playout_g3(a, s); break;
+    default: e = launch_playout_g4(a, s); break;
   }
+  if (e != cudaSuccess || a.start == nullptr || a.n < kPlayoutDeriveMinN) return e;
+  return launch_derive_blocked(a.records, a.count, a.n, a.start, s);
 }
 
 }  // namespace twixt

@@ -6,7 +6,8 @@
 //                        simulation first reaches, and write the leaf record to its evaluator: R rollout slots
 //                        (built-in evaluator) or a batch env (stepwise form)
 //   launch_playout       the EXISTING fused playout kernel over the rollout slots, with the stream ids the
-//                        select kernel wrote (twixt_kernel_playout.cu, unchanged)
+//                        select kernel wrote (twixt_kernel_playout.cu, unchanged; without the blocked-plane
+//                        pass of twixt_playout, since only the returns of a rollout are read)
 //   mcts_backup_kernel   the leaf value (mean rollout return, caller's value or terminal Returns()) added to
 //                        every edge on the path, lanes over the path; a PUCT search expands the leaf here, a
 //                        solver search proves nodes up the path from a terminal leaf
