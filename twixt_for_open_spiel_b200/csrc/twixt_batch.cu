@@ -13,8 +13,10 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/twixt_b200.h"
@@ -301,9 +303,7 @@ class TwixTBatch {
     TW_CUDA(launch_legal_actions(rec(first), count, n_, acts.dev, elem_bytes, stride,
                                  static_cast<int32_t*>(cnts.dev), stream_));
     launches_ += 1;
-    TW_TRY(Finish(&acts));
-    TW_TRY(Finish(&cnts));
-    return SyncIfHost(acts, cnts);
+    return FinishOutputs({&acts, &cnts});
   }
 
   int LegalMask(int64_t first, int64_t count, uint8_t* out) {
@@ -316,8 +316,7 @@ class TwixTBatch {
     TW_TRY(StageOut(out, static_cast<size_t>(count) * n_ * n_, &m, false));
     TW_CUDA(launch_legal_mask(rec(first), count, n_, static_cast<uint8_t*>(m.dev), stream_));
     launches_ += 1;
-    TW_TRY(Finish(&m));
-    return SyncIfHost(m, m);
+    return FinishOutputs({&m});
   }
 
   int Apply(int64_t first, int64_t count, const int32_t* actions, int32_t* out_status) {
@@ -333,32 +332,13 @@ class TwixTBatch {
     else TW_TRY(StageOut(out_status, status_bytes, &st, false));
     // Where the statuses end up in host-visible memory the first illegal action is found by reading them;
     // otherwise the kernel's device-side flag is reset, and read back after the launch.
-    const bool scan_host = st.pin != nullptr;
-    if (!scan_host) TW_CUDA(cudaMemsetAsync(&d_stats_->illegal_index, 0xFF, sizeof(unsigned int), stream_));
+    if (st.pin == nullptr) TW_CUDA(cudaMemsetAsync(&d_stats_->illegal_index, 0xFF, sizeof(unsigned int), stream_));
     TW_CUDA(launch_apply(rec(first), count, n_, static_cast<const int32_t*>(in.dev), static_cast<int32_t*>(st.dev),
                          d_stats_, stream_));
     launches_ += 1;
     TW_TRY(Finish(&st));
     if (out_status != nullptr && !st.host) return TWIXT_OK;  // fully asynchronous: caller inspects the statuses
-    int64_t bad = -1;
-    if (scan_host) {
-      TW_TRY(Sync());
-      const int32_t* seen = static_cast<const int32_t*>(st.pin);
-      for (int64_t i = 0; i < count && bad < 0; ++i)
-        if (seen[i] == 1) bad = i;
-    } else {
-      unsigned int flag = 0xFFFFFFFFu;
-      TW_CUDA(cudaMemcpyAsync(&flag, &d_stats_->illegal_index, sizeof(flag), cudaMemcpyDeviceToHost, stream_));
-      TW_TRY(Sync());
-      if (flag != 0xFFFFFFFFu) bad = flag;
-    }
-    if (bad >= 0) {
-      int32_t a = 0;
-      if (in.host) a = actions[bad];
-      else TW_CUDA(cudaMemcpy(&a, actions + bad, sizeof(a), cudaMemcpyDeviceToHost));
-      return fail(TWIXT_EILLEGAL, "Not a legal action: %d", a);  // twixt.h:96, same text
-    }
-    return TWIXT_OK;
+    return ReportIllegal(st, in, actions, count);
   }
 
   int Query(int64_t first, int64_t count, int8_t* player, uint8_t* terminal, float* returns) {
@@ -373,11 +353,7 @@ class TwixTBatch {
     TW_CUDA(launch_query(rec(first), count, n_, static_cast<int8_t*>(p.dev), static_cast<uint8_t*>(t.dev),
                          static_cast<float*>(r.dev), stream_));
     launches_ += 1;
-    TW_TRY(Finish(&p));
-    TW_TRY(Finish(&t));
-    TW_TRY(Finish(&r));
-    if (p.host || t.host || r.host) TW_TRY(Sync());
-    return TWIXT_OK;
+    return FinishOutputs({&p, &t, &r});
   }
 
   // out_mask != nullptr: the fused producer (tensor + legal mask in one pass over the records)
@@ -393,9 +369,7 @@ class TwixTBatch {
     TW_CUDA(launch_observation(rec(first), count, n_, static_cast<float*>(o.dev), static_cast<uint8_t*>(m.dev),
                                stream_));
     launches_ += 1;
-    TW_TRY(Finish(&o));
-    TW_TRY(Finish(&m));
-    return SyncIfHost(o, m);
+    return FinishOutputs({&o, &m});
   }
 
   int Replay(int64_t first, int64_t count, const int32_t* actions, int64_t stride, const int32_t* lengths,
@@ -650,9 +624,39 @@ class TwixTBatch {
     return TWIXT_OK;
   }
 
-  int SyncIfHost(const Staged& a, const Staged& b) {
-    if (a.host || b.host) TW_TRY(Sync());
+  // Finishes every staged output, then synchronises once if any of them is host memory
+  int FinishOutputs(std::initializer_list<Staged*> outs) {
+    bool host = false;
+    for (Staged* s : outs) {
+      TW_TRY(Finish(s));
+      host = host || s->host;
+    }
+    if (host) TW_TRY(Sync());
     return TWIXT_OK;
+  }
+
+  // After a launch that marks an illegal action with status 1 (apply's statuses, tree advance's kRootIllegal) and
+  // lowers d_stats_->illegal_index to its position: the first one from the statuses where they are in the pinned
+  // arena (st.pin), else from the device flag, named as twixt.h:96 names it.  Synchronises the stream.
+  int ReportIllegal(const Staged& st, const Staged& in, const int32_t* actions, int64_t count) {
+    static_assert(kRootIllegal == 1, "apply and tree advance mark an illegal action alike");
+    int64_t bad = -1;
+    if (st.pin != nullptr) {
+      TW_TRY(Sync());
+      const int32_t* seen = static_cast<const int32_t*>(st.pin);
+      for (int64_t i = 0; i < count && bad < 0; ++i)
+        if (seen[i] == 1) bad = i;
+    } else {
+      unsigned int flag = 0xFFFFFFFFu;
+      TW_CUDA(cudaMemcpyAsync(&flag, &d_stats_->illegal_index, sizeof(flag), cudaMemcpyDeviceToHost, stream_));
+      TW_TRY(Sync());
+      if (flag != 0xFFFFFFFFu) bad = flag;
+    }
+    if (bad < 0) return TWIXT_OK;
+    int32_t a = 0;
+    if (in.host) a = actions[bad];
+    else TW_CUDA(cudaMemcpy(&a, actions + bad, sizeof(a), cudaMemcpyDeviceToHost));
+    return fail(TWIXT_EILLEGAL, "Not a legal action: %d", a);  // twixt.h:96, same text
   }
 
   int n_ = 0;
@@ -734,38 +738,58 @@ class TwixTMCTS {
     const int cols = gumbel ? max_simulations - 1 : 0;
     std::vector<int32_t> considered(gumbel ? static_cast<size_t>(mc + 1) * cols : 0);
     for (int m = 0; gumbel && m <= mc; ++m) mcts_considered_visits(m, cols, considered.data() + static_cast<size_t>(m) * cols);
-    // carve one allocation; each array starts on a 256-byte boundary (priors and tie keys are PUCT's, the outcome
-    // bytes PUCT's and the solver's, the root codes the solver's, the virtual counts those of K > 1: empty
-    // otherwise).  Tree entries, paths and rollout slots are per leaf row: K per tree.
+    // One allocation, carved by the same list twice: a sizing pass, then (base set) the pointer pass.  Each array
+    // starts on a 256-byte boundary; those of other search kinds stay nullptr (priors and tie keys are PUCT's, the
+    // outcome bytes PUCT's and the solver's, the root codes the solver's, the virtual counts those of K > 1, the last
+    // four Gumbel's).  Tree entries, paths and rollout slots are per leaf row: K per tree.
     const int64_t T = num_trees, nodes = T * s.slots, edges = nodes * s.edges, rows = T * K, rolls = rows * s.rollouts;
-    const int64_t pe = puct ? edges : 0, oe = (puct || solve) ? edges : 0, rt = solve ? T : 0;
-    const int64_t vn = K > 1 ? nodes : 0, ve = K > 1 ? edges : 0;
-    const int64_t ge = gumbel ? edges : 0, gn = gumbel ? nodes : 0, gt = gumbel ? T * cells : 0;
-    const int64_t sizes[23] = {nodes * s.rw * 4, nodes * 4, nodes * 4, edges * 2, edges * 4, edges * 8, edges * 4,
-                               rows * 16, rows * s.path * 8, rolls * s.rw * 4, rolls * 8, rolls * 8, s.slots * 8,
-                               pe * 4, pe * 4, oe, rt, vn * 2, ve * 2,
-                               ge * 4, gn * 8, gt * 4, static_cast<int64_t>(considered.size()) * 4};
-    int64_t offs[23], total = 0;
-    for (int i = 0; i < 23; ++i) {
-      offs[i] = total;
-      total += (sizes[i] + 255) & ~static_cast<int64_t>(255);
-    }
+    char* base = nullptr;
+    int64_t total = 0;
+    auto take = [&](auto*& p, int64_t count, bool used = true) {  // count elements of *p
+      using E = std::remove_reference_t<decltype(*p)>;
+      p = used && base != nullptr ? reinterpret_cast<E*>(base + total) : nullptr;
+      if (used) total += (count * static_cast<int64_t>(sizeof(E)) + 255) & ~static_cast<int64_t>(255);
+    };
+    double* log_table = nullptr;
+    int32_t* considered_table = nullptr;
+    auto carve = [&] {
+      total = 0;
+      take(a_.node_rec, nodes * s.rw);
+      take(a_.node_legal, nodes);
+      take(a_.node_n, nodes);
+      take(a_.edge_action, edges);
+      take(a_.edge_n, edges);
+      take(a_.edge_w, edges);
+      take(a_.edge_child, edges);
+      take(a_.tree, rows);
+      take(a_.path, rows * s.path);
+      take(a_.roll_rec, rolls * s.rw);
+      take(a_.roll_ids, rolls);
+      take(a_.roll_ret, rolls * 2);
+      take(log_table, s.slots);
+      take(a_.edge_p, edges, puct);
+      take(a_.edge_key, edges, puct);
+      take(a_.edge_out, edges, puct || solve);
+      take(a_.root_out, T, solve);
+      take(a_.node_v, nodes, K > 1);
+      take(a_.edge_v, edges, K > 1);
+      take(gm_.edge_logit, edges, gumbel);
+      take(gm_.node_value, nodes, gumbel);
+      take(gm_.root_gumbel, T * cells, gumbel);
+      take(considered_table, static_cast<int64_t>(considered.size()), gumbel);
+    };
+    carve();
     DeviceGuard g(b->device_);
     size_t free_bytes = 0, total_bytes = 0;
     TW_CUDA(cudaMemGetInfo(&free_bytes, &total_bytes));
-    if (gumbel && static_cast<uint64_t>(total) > free_bytes)
-      return fail(TWIXT_ENOMEM,
-                  "Gumbel MCTS arena of %lld bytes (%lld trees x %lld bytes per tree = S*(rw*4 + 16 + 22*M) + 16 + 8*P "
-                  "+ R*(rw*4 + 16) + 4*n*n at n = %d, %d simulations, %d rollouts; plus a %lld-byte considered-visits "
-                  "table) exceeds the %zu bytes free on device %d",
-                  static_cast<long long>(total), static_cast<long long>(T), static_cast<long long>(per_tree), n,
-                  max_simulations, n_rollouts, static_cast<long long>(considered.size() * 4), free_bytes, b->device_);
     if (static_cast<uint64_t>(total) > free_bytes)
       return fail(TWIXT_ENOMEM,
-                  "MCTS arena of %lld bytes (%lld trees x %lld bytes per tree at n = %d, %d simulations, %d rollouts, "
-                  "%d leaves per step) exceeds the %zu bytes free on device %d",
-                  static_cast<long long>(total), static_cast<long long>(T), static_cast<long long>(per_tree), n,
-                  max_simulations, n_rollouts, K, free_bytes, b->device_);
+                  "%sMCTS arena of %lld bytes (%lld trees x %lld bytes per tree at n = %d, %d simulations, "
+                  "%d rollouts, %d leaves per step; plus a %lld-byte considered-visits table) exceeds the %zu bytes "
+                  "free on device %d",
+                  gumbel ? "Gumbel " : "", static_cast<long long>(total), static_cast<long long>(T),
+                  static_cast<long long>(per_tree), n, max_simulations, n_rollouts, K,
+                  static_cast<long long>(considered.size() * 4), free_bytes, b->device_);
     cudaError_t e = cudaMalloc(&arena_mem_, static_cast<size_t>(total));
     if (e != cudaSuccess) {
       cudaGetLastError();
@@ -773,55 +797,35 @@ class TwixTMCTS {
       return fail(TWIXT_ENOMEM, "cudaMalloc of %lld bytes for the MCTS arena failed: %s", static_cast<long long>(total),
                   cudaGetErrorString(e));
     }
-    char* base = static_cast<char*>(arena_mem_);
+    base = static_cast<char*>(arena_mem_);
+    carve();
     a_.n = n;
     a_.rw = static_cast<int>(s.rw);
     a_.M = static_cast<int>(s.edges);
     a_.S = static_cast<int>(s.slots);
     a_.P = static_cast<int>(s.path);
     a_.R = n_rollouts;
-    a_.node_rec = reinterpret_cast<uint32_t*>(base + offs[0]);
-    a_.node_legal = reinterpret_cast<int32_t*>(base + offs[1]);
-    a_.node_n = reinterpret_cast<uint32_t*>(base + offs[2]);
-    a_.edge_action = reinterpret_cast<uint16_t*>(base + offs[3]);
-    a_.edge_n = reinterpret_cast<uint32_t*>(base + offs[4]);
-    a_.edge_w = reinterpret_cast<double*>(base + offs[5]);
-    a_.edge_child = reinterpret_cast<int32_t*>(base + offs[6]);
-    a_.tree = reinterpret_cast<int4*>(base + offs[7]);
-    a_.path = reinterpret_cast<int2*>(base + offs[8]);
-    a_.roll_rec = reinterpret_cast<uint32_t*>(base + offs[9]);
-    a_.roll_ids = reinterpret_cast<uint64_t*>(base + offs[10]);
-    a_.roll_ret = reinterpret_cast<float*>(base + offs[11]);
-    double* table = reinterpret_cast<double*>(base + offs[12]);
-    a_.log_table = table;
-    a_.edge_p = puct ? reinterpret_cast<float*>(base + offs[13]) : nullptr;
-    a_.edge_key = puct ? reinterpret_cast<uint32_t*>(base + offs[14]) : nullptr;
-    a_.edge_out = (puct || solve) ? reinterpret_cast<uint8_t*>(base + offs[15]) : nullptr;
-    a_.root_out = solve ? reinterpret_cast<uint8_t*>(base + offs[16]) : nullptr;
-    a_.node_v = K > 1 ? reinterpret_cast<uint16_t*>(base + offs[17]) : nullptr;
-    a_.edge_v = K > 1 ? reinterpret_cast<uint16_t*>(base + offs[18]) : nullptr;
+    a_.log_table = log_table;
     a_.K = K;
     a_.vl = virtual_loss;
     K_ = K;
     gumbel_ = gumbel;
     if (gumbel) {
-      gm_.edge_logit = reinterpret_cast<float*>(base + offs[19]);
-      gm_.node_value = reinterpret_cast<double*>(base + offs[20]);
-      gm_.root_gumbel = reinterpret_cast<float*>(base + offs[21]);
-      gm_.table = reinterpret_cast<const int32_t*>(base + offs[22]);
+      gm_.table = considered_table;
       gm_.max_considered = mc;
       gm_.cols = cols;
       gm_.c_visit = c_visit;
       gm_.c_scale = c_scale;
       if (!considered.empty())
-        TW_CUDA(cudaMemcpyAsync(base + offs[22], considered.data(), considered.size() * sizeof(int32_t),
+        TW_CUDA(cudaMemcpyAsync(considered_table, considered.data(), considered.size() * sizeof(int32_t),
                                 cudaMemcpyHostToDevice, b->stream_));
     }
     log_size_ = s.slots;
     // ln N(s) from the host's libm, so that a CPU restatement of the search computes the same scores
     std::vector<double> logs(static_cast<size_t>(s.slots));
     for (size_t i = 0; i < logs.size(); ++i) logs[i] = std::log(static_cast<double>(i));
-    TW_CUDA(cudaMemcpyAsync(table, logs.data(), logs.size() * sizeof(double), cudaMemcpyHostToDevice, b->stream_));
+    TW_CUDA(cudaMemcpyAsync(log_table, logs.data(), logs.size() * sizeof(double), cudaMemcpyHostToDevice,
+                            b->stream_));
     TW_CUDA(cudaStreamSynchronize(b->stream_));
     return TWIXT_OK;
   }
@@ -916,9 +920,7 @@ class TwixTMCTS {
     pending_ = true;
     leaf_first_ = leaf_first;
     node_bound_ += K_;
-    TW_TRY(b.Finish(&st));
-    if (st.host) TW_TRY(b.Sync());
-    return TWIXT_OK;
+    return b.FinishOutputs({&st});
   }
 
   // values [count*K, 2], priors: [count*K, n*n] float32 or nullptr (uniform); host priors are checked before anything
@@ -930,16 +932,8 @@ class TwixTMCTS {
     if (priors != nullptr && a_.edge_p == nullptr && !gumbel_)
       return fail(TWIXT_EINVAL, "twixt_mcts_backup_priors: priors given to a UCT search (use twixt_mcts_create_puct)");
     const size_t cells = static_cast<size_t>(a_.n) * a_.n;
-    if (gumbel_ && priors != nullptr && count_ > 0 && !is_device_pointer(priors)) {
-      TW_TRY(CheckHostLogits(priors));
-    } else if (priors != nullptr && count_ > 0 && !is_device_pointer(priors)) {
-      const size_t total = static_cast<size_t>(count_ * K_) * cells;
-      for (size_t i = 0; i < total; ++i)
-        if (!std::isfinite(priors[i]) || priors[i] < 0.0f)
-          return fail(TWIXT_EINVAL, "prior [%lld, %lld] = %g: priors must be finite and >= 0",
-                      static_cast<long long>(i / cells), static_cast<long long>(i % cells),
-                      static_cast<double>(priors[i]));
-    }
+    if (priors != nullptr && count_ > 0 && !is_device_pointer(priors))
+      TW_TRY(gumbel_ ? CheckHostLogits(priors) : CheckHostPriors(priors, count_ * K_));
     if (count_ > 0) {
       DeviceGuard g(b_->device_);
       TwixTBatch& b = *b_;
@@ -988,19 +982,14 @@ class TwixTMCTS {
                                      static_cast<int32_t*>(best.dev), b.stream_));
       b.launches_ += 1;
     }
-    TW_TRY(b.Finish(&v));
-    TW_TRY(b.Finish(&w));
-    TW_TRY(b.Finish(&best));
-    if (v.host || w.host || best.host) TW_TRY(b.Sync());
-    return TWIXT_OK;
+    return b.FinishOutputs({&v, &w, &best});
   }
 
   // MCTS-Solver results of a solver search; every output nullable, host or device
   int SolverStats(uint8_t* out_proven, float* out_returns, int8_t* out_edge_values, int32_t* out_simulations) {
     if (a_.root_out == nullptr)
       return fail(TWIXT_EINVAL, "twixt_mcts_solver_stats: the search was not created with TWIXT_MCTS_SOLVE");
-    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_solver_stats: no search begun");
-    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_solver_stats while a twixt_mcts_select awaits its backup");
+    TW_TRY(CheckIdle("solver_stats"));
     if (count_ == 0) return TWIXT_OK;
     DeviceGuard g(b_->device_);
     TwixTBatch& b = *b_;
@@ -1014,12 +1003,7 @@ class TwixTMCTS {
     TW_CUDA(launch_mcts_solver_stats(a_, count_, static_cast<uint8_t*>(pr.dev), static_cast<float*>(re.dev),
                                      static_cast<int8_t*>(ev.dev), static_cast<int32_t*>(sm.dev), b.stream_));
     b.launches_ += 1;
-    TW_TRY(b.Finish(&pr));
-    TW_TRY(b.Finish(&re));
-    TW_TRY(b.Finish(&ev));
-    TW_TRY(b.Finish(&sm));
-    if (pr.host || re.host || ev.host || sm.host) TW_TRY(b.Sync());
-    return TWIXT_OK;
+    return b.FinishOutputs({&pr, &re, &ev, &sm});
   }
 
   // Tree reuse: actions [count] int32 (host or device), 1 <= keep_nodes <= S, out_status [count] int32 or nullptr.
@@ -1029,8 +1013,7 @@ class TwixTMCTS {
     if (gumbel_)
       return fail(TWIXT_EINVAL, "twixt_mcts_advance: a Gumbel search does not reuse trees (Sequential Halving needs a "
                                 "fresh root); begin it again");
-    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_advance: no search begun");
-    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_advance while a twixt_mcts_select awaits its backup");
+    TW_TRY(CheckIdle("advance"));
     if (keep_nodes < 1 || keep_nodes > a_.S)
       return fail(TWIXT_EINVAL, "keep_nodes must be in [1, max_simulations + 1 = %d]: %d", a_.S, keep_nodes);
     if (count_ == 0) return TWIXT_OK;
@@ -1053,8 +1036,7 @@ class TwixTMCTS {
     const size_t status_bytes = static_cast<size_t>(count_) * sizeof(int32_t);
     if (out_status == nullptr) b.PinAlloc(status_bytes, &st);  // as twixt_apply: statuses read below
     else TW_TRY(b.StageOut(out_status, status_bytes, &st, false));
-    const bool scan_host = st.pin != nullptr;
-    if (!scan_host) TW_CUDA(cudaMemsetAsync(&b.d_stats_->illegal_index, 0xFF, sizeof(unsigned int), b.stream_));
+    if (st.pin == nullptr) TW_CUDA(cudaMemsetAsync(&b.d_stats_->illegal_index, 0xFF, sizeof(unsigned int), b.stream_));
     TW_CUDA(launch_mcts_advance(a_, count_, static_cast<const int32_t*>(in.dev), keep_nodes, map_,
                                 static_cast<int32_t*>(st.dev), &b.d_stats_->illegal_index, b.stream_));
     b.launches_ += 1;
@@ -1068,24 +1050,7 @@ class TwixTMCTS {
       if (in.host) TW_TRY(b.Sync());  // the staged actions are reused by the next call
       return TWIXT_OK;
     }
-    int64_t bad = -1;
-    if (scan_host) {
-      TW_TRY(b.Sync());
-      const int32_t* seen = static_cast<const int32_t*>(st.pin);
-      for (int64_t i = 0; i < count_ && bad < 0; ++i)
-        if (seen[i] == kRootIllegal) bad = i;
-    } else {
-      unsigned int flag = 0xFFFFFFFFu;
-      TW_CUDA(cudaMemcpyAsync(&flag, &b.d_stats_->illegal_index, sizeof(flag), cudaMemcpyDeviceToHost, b.stream_));
-      TW_TRY(b.Sync());
-      if (flag != 0xFFFFFFFFu) bad = flag;
-    }
-    if (bad >= 0) {
-      int32_t act = 0;
-      if (in.host) act = actions[bad];
-      else TW_CUDA(cudaMemcpy(&act, actions + bad, sizeof(act), cudaMemcpyDeviceToHost));
-      return fail(TWIXT_EILLEGAL, "Not a legal action: %d", act);  // twixt.h:96, as twixt_apply
-    }
+    TW_TRY(b.ReportIllegal(st, in, actions, count_));
     node_bound_ = truncated;
     return TWIXT_OK;
   }
@@ -1097,20 +1062,11 @@ class TwixTMCTS {
                                 "and its root noise from twixt_mcts_set_root_gumbel");
     if (a_.edge_p == nullptr)
       return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors: the search is not a PUCT search");
-    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors: no search begun");
-    if (pending_)
-      return fail(TWIXT_EINVAL, "twixt_mcts_set_root_priors while a twixt_mcts_select awaits its backup");
+    TW_TRY(CheckIdle("set_root_priors"));
     if (count_ == 0) return TWIXT_OK;
     if (priors == nullptr) return fail(TWIXT_EINVAL, "null priors pointer");
     const size_t cells = static_cast<size_t>(a_.n) * a_.n;
-    if (!is_device_pointer(priors)) {
-      const size_t total = static_cast<size_t>(count_) * cells;
-      for (size_t i = 0; i < total; ++i)
-        if (!std::isfinite(priors[i]) || priors[i] < 0.0f)
-          return fail(TWIXT_EINVAL, "prior [%lld, %lld] = %g: priors must be finite and >= 0",
-                      static_cast<long long>(i / cells), static_cast<long long>(i % cells),
-                      static_cast<double>(priors[i]));
-    }
+    if (!is_device_pointer(priors)) TW_TRY(CheckHostPriors(priors, count_));
     DeviceGuard g(b_->device_);
     TwixTBatch& b = *b_;
     b.ScratchReset();
@@ -1125,8 +1081,7 @@ class TwixTMCTS {
   // Gumbel searches: the root noise g [count, n*n] float32 (host or device; host values must be finite)
   int SetRootGumbel(const float* gumbel) {
     if (!gumbel_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_gumbel: the search is not a Gumbel search");
-    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_gumbel: no search begun");
-    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_set_root_gumbel while a twixt_mcts_select awaits its backup");
+    TW_TRY(CheckIdle("set_root_gumbel"));
     if (count_ == 0) return TWIXT_OK;
     if (gumbel == nullptr) return fail(TWIXT_EINVAL, "null gumbel pointer");
     const size_t cells = static_cast<size_t>(a_.n) * a_.n, total = static_cast<size_t>(count_) * cells;
@@ -1151,8 +1106,7 @@ class TwixTMCTS {
   // device
   int GumbelStats(int32_t* out_action, float* out_policy) {
     if (!gumbel_) return fail(TWIXT_EINVAL, "twixt_mcts_gumbel_stats: the search is not a Gumbel search");
-    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_gumbel_stats: no search begun");
-    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_gumbel_stats while a twixt_mcts_select awaits its backup");
+    TW_TRY(CheckIdle("gumbel_stats"));
     if (count_ == 0) return TWIXT_OK;
     DeviceGuard g(b_->device_);
     TwixTBatch& b = *b_;
@@ -1164,16 +1118,31 @@ class TwixTMCTS {
     TW_CUDA(launch_mcts_gumbel_stats(a_, gm_, count_, static_cast<int32_t*>(ac.dev), static_cast<float*>(po.dev),
                                      b.stream_));
     b.launches_ += 1;
-    TW_TRY(b.Finish(&ac));
-    TW_TRY(b.Finish(&po));
-    if (ac.host || po.host) TW_TRY(b.Sync());
-    return TWIXT_OK;
+    return b.FinishOutputs({&ac, &po});
   }
 
   int64_t count() const { return count_; }
   int64_t simulations() const { return sims_; }
 
  private:
+  // twixt_mcts_<what> needs a begun search without a select pending
+  int CheckIdle(const char* what) const {
+    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_%s: no search begun", what);
+    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_%s while a twixt_mcts_select awaits its backup", what);
+    return TWIXT_OK;
+  }
+
+  // Host priors [rows, n*n] must be finite and >= 0
+  int CheckHostPriors(const float* priors, int64_t rows) const {
+    const size_t cells = static_cast<size_t>(a_.n) * a_.n, total = static_cast<size_t>(rows) * cells;
+    for (size_t i = 0; i < total; ++i)
+      if (!std::isfinite(priors[i]) || priors[i] < 0.0f)
+        return fail(TWIXT_EINVAL, "prior [%lld, %lld] = %g: priors must be finite and >= 0",
+                    static_cast<long long>(i / cells), static_cast<long long>(i % cells),
+                    static_cast<double>(priors[i]));
+    return TWIXT_OK;
+  }
+
   // Host logits of a Gumbel backup must be finite on the legal actions of every non-terminal leaf: the leaf records
   // select wrote to envs [leaf_first_, leaf_first_ + count) are read back and their legal lists computed here.
   int CheckHostLogits(const float* logits) {
@@ -1207,8 +1176,7 @@ class TwixTMCTS {
   // +K per step) keeps every step inside the S node slots without reading the trees back.  Without an advance this
   // is "at most max_simulations simulations since begin".
   int CheckSimulations(int32_t num, const char* what) const {
-    if (!begun_) return fail(TWIXT_EINVAL, "twixt_mcts_%s: no search begun", what);
-    if (pending_) return fail(TWIXT_EINVAL, "twixt_mcts_%s while a twixt_mcts_select awaits its backup", what);
+    TW_TRY(CheckIdle(what));
     if (num < 0) return fail(TWIXT_EINVAL, "num_simulations must be >= 0: %d", num);
     if (!advanced_ && sims_ + num > max_sims_)
       return fail(TWIXT_EINVAL, "%lld simulations since begin would exceed max_simulations %d",

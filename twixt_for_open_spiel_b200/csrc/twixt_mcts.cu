@@ -15,6 +15,8 @@
 // draw) and expands a non-terminal leaf in the backup kernel, where the caller's priors for it are known.
 // A solver search (a.root_out != nullptr, MCTS-Solver) keeps an outcome code per edge and per root: a proven child
 // is scored by its outcome, and a tree whose root is proven is finished and takes no further part.
+// The select and backup kernels are templates on the search kind; the kernels that run once per search or per move
+// (begin, root stats, advance, ...) are one kernel each and test the arena's optional arrays for nullptr.
 // The scalar arithmetic (scores, draw, tie keys, stream ids, best child) is in twixt_mcts.cuh, shared with the
 // host harnesses that check it without a GPU.
 #include <cuda_runtime.h>
@@ -76,8 +78,8 @@ __device__ __forceinline__ int warp_expand(const MctsArena& a, int64_t g, const 
 
 // ----------------------------------------------------------------- begin ---
 // The root of tree t is a COPY of env roots + t; every tree is cleared to its root alone (a solver search: and its
-// root code to unproven; kVirtual: its V(s) to 0, and the node count goes to tree entry t*K).
-template <bool kSolve, bool kVirtual>
+// root code to unproven; K > 1: its V(s) to 0).  The node count goes to tree entry t*K, and K = 1 without virtual
+// visits.
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a, const uint32_t* __restrict__ roots,
                                                                      int64_t count) {
   const int lane = threadIdx.x & 31;
@@ -88,13 +90,9 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_begin_kernel(MctsArena a
   if (lane == 0) {
     a.node_legal[root] = -1;
     a.node_n[root] = 0u;
-    if constexpr (kVirtual) {
-      a.node_v[root] = 0;
-      a.tree[t * a.K] = make_int4(1, 0, 0, kLeafNeedsValue);
-    } else {
-      a.tree[t] = make_int4(1, 0, 0, kLeafNeedsValue);
-    }
-    if constexpr (kSolve) a.root_out[t] = 0;
+    if (a.node_v != nullptr) a.node_v[root] = 0;
+    a.tree[t * a.K] = make_int4(1, 0, 0, kLeafNeedsValue);
+    if (a.root_out != nullptr) a.root_out[t] = 0;
   }
 }
 
@@ -569,8 +567,10 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_backup_kernel(MctsArena 
 }
 
 // ------------------------------------------------------------ root stats ---
-// kSolve: a UCT solver search ranks by open_spiel's sort_key (outcome value, N, W), then the lower edge
-template <bool kSolve>
+// BestChild of every search kind, open_spiel's sort_key (outcome value, N, W), then the tie key, then the lower edge:
+// without outcome codes (UCT) every edge's outcome counts as 0, without tie keys (UCT, UCT solver) every key as 0.
+// A PUCT root has no best move (-1) while no edge has a visit, a UCT root only while it has no edges, so that an
+// expanded root queried between select and backup still reports edge 0.
 __global__ void __launch_bounds__(kMctsWarps * 32) mcts_root_stats_kernel(MctsArena a, int64_t count,
                                                                           int32_t* __restrict__ out_visits,
                                                                           double* __restrict__ out_value_sums,
@@ -586,113 +586,45 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_root_stats_kernel(MctsAr
     if (out_value_sums != nullptr) out_value_sums[t * cells + c] = 0.0;
   }
   __syncwarp();
-  if (a.edge_p != nullptr) {
-    // PUCT BestChild: (terminal outcome, N, W), then the tie key, then the lower edge; -1 while no N > 0
-    int bo = 0;
-    uint32_t bn = 0u, bk = 0u, nmax = 0u;
-    double bw = 0.0;
-    int bi = 0x7FFFFFFF;
-    for (int i = lane; i < legal; i += 32) {
-      const int action = a.edge_action[e0 + i];
-      const uint32_t en = a.edge_n[e0 + i];
-      const double ew = a.edge_w[e0 + i];
-      const int eo = mcts_outcome_value(a.edge_out[e0 + i]);
-      const uint32_t ek = a.edge_key[e0 + i];
-      if (out_visits != nullptr) out_visits[t * cells + action] = static_cast<int32_t>(en);
-      if (out_value_sums != nullptr) out_value_sums[t * cells + action] = ew;
-      nmax = en > nmax ? en : nmax;
-      if (bi == 0x7FFFFFFF || mcts_puct_best_beats(eo, en, ew, ek, i, bo, bn, bw, bk, bi)) {
-        bo = eo;
-        bn = en;
-        bw = ew;
-        bk = ek;
-        bi = i;
-      }
-    }
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      const int oo = __shfl_xor_sync(kFullMask, bo, d);
-      const uint32_t on = __shfl_xor_sync(kFullMask, bn, d);
-      const double ow = __shfl_xor_sync(kFullMask, bw, d);
-      const uint32_t ok = __shfl_xor_sync(kFullMask, bk, d);
-      const int oi = __shfl_xor_sync(kFullMask, bi, d);
-      if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_puct_best_beats(oo, on, ow, ok, oi, bo, bn, bw, bk, bi))) {
-        bo = oo;
-        bn = on;
-        bw = ow;
-        bk = ok;
-        bi = oi;
-      }
-    }
-    nmax = __reduce_max_sync(kFullMask, nmax);
-    if (out_best != nullptr && lane == 0)
-      out_best[t] = nmax > 0u ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
-    return;
-  }
-  if constexpr (kSolve) {
-    int bo = 0;
-    uint32_t bn = 0u;
-    double bw = 0.0;
-    int bi = 0x7FFFFFFF;
-    for (int i = lane; i < legal; i += 32) {
-      const int action = a.edge_action[e0 + i];
-      const uint32_t en = a.edge_n[e0 + i];
-      const double ew = a.edge_w[e0 + i];
-      const int eo = mcts_outcome_value(a.edge_out[e0 + i]);
-      if (out_visits != nullptr) out_visits[t * cells + action] = static_cast<int32_t>(en);
-      if (out_value_sums != nullptr) out_value_sums[t * cells + action] = ew;
-      if (bi == 0x7FFFFFFF || mcts_puct_best_beats(eo, en, ew, 0u, i, bo, bn, bw, 0u, bi)) {
-        bo = eo;
-        bn = en;
-        bw = ew;
-        bi = i;
-      }
-    }
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      const int oo = __shfl_xor_sync(kFullMask, bo, d);
-      const uint32_t on = __shfl_xor_sync(kFullMask, bn, d);
-      const double ow = __shfl_xor_sync(kFullMask, bw, d);
-      const int oi = __shfl_xor_sync(kFullMask, bi, d);
-      if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_puct_best_beats(oo, on, ow, 0u, oi, bo, bn, bw, 0u, bi))) {
-        bo = oo;
-        bn = on;
-        bw = ow;
-        bi = oi;
-      }
-    }
-    if (out_best != nullptr && lane == 0)
-      out_best[t] = (legal > 0 && bi != 0x7FFFFFFF) ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
-    return;
-  }
-  uint32_t bn = 0u;
+  int bo = 0;
+  uint32_t bn = 0u, bk = 0u, nmax = 0u;
   double bw = 0.0;
   int bi = 0x7FFFFFFF;
   for (int i = lane; i < legal; i += 32) {
     const int action = a.edge_action[e0 + i];
     const uint32_t en = a.edge_n[e0 + i];
     const double ew = a.edge_w[e0 + i];
+    const int eo = a.edge_out != nullptr ? mcts_outcome_value(a.edge_out[e0 + i]) : 0;
+    const uint32_t ek = a.edge_key != nullptr ? a.edge_key[e0 + i] : 0u;
     if (out_visits != nullptr) out_visits[t * cells + action] = static_cast<int32_t>(en);
     if (out_value_sums != nullptr) out_value_sums[t * cells + action] = ew;
-    if (bi == 0x7FFFFFFF || mcts_best_beats(en, ew, i, bn, bw, bi)) {
+    nmax = en > nmax ? en : nmax;
+    if (bi == 0x7FFFFFFF || mcts_puct_best_beats(eo, en, ew, ek, i, bo, bn, bw, bk, bi)) {
+      bo = eo;
       bn = en;
       bw = ew;
+      bk = ek;
       bi = i;
     }
   }
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) {
+    const int oo = __shfl_xor_sync(kFullMask, bo, d);
     const uint32_t on = __shfl_xor_sync(kFullMask, bn, d);
     const double ow = __shfl_xor_sync(kFullMask, bw, d);
+    const uint32_t ok = __shfl_xor_sync(kFullMask, bk, d);
     const int oi = __shfl_xor_sync(kFullMask, bi, d);
-    if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_best_beats(on, ow, oi, bn, bw, bi))) {
+    if (oi != 0x7FFFFFFF && (bi == 0x7FFFFFFF || mcts_puct_best_beats(oo, on, ow, ok, oi, bo, bn, bw, bk, bi))) {
+      bo = oo;
       bn = on;
       bw = ow;
+      bk = ok;
       bi = oi;
     }
   }
-  if (out_best != nullptr && lane == 0)
-    out_best[t] = (legal > 0 && bi != 0x7FFFFFFF) ? static_cast<int32_t>(a.edge_action[e0 + bi]) : -1;
+  nmax = __reduce_max_sync(kFullMask, nmax);
+  const bool none = a.edge_p != nullptr ? nmax == 0u : legal <= 0;
+  if (out_best != nullptr && lane == 0) out_best[t] = none ? -1 : static_cast<int32_t>(a.edge_action[e0 + bi]);
 }
 
 // ---------------------------------------------------------- solver stats ---
@@ -1220,102 +1152,77 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_gumbel_stats_kernel(Mcts
   }
 }
 
-unsigned mcts_blocks(int64_t count) { return static_cast<unsigned>((count + kMctsWarps - 1) / kMctsWarps); }
+// One warp per tree: count trees in blocks of kMctsWarps warps, nothing to launch for none
+template <typename... Params, typename... Args>
+cudaError_t launch_per_tree(void (*kernel)(Params...), int64_t count, cudaStream_t s, Args... args) {
+  if (count <= 0) return cudaSuccess;
+  kernel<<<static_cast<unsigned>((count + kMctsWarps - 1) / kMctsWarps), kMctsWarps * 32, 0, s>>>(args...);
+  return cudaGetLastError();
+}
 
 }  // namespace
 
 cudaError_t launch_mcts_begin(const MctsArena& a, const uint32_t* roots, int64_t count, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  auto kernel = a.node_v != nullptr ? mcts_begin_kernel<false, true>
-                                    : (a.root_out != nullptr ? mcts_begin_kernel<true, false>
-                                                             : mcts_begin_kernel<false, false>);
-  kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, roots, count);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_begin_kernel, count, s, a, roots, count);
 }
 
 cudaError_t launch_mcts_select(const MctsArena& a, int64_t count, uint64_t seed, uint32_t stream0, uint32_t k,
                                double uct_c, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
   const bool puct = a.edge_p != nullptr, solve = a.root_out != nullptr;
   auto kernel = a.node_v != nullptr
                     ? (puct ? mcts_select_kernel<true, false, true> : mcts_select_kernel<false, false, true>)
                 : puct ? (solve ? mcts_select_kernel<true, true, false> : mcts_select_kernel<true, false, false>)
                        : (solve ? mcts_select_kernel<false, true, false> : mcts_select_kernel<false, false, false>);
-  kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, seed, stream0, k, uct_c, leaf_dst, out_status);
-  return cudaGetLastError();
+  return launch_per_tree(kernel, count, s, a, count, seed, stream0, k, uct_c, leaf_dst, out_status);
 }
 
 cudaError_t launch_mcts_backup(const MctsArena& a, int64_t count, const float* values, const float* priors,
                                uint64_t seed, uint32_t stream0, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
   auto kernel = a.node_v != nullptr ? mcts_backup_kernel<false, true>
                                     : (a.root_out != nullptr ? mcts_backup_kernel<true, false>
                                                              : mcts_backup_kernel<false, false>);
-  kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, values, priors, seed, stream0);
-  return cudaGetLastError();
+  return launch_per_tree(kernel, count, s, a, count, values, priors, seed, stream0);
 }
 
 cudaError_t launch_mcts_root_stats(const MctsArena& a, int64_t count, int32_t* out_visits, double* out_value_sums,
                                    int32_t* out_best, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  if (a.root_out != nullptr)
-    mcts_root_stats_kernel<true><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_visits, out_value_sums,
-                                                                                out_best);
-  else
-    mcts_root_stats_kernel<false><<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_visits,
-                                                                                 out_value_sums, out_best);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_root_stats_kernel, count, s, a, count, out_visits, out_value_sums, out_best);
 }
 
 cudaError_t launch_mcts_solver_stats(const MctsArena& a, int64_t count, uint8_t* out_proven, float* out_returns,
                                      int8_t* out_edge_values, int32_t* out_simulations, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  mcts_solver_stats_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, out_proven, out_returns,
-                                                                           out_edge_values, out_simulations);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_solver_stats_kernel, count, s, a, count, out_proven, out_returns, out_edge_values,
+                         out_simulations);
 }
 
 cudaError_t launch_mcts_advance(const MctsArena& a, int64_t count, const int32_t* actions, int keep_nodes,
                                 int32_t* map, int32_t* out_status, unsigned int* illegal_index, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  mcts_advance_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, actions, keep_nodes, map, out_status,
-                                                                      illegal_index);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_advance_kernel, count, s, a, count, actions, keep_nodes, map, out_status,
+                         illegal_index);
 }
 
 cudaError_t launch_mcts_set_root_priors(const MctsArena& a, int64_t count, const float* priors, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  mcts_set_root_priors_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, count, priors);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_set_root_priors_kernel, count, s, a, count, priors);
 }
 
 cudaError_t launch_mcts_gumbel_select(const MctsArena& a, const MctsGumbel& gm, int64_t count, uint32_t stream0,
                                       uint32_t k, uint32_t* leaf_dst, int32_t* out_status, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  mcts_gumbel_select_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, stream0, k, leaf_dst,
-                                                                            out_status);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_gumbel_select_kernel, count, s, a, gm, count, stream0, k, leaf_dst, out_status);
 }
 
 cudaError_t launch_mcts_gumbel_backup(const MctsArena& a, const MctsGumbel& gm, int64_t count, const float* values,
                                       const float* logits, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  mcts_gumbel_backup_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, values, logits);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_gumbel_backup_kernel, count, s, a, gm, count, values, logits);
 }
 
 cudaError_t launch_mcts_set_root_gumbel(const MctsArena& a, const MctsGumbel& gm, int64_t count, const float* gumbel,
                                         cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  mcts_set_root_gumbel_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, gumbel);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_set_root_gumbel_kernel, count, s, a, gm, count, gumbel);
 }
 
 cudaError_t launch_mcts_gumbel_stats(const MctsArena& a, const MctsGumbel& gm, int64_t count, int32_t* out_action,
                                      float* out_policy, cudaStream_t s) {
-  if (count <= 0) return cudaSuccess;
-  mcts_gumbel_stats_kernel<<<mcts_blocks(count), kMctsWarps * 32, 0, s>>>(a, gm, count, out_action, out_policy);
-  return cudaGetLastError();
+  return launch_per_tree(mcts_gumbel_stats_kernel, count, s, a, gm, count, out_action, out_policy);
 }
 
 }  // namespace twixt

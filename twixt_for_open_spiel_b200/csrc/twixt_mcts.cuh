@@ -172,13 +172,6 @@ TW_HD double mcts_uct_score(double w, uint32_t n, double log_parent, double c) {
 // (score a, edge ia) beats (score b, edge ib): the larger score, then the lower edge (= lower action)
 TW_HD bool mcts_score_beats(double a, int ia, double b, int ib) { return a > b || (a == b && ia < ib); }
 
-// BestChild: (visits, value sum, edge) beats another: most visits, then larger W, then the lower action
-TW_HD bool mcts_best_beats(uint32_t na, double wa, int ia, uint32_t nb, double wb, int ib) {
-  if (na != nb) return na > nb;
-  if (wa != wb) return wa > wb;
-  return ia < ib;
-}
-
 // sqrt(N(s)) of the PUCT score, once per node
 TW_HD double mcts_sqrt_visits(uint32_t parent_visits) {
 #if defined(__CUDA_ARCH__)
@@ -246,8 +239,8 @@ TW_HD int mcts_proven_value(int max_code, bool all_proven) {
 // the code of the parent's edge into a node proven with value v (zero-sum, players alternate by ply)
 TW_HD uint8_t mcts_parent_code(int v) { return static_cast<uint8_t>(2 - v); }
 
-// PUCT BestChild (open_spiel SearchNode.sort_key): (outcome value, N, W), then the smaller key, then the
-// lower edge
+// BestChild (open_spiel SearchNode.sort_key): (outcome value, N, W), then the smaller key, then the lower edge; a
+// search without outcome codes or tie keys passes 0 for them
 TW_HD bool mcts_puct_best_beats(int oa, uint32_t na, double wa, uint32_t ka, int ia, int ob, uint32_t nb, double wb,
                                 uint32_t kb, int ib) {
   if (oa != ob) return oa > ob;
@@ -255,6 +248,12 @@ TW_HD bool mcts_puct_best_beats(int oa, uint32_t na, double wa, uint32_t ka, int
   if (wa != wb) return wa > wb;
   if (ka != kb) return ka < kb;
   return ia < ib;
+}
+
+// UCT BestChild: most visits, then larger W, then the lower action; the order above without outcome codes or keys,
+// which is how mcts_root_stats_kernel ranks a UCT root
+TW_HD bool mcts_best_beats(uint32_t na, double wa, int ia, uint32_t nb, double wb, int ib) {
+  return mcts_puct_best_beats(0, na, wa, 0u, ia, 0, nb, wb, 0u, ib);
 }
 
 // the one random draw of simulation k of the tree with stream id T: the index of the unvisited edge taken,
